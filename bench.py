@@ -519,6 +519,18 @@ def bench_json_e2e(pb, max_sites):
     return out
 
 
+def dump_outputs(path, m):
+    """The last timed step of each cfg2 loop as a caller of include/plf.h receives it (all ranks' sums when N > 1): ll + deriv
+    with resident inputs (the headline), the same query end to end, and ll alone.  The inputs are seeded, so two builds of
+    the project can be compared array for array."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"sum_ll": [m["res"]["sum_ll"]], "sum_deriv": m["res"]["sum_deriv"],
+              "e2e_sum_ll": [m["res2"]["sum_ll"]], "e2e_sum_deriv": m["res2"]["sum_deriv"],
+              "ll_only_sum_ll": [m["res3"][1]]}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -598,7 +610,7 @@ def run_ours(args):
                    kern_ms=float(np.mean(kern_ms)), mat_ms=float(np.mean(mat_ms)), site_ms=float(np.mean(site_ms)),
                    kernel=eng.last_kernel_name())
         if want_e2e:
-            e2e_steps = max(1, min(steps, 50))
+            e2e_steps = steps
             for _ in range(min(args.warmup, 3)):
                 step_e2e()
             barrier()
@@ -611,7 +623,7 @@ def run_ours(args):
             barrier()
             out.update(e2e_steps=e2e_steps, ms_e2e=f0.elapsed_time(f1), t1=t1, t1_end=time.perf_counter(), res2=res2)
         if want_ll:
-            ll_steps = max(1, min(steps, 50))
+            ll_steps = steps
             for _ in range(3):
                 step_ll()
             barrier()
@@ -619,11 +631,12 @@ def run_ours(args):
             ll_kern = []
             g0.record(stream)
             for _ in range(ll_steps):
-                step_ll()
+                res3 = step_ll()
                 ll_kern.append(eng.last_kernel_ms())
             g1.record(stream)
             barrier()
-            out.update(ll_steps=ll_steps, ms_ll=g0.elapsed_time(g1), ll_kern=float(np.mean(ll_kern)), ll_kernel=eng.last_kernel_name())
+            out.update(ll_steps=ll_steps, ms_ll=g0.elapsed_time(g1), ll_kern=float(np.mean(ll_kern)), ll_kernel=eng.last_kernel_name(),
+                       res3=res3)
         return out
 
     def max_over_ranks(vals):
@@ -663,7 +676,7 @@ def run_ours(args):
     # ---- weak scaling beside it (N > 1 only): every rank owns a whole alignment of args.sites patterns ----
     weak = None
     if world > 1:
-        mw = measure(0, S_total, max(3, min(args.steps, 20)), True, False)
+        mw = measure(0, S_total, args.steps, True, False)
         ms_w, ms_w_e2e = max_over_ranks([mw["ms"], mw["ms_e2e"]])
         weak = {"scaling": "weak", "sites_per_gpu": S_total, "steps": mw["steps"], "ms_per_step": ms_w / mw["steps"],
                 "value": float(S_total) * Eg * C * world * mw["steps"] / (ms_w * 1e-3), "unit": "updates/s",
@@ -676,6 +689,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m)
     S = m["S"]
     updates_per_step = float(S_total) * Eg * C
     value = updates_per_step * args.steps / (ms * 1e-3)
@@ -914,7 +929,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg4 and JSON drop-in measurements (N = 1)")
     ap.add_argument("--json-sites", type=int, default=1000000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each cfg2 loop returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a site sample and keeps no outputs")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
