@@ -840,12 +840,21 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
             const F4Op op = F4_OP(o);
             /* fn_a comes from "cur" if this node was consumed from registers by its parent, else from its slot */
             const bool from_slot = (o != a.nops - 1) && F4_OP(o + 1).spill_before;
-            /* the next node (o-1) reads these slab lines: start fetching them */
+            /* the next node (o-1) reads these slab lines: start fetching them.  That includes the scale words of the
+             * node and of its internal children and, when this op does not consume the node (spill_before), the fn its
+             * parent left in its slot: they head the dependent chain of its step (the scale of fa, fa itself, the
+             * constant-column flags), and without the prefetch each is a full L2 / DRAM round trip at its start. */
             if (o > 0) {
                 const F4Op nx = F4_OP(o - 1);
+                f4_prefetch(&a.scratchS[(size_t)nx.slot * T + gtid]);
+                if (op.spill_before) {
+#pragma unroll
+                    for (int c = 0; c < C; c++) f4_prefetch(&a.scratch[((size_t)nx.slot * C + c) * T + gtid]);
+                }
                 for (int j = 0; j < nx.nchild; j++) {
                     const F4Child nc = F4_CH(nx.first_child + j);
                     if (nc.kind != F4_KIND_TIP) {
+                        f4_prefetch(&a.scratchS[(size_t)nc.slot * T + gtid]);
 #pragma unroll
                         for (int c = 0; c < C; c++) f4_prefetch(&a.scratch[((size_t)nc.slot * C + c) * T + gtid]);
                     }
