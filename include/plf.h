@@ -171,6 +171,27 @@ int plf_edge_expect(plf_engine *e, int kind,
                     const unsigned char *edge_mask,
                     double *site_out /*[S][E]*/, double *sum_out /*[E]*/);
 
+/*
+ * All Frechet directions of plf_edge_expect at once, summed over the sites with the site weights (edges in csr order,
+ * no edge mask, no per-site output):
+ *   dwell[e][i][j] = what plf_edge_expect(PLF_KIND_DWELL, L = E_ij) returns in sum_out[e]
+ *   trans[e][i][j] = what plf_edge_expect(PLF_KIND_TRANS, L = E_ij) returns in sum_out[e]
+ * so plf_edge_expect(kind, L)[e] == sum_ij L_ij X_kind[e][i][j] for every L; sum_ll = sum_s w_s log L_s.  Any output
+ * may be NULL.  As in plf_edge_expect, a rate category of zero likelihood at a site adds nothing there (which only
+ * shows in the off-diagonal dwell entries of a category of rate 0).  One pass over the sites: the edge form is bilinear in the outside and inside vectors, so the pass sums
+ * G_{e,c} = sum_s w_s prior_c fe L_b^T / L_s and the directions come from the adjoint Frechet derivative at A^T.
+ *
+ * Gradient of the log-likelihood with respect to the rate matrix:
+ *   d sum_ll / d Q_ij = sum_e trans[e][i][j]
+ * where Q is the scaled matrix given to plf_set_model with its n^2 entries treated as independent, and the category
+ * rates, category priors and root prior are held fixed.  The dependence of an equilibrium root prior on Q is not
+ * included; the caller applies the chain rule for the rate divisor, the diagonal and the equilibrium.
+ *
+ * Errors as for the other queries (no configuration; a site of zero likelihood with non-zero weight).  After
+ * plf_comm_init the sums are all-reduced like every other *_sum output.
+ */
+int plf_edge_expect_all(plf_engine *e, double *sum_ll, double *dwell /*[E][n][n]*/, double *trans /*[E][n][n]*/);
+
 /* Copies of device-computed matrices, for tests: P[C][E][n][n] (row major). */
 int plf_get_transition_matrices(plf_engine *e, double *p_out);
 /* rate_c * Q * P, the matrices used by plf_deriv */

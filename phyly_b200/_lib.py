@@ -44,6 +44,7 @@ def load():
     lib.plf_deriv.argtypes = [P, P, P, P, P, P]
     lib.plf_marginal.argtypes = [P, P, P]
     lib.plf_edge_expect.argtypes = [P, c.c_int, P, P, P, P, P]
+    lib.plf_edge_expect_all.argtypes = [P, P, P, P]
     lib.plf_get_transition_matrices.argtypes = [P, P]
     lib.plf_get_derivative_matrices.argtypes = [P, P]
     lib.plf_get_frechet_matrices.argtypes = [P, P, P, P]
@@ -68,7 +69,7 @@ def load():
     lib.plf_stream.restype = P
     lib.plf_synchronize.argtypes = [P]
     for name in ("plf_set_path", "plf_set_tree", "plf_set_model", "plf_set_edge_rates", "plf_set_data", "plf_set_data_async",
-                 "plf_set_site_weights", "plf_ll", "plf_deriv", "plf_marginal", "plf_edge_expect",
+                 "plf_set_site_weights", "plf_ll", "plf_deriv", "plf_marginal", "plf_edge_expect", "plf_edge_expect_all",
                  "plf_get_transition_matrices", "plf_get_derivative_matrices", "plf_get_frechet_matrices",
                  "plf_last_timing", "plf_comm_unique_id", "plf_comm_init", "plf_synchronize"):
         getattr(lib, name).restype = c.c_int

@@ -32,6 +32,10 @@ struct ExpmArgs {
     double *F;                       /* [C][E][n][n] Frechet block, or NULL */
     int f_scale_mode;                /* 0: F ; 1: F * cat_rate * edge_rate */
     dd_t *ws;                        /* global workspace (8*n*n dd per CTA) or NULL => shared */
+    /* adjoint form (plf_edge_expect_all): a direction per matrix, l_per[C][E][n][n] (fp64, replaces l_hi / l_lo),
+     * and the Frechet derivative taken at A^T = r_c t_e Q^T -- the adjoint of L -> Frechet(A, L) */
+    const double *l_per = nullptr;
+    int q_transpose = 0;
 };
 
 __device__ __forceinline__ void dd_matmul(dd_t *Cm, const dd_t *A, const dd_t *B, int n, dd_t scale, bool use_scale)
@@ -134,7 +138,8 @@ __global__ void __launch_bounds__(256) expm_dd_kernel(ExpmArgs a)
 
     for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
         int i = idx / n, j = idx - i * n;
-        dd_t q = dd_make(a.q_hi[idx], a.q_lo ? a.q_lo[idx] : 0.0);
+        const int qidx = a.q_transpose ? j * n + i : idx;
+        dd_t q = dd_make(a.q_hi[qidx], a.q_lo ? a.q_lo[qidx] : 0.0);
         dd_t v = dd_mul_pwr2(dd_mul(q, rt), inv2s);
         if (i == j) v = dd_add(v, mus);
         if (v.hi < 0.0) v = dd_make(0.0, 0.0);   /* the diagonal entry that defines mu */
@@ -142,7 +147,8 @@ __global__ void __launch_bounds__(256) expm_dd_kernel(ExpmArgs a)
         dd_t id = dd_make(i == j ? 1.0 : 0.0, 0.0);
         X[idx] = id; SX[idx] = id;
         if (want_f) {
-            dd_t l = dd_make(a.l_hi[idx], a.l_lo ? a.l_lo[idx] : 0.0);
+            dd_t l = a.l_per ? dd_make(a.l_per[((size_t)c * a.E + e) * nn + idx], 0.0)
+                             : dd_make(a.l_hi[idx], a.l_lo ? a.l_lo[idx] : 0.0);
             Ls[idx] = dd_mul_pwr2(l, inv2s);
             Y[idx] = dd_make(0.0, 0.0); SY[idx] = dd_make(0.0, 0.0);
         }

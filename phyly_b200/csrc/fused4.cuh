@@ -215,15 +215,50 @@ __device__ __forceinline__ double f4_warp_sum2(double a, double b, int lane)
 }
 
 /*
+ * Mode 3 (plf_edge_expect_all): adds the warp's sum of the outer product fe (x) lb -- entry 4 i + j = fe_i lb_j -- to the
+ * 16 accumulators at row.  A reduce-scatter butterfly halves the live products at every step (16 shuffles instead of
+ * 16 x 5) and leaves the sum of entry m = lane >> 1 in lanes lane and lane ^ 1; the even lanes add it.  Every lane
+ * stores entry k ^ m at position k (fe and lb permuted by the bits of m), so that at every step the half it keeps is
+ * its lower half and the half it sends its upper one: no selects.  Fixed order: the bits do not depend on timing.
+ */
+__device__ __forceinline__ void f4_gm_add(double *row, const double fe[4], const double lb[4], int lane)
+{
+    const int m = (lane >> 1) & 15;
+    double f[4], l[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const double f1 = (m & 4) ? fe[i ^ 1] : fe[i], l1 = (m & 1) ? lb[i ^ 1] : lb[i];
+        f[i] = f1; l[i] = l1;
+    }
+#pragma unroll
+    for (int i = 0; i < 2; i++) {
+        const double fa = f[i], fb = f[i + 2], la = l[i], lbv = l[i + 2];
+        if (m & 8) { f[i] = fb; f[i + 2] = fa; }
+        if (m & 2) { l[i] = lbv; l[i + 2] = la; }
+    }
+    double v[16];
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+#pragma unroll
+        for (int j = 0; j < 4; j++) v[4 * i + j] = f[i] * l[j];
+#pragma unroll
+    for (int h = 8; h >= 1; h >>= 1)
+#pragma unroll
+        for (int k = 0; k < h; k++) v[k] += __shfl_xor_sync(0xffffffffu, v[h + k], 2 * h);
+    const double sum = v[0] + __shfl_xor_sync(0xffffffffu, v[0], 1);
+    if (!(lane & 1)) row[lane >> 1] += sum;
+}
+
+/*
  * Outside step specialised for a node with exactly two children of kinds (K0, K1) in
  * {(CUR, TIP), (CUR, STACK), (TIP, TIP)}: straight-line code, no filler factors.
  */
-template <int C, int BD, int K0, int K1, bool PACK, bool CM, bool MARG>
+template <int C, int BD, int K0, int K1, bool PACK, bool CM, bool MARG, bool GM>
 __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, const F4Child &c0, const F4Child &c1,
                                             bool from_slot, double *cur, const unsigned char *tile, const double *defs_s,
                                             const double *Pint, const double *Fint, const double *TP, const double *TF,
                                             int pstride, int tpstride, size_t T, size_t gtid, int tid,
-                                            double &x0, double &x1, double *mgo)
+                                            double &x0, double &x1, double *mgo, double *accG)
 {
     double basev[4] = {1.0, 1.0, 1.0, 1.0};
     const bool has_base = op.code_row >= 0;
@@ -236,7 +271,8 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
     /* marginal mode: posterior state distribution of this node and of its tip children, summed over categories */
     double mg[4] = {0.0, 0.0, 0.0, 0.0}, mt0[4] = {0.0, 0.0, 0.0, 0.0}, mt1[4] = {0.0, 0.0, 0.0, 0.0};
     const int ptstride = a.Et * 16;
-#pragma unroll (CM ? 1 : 2)
+    /* (mode 3 walks the categories one at a time: its 16 outer products per edge leave no room for two in flight) */
+#pragma unroll ((CM || GM) ? 1 : 2)
     for (int c = 0; c < C; c++) {
         /* loads of this category first */
         double l0[4], l1[4], fa[4];
@@ -268,30 +304,36 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
         double em0[4], y0[4], em1[4], y1[4];
         if (K0 == F4_KIND_TIP) {
             f4_ld4(TP + c * tpstride + (c0.mat * a.K + code0) * 4, em0);
-            if (!MARG) f4_ld4(TF + c * tpstride + (c0.mat * a.K + code0) * 4, y0);
+            if (!MARG && !GM) f4_ld4(TF + c * tpstride + (c0.mat * a.K + code0) * 4, y0);
         } else {
             f4_mv<CM, 0>(Pint, c * pstride + c0.mat * 16, l0, em0);
-            if (!MARG) f4_mv<CM, 1>(Fint, c * pstride + c0.mat * 16, l0, y0);
+            if (!MARG && !GM) f4_mv<CM, 1>(Fint, c * pstride + c0.mat * 16, l0, y0);
             if (bc0) {
 #pragma unroll
-                for (int i = 0; i < 4; i++) { em0[i] = l0[i]; if (!MARG && a.f_zero_rowsum) y0[i] = 0.0; }
+                for (int i = 0; i < 4; i++) { em0[i] = l0[i]; if (!MARG && !GM && a.f_zero_rowsum) y0[i] = 0.0; }
             }
         }
         if (K1 == F4_KIND_TIP) {
             f4_ld4(TP + c * tpstride + (c1.mat * a.K + code1) * 4, em1);
-            if (!MARG) f4_ld4(TF + c * tpstride + (c1.mat * a.K + code1) * 4, y1);
+            if (!MARG && !GM) f4_ld4(TF + c * tpstride + (c1.mat * a.K + code1) * 4, y1);
         } else {
             f4_mv<CM, 0>(Pint, c * pstride + c1.mat * 16, l1, em1);
-            if (!MARG) f4_mv<CM, 1>(Fint, c * pstride + c1.mat * 16, l1, y1);
+            if (!MARG && !GM) f4_mv<CM, 1>(Fint, c * pstride + c1.mat * 16, l1, y1);
             if (bc1) {
 #pragma unroll
-                for (int i = 0; i < 4; i++) { em1[i] = l1[i]; if (!MARG && a.f_zero_rowsum) y1[i] = 0.0; }
+                for (int i = 0; i < 4; i++) { em1[i] = l1[i]; if (!MARG && !GM && a.f_zero_rowsum) y1[i] = 0.0; }
             }
         }
         double fe0[4], fe1[4];
 #pragma unroll
         for (int i = 0; i < 4; i++) { fe0[i] = fa[i] * em1[i]; fe1[i] = fa[i] * em0[i]; }
-        if (!MARG) {
+        if (GM) {
+            /* the child's inside vector: the slab line, or the definition row of a tip's character */
+            if (K0 == F4_KIND_TIP) f4_ld4(defs_s + code0 * 4, l0);
+            if (K1 == F4_KIND_TIP) f4_ld4(defs_s + code1 * 4, l1);
+            f4_gm_add(accG + ((size_t)c * a.E + c0.edge) * 16, fe0, l0, tid & 31);
+            f4_gm_add(accG + ((size_t)c * a.E + c1.edge) * 16, fe1, l1, tid & 31);
+        } else if (!MARG) {
             double xv = fe0[0] * y0[0];
             xv = fma(fe0[1], y0[1], xv); xv = fma(fe0[2], y0[2], xv); xv = fma(fe0[3], y0[3], xv);
             x0 += xv;
@@ -412,7 +454,7 @@ __device__ __forceinline__ void f4_root_site(const F4Args &a, const double *cur,
 
 /* values of the kernel's frame that the out-of-line outside step needs */
 struct F4Ctx {
-    double *cur, *accE, *accM;
+    double *cur, *accE, *accM, *accG;
     const unsigned char *tile;
     const double *defs_s, *Pint, *Fint, *TP, *TF;
     const F4Child *chp;
@@ -425,11 +467,11 @@ struct F4Ctx {
 /*
  * Outside step for a node with any number of children (1..F4_MAXD) of any kind (non-CM kernels only).
  */
-template <int C, int BD, bool PACK, bool CM, bool MARG>
+template <int C, int BD, bool PACK, bool CM, bool MARG, bool GM>
 __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &op, bool from_slot, const F4Ctx &k)
 {
     constexpr int bd = BD;
-    double *cur = k.cur, *accE = k.accE, *accM = k.accM;
+    double *cur = k.cur, *accE = k.accE, *accM = k.accM, *accG = k.accG;
     const unsigned char *tile = k.tile;
     const double *defs_s = k.defs_s, *Pint = k.Pint, *Fint = k.Fint, *TP = k.TP, *TF = k.TF;
     const F4Child *chp = k.chp;
@@ -483,7 +525,7 @@ __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &
             for (int i = 0; i < 4; i++) { em[j][i] = 1.0; y[j][i] = 0.0; }
             if (kinds[j] == F4_KIND_TIP) {
                 f4_ld4(TP + c * tpstride + (mats[j] * a.K + codes[j]) * 4, em[j]);
-                if (!MARG) f4_ld4(TF + c * tpstride + (mats[j] * a.K + codes[j]) * 4, y[j]);
+                if (!MARG && !GM) f4_ld4(TF + c * tpstride + (mats[j] * a.K + codes[j]) * 4, y[j]);
             } else if (kinds[j] >= 0) {
                 double4 l4 = f4_slab_ld(&a.scratch[((size_t)slots[j] * C + c) * T + gtid]);
                 double lv[4] = {l4.x, l4.y, l4.z, l4.w};
@@ -493,7 +535,7 @@ __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &
                 } else {
                     f4_mv<CM, 0>(Pint, c * pstride + mats[j] * 16, lv, em[j]);
                 }
-                if (!MARG && !(bcs[j] && a.f_zero_rowsum)) f4_mv<CM, 1>(Fint, c * pstride + mats[j] * 16, lv, y[j]);
+                if (!MARG && !GM && !(bcs[j] && a.f_zero_rowsum)) f4_mv<CM, 1>(Fint, c * pstride + mats[j] * 16, lv, y[j]);
             }
         }
 #pragma unroll
@@ -507,7 +549,17 @@ __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &
                     for (int j2 = 0; j2 < F4_MAXD; j2++) if (j2 != j) f *= em[j2][i];
                     fe[i] = f;
                 }
-                if (!MARG) {
+                if (GM) {
+                    /* the child's inside vector, read again (its slot is rewritten below): fewer live registers */
+                    double lb[4];
+                    if (kinds[j] == F4_KIND_TIP) {
+                        f4_ld4(defs_s + codes[j] * 4, lb);
+                    } else {
+                        const double4 l4 = f4_slab_ld(&a.scratch[((size_t)slots[j] * C + c) * T + gtid]);
+                        lb[0] = l4.x; lb[1] = l4.y; lb[2] = l4.z; lb[3] = l4.w;
+                    }
+                    f4_gm_add(accG + ((size_t)c * a.E + edges[j]) * 16, fe, lb, lane);
+                } else if (!MARG) {
                     double xv = fe[0] * y[j][0];
                     xv = fma(fe[1], y[j][1], xv);
                     xv = fma(fe[2], y[j][2], xv);
@@ -553,7 +605,7 @@ __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &
         }
     }
 #pragma unroll
-    for (int j = 0; j < (MARG ? 0 : F4_MAXD); j++) {
+    for (int j = 0; j < ((MARG || GM) ? 0 : F4_MAXD); j++) {
         if (kinds[j] >= 0) {
             const int e = edges[j];
             const bool me = !a.edge_mask || a.edge_mask[e];
@@ -570,7 +622,9 @@ __device__ __forceinline__ void f4_outside_general(const F4Args &a, const F4Op &
 /*
  * C     : number of rate categories (1..4)
  * MODE  : 0 = log-likelihood only; 1 = log-likelihood + per-edge bilinear forms (deriv / dwell / trans);
- *         2 = log-likelihood + posterior marginals of every node
+ *         2 = log-likelihood + posterior marginals of every node;
+ *         3 = log-likelihood + the matrices G_{e,c} = sum_s fe (x) L_b of every edge and category (plf_edge_expect_all):
+ *             the outside pass of mode 2, with the outer products summed per warp into block_gmat
  * The dynamic shared memory layout below is mirrored on the host by f4_smem_bytes().
  */
 /* STAGED: 2 = all tables in shared memory, 1 = all but TF (read through L1), 0 = none.
@@ -582,6 +636,7 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
 {
     constexpr bool EDGE = MODE != 0;     /* an outside pass runs */
     constexpr bool MARG = MODE == 2;     /* ... and produces node marginals instead of per-edge forms */
+    constexpr bool GM = MODE == 3;       /* ... or the per-edge outer-product matrices (no edge-form tables) */
     extern __shared__ __align__(16) unsigned char f4_smem[];
     const int tid = threadIdx.x;
     constexpr int bd = BD;
@@ -604,7 +659,7 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
 #define F4_OP(i) (CM ? prog.ops[i] : ops_s[i])
 #define F4_CH(i) (CM ? prog.ch[i] : chs_s[i])
     double *cur = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + sizeof(double) * 4 * C * bd);   /* [C][4][bd] */
-    double *accE = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + ((EDGE && !MARG) ? sizeof(double) * nwarp * a.E : 0));
+    double *accE = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + ((EDGE && !MARG && !GM) ? sizeof(double) * nwarp * a.E : 0));
     double *stack = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + (EDGE ? 0 : sizeof(double) * 4 * C * bd * a.stack_depth));
     int *stackf = reinterpret_cast<int *>(f4_smem + off); off = f4_align16(off + (EDGE ? 0 : sizeof(int) * bd * a.stack_depth));
     unsigned char *tile = f4_smem + off; off = f4_align16(off + (size_t)(PACK ? (a.ncode_rows + 1) / 2 : a.ncode_rows) * bd);
@@ -616,14 +671,14 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
         const size_t nF = MARG ? (size_t)C * a.Et * 16 : nP;       /* marginal mode: P of the tip edges */
         double *sP = reinterpret_cast<double *>(f4_smem + off); off += sizeof(double) * nP;
         double *sT = reinterpret_cast<double *>(f4_smem + off); off += sizeof(double) * nT;
-        double *sF = reinterpret_cast<double *>(f4_smem + off); off += EDGE ? sizeof(double) * nF : 0;
-        double *sTF = reinterpret_cast<double *>(f4_smem + off); off += (EDGE && !MARG && STAGED == 2) ? sizeof(double) * nT : 0;
+        double *sF = reinterpret_cast<double *>(f4_smem + off); off += (EDGE && !GM) ? sizeof(double) * nF : 0;
+        double *sTF = reinterpret_cast<double *>(f4_smem + off); off += (EDGE && !MARG && !GM && STAGED == 2) ? sizeof(double) * nT : 0;
         /* (counts as int: a compile-time zero count would make the loop test an unsigned comparison with 0) */
         for (int i = tid; i < (int)nP; i += bd) sP[i] = a.Pint[i];
-        for (int i = tid; i < (EDGE ? (int)nF : 0); i += bd) sF[i] = a.Fint[i];
-        for (size_t i = tid; i < nT; i += bd) { sT[i] = a.TP[i]; if (EDGE && !MARG && STAGED == 2) sTF[i] = a.TF[i]; }
+        for (int i = tid; i < ((EDGE && !GM) ? (int)nF : 0); i += bd) sF[i] = a.Fint[i];
+        for (size_t i = tid; i < nT; i += bd) { sT[i] = a.TP[i]; if (EDGE && !MARG && !GM && STAGED == 2) sTF[i] = a.TF[i]; }
         Pint = sP; TP = sT; Fint = sF;
-        if (STAGED == 2 && !MARG) TF = sTF;
+        if (STAGED == 2 && !MARG && !GM) TF = sTF;
     }
     if (!CM) {
         for (int i = tid; i < a.nops; i += bd) ops_s[i] = a.ops[i];
@@ -631,8 +686,9 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
     }
     for (int i = tid; i < a.K; i += bd) dconst[i] = a.def_const[i];
     for (int i = tid; i < 4 * a.K; i += bd) defs_s[i] = a.defs[i];
-    if (EDGE && !MARG) for (int i = tid; i < nwarp * a.E; i += bd) accE[i] = 0.0;
+    if (EDGE && !MARG && !GM) for (int i = tid; i < nwarp * a.E; i += bd) accE[i] = 0.0;
     double *accM = MARG ? a.block_marg + ((size_t)blockIdx.x * nwarp + warp) * ((size_t)a.N * 4) : nullptr;
+    double *accG = GM ? a.block_gmat + ((size_t)blockIdx.x * nwarp + warp) * ((size_t)C * a.E * 16) : nullptr;
     __syncthreads();
 
     const int tpstride = a.Et * a.K * 4;     /* doubles per category in the tip tables */
@@ -859,27 +915,28 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
                         for (int c = 0; c < C; c++) f4_prefetch(&a.scratch[((size_t)nc.slot * C + c) * T + gtid]);
                     }
                     if (STAGED == 0 && !CM)
-                        f4_prefetch_tables<C, BD, PACK, !MARG>(a, nc, tile, Pint, Fint, TP, TF, pstride, tpstride, tid, lane);
+                        f4_prefetch_tables<C, BD, PACK, !MARG && !GM>(a, nc, tile, Pint, Fint, TP, TF, pstride, tpstride, tid, lane);
                 }
             }
             if (op.nchild == 2) {
                 const F4Child c0 = F4_CH(op.first_child), c1 = F4_CH(op.first_child + 1);
                 double x0, x1, mgo[12];
                 if (c0.kind == F4_KIND_CUR && c1.kind == F4_KIND_TIP)
-                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_TIP, PACK, CM, MARG>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo);
+                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_TIP, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
+                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
                 else if (c0.kind == F4_KIND_CUR)
-                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_STACK, PACK, CM, MARG>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                   pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo);
+                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_STACK, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
+                                                                   pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
                 else
-                    f4_outside2<C, BD, F4_KIND_TIP, F4_KIND_TIP, PACK, CM, MARG>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo);
+                    f4_outside2<C, BD, F4_KIND_TIP, F4_KIND_TIP, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
+                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
                 if (MARG) {
                     f4_marg_out(a, accM, op.node, mgo, valid, site, lane);
                     if (c0.kind == F4_KIND_TIP) f4_marg_out(a, accM, c0.node, mgo + 4, valid, site, lane);
                     if (c1.kind == F4_KIND_TIP) f4_marg_out(a, accM, c1.node, mgo + 8, valid, site, lane);
                     continue;
                 }
+                if (GM) continue;
                 const bool m0 = !a.edge_mask || a.edge_mask[c0.edge];
                 const bool m1 = !a.edge_mask || a.edge_mask[c1.edge];
                 if (a.edge_site_out) {
@@ -896,11 +953,11 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
             }
             if (!CM) {      /* the host selects a CM kernel only for programs made of two-children nodes */
                 F4Ctx k;
-                k.cur = cur; k.accE = accE; k.accM = accM; k.tile = tile; k.defs_s = defs_s; k.Pint = Pint; k.Fint = Fint; k.TP = TP; k.TF = TF;
+                k.cur = cur; k.accE = accE; k.accM = accM; k.accG = accG; k.tile = tile; k.defs_s = defs_s; k.Pint = Pint; k.Fint = Fint; k.TP = TP; k.TF = TF;
                 k.chp = CM ? prog.ch : chs_s;
                 k.pstride = pstride; k.tpstride = tpstride; k.tid = tid; k.lane = lane; k.warp = warp;
                 k.T = (size_t)T; k.gtid = (size_t)gtid; k.site = site; k.valid = valid;
-                f4_outside_general<C, BD, PACK, CM, MARG>(a, op, from_slot, k);
+                f4_outside_general<C, BD, PACK, CM, MARG, GM>(a, op, from_slot, k);
             }
         }
     }
@@ -916,7 +973,7 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
             for (int i = 0; i < nwarp; i++) s += red[i];
             a.block_ll[blockIdx.x] = s;
         }
-        if (EDGE && !MARG && !a.edge_site_out) {
+        if (EDGE && !MARG && !GM && !a.edge_site_out) {
             for (int e = tid; e < a.E; e += bd) {
                 double s = 0.0;
                 for (int wv = 0; wv < nwarp; wv++) s += accE[wv * a.E + e];

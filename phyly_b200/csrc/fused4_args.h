@@ -42,6 +42,7 @@ struct F4Args {
     double *block_ll;                /* [grid] */
     double *block_edge;              /* [grid][E] */
     int *error_flag;
+    double *block_gmat;              /* mode 3: [grid * warps][C][E][16], zeroed by the host, accumulated here */
 };
 
 /*
@@ -65,7 +66,8 @@ __host__ __device__ inline size_t f4_align16(size_t x) { return (x + 15) & ~(siz
 typedef void (*f4_kernel_t)(const F4Args, const F4Prog);
 
 /* kernel instantiation for (block size, staging level, packed codes, constant-memory matrices, categories, mode):
- * mode 0 = ll only, 1 = ll + edge forms, 2 = ll + marginals; NULL when the combination is not instantiated */
+ * mode 0 = ll only, 1 = ll + edge forms, 2 = ll + marginals, 3 = ll + per-edge outer-product matrices (the 256- and
+ * 128-thread configurations of mode 2); NULL when the combination is not instantiated */
 f4_kernel_t f4_get_kernel(int bd, int staged, bool pack, bool cm, int C, int mode);
 /* copy the compact matrices of the internal-child edges into the constant bank (device to device, in-stream) */
 cudaError_t f4_upload_const(const double *Pint, const double *Fint, size_t bytes, cudaStream_t st);

@@ -6,14 +6,29 @@
 #include <cuda_runtime.h>
 #include "fused4.cuh"
 
-template <int BD, int STAGED, bool PACK>
-static f4_kernel_t f4_select_marg(int C)
+/* mode 3: the configurations of mode 2 less the four in which ptxas (CUDA 12.9) spills at the register cap
+ * (-Xptxas -v); the tuning in run_fused picks among the others */
+template <int C, int BD, int STAGED, bool PACK>
+static f4_kernel_t f4_gm_kernel()
 {
-    switch (C) {
-    case 1: return fused4_kernel<1, 2, BD, STAGED, PACK, false>;
-    case 2: return fused4_kernel<2, 2, BD, STAGED, PACK, false>;
-    case 3: return fused4_kernel<3, 2, BD, STAGED, PACK, false>;
-    case 4: return fused4_kernel<4, 2, BD, STAGED, PACK, false>;
+    constexpr bool spills = (C == 4 && BD == 384 && STAGED <= 1 && PACK == (STAGED == 0)) || (C == 2 && BD <= 256 && STAGED == 0);
+    if constexpr (spills) return nullptr;
+    else return fused4_kernel<C, 3, BD, STAGED, PACK, false>;
+}
+
+/* the outside-pass modes without edge-form tables: 2 (marginals) and 3 (per-edge outer-product matrices) */
+template <int BD, int STAGED, bool PACK>
+static f4_kernel_t f4_select_marg(int C, int mode)
+{
+    switch (C * 2 + (mode == 3 ? 1 : 0)) {
+    case 2: return fused4_kernel<1, 2, BD, STAGED, PACK, false>;
+    case 3: return f4_gm_kernel<1, BD, STAGED, PACK>();
+    case 4: return fused4_kernel<2, 2, BD, STAGED, PACK, false>;
+    case 5: return f4_gm_kernel<2, BD, STAGED, PACK>();
+    case 6: return fused4_kernel<3, 2, BD, STAGED, PACK, false>;
+    case 7: return f4_gm_kernel<3, BD, STAGED, PACK>();
+    case 8: return fused4_kernel<4, 2, BD, STAGED, PACK, false>;
+    case 9: return f4_gm_kernel<4, BD, STAGED, PACK>();
     }
     return nullptr;
 }
@@ -39,15 +54,15 @@ static f4_kernel_t f4_select_c(int C, bool edge)
 f4_kernel_t f4_get_kernel(int bd, int staged, bool pack, bool cm, int C, int mode)
 {
     const int key = F4_KEY(bd, staged, pack, cm);
-    if (mode == 2) {
+    if (mode == 2 || mode == 3) {
         switch (key) {
-        case F4_KEY(384, 1, true, false): return f4_select_marg<384, 1, true>(C);
-        case F4_KEY(384, 1, false, false): return f4_select_marg<384, 1, false>(C);
-        case F4_KEY(256, 1, false, false): return f4_select_marg<256, 1, false>(C);
-        case F4_KEY(384, 0, true, false): return f4_select_marg<384, 0, true>(C);
-        case F4_KEY(384, 0, false, false): return f4_select_marg<384, 0, false>(C);
-        case F4_KEY(256, 0, false, false): return f4_select_marg<256, 0, false>(C);
-        case F4_KEY(128, 0, false, false): return f4_select_marg<128, 0, false>(C);
+        case F4_KEY(384, 1, true, false): return f4_select_marg<384, 1, true>(C, mode);
+        case F4_KEY(384, 1, false, false): return f4_select_marg<384, 1, false>(C, mode);
+        case F4_KEY(256, 1, false, false): return f4_select_marg<256, 1, false>(C, mode);
+        case F4_KEY(384, 0, true, false): return f4_select_marg<384, 0, true>(C, mode);
+        case F4_KEY(384, 0, false, false): return f4_select_marg<384, 0, false>(C, mode);
+        case F4_KEY(256, 0, false, false): return f4_select_marg<256, 0, false>(C, mode);
+        case F4_KEY(128, 0, false, false): return f4_select_marg<128, 0, false>(C, mode);
         }
         return nullptr;
     }

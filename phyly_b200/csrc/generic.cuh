@@ -70,6 +70,10 @@ struct GenericArgs {
     /* tile_inside_kernel stages the tile's tip codes in shared memory (1-byte codes, Et * 64 bytes) */
     int tip_stage;
     const int *tip_edge_csr;      /* [Et] csr index of each tip edge */
+    /* plf_edge_expect_all: the outside pass writes the scaled outside edge vectors w_s prior_c fe / L_s (exponents
+     * applied, the child's included) to fe_out [C][E][n][Sc]; generic_gmat_kernel multiplies them into the L_b */
+    double *fe_out;
+    const double *site_w;         /* [S] or NULL, read with fe_out */
 };
 
 __device__ __forceinline__ int plf_code_at(const void *codes, int code_bytes, int64_t S, int node, int64_t site)
@@ -272,6 +276,12 @@ __global__ void __launch_bounds__(PLF_TS) generic_outside_kernel(GenericArgs a)
                 const double *Lb = a.Lg + ((cN + b) * n) * Sc + s;
                 const int kb = a.Kg[(cN + b) * Sc + s];
                 const int bc = a.Cg[(cN + b) * Sc + s];
+                if (a.fe_out) {
+                    const double wv = a.site_w ? a.site_w[gs] : 1.0;
+                    double *Fo = a.fe_out + ((cE + idx) * n) * Sc + s;
+                    const int sh = PLF_SCALE_BITS * (kfe + kb - site_k);
+                    for (int i = 0; i < n; i++) Fo[(size_t)i * Sc] = (wv == 0.0) ? 0.0 : scalbn(fe[i * PLF_TS] * coef * wv, sh);
+                }
                 if (a.want_edge && (!a.edge_mask || a.edge_mask[idx])) {
                     /* evaluate_site_frechet.c:18-39: fe^T F L_b */
                     double x = 0.0;
@@ -306,6 +316,54 @@ __global__ void __launch_bounds__(PLF_TS) generic_outside_kernel(GenericArgs a)
                     a.FK[(cN + b) * Sc + s] = kfb;
                 }
             }
+        }
+    }
+}
+
+/*
+ * plf_edge_expect_all: G[c][e][i][j] += sum_s fe_out[c][e][i][s] L_b[c][b][j][s] over the sites of a chunk (b = child of
+ * edge e).  One CTA per (edge, category); the entries in blocks of 4 x 4, every thread a fixed slice of the sites, the
+ * slices added in a fixed tree order, the chunks in order: the same bits on every run.
+ */
+__global__ void __launch_bounds__(256) generic_gmat_kernel(GenericArgs a, double *G)
+{
+    __shared__ double red[16][256];
+    const int e = blockIdx.x, c = blockIdx.y, tid = threadIdx.x, n = a.n, Sc = a.Sc;
+    const int b = a.t.indices[e];
+    const double *FE = a.fe_out + (((size_t)c * a.t.E + e) * n) * Sc;
+    const double *Lb = a.Lg + (((size_t)c * a.t.N + b) * n) * Sc;
+    double *Ge = G + ((size_t)c * a.t.E + e) * n * n;
+    for (int i0 = 0; i0 < n; i0 += 4) {
+        for (int j0 = 0; j0 < n; j0 += 4) {
+            double acc[16];
+#pragma unroll
+            for (int k = 0; k < 16; k++) acc[k] = 0.0;
+            for (int s = tid; s < Sc; s += 256) {
+                double f[4], l[4];
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    f[k] = (i0 + k < n) ? FE[(size_t)(i0 + k) * Sc + s] : 0.0;
+                    l[k] = (j0 + k < n) ? Lb[(size_t)(j0 + k) * Sc + s] : 0.0;
+                }
+#pragma unroll
+                for (int ii = 0; ii < 4; ii++)
+#pragma unroll
+                    for (int jj = 0; jj < 4; jj++) acc[4 * ii + jj] = fma(f[ii], l[jj], acc[4 * ii + jj]);
+            }
+#pragma unroll
+            for (int k = 0; k < 16; k++) red[k][tid] = acc[k];
+            __syncthreads();
+            for (int o = 128; o > 0; o >>= 1) {
+                if (tid < o)
+#pragma unroll
+                    for (int k = 0; k < 16; k++) red[k][tid] += red[k][tid + o];
+                __syncthreads();
+            }
+            if (tid < 16) {
+                const int i = i0 + (tid >> 2), j = j0 + (tid & 3);
+                if (i < n && j < n) Ge[(size_t)i * n + j] += red[tid][0];
+            }
+            __syncthreads();
         }
     }
 }

@@ -144,14 +144,16 @@ struct plf_engine {
     DevBuf d_dmPf, d_dmTPf, d_dmTFf, d_dm_defsf, d_dm_rootf, d_dm_stack, d_dm_stackmeta, d_dm_slab, d_dm_slabmeta, d_dm_Of, d_dm_oidx, d_dm_otr, d_dm_ops, d_dm_ch;
     int dm_out_depth = 0;
     F4Prog prog_h;
-    /* tuning / candidate caches of the fused kernel: slot = 5 * kind (ll, edge forms, marginals) + categories of the launch */
-    uint64_t program_version = 0, f4_tuned_version[15];
-    size_t f4_tuned_pick[15] = {0};
-    int f4_tuned_C[15] = {0}, f4_tuned_K[15] = {0};
-    std::string f4_cand_key[15];
-    std::vector<Cand> f4_cands[15];
+    /* tuning / candidate caches of the fused kernel: slot = 5 * kind (ll, edge forms, marginals, edge matrices) +
+     * categories of the launch */
+    uint64_t program_version = 0, f4_tuned_version[20];
+    size_t f4_tuned_pick[20] = {0};
+    int f4_tuned_C[20] = {0}, f4_tuned_K[20] = {0};
+    std::string f4_cand_key[20];
+    std::vector<Cand> f4_cands[20];
     DevBuf f4w_ll, f4w_edge, f4w_marg;      /* per-window per-site outputs when C > 4 (run_fused_windows) */
-    plf_engine() { for (int i = 0; i < 15; i++) f4_tuned_version[i] = ~(uint64_t)0; }
+    DevBuf d_block_gmat, g_fe, d_gmat_W, d_gmat_out;   /* plf_edge_expect_all */
+    plf_engine() { for (int i = 0; i < 20; i++) f4_tuned_version[i] = ~(uint64_t)0; }
 
     /* scratch */
     DevBuf d_scratch, d_scratchS, d_block_ll, d_block_edge, d_edge_site, d_sum, d_site_ll, d_err, d_mask, d_retry;
@@ -856,12 +858,13 @@ extern "C" int plf_set_edge_rates(plf_engine *e, const double *edge_rates)
 
 /* launch the expm kernel; which outputs are produced depends on the pointers */
 static int run_expm(plf_engine *e, double *P, double *D, double *F, int f_scale_mode, const unsigned char *d_mask,
-                    const double *d_lhi, const double *d_llo)
+                    const double *d_lhi, const double *d_llo, const double *d_lper = nullptr, int q_transpose = 0)
 {
     ExpmArgs a;
     a.n = e->n; a.E = e->E; a.C = e->C;
     a.q_hi = e->d_qhi.as<double>(); a.q_lo = e->d_qlo.as<double>();
     a.l_hi = d_lhi; a.l_lo = d_llo;
+    a.l_per = d_lper; a.q_transpose = q_transpose;
     a.edge_rate = e->d_edge_rates.as<double>(); a.cat_rate = e->d_cat_rates.as<double>();
     a.edge_mask = d_mask;
     a.P = P; a.D = D; a.F = F; a.f_scale_mode = f_scale_mode;
@@ -1133,6 +1136,9 @@ struct Query {
     double *site_edge = nullptr, *sum_edge = nullptr;   /* [S][E], [E] */
     double *site_marg = nullptr, *sum_marg = nullptr;   /* [S][N][n], [N][n] */
     double *sum_hess = nullptr;                         /* [E][E]: Hessian of the weighted log likelihood (generic path) */
+    /* plf_edge_expect_all: [sum_ll | G] is reduced, then run_gmat_adjoint turns G into the dwell / trans matrices */
+    bool want_gmat = false;
+    double *dwell_out = nullptr, *trans_out = nullptr;  /* [E][n][n] */
 };
 
 static bool fused_applicable(const plf_engine *e)
@@ -1281,7 +1287,7 @@ static cudaEvent_t g_cm_done[64];
 
 /* mirrors the shared-memory carve-up at the top of fused4_kernel */
 static size_t f4_smem_bytes(const plf_engine *e, bool edge, int bd, int staged, bool pack = false, bool cm = false,
-                            bool marg = false, bool gstack = false)
+                            bool marg = false, bool gstack = false, bool gm = false)
 {
     const int sdepth = gstack ? 0 : e->stack_depth;
     const int C = std::min(e->C, 4), Ei = cm ? 0 : (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
@@ -1289,7 +1295,7 @@ static size_t f4_smem_bytes(const plf_engine *e, bool edge, int bd, int staged, 
     off = f4_align16(off + (cm ? 0 : sizeof(F4Op) * e->ops.size()));
     off = f4_align16(off + (cm ? 0 : sizeof(F4Child) * e->children.size()));
     off = f4_align16(off + sizeof(double) * 4 * C * bd);
-    off = f4_align16(off + ((edge && !marg) ? sizeof(double) * (bd / 32) * e->E : 0));
+    off = f4_align16(off + ((edge && !marg && !gm) ? sizeof(double) * (bd / 32) * e->E : 0));
     off = f4_align16(off + (edge ? 0 : sizeof(double) * 4 * C * bd * sdepth));
     off = f4_align16(off + (edge ? 0 : sizeof(int) * bd * sdepth));
     off = f4_align16(off + (pack ? (e->code_row_node.size() + 1) / 2 : e->code_row_node.size()) * bd);
@@ -1297,13 +1303,58 @@ static size_t f4_smem_bytes(const plf_engine *e, bool edge, int bd, int staged, 
     off = f4_align16(off + sizeof(double) * 4 * e->K);
     const size_t nP = (size_t)C * Ei * 16 * sizeof(double), nT = (size_t)C * Et * e->K * 4 * sizeof(double);
     const size_t nF = marg ? (size_t)C * Et * 16 * sizeof(double) : nP;
-    if (staged) off += nP + nT + (edge ? nF : 0) + ((edge && !marg && staged == 2) ? nT : 0);
+    if (staged) off += nP + nT + ((edge && !gm) ? nF : 0) + ((edge && !marg && !gm && staged == 2) ? nT : 0);
     return off + 16;
 }
 
 static bool fused_fits(const plf_engine *e, bool edge)
 {
     return f4_smem_bytes(e, edge, 128, 0) <= 227 * 1024;
+}
+
+/* dwell[e] = sum_c W[c][e], trans[e] = sum_c rate_c t_e W[c][e] (categories in order) */
+__global__ void gmat_combine_kernel(const double *W, const double *cat_rate, const double *edge_rate, int C, int E, int nn,
+                                    double *dwell, double *trans)
+{
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= E * nn) return;
+    const double t = edge_rate[idx / nn];
+    double d = 0.0, x = 0.0;
+    for (int c = 0; c < C; c++) {
+        const double w = W[(size_t)c * E * nn + idx];
+        d += w;
+        x = fma(cat_rate[c] * t, w, x);
+    }
+    dwell[idx] = d;
+    trans[idx] = x;
+}
+
+/*
+ * plf_edge_expect_all, after the all-reduce of G: the edge form is bilinear, fe^T F_A(L) L_b = <L, F_{A^T}(fe L_b^T)>
+ * (the adjoint of the Frechet derivative of exp at A is the one at A^T), so W_{e,c} = F_{A_{e,c}^T}(G_{e,c}) (double-
+ * double, one CTA per matrix) holds the values of every direction at once.  Every rank runs it on the same bits.
+ */
+static int run_gmat_adjoint(plf_engine *e, const double *d_G)
+{
+    const size_t nn = (size_t)e->n * e->n;
+    ENSURE(e, e->d_gmat_W, sizeof(double) * (size_t)e->C * e->E * nn);
+    ENSURE(e, e->d_gmat_out, sizeof(double) * 2 * (size_t)e->E * nn);
+    if (run_expm(e, nullptr, nullptr, e->d_gmat_W.as<double>(), 0, nullptr, nullptr, nullptr, d_G, 1)) return -1;
+    const int total = (int)(e->E * nn);
+    double *out = e->d_gmat_out.as<double>();
+    gmat_combine_kernel<<<(total + 255) / 256, 256, 0, e->stream>>>(e->d_gmat_W.as<double>(), e->d_cat_rates.as<double>(),
+                                                                   e->d_edge_rates.as<double>(), e->C, e->E, (int)nn, out, out + total);
+    KCHECK(e);
+    return 0;
+}
+
+/* host copies of the matrices of run_gmat_adjoint (in stream: final after the query's synchronisation) */
+static int copy_gmat_out(plf_engine *e, const Query &q)
+{
+    const size_t cnt = (size_t)e->E * e->n * e->n;
+    if (q.dwell_out) CK(e, cudaMemcpyAsync(q.dwell_out, e->d_gmat_out.p, sizeof(double) * cnt, cudaMemcpyDeviceToHost, e->stream));
+    if (q.trans_out) CK(e, cudaMemcpyAsync(q.trans_out, e->d_gmat_out.as<double>() + cnt, sizeof(double) * cnt, cudaMemcpyDeviceToHost, e->stream));
+    return 0;
 }
 
 /* A launch over a window of <= 4 rate categories [c0, c0 + e->C) of a model with more (run_fused_windows): per-site
@@ -1316,7 +1367,9 @@ struct F4Window {
 static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
 {
     const bool marg = q.want_marg;              /* outside pass producing node marginals */
-    const bool edge = q.want_edge || marg;      /* an outside pass runs (slab, no stack) */
+    const bool gm = q.want_gmat;                /* outside pass producing the per-edge matrices G (mode 3) */
+    const bool edge = q.want_edge || marg || gm;      /* an outside pass runs (slab, no stack) */
+    const int kind = gm ? 3 : (marg ? 2 : (edge ? 1 : 0));
     F4Args a;
     memset(&a, 0, sizeof(a));
     a.nops = (int)e->ops.size(); a.nchildren = (int)e->children.size();
@@ -1328,8 +1381,8 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     a.codes = e->d_codes.as<unsigned char>();
     a.defs = e->d_defs.as<double>(); a.def_const = e->d_def_const.as<unsigned char>();
     a.Pint = e->d_Pint.as<double>(); a.TP = e->d_TP.as<double>();
-    a.Fint = marg ? e->d_Ptip.as<double>() : (edge ? e->d_Fint.as<double>() : nullptr);
-    a.TF = (edge && !marg) ? e->d_TF.as<double>() : nullptr;
+    a.Fint = marg ? e->d_Ptip.as<double>() : ((edge && !gm) ? e->d_Fint.as<double>() : nullptr);
+    a.TF = (edge && !marg && !gm) ? e->d_TF.as<double>() : nullptr;
     a.f_zero_rowsum = q.f_zero_rowsum;
     a.cat_prior = e->d_cat_prior.as<double>();
     a.root_mode = e->root_mode;
@@ -1350,8 +1403,8 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     /* the candidates that fit (shared memory, occupancy) depend only on the program, the model's shape and the query
      * kind: scanned once and remembered -- the occupancy queries of a dozen instantiations cost more host time per
      * query than the matrix kernels take on the device */
-    const int tm0 = 5 * (marg ? 2 : (edge ? 1 : 0)) + e->C;
-    const char *force0 = getenv(marg ? "PLF_F4_CONFIG_MARG" : (edge ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
+    const int tm0 = 5 * kind + e->C;
+    const char *force0 = getenv((marg || gm) ? "PLF_F4_CONFIG_MARG" : (edge ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
     const std::string cand_key = std::to_string(e->program_version) + "/" + std::to_string(e->C) + "/" + std::to_string(e->K) + "/" +
                                  std::to_string(e->E) + "/" + (force0 ? force0 : "");
     std::vector<Cand> viable;
@@ -1362,15 +1415,17 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         bool can_cm = (size_t)e->C * e->edge_of_int.size() * 16 <= F4_CM_MAXD && e->ops.size() <= F4_CM_MAXOPS &&
                       e->children.size() <= F4_CM_MAXCH && e->device < 64;
         for (const F4Op &op : e->ops) if (op.nchild != 2) can_cm = false;     /* CM kernels carry the two-children step only */
+        /* marginals and edge matrices (modes 2 and 3): the same configurations (mode 3 has the 256- and 128-thread ones) */
+        const int mm = gm ? 3 : 2;
         const Cand mcands[] = {
-            {384, 1, true, false, can_pack ? f4_get_kernel(384, 1, true, false, e->C, 2) : nullptr, 0, 0},
-            {384, 1, false, false, f4_get_kernel(384, 1, false, false, e->C, 2), 0, 0},
-            {256, 1, false, false, f4_get_kernel(256, 1, false, false, e->C, 2), 0, 0},
+            {384, 1, true, false, can_pack ? f4_get_kernel(384, 1, true, false, e->C, mm) : nullptr, 0, 0},
+            {384, 1, false, false, f4_get_kernel(384, 1, false, false, e->C, mm), 0, 0},
+            {256, 1, false, false, f4_get_kernel(256, 1, false, false, e->C, mm), 0, 0},
             /* larger trees: tables through L1 / L2, CTAs stay large */
-            {384, 0, true, false, can_pack ? f4_get_kernel(384, 0, true, false, e->C, 2) : nullptr, 0, 0},
-            {384, 0, false, false, f4_get_kernel(384, 0, false, false, e->C, 2), 0, 0},
-            {256, 0, false, false, f4_get_kernel(256, 0, false, false, e->C, 2), 0, 0},
-            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, 2), 0, 0},
+            {384, 0, true, false, can_pack ? f4_get_kernel(384, 0, true, false, e->C, mm) : nullptr, 0, 0},
+            {384, 0, false, false, f4_get_kernel(384, 0, false, false, e->C, mm), 0, 0},
+            {256, 0, false, false, f4_get_kernel(256, 0, false, false, e->C, mm), 0, 0},
+            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, mm), 0, 0},
         };
         const Cand ecands[] = {
             {512, 2, true, true, (can_cm && can_pack) ? f4_get_kernel(512, 2, true, true, e->C, edge ? 1 : 0) : nullptr, 0, 0},
@@ -1405,16 +1460,16 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
             {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, 0), 0, 0, true},
             {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, 0), 0, 0, false},
         };
-        const Cand *cands = marg ? mcands : (edge ? ecands : lcands);
-        const int ncand = marg ? (int)(sizeof(mcands) / sizeof(mcands[0]))
-                               : (edge ? (int)(sizeof(ecands) / sizeof(ecands[0])) : (int)(sizeof(lcands) / sizeof(lcands[0])));
-        const char *force = getenv(marg ? "PLF_F4_CONFIG_MARG" : (edge ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
+        const Cand *cands = (marg || gm) ? mcands : (edge ? ecands : lcands);
+        const int ncand = (marg || gm) ? (int)(sizeof(mcands) / sizeof(mcands[0]))
+                                       : (edge ? (int)(sizeof(ecands) / sizeof(ecands[0])) : (int)(sizeof(lcands) / sizeof(lcands[0])));
+        const char *force = force0;
         size_t smem = 0;
         for (int i = 0; i < ncand; i++) {
             if (force && atoi(force) != i) continue;
             if (!cands[i].k) continue;
             Cand c = cands[i];
-            c.smem = smem = f4_smem_bytes(e, edge, c.bd, c.staged, c.pack, c.cm, marg, c.gstack);
+            c.smem = smem = f4_smem_bytes(e, edge, c.bd, c.staged, c.pack, c.cm, marg, c.gstack, gm);
             if (c.smem > smem_cap) continue;
             CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
             CK(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.per_sm, c.k, c.bd, c.smem));
@@ -1440,7 +1495,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
      * on a sample of the sites and keeps the fastest. */
     const int64_t tune_sites = (int64_t)e->sm_count * 512 * 2;
     const bool can_tune = viable.size() > 1 && e->S >= tune_sites / 2 && !getenv("PLF_F4_NOTUNE");
-    const int tm = 5 * (marg ? 2 : (edge ? 1 : 0)) + e->C;      /* tuning slot: (ll, edge forms, marginals) x categories */
+    const int tm = tm0;      /* tuning slot: (ll, edge forms, marginals, edge matrices) x categories */
     size_t pick = 0;
     bool tune = false;
     if (can_tune) {
@@ -1460,7 +1515,8 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     }
 
     ENSURE(e, e->d_block_ll, sizeof(double) * gmax * nchunk);
-    ENSURE(e, e->d_sum, sizeof(double) * (2 + e->E + (size_t)e->N * e->n));
+    const size_t ngm = gm ? (size_t)e->C * e->E * 16 : 0;     /* mode 3: G[C][E][16] follows sum_ll */
+    ENSURE(e, e->d_sum, sizeof(double) * (2 + std::max((size_t)e->E + (size_t)e->N * e->n, ngm)));
     ENSURE(e, e->d_err, sizeof(int) * (e->N + 4));
     CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
     a.block_ll = e->d_block_ll.as<double>();
@@ -1471,7 +1527,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     if (edge) {
         ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * e->nslots * Tmax);
         ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)e->nslots * Tmax);
-        if (!marg) ENSURE(e, e->d_block_edge, sizeof(double) * (size_t)gmax * e->E * nchunk);
+        if (!marg && !gm) ENSURE(e, e->d_block_edge, sizeof(double) * (size_t)gmax * e->E * nchunk);
         a.scratch = e->d_scratch.as<double4>(); a.scratchS = e->d_scratchS.as<unsigned int>();
         a.block_edge = e->d_block_edge.as<double>();
         if (marg && win) {
@@ -1487,6 +1543,11 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
             ENSURE(e, e->d_block_marg, sizeof(double) * rows * e->N * 4);
             CK(e, cudaMemsetAsync(e->d_block_marg.p, 0, sizeof(double) * rows * e->N * 4, e->stream));
             a.block_marg = e->d_block_marg.as<double>();
+        } else if (gm) {
+            /* the same for the matrices G: a row [C][E][16] per warp */
+            ENSURE(e, e->d_block_gmat, sizeof(double) * (size_t)gmax * 16 * ngm);
+            CK(e, cudaMemsetAsync(e->d_block_gmat.p, 0, sizeof(double) * (size_t)gmax * 16 * ngm, e->stream));
+            a.block_gmat = e->d_block_gmat.as<double>();
         }
         if (q.edge_mask_h) {
             ENSURE(e, e->d_mask, e->E);
@@ -1561,12 +1622,13 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         /* the marginal accumulators are added to by every launch: forget what the timing runs left there */
         if (marg && a.block_marg)
             CK(e, cudaMemsetAsync(e->d_block_marg.p, 0, sizeof(double) * (size_t)gmax * 16 * e->N * 4, e->stream));
+        if (gm) CK(e, cudaMemsetAsync(e->d_block_gmat.p, 0, sizeof(double) * (size_t)gmax * 16 * ngm, e->stream));
     }
     const Cand &use = viable[pick];
     const int grid = grid_of(use);
     {
         char nm[96];
-        snprintf(nm, sizeof nm, "fused4_kernel<%d,%d,%d,%d,%d,%d>", e->C, marg ? 2 : (edge ? 1 : 0), use.bd, use.staged, use.pack ? 1 : 0, use.cm ? 1 : 0);
+        snprintf(nm, sizeof nm, "fused4_kernel<%d,%d,%d,%d,%d,%d>", e->C, kind, use.bd, use.staged, use.pack ? 1 : 0, use.cm ? 1 : 0);
         e->last_kernel = nm;
     }
     a.gstack = use.gstack ? 1 : 0; a.stack_depth = use.gstack ? 0 : e->stack_depth;
@@ -1575,7 +1637,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     for (size_t k = 0; k < nchunk; k++) {
         a.s_begin = bounds[k]; a.s_end = bounds[k + 1];
         a.block_ll = e->d_block_ll.as<double>() + k * (size_t)grid;
-        if (edge && !marg) a.block_edge = e->d_block_edge.as<double>() + k * (size_t)grid * e->E;
+        if (edge && !marg && !gm) a.block_edge = e->d_block_edge.as<double>() + k * (size_t)grid * e->E;
         if (pipelined) {
             /* this chunk's codes and weights have arrived; bring them into the node-major layout */
             CK(e, cudaStreamWaitEvent(e->stream, e->chunk_ev[k], 0));
@@ -1611,7 +1673,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     if (edge) a.block_edge = e->d_block_edge.as<double>();
     double *dsum = e->d_sum.as<double>();
     /* ll / ll + edge sums with a communicator: second-stage reduction and all-reduce are one kernel over peer memory */
-    const bool fuse_reduce = !marg && !q.site_edge && !pipelined && peer_path(e, 1 + (size_t)(edge ? e->E : 0));
+    const bool fuse_reduce = !marg && !gm && !q.site_edge && !pipelined && peer_path(e, 1 + (size_t)(edge ? e->E : 0));
     if (!fuse_reduce) {
         sum_rows_kernel<<<1, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_ll, rows, 1, dsum);
         KCHECK(e);
@@ -1632,7 +1694,12 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         }
         nsum = 1 + e->E + cols;
     }
-    if (edge && !marg && !q.site_edge) {
+    if (gm) {
+        sum_rows_kernel<<<(unsigned)((ngm + 31) / 32), dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_gmat, grid * (use.bd / 32), (int)ngm, dsum + 1);
+        KCHECK(e);
+        nsum = 1 + ngm;
+    }
+    if (edge && !marg && !gm && !q.site_edge) {
         if (!fuse_reduce) {
             sum_rows_kernel<<<(e->E + 31) / 32, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_edge, rows, e->E, dsum + 1);
             KCHECK(e);
@@ -1653,6 +1720,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
                                                                          e->d_err.as<int>(), a.block_ll, edge ? a.block_edge : nullptr, rows, e->E);
         KCHECK(e);
     } else if (finish_sums(e, dsum, nsum + (shared_retry ? 1 : 0))) return -1;
+    if (gm && (run_gmat_adjoint(e, dsum + 1) || copy_gmat_out(e, q))) return -1;
     CK(e, cudaEventRecord(e->ev[2], e->stream));
     std::vector<double> hs(nsum + 1, 0.0);
     int herr = 0;
@@ -1671,7 +1739,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     }
     if (q.site_edge && copy_site_matrix(e, e->d_edge_site.as<double>(), e->E, e->S, q.site_edge)) return -1;
     if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg)) FAIL(e, "a site with non-zero weight has zero likelihood");
+    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg || gm)) FAIL(e, "a site with non-zero weight has zero likelihood");
     if (q.sum_ll) *q.sum_ll = hs[0];
     if (q.sum_edge && !marg && nsum > 1) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * e->E);
     if (marg && q.site_marg && copy_site_matrix(e, e->d_marg_site.as<double>(), e->N * 4, e->S, q.site_marg)) return -1;
@@ -1782,12 +1850,17 @@ static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
 static int run_generic(plf_engine *e, Query &q)
 {
     const int n = e->n, C = e->C, N = e->N, E = e->E;
-    const bool outside = q.want_edge || q.want_marg;
-    e->last_kernel = (n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE")) ? "tile_inside_kernel / tile_outside_kernel" : "generic_inside_kernel / generic_outside_kernel";
+    const bool gm = q.want_gmat;        /* plf_edge_expect_all: generic kernels only (generic_gmat_kernel) */
+    const bool outside = q.want_edge || q.want_marg || gm;
+    e->last_kernel = (n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !gm) ? "tile_inside_kernel / tile_outside_kernel"
+                                                                               : "generic_inside_kernel / generic_outside_kernel";
+    const size_t ngm = gm ? (size_t)C * E * n * n : 0;     /* G[C][E][n][n] follows sum_ll */
+    const size_t nsum_all = 1 + std::max((size_t)E + (size_t)N * n, ngm);
     /* chunk size from a memory budget */
     size_t per_site = (size_t)C * ((size_t)N * n * 8 + N * 5 + (size_t)E * n * 8 + 16) + 16;
     if (outside) per_site += (size_t)C * ((size_t)N * n * 8 + N * 4) + (size_t)E * 8 + (size_t)N * n * 8;
     if (q.sum_hess) per_site += (size_t)C * E * n * 8 + (size_t)N * n * 8 + (size_t)N * 4;
+    if (gm) per_site += (size_t)C * E * n * 8;
     size_t free_b = 0, total_b = 0;
     CK(e, cudaMemGetInfo(&free_b, &total_b));
     size_t budget = std::min<size_t>((size_t)24 << 30, free_b / 2);
@@ -1804,8 +1877,9 @@ static int run_generic(plf_engine *e, Query &q)
     ENSURE(e, e->g_site_m, sizeof(double) * Sc);
     ENSURE(e, e->g_site_k, sizeof(int) * Sc);
     ENSURE(e, e->d_site_ll, sizeof(double) * e->S);
-    ENSURE(e, e->d_sum, sizeof(double) * (1 + E + (size_t)N * n));
+    ENSURE(e, e->d_sum, sizeof(double) * nsum_all);
     ENSURE(e, e->d_err, sizeof(int) * (N + 4));
+    if (gm) ENSURE(e, e->g_fe, sizeof(double) * (size_t)C * E * n * Sc);
     if (outside) {
         ENSURE(e, e->g_Fg, sizeof(double) * (size_t)C * N * n * Sc);
         ENSURE(e, e->g_FK, sizeof(int) * (size_t)C * N * Sc);
@@ -1817,7 +1891,7 @@ static int run_generic(plf_engine *e, Query &q)
         CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, E, cudaMemcpyHostToDevice, e->stream));
     }
     double *dsum = e->d_sum.as<double>();
-    CK(e, cudaMemsetAsync(dsum, 0, sizeof(double) * (1 + E + (size_t)N * n), e->stream));
+    CK(e, cudaMemsetAsync(dsum, 0, sizeof(double) * nsum_all, e->stream));
     CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
 
     GenericArgs a;
@@ -1841,6 +1915,7 @@ static int run_generic(plf_engine *e, Query &q)
     a.edge_out = q.want_edge ? e->g_edge_out.as<double>() : nullptr;
     a.marg_out = q.want_marg ? e->g_marg_out.as<double>() : nullptr;
     a.want_edge = q.want_edge; a.want_marg = q.want_marg;
+    if (gm) { a.fe_out = e->g_fe.as<double>(); a.site_w = e->have_w ? e->d_site_w.as<double>() : nullptr; }
 
     const size_t smem_in = sizeof(double) * 2 * n * PLF_TS, smem_out = sizeof(double) * 3 * n * PLF_TS;
     if (smem_in > 48 * 1024) CK(e, cudaFuncSetAttribute(generic_inside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_in));
@@ -1848,7 +1923,7 @@ static int run_generic(plf_engine *e, Query &q)
     if (smem_out > 227 * 1024) FAIL(e, "state count %d is too large for the generic kernels", n);
     const double *w = e->have_w ? e->d_site_w.as<double>() : nullptr;
     /* 16 < n <= 64 (amino-acid, codon): inside pass on the FP64 tensor pipe (tile.cuh) */
-    const bool use_tile = n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess;
+    const bool use_tile = n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess && !gm;
     if (use_tile && e->K <= 4096 && !getenv("PLF_NO_TIPTABLE")) {
         /* tip tables (P_e def_k) so that tip children need no GEMM */
         if (ensure_program(e)) return -1;
@@ -1999,6 +2074,7 @@ static int run_generic(plf_engine *e, Query &q)
         if (outside) {
             if (q.want_edge) CK(e, cudaMemsetAsync(a.edge_out, 0, sizeof(double) * (size_t)E * a.Sc, e->stream));
             if (q.want_marg) CK(e, cudaMemsetAsync(a.marg_out, 0, sizeof(double) * (size_t)N * n * a.Sc, e->stream));
+            if (gm) CK(e, cudaMemsetAsync(a.fe_out, 0, sizeof(double) * (size_t)C * E * n * a.Sc, e->stream));
             if (use_tile) {
                 if (tnp == 32) tile_outside_kernel<32><<<(a.Sc + TL_TS - 1) / TL_TS, 128, smem_tile_out, e->stream>>>(a);
                 else tile_outside_kernel<64><<<(a.Sc + TL_TS - 1) / TL_TS, 256, smem_tile_out, e->stream>>>(a);
@@ -2010,6 +2086,10 @@ static int run_generic(plf_engine *e, Query &q)
             zero_lik_rows_kernel<<<(a.Sc + 255) / 256, 256, 0, e->stream>>>(a.site_ll + s0, w, s0, a.Sc, e->d_err.as<int>(),
                                                                             a.edge_out, q.want_edge ? E : 0, a.marg_out, q.want_marg ? N * n : 0);
             KCHECK(e);
+            if (gm && E > 0) {
+                generic_gmat_kernel<<<dim3(E, C), 256, 0, e->stream>>>(a, dsum + 1);
+                KCHECK(e);
+            }
             if (q.want_edge && q.sum_edge) {
                 wsum_rows_kernel<<<E, 256, 0, e->stream>>>(a.edge_out, w, s0, a.Sc, dsum + 1, e->d_err.as<int>(), 0);
                 KCHECK(e);
@@ -2038,8 +2118,9 @@ static int run_generic(plf_engine *e, Query &q)
             }
         }
     }
-    const size_t nsum = 1 + E + (size_t)N * n;
+    const size_t nsum = gm ? 1 + ngm : 1 + E + (size_t)N * n;
     if (finish_sums(e, dsum, nsum)) return -1;
+    if (gm && (run_gmat_adjoint(e, dsum + 1) || copy_gmat_out(e, q))) return -1;
     if (q.sum_hess) {
         /* H = sum of the per-CTA parts - Gram matrix of the per-site derivatives (lower triangle, csr order) */
         sum_rows_kernel<<<(unsigned)(((size_t)E * E + 31) / 32), dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(e->h_part.as<double>(), hgrid, E * E, e->h_out.as<double>());
@@ -2058,7 +2139,7 @@ static int run_generic(plf_engine *e, Query &q)
     CK(e, cudaStreamSynchronize(e->stream));
     if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
     if ((herr & 2) && q.sum_hess) FAIL(e, "infeasible: a rate category with a non-zero rate has zero likelihood at a weighted site");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg)) FAIL(e, "a site with non-zero weight has zero likelihood");
+    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg || gm)) FAIL(e, "a site with non-zero weight has zero likelihood");
     if (q.sum_hess) {
         for (int i = 0; i < E; i++) for (int j = 0; j < i; j++) q.sum_hess[(size_t)j * E + i] = q.sum_hess[(size_t)i * E + j];
     }
@@ -2307,7 +2388,8 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
 {
     if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
     CK(e, cudaSetDevice(e->device));
-    bool use_fused = fused_applicable(e) && !q.sum_hess;
+    /* the edge matrices need the whole site likelihood: no category windows (n = 4 with C > 4 goes to the generic path) */
+    bool use_fused = fused_applicable(e) && !q.sum_hess && !(q.want_gmat && e->C > 4);
     /* per-site marginals of a huge alignment: the generic path works in chunks of sites */
     if (q.want_marg && q.site_marg && (size_t)e->N * 4 * e->S * sizeof(double) > ((size_t)32 << 30)) use_fused = false;
     if (e->path == PLF_PATH_GENERIC) use_fused = false;
@@ -2315,7 +2397,7 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
     if (e->pend_active && !(use_fused && e->node_has_data_h.size() == (size_t)e->N) && resolve_pending(e)) return -1;
     if (use_fused) {
         if (ensure_program(e)) return -1;
-        if (!fused_fits(e, q.want_edge || q.want_marg)) use_fused = false;
+        if (!fused_fits(e, q.want_edge || q.want_marg || q.want_gmat)) use_fused = false;
     }
     if (!use_fused && resolve_pending(e)) return -1;
     if (e->path == PLF_PATH_FUSED4 && !use_fused) FAIL(e, "the fused 4-state path does not apply to this query");
@@ -2342,8 +2424,10 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
      * constant-memory kernels at the price of per-site outputs and a combination pass) */
     int wforce = 0;
     if (const char *wf = getenv("PLF_F4_WINDOW")) wforce = std::max(1, std::min(4, atoi(wf)));
-    int rc = use_fused ? ((e->C > 4 || (wforce && wforce < e->C)) ? run_fused_windows(e, q, wforce ? wforce : 4) : run_fused(e, q))
-                       : (e->path != PLF_PATH_GENERIC && !q.sum_hess && dmma_applicable(e, q)) ? run_dmma(e, q) : run_generic(e, q);
+    int rc = use_fused ? ((!q.want_gmat && (e->C > 4 || (wforce && wforce < e->C))) ? run_fused_windows(e, q, wforce ? wforce : 4)
+                                                                                : run_fused(e, q))
+                       : (e->path != PLF_PATH_GENERIC && !q.sum_hess && !q.want_gmat && dmma_applicable(e, q)) ? run_dmma(e, q)
+                                                                                                              : run_generic(e, q);
     if (rc) return rc;
     cudaEventElapsedTime(&e->ms_mat, e->ev[0], e->ev[1]);
     cudaEventElapsedTime(&e->ms_sites, e->ev[1], e->ev[2]);
@@ -2407,6 +2491,14 @@ extern "C" int plf_edge_expect(plf_engine *e, int kind, const double *l_hi, cons
     Query q;
     q.want_edge = true; q.edge_mask_h = edge_mask; q.site_edge = site_out; q.sum_edge = sum_out;
     return run_query(e, q, false, l_hi, l_lo, kind);
+}
+
+extern "C" int plf_edge_expect_all(plf_engine *e, double *sum_ll, double *dwell, double *trans)
+{
+    if (!e) return -1;
+    Query q;
+    q.want_gmat = true; q.sum_ll = sum_ll; q.dwell_out = dwell; q.trans_out = trans;
+    return run_query(e, q, false, nullptr, nullptr, 0);
 }
 
 extern "C" int plf_get_transition_matrices(plf_engine *e, double *p_out)

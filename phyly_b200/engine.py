@@ -175,6 +175,17 @@ class Engine:
         self._ck(self._lib.plf_edge_expect(self._h, kind, _ptr(_f64(l_hi)), _ptr(_f64(l_lo)), _ptr(m), _ptr(so), _ptr(tot)))
         return so, tot
 
+    def edge_expect_all(self):
+        """Every Frechet direction of edge_expect in one pass, site-summed with the site weights (plf_edge_expect_all):
+        sum_ll, dwell [E, n, n] and trans [E, n, n] with edge_expect(kind, L)[1][e] == (L * X_kind[e]).sum(), and
+        q_grad = trans.sum(0), the gradient of sum_ll with respect to the entries of the scaled rate matrix (category
+        rates, category priors and root prior held fixed)."""
+        sll = np.zeros(1)
+        dwell = np.zeros((self.E, self.n, self.n))
+        trans = np.zeros((self.E, self.n, self.n))
+        self._ck(self._lib.plf_edge_expect_all(self._h, _ptr(sll), _ptr(dwell), _ptr(trans)))
+        return dict(sum_ll=float(sll[0]), dwell=dwell, trans=trans, q_grad=trans.sum(axis=0))
+
     def transition_matrices(self):
         out = np.empty((self.C, self.E, self.n, self.n))
         self._ck(self._lib.plf_get_transition_matrices(self._h, _ptr(out)))
