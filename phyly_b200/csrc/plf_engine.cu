@@ -94,7 +94,19 @@ static NcclApi g_nccl;
 #define PLF_PEER_MAX 16
 #define PLF_PEER_CAP 8192          /* doubles per (sender, parity) slot of an inbox */
 
-struct Cand { int bd, staged; bool pack, cm; f4_kernel_t k; size_t smem; int per_sm; bool gstack; };
+/* a configuration of the fused kernel: block size, tables staged in shared memory (0: read through L1 / L2),
+ * packed codes, matrices in constant memory, pending partials of the ll-only walk in a global stack */
+struct F4Config { int bd, staged; bool pack, cm, gstack; };
+/* one that exists for the model's category count and fits the program: its kernel, shared memory and CTAs per SM */
+struct Cand : F4Config { f4_kernel_t k; size_t smem; int per_sm; };
+/* tuning / candidate cache of the fused kernel for one query kind and category count */
+struct F4Slot {
+    std::string cand_key;             /* program version / C / K / E / forced index the candidates were scanned for */
+    std::vector<Cand> cands;
+    uint64_t tuned_version = ~(uint64_t)0;
+    size_t tuned_pick = 0;
+    int tuned_C = 0, tuned_K = 0;
+};
 
 struct plf_engine {
     int device = 0;
@@ -144,16 +156,11 @@ struct plf_engine {
     DevBuf d_dmPf, d_dmTPf, d_dmTFf, d_dm_defsf, d_dm_rootf, d_dm_stack, d_dm_stackmeta, d_dm_slab, d_dm_slabmeta, d_dm_Of, d_dm_oidx, d_dm_otr, d_dm_ops, d_dm_ch;
     int dm_out_depth = 0;
     F4Prog prog_h;
-    /* tuning / candidate caches of the fused kernel: slot = 5 * kind (ll, edge forms, marginals, edge matrices) +
-     * categories of the launch */
-    uint64_t program_version = 0, f4_tuned_version[20];
-    size_t f4_tuned_pick[20] = {0};
-    int f4_tuned_C[20] = {0}, f4_tuned_K[20] = {0};
-    std::string f4_cand_key[20];
-    std::vector<Cand> f4_cands[20];
+    uint64_t program_version = 0;
+    /* slot = 5 * kind (ll, edge forms, marginals, edge matrices) + categories of the launch */
+    F4Slot f4_slot[20];
     DevBuf f4w_ll, f4w_edge, f4w_marg;      /* per-window per-site outputs when C > 4 (run_fused_windows) */
     DevBuf d_block_gmat, g_fe, d_gmat_W, d_gmat_out;   /* plf_edge_expect_all */
-    plf_engine() { for (int i = 0; i < 20; i++) f4_tuned_version[i] = ~(uint64_t)0; }
 
     /* scratch */
     DevBuf d_scratch, d_scratchS, d_block_ll, d_block_edge, d_edge_site, d_sum, d_site_ll, d_err, d_mask, d_retry;
@@ -1147,9 +1154,6 @@ static bool fused_applicable(const plf_engine *e)
     return e->n == 4 && e->C <= 16 && e->code_bytes == 1 && e->K <= 256 && e->max_degree <= F4_MAXD;
 }
 
-static bool fused_fits(const plf_engine *e, bool edge);
-static int ensure_program(plf_engine *e);
-
 static int ensure_program(plf_engine *e)
 {
     if (!e->program_dirty) return 0;
@@ -1244,7 +1248,7 @@ static bool peer_path(const plf_engine *e, size_t count)
 
 static int finish_sums(plf_engine *e, double *d_sum, size_t count)
 {
-    if (e->comm && !e->comm_paused && e->peer_ready && count <= PLF_PEER_CAP && !getenv("PLF_NO_PEER_ALLREDUCE")) {
+    if (peer_path(e, count)) {
         ENSURE(e, e->d_err, sizeof(int) * (e->N + 4));
         e->peer_seq++;
         peer_allreduce_kernel<<<1, 256, 0, e->stream>>>(d_sum, (int)count, e->peer_seq, e->rank, e->nranks,
@@ -1280,14 +1284,58 @@ static int copy_site_matrix(plf_engine *e, const double *d_rows /*[R][cols]*/, i
     return 0;
 }
 
+/* the buffers every query path ends in: site log-likelihoods, the sum vector (sum_doubles of it) and the error word
+ * (bit 0: a weighted site with zero likelihood, 1: Hessian infeasible, 2: peer all-reduce timed out), cleared */
+static int prepare_sums(plf_engine *e, size_t sum_doubles)
+{
+    ENSURE(e, e->d_site_ll, sizeof(double) * e->S);
+    ENSURE(e, e->d_sum, sizeof(double) * sum_doubles);
+    ENSURE(e, e->d_err, sizeof(int) * (e->N + 4));
+    CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
+    return 0;
+}
+
+/* the end of every query path: the first count doubles of d_sum, the error word, the site log-likelihoods and the
+ * Hessian to the host */
+static int read_back(plf_engine *e, const Query &q, const double *d_sum, size_t count, std::vector<double> &hs, int &herr)
+{
+    CK(e, cudaEventRecord(e->ev[2], e->stream));
+    hs.assign(count, 0.0); herr = 0;
+    CK(e, cudaMemcpyAsync(hs.data(), d_sum, sizeof(double) * count, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaMemcpyAsync(&herr, e->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+    if (q.site_ll) CK(e, cudaMemcpyAsync(q.site_ll, e->d_site_ll.p, sizeof(double) * e->S, cudaMemcpyDeviceToHost, e->stream));
+    if (q.sum_hess) CK(e, cudaMemcpyAsync(q.sum_hess, e->h_out.p, sizeof(double) * (size_t)e->E * e->E, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+/* errors of the query, then the host sums from the read-back sum vector [ll | edge (E) | marginals (N n)] */
+static int unpack_sums(plf_engine *e, const Query &q, const std::vector<double> &hs, int herr)
+{
+    const int E = e->E;
+    if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
+    if ((herr & 2) && q.sum_hess) FAIL(e, "infeasible: a rate category with a non-zero rate has zero likelihood at a weighted site");
+    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg || q.want_gmat)) FAIL(e, "a site with non-zero weight has zero likelihood");
+    if (q.sum_ll) *q.sum_ll = hs[0];
+    if (q.sum_edge) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * E);
+    if (q.sum_marg) memcpy(q.sum_marg, hs.data() + 1 + E, sizeof(double) * (size_t)e->N * e->n);
+    if (q.sum_hess)
+        for (int i = 0; i < E; i++) for (int j = 0; j < i; j++) q.sum_hess[(size_t)j * E + i] = q.sum_hess[(size_t)i * E + j];
+    return 0;
+}
+
 /* the constant-memory matrices are one per device and context: queries of different engines (different
  * streams) that use them are ordered through this event */
 static std::mutex g_cm_mutex;
 static cudaEvent_t g_cm_done[64];
 
+/* query kind of the fused path, the kernel's mode: 0 = ll, 1 = edge forms, 2 = marginals, 3 = edge matrices
+ * (1 to 3 run an outside pass: slab, no stack) */
+static int f4_kind(const Query &q) { return q.want_gmat ? 3 : (q.want_marg ? 2 : (q.want_edge ? 1 : 0)); }
+
 /* mirrors the shared-memory carve-up at the top of fused4_kernel */
-static size_t f4_smem_bytes(const plf_engine *e, bool edge, int bd, int staged, bool pack = false, bool cm = false,
-                            bool marg = false, bool gstack = false, bool gm = false)
+static size_t f4_smem_bytes(const plf_engine *e, int kind, int bd, int staged, bool pack = false, bool cm = false,
+                            bool gstack = false)
 {
     const int sdepth = gstack ? 0 : e->stack_depth;
     const int C = std::min(e->C, 4), Ei = cm ? 0 : (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
@@ -1295,21 +1343,22 @@ static size_t f4_smem_bytes(const plf_engine *e, bool edge, int bd, int staged, 
     off = f4_align16(off + (cm ? 0 : sizeof(F4Op) * e->ops.size()));
     off = f4_align16(off + (cm ? 0 : sizeof(F4Child) * e->children.size()));
     off = f4_align16(off + sizeof(double) * 4 * C * bd);
-    off = f4_align16(off + ((edge && !marg && !gm) ? sizeof(double) * (bd / 32) * e->E : 0));
-    off = f4_align16(off + (edge ? 0 : sizeof(double) * 4 * C * bd * sdepth));
-    off = f4_align16(off + (edge ? 0 : sizeof(int) * bd * sdepth));
+    off = f4_align16(off + (kind == 1 ? sizeof(double) * (bd / 32) * e->E : 0));
+    off = f4_align16(off + (kind ? 0 : sizeof(double) * 4 * C * bd * sdepth));
+    off = f4_align16(off + (kind ? 0 : sizeof(int) * bd * sdepth));
     off = f4_align16(off + (pack ? (e->code_row_node.size() + 1) / 2 : e->code_row_node.size()) * bd);
     off = f4_align16(off + e->K);
     off = f4_align16(off + sizeof(double) * 4 * e->K);
     const size_t nP = (size_t)C * Ei * 16 * sizeof(double), nT = (size_t)C * Et * e->K * 4 * sizeof(double);
-    const size_t nF = marg ? (size_t)C * Et * 16 * sizeof(double) : nP;
-    if (staged) off += nP + nT + ((edge && !gm) ? nF : 0) + ((edge && !marg && !gm && staged == 2) ? nT : 0);
+    const size_t nF = kind == 2 ? (size_t)C * Et * 16 * sizeof(double) : nP;
+    if (staged) off += nP + nT + ((kind == 1 || kind == 2) ? nF : 0) + ((kind == 1 && staged == 2) ? nT : 0);
     return off + 16;
 }
 
-static bool fused_fits(const plf_engine *e, bool edge)
+/* an outside pass is checked with the layout of the edge forms, the largest unstaged one */
+static bool fused_fits(const plf_engine *e, bool outside)
 {
-    return f4_smem_bytes(e, edge, 128, 0) <= 227 * 1024;
+    return f4_smem_bytes(e, outside ? 1 : 0, 128, 0) <= 227 * 1024;
 }
 
 /* dwell[e] = sum_c W[c][e], trans[e] = sum_c rate_c t_e W[c][e] (categories in order) */
@@ -1357,20 +1406,90 @@ static int copy_gmat_out(plf_engine *e, const Query &q)
     return 0;
 }
 
-/* A launch over a window of <= 4 rate categories [c0, c0 + e->C) of a model with more (run_fused_windows): per-site
- * outputs go to device buffers and nothing is reduced or copied here. */
-struct F4Window {
-    int c0 = 0;
-    double *site_ll = nullptr, *site_edge = nullptr, *site_marg = nullptr;
+/* candidate configurations of the fused kernel per query kind, preferred first.  PLF_F4_CONFIG (edge forms),
+ * PLF_F4_CONFIG_LL and PLF_F4_CONFIG_MARG (marginals, edge matrices) force one by its index here (tuning aid): an
+ * entry keeps its place where it has no kernel (pack needs K <= 16, cm a small binary tree). */
+static const std::vector<F4Config> f4_configs[3] = {
+    /* log-likelihood only: no slab; the pending partials of the post-order walk either sit in shared
+     * memory (which limits the CTA to 256 threads at depth 3) or in a small L2-resident global stack */
+    {{512, 2, true, true, true}, {512, 2, true, false, true}, {512, 2, false, true, true}, {384, 2, true, false, true},
+     {384, 2, true, false, false}, {384, 1, false, false, false}, {256, 2, false, false, false}, {256, 2, false, false, true},
+     {512, 0, true, false, true}, {384, 0, true, false, true}, {384, 0, false, false, true}, {256, 0, false, false, true},
+     {128, 0, false, false, true}, {128, 0, false, false, false}},
+    /* edge forms; from index 7 on, for larger trees (the tables no longer fit shared memory): tables through L1 / L2,
+     * CTAs stay large */
+    {{512, 2, true, true}, {512, 2, false, true}, {384, 2, false, true}, {384, 2, true, false}, {384, 1, false, false},
+     {512, 1, false, false}, {256, 2, false, false},
+     {512, 0, true, false}, {384, 0, true, false}, {384, 0, false, false}, {256, 0, false, false}, {128, 0, false, false}},
+    /* marginals and edge matrices (modes 2 and 3): the same configurations (mode 3 has the 256- and 128-thread ones) */
+    {{384, 1, true, false}, {384, 1, false, false}, {256, 1, false, false},
+     {384, 0, true, false}, {384, 0, false, false}, {256, 0, false, false}, {128, 0, false, false}},
 };
 
-static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
+/* sites of the tuning sample */
+static int64_t f4_tune_sites(const plf_engine *e) { return (int64_t)e->sm_count * 512 * 2; }
+
+/*
+ * Which configuration a fused query of this kind runs: the slot with its viable candidates, the index of the one to
+ * run or tune = true.  The candidates that fit (shared memory, occupancy) depend only on the program, the model's
+ * shape and the query kind: scanned once and remembered -- the occupancy queries of a dozen instantiations cost more
+ * host time per query than the matrix kernels take on the device.  The pick is the tuned one if this program has been
+ * tuned, else the first.  Whether the constant-memory kernels beat the shared-memory ones depends on what the compiler
+ * made of each instantiation (tools/check_cm_uniform.sh), so the first large query times the leading candidates on a
+ * sample of the sites and keeps the fastest.
+ */
+static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool &tune)
 {
-    const bool marg = q.want_marg;              /* outside pass producing node marginals */
-    const bool gm = q.want_gmat;                /* outside pass producing the per-edge matrices G (mode 3) */
-    const bool edge = q.want_edge || marg || gm;      /* an outside pass runs (slab, no stack) */
-    const int kind = gm ? 3 : (marg ? 2 : (edge ? 1 : 0));
-    F4Args a;
+    slot = &e->f4_slot[5 * kind + e->C];
+    const char *force = getenv(kind >= 2 ? "PLF_F4_CONFIG_MARG" : (kind ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
+    const std::string cand_key = std::to_string(e->program_version) + "/" + std::to_string(e->C) + "/" + std::to_string(e->K) + "/" +
+                                 std::to_string(e->E) + "/" + (force ? force : "");
+    if (slot->cand_key != cand_key) {
+        const bool can_pack = e->K <= 16;
+        bool can_cm = (size_t)e->C * e->edge_of_int.size() * 16 <= F4_CM_MAXD && e->ops.size() <= F4_CM_MAXOPS &&
+                      e->children.size() <= F4_CM_MAXCH && e->device < 64;
+        for (const F4Op &op : e->ops) if (op.nchild != 2) can_cm = false;     /* CM kernels carry the two-children step only */
+        const std::vector<F4Config> &cfgs = f4_configs[std::min(kind, 2)];
+        std::vector<Cand> viable;
+        size_t smem = 0;
+        for (int i = 0; i < (int)cfgs.size(); i++) {
+            const F4Config &f = cfgs[i];
+            if ((force && atoi(force) != i) || (f.pack && !can_pack) || (f.cm && !can_cm)) continue;
+            Cand c{f, f4_get_kernel(f.bd, f.staged, f.pack, f.cm, e->C, kind), 0, 0};
+            if (!c.k) continue;
+            c.smem = smem = f4_smem_bytes(e, kind, c.bd, c.staged, c.pack, c.cm, c.gstack);
+            if (c.smem > 227 * 1024) continue;
+            CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
+            CK(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.per_sm, c.k, c.bd, c.smem));
+            if (c.per_sm >= 1) viable.push_back(c);
+        }
+        if (viable.empty()) FAIL(e, "fused kernel: no configuration fits (C = %d, %zu bytes of shared memory)", e->C, smem);
+        slot->cand_key = cand_key;
+        slot->cands = std::move(viable);
+    }
+    const std::vector<Cand> &viable = slot->cands;
+    const bool can_tune = viable.size() > 1 && e->S >= f4_tune_sites(e) / 2 && !getenv("PLF_F4_NOTUNE");
+    pick = 0; tune = false;
+    if (can_tune && slot->tuned_version == e->program_version && slot->tuned_C == e->C && slot->tuned_K == e->K &&
+        slot->tuned_pick < viable.size())
+        pick = slot->tuned_pick;
+    else if (can_tune && !e->pend_active)
+        tune = true;
+    else        /* small problems, or untuned with the data still in flight: no constant-memory kernels */
+        while (pick + 1 < viable.size() && viable[pick].cm) pick++;
+    return 0;
+}
+
+/* A launch over a window of <= 4 rate categories [c0, c0 + e->C) of a model with more (run_fused_windows): per-site
+ * outputs go to these device buffers. */
+struct F4Window { int c0; double *site_ll, *site_edge, *site_marg; };
+
+/* what the reduction of a fused query needs from its launches */
+struct F4Launch { F4Args a; const Cand *use; int grid; size_t nchunk; bool pipelined; };
+
+/* the arguments of a fused launch that do not depend on its configuration */
+static void f4_fill_args(const plf_engine *e, const Query &q, int kind, const F4Window *win, F4Args &a)
+{
     memset(&a, 0, sizeof(a));
     a.nops = (int)e->ops.size(); a.nchildren = (int)e->children.size();
     a.ops = e->d_ops.as<F4Op>(); a.children = e->d_children.as<F4Child>();
@@ -1381,8 +1500,8 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     a.codes = e->d_codes.as<unsigned char>();
     a.defs = e->d_defs.as<double>(); a.def_const = e->d_def_const.as<unsigned char>();
     a.Pint = e->d_Pint.as<double>(); a.TP = e->d_TP.as<double>();
-    a.Fint = marg ? e->d_Ptip.as<double>() : ((edge && !gm) ? e->d_Fint.as<double>() : nullptr);
-    a.TF = (edge && !marg && !gm) ? e->d_TF.as<double>() : nullptr;
+    a.Fint = kind == 2 ? e->d_Ptip.as<double>() : (kind == 1 ? e->d_Fint.as<double>() : nullptr);
+    a.TF = kind == 1 ? e->d_TF.as<double>() : nullptr;
     a.f_zero_rowsum = q.f_zero_rowsum;
     a.cat_prior = e->d_cat_prior.as<double>();
     a.root_mode = e->root_mode;
@@ -1393,168 +1512,110 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         /* the tables are laid out [category][...]: a window is a pointer offset */
         const size_t c0 = (size_t)win->c0;
         a.Pint += c0 * a.Ei * 16; a.TP += c0 * a.Et * a.K * 4;
-        if (a.Fint) a.Fint += marg ? c0 * a.Et * 16 : c0 * a.Ei * 16;
+        if (a.Fint) a.Fint += kind == 2 ? c0 * a.Et * 16 : c0 * a.Ei * 16;
         if (a.TF) a.TF += c0 * a.Et * a.K * 4;
         a.cat_prior += c0;
     }
+}
 
-    /* candidate configurations (block size, which tables are staged in shared memory, packed codes, matrices
-     * in constant memory), preferred first.  PLF_F4_CONFIG=<index> forces one (tuning aid, edge queries). */
-    /* the candidates that fit (shared memory, occupancy) depend only on the program, the model's shape and the query
-     * kind: scanned once and remembered -- the occupancy queries of a dozen instantiations cost more host time per
-     * query than the matrix kernels take on the device */
-    const int tm0 = 5 * kind + e->C;
-    const char *force0 = getenv((marg || gm) ? "PLF_F4_CONFIG_MARG" : (edge ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
-    const std::string cand_key = std::to_string(e->program_version) + "/" + std::to_string(e->C) + "/" + std::to_string(e->K) + "/" +
-                                 std::to_string(e->E) + "/" + (force0 ? force0 : "");
-    std::vector<Cand> viable;
-    if (e->f4_cand_key[tm0] == cand_key) viable = e->f4_cands[tm0];
-    if (viable.empty()) {
-        const size_t smem_cap = 227 * 1024;
-        const bool can_pack = e->K <= 16;
-        bool can_cm = (size_t)e->C * e->edge_of_int.size() * 16 <= F4_CM_MAXD && e->ops.size() <= F4_CM_MAXOPS &&
-                      e->children.size() <= F4_CM_MAXCH && e->device < 64;
-        for (const F4Op &op : e->ops) if (op.nchild != 2) can_cm = false;     /* CM kernels carry the two-children step only */
-        /* marginals and edge matrices (modes 2 and 3): the same configurations (mode 3 has the 256- and 128-thread ones) */
-        const int mm = gm ? 3 : 2;
-        const Cand mcands[] = {
-            {384, 1, true, false, can_pack ? f4_get_kernel(384, 1, true, false, e->C, mm) : nullptr, 0, 0},
-            {384, 1, false, false, f4_get_kernel(384, 1, false, false, e->C, mm), 0, 0},
-            {256, 1, false, false, f4_get_kernel(256, 1, false, false, e->C, mm), 0, 0},
-            /* larger trees: tables through L1 / L2, CTAs stay large */
-            {384, 0, true, false, can_pack ? f4_get_kernel(384, 0, true, false, e->C, mm) : nullptr, 0, 0},
-            {384, 0, false, false, f4_get_kernel(384, 0, false, false, e->C, mm), 0, 0},
-            {256, 0, false, false, f4_get_kernel(256, 0, false, false, e->C, mm), 0, 0},
-            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, mm), 0, 0},
-        };
-        const Cand ecands[] = {
-            {512, 2, true, true, (can_cm && can_pack) ? f4_get_kernel(512, 2, true, true, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {512, 2, false, true, can_cm ? f4_get_kernel(512, 2, false, true, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {384, 2, false, true, can_cm ? f4_get_kernel(384, 2, false, true, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {384, 2, true, false, can_pack ? f4_get_kernel(384, 2, true, false, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {384, 1, false, false, f4_get_kernel(384, 1, false, false, e->C, edge ? 1 : 0), 0, 0},
-            {512, 1, false, false, f4_get_kernel(512, 1, false, false, e->C, edge ? 1 : 0), 0, 0},
-            {256, 2, false, false, f4_get_kernel(256, 2, false, false, e->C, edge ? 1 : 0), 0, 0},
-            /* larger trees (the tables no longer fit shared memory): tables through L1 / L2, CTAs stay large */
-            {512, 0, true, false, can_pack ? f4_get_kernel(512, 0, true, false, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {384, 0, true, false, can_pack ? f4_get_kernel(384, 0, true, false, e->C, edge ? 1 : 0) : nullptr, 0, 0},
-            {384, 0, false, false, f4_get_kernel(384, 0, false, false, e->C, edge ? 1 : 0), 0, 0},
-            {256, 0, false, false, f4_get_kernel(256, 0, false, false, e->C, edge ? 1 : 0), 0, 0},
-            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, edge ? 1 : 0), 0, 0},
-        };
-        /* log-likelihood only: no slab; the pending partials of the post-order walk either sit in shared
-         * memory (which limits the CTA to 256 threads at depth 3) or in a small L2-resident global stack */
-        const Cand lcands[] = {
-            {512, 2, true, true, (can_cm && can_pack) ? f4_get_kernel(512, 2, true, true, e->C, 0) : nullptr, 0, 0, true},
-            {512, 2, true, false, can_pack ? f4_get_kernel(512, 2, true, false, e->C, 0) : nullptr, 0, 0, true},
-            {512, 2, false, true, can_cm ? f4_get_kernel(512, 2, false, true, e->C, 0) : nullptr, 0, 0, true},
-            {384, 2, true, false, can_pack ? f4_get_kernel(384, 2, true, false, e->C, 0) : nullptr, 0, 0, true},
-            {384, 2, true, false, can_pack ? f4_get_kernel(384, 2, true, false, e->C, 0) : nullptr, 0, 0, false},
-            {384, 1, false, false, f4_get_kernel(384, 1, false, false, e->C, 0), 0, 0, false},
-            {256, 2, false, false, f4_get_kernel(256, 2, false, false, e->C, 0), 0, 0, false},
-            {256, 2, false, false, f4_get_kernel(256, 2, false, false, e->C, 0), 0, 0, true},
-            {512, 0, true, false, can_pack ? f4_get_kernel(512, 0, true, false, e->C, 0) : nullptr, 0, 0, true},
-            {384, 0, true, false, can_pack ? f4_get_kernel(384, 0, true, false, e->C, 0) : nullptr, 0, 0, true},
-            {384, 0, false, false, f4_get_kernel(384, 0, false, false, e->C, 0), 0, 0, true},
-            {256, 0, false, false, f4_get_kernel(256, 0, false, false, e->C, 0), 0, 0, true},
-            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, 0), 0, 0, true},
-            {128, 0, false, false, f4_get_kernel(128, 0, false, false, e->C, 0), 0, 0, false},
-        };
-        const Cand *cands = (marg || gm) ? mcands : (edge ? ecands : lcands);
-        const int ncand = (marg || gm) ? (int)(sizeof(mcands) / sizeof(mcands[0]))
-                                       : (edge ? (int)(sizeof(ecands) / sizeof(ecands[0])) : (int)(sizeof(lcands) / sizeof(lcands[0])));
-        const char *force = force0;
-        size_t smem = 0;
-        for (int i = 0; i < ncand; i++) {
-            if (force && atoi(force) != i) continue;
-            if (!cands[i].k) continue;
-            Cand c = cands[i];
-            c.smem = smem = f4_smem_bytes(e, edge, c.bd, c.staged, c.pack, c.cm, marg, c.gstack, gm);
-            if (c.smem > smem_cap) continue;
-            CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
-            CK(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.per_sm, c.k, c.bd, c.smem));
-            if (c.per_sm >= 1) viable.push_back(c);
+/* grid of a fused launch over at most longest sites */
+static int f4_grid(const plf_engine *e, const Cand &c, int64_t longest)
+{
+    return (int)std::min<int64_t>((longest + c.bd - 1) / c.bd, (int64_t)c.per_sm * e->sm_count);
+}
+
+/* times each leading candidate on the first sites (results are overwritten by the real run) and keeps the fastest */
+static int f4_tune(plf_engine *e, F4Slot *slot, F4Args &a, int64_t longest, size_t &pick)
+{
+    const std::vector<Cand> &viable = slot->cands;
+    float best = 0.f;
+    const size_t ntry = std::min<size_t>(viable.size(), 5);
+    a.s_begin = 0; a.s_end = std::min<int64_t>(e->S, f4_tune_sites(e));
+    for (size_t i = 0; i < ntry; i++) {
+        const Cand &c = viable[i];
+        a.gstack = c.gstack ? 1 : 0; a.stack_depth = c.gstack ? 0 : e->stack_depth;
+        /* candidates may share a kernel function with different amounts of dynamic shared memory */
+        CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
+        float ms = 0.f;
+        for (int rep = 0; rep < 4; rep++) {      /* the first launch pays for loading the code; then the best of three */
+            float t = 0.f;
+            CK(e, cudaEventRecord(e->ev[3], e->stream));
+            c.k<<<f4_grid(e, c, longest), c.bd, c.smem, e->stream>>>(a, e->prog_h);
+            KCHECK(e);
+            CK(e, cudaEventRecord(e->ev[4], e->stream));
+            CK(e, cudaEventSynchronize(e->ev[4]));
+            CK(e, cudaEventElapsedTime(&t, e->ev[3], e->ev[4]));
+            if (rep == 1 || (rep > 1 && t < ms)) ms = t;
         }
-        if (viable.empty()) FAIL(e, "fused kernel: no configuration fits (C = %d, %zu bytes of shared memory)", e->C, smem);
-        e->f4_cand_key[tm0] = cand_key;
-        e->f4_cands[tm0] = viable;
+        if (i == 0 || ms < best) { best = ms; pick = i; }
     }
-    /* one launch per chunk of sites: a single chunk normally, the upload's chunks while it is still in flight */
-    const bool pipelined = e->pend_active;
+    slot->tuned_version = e->program_version; slot->tuned_C = e->C; slot->tuned_K = e->K;
+    slot->tuned_pick = pick;
+    return 0;
+}
+
+/*
+ * The fused kernel over all sites for a query of this kind: arguments, the per-kind buffers, tuning when it is due,
+ * then one launch per chunk of sites -- a single chunk normally, the upload's chunks while it is still in flight.
+ * Nothing is reduced here.  prepare_sums has sized the site log-likelihoods and the error word.
+ */
+static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *win, F4Launch &L)
+{
+    F4Slot *slot = nullptr; size_t pick = 0; bool tune = false;
+    if (f4_choose(e, kind, slot, pick, tune)) return -1;
+    const std::vector<Cand> &viable = slot->cands;
+    F4Args &a = L.a;
+    f4_fill_args(e, q, kind, win, a);
+    L.pipelined = e->pend_active;
     std::vector<int64_t> bounds;
-    if (pipelined) bounds = e->pend_bounds; else { bounds.push_back(0); bounds.push_back(e->S); }
-    const size_t nchunk = bounds.size() - 1;
+    if (L.pipelined) bounds = e->pend_bounds; else { bounds.push_back(0); bounds.push_back(e->S); }
+    L.nchunk = bounds.size() - 1;
     int64_t longest = 0;
-    for (size_t k = 0; k < nchunk; k++) longest = std::max(longest, bounds[k + 1] - bounds[k]);
-    auto grid_of = [&](const Cand &c) {
-        return (int)std::min<int64_t>((longest + c.bd - 1) / c.bd, (int64_t)c.per_sm * e->sm_count);
-    };
-    /* Which candidate: the tuned one if this program has been tuned, else the first.  Whether the
-     * constant-memory kernels beat the shared-memory ones depends on what the compiler made of each
-     * instantiation (tools/check_cm_uniform.sh), so the first large query times the leading candidates
-     * on a sample of the sites and keeps the fastest. */
-    const int64_t tune_sites = (int64_t)e->sm_count * 512 * 2;
-    const bool can_tune = viable.size() > 1 && e->S >= tune_sites / 2 && !getenv("PLF_F4_NOTUNE");
-    const int tm = tm0;      /* tuning slot: (ll, edge forms, marginals, edge matrices) x categories */
-    size_t pick = 0;
-    bool tune = false;
-    if (can_tune) {
-        if (e->f4_tuned_version[tm] == e->program_version && e->f4_tuned_C[tm] == e->C && e->f4_tuned_K[tm] == e->K &&
-            e->f4_tuned_pick[tm] < viable.size()) pick = e->f4_tuned_pick[tm];
-        else if (!pipelined) tune = true;
-        else while (pick + 1 < viable.size() && viable[pick].cm) pick++;      /* untuned and data still in flight */
-    } else {
-        while (pick + 1 < viable.size() && viable[pick].cm) pick++;          /* small problems: no constant-memory kernels */
-    }
+    for (size_t k = 0; k < L.nchunk; k++) longest = std::max(longest, bounds[k + 1] - bounds[k]);
     size_t Tmax = 0;
     int gmax = 0;
+    bool any_cm = false, any_gstack = false;
     for (size_t i = 0; i < viable.size(); i++) {
         if (!tune && i != pick) continue;
-        Tmax = std::max(Tmax, (size_t)grid_of(viable[i]) * viable[i].bd);
-        gmax = std::max(gmax, grid_of(viable[i]));
+        Tmax = std::max(Tmax, (size_t)f4_grid(e, viable[i], longest) * viable[i].bd);
+        gmax = std::max(gmax, f4_grid(e, viable[i], longest));
+        if (viable[i].cm) any_cm = true;
+        if (viable[i].gstack) any_gstack = true;
     }
 
-    ENSURE(e, e->d_block_ll, sizeof(double) * gmax * nchunk);
-    const size_t ngm = gm ? (size_t)e->C * e->E * 16 : 0;     /* mode 3: G[C][E][16] follows sum_ll */
-    ENSURE(e, e->d_sum, sizeof(double) * (2 + std::max((size_t)e->E + (size_t)e->N * e->n, ngm)));
-    ENSURE(e, e->d_err, sizeof(int) * (e->N + 4));
-    CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
+    ENSURE(e, e->d_block_ll, sizeof(double) * gmax * L.nchunk);
+    const size_t ngm = kind == 3 ? (size_t)e->C * e->E * 16 : 0;     /* mode 3: a row [C][E][16] of G per warp */
     a.block_ll = e->d_block_ll.as<double>();
     a.error_flag = e->d_err.as<int>();
     /* the site log-likelihoods are always kept: the zero-likelihood check of every query kind reads them */
-    ENSURE(e, e->d_site_ll, sizeof(double) * e->S);
     a.site_ll = win ? win->site_ll : e->d_site_ll.as<double>();
-    if (edge) {
+    if (kind) {
         ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * e->nslots * Tmax);
         ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)e->nslots * Tmax);
-        if (!marg && !gm) ENSURE(e, e->d_block_edge, sizeof(double) * (size_t)gmax * e->E * nchunk);
+        if (kind == 1) ENSURE(e, e->d_block_edge, sizeof(double) * (size_t)gmax * e->E * L.nchunk);
         a.scratch = e->d_scratch.as<double4>(); a.scratchS = e->d_scratchS.as<unsigned int>();
         a.block_edge = e->d_block_edge.as<double>();
-        if (marg && win) {
+        if (kind == 2 && win) {
             CK(e, cudaMemsetAsync(win->site_marg, 0, sizeof(double) * (size_t)e->N * 4 * e->S, e->stream));
             a.marg_site_out = win->site_marg;
-        } else if (marg && q.site_marg) {
+        } else if (kind == 2 && q.site_marg) {
             ENSURE(e, e->d_marg_site, sizeof(double) * (size_t)e->N * 4 * e->S);
             CK(e, cudaMemsetAsync(e->d_marg_site.p, 0, sizeof(double) * (size_t)e->N * 4 * e->S, e->stream));
             a.marg_site_out = e->d_marg_site.as<double>();
-        } else if (marg) {
+        } else if (kind == 2) {
             /* one row of accumulators per warp of the grid; every launch of this query adds into them */
             const size_t rows = (size_t)gmax * 16;
             ENSURE(e, e->d_block_marg, sizeof(double) * rows * e->N * 4);
             CK(e, cudaMemsetAsync(e->d_block_marg.p, 0, sizeof(double) * rows * e->N * 4, e->stream));
             a.block_marg = e->d_block_marg.as<double>();
-        } else if (gm) {
-            /* the same for the matrices G: a row [C][E][16] per warp */
+        } else if (kind == 3) {
+            /* the same for the matrices G */
             ENSURE(e, e->d_block_gmat, sizeof(double) * (size_t)gmax * 16 * ngm);
             CK(e, cudaMemsetAsync(e->d_block_gmat.p, 0, sizeof(double) * (size_t)gmax * 16 * ngm, e->stream));
             a.block_gmat = e->d_block_gmat.as<double>();
         }
-        if (q.edge_mask_h) {
-            ENSURE(e, e->d_mask, e->E);
-            CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, e->E, cudaMemcpyHostToDevice, e->stream));
-            a.edge_mask = e->d_mask.as<unsigned char>();
-        }
-        if (win && !marg) {
+        a.edge_mask = q.edge_mask_h ? e->d_mask.as<unsigned char>() : nullptr;
+        if (win && kind != 2) {
             CK(e, cudaMemsetAsync(win->site_edge, 0, sizeof(double) * (size_t)e->E * e->S, e->stream));
             a.edge_site_out = win->site_edge;
         } else if (q.site_edge) {
@@ -1563,13 +1624,7 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
             a.edge_site_out = e->d_edge_site.as<double>();
         }
     }
-    bool any_cm = false, any_gstack = false;
-    for (size_t i = 0; i < viable.size(); i++) {
-        if (!(tune || i == pick)) continue;
-        if (viable[i].cm) any_cm = true;
-        if (viable[i].gstack) any_gstack = true;
-    }
-    if (!edge && any_gstack && e->stack_depth > 0) {
+    if (!kind && any_gstack && e->stack_depth > 0) {
         ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * e->stack_depth * Tmax);
         ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)e->stack_depth * Tmax);
         a.scratch = e->d_scratch.as<double4>(); a.scratchS = e->d_scratchS.as<unsigned int>();
@@ -1591,41 +1646,18 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         CK(e, cudaStreamWaitEvent(e->stream, g_cm_done[e->device], 0));
         cm_guard.ev = &g_cm_done[e->device]; cm_guard.st = e->stream;
         const size_t nP = sizeof(double) * (size_t)e->C * e->edge_of_int.size() * 16;
-        CK(e, f4_upload_const(a.Pint, edge ? a.Fint : nullptr, nP, e->stream));
+        CK(e, f4_upload_const(a.Pint, kind ? a.Fint : nullptr, nP, e->stream));
     }
     if (tune) {
-        /* time each leading candidate on the first tune_sites sites (results are overwritten by the real run) */
-        float best = 0.f;
-        const size_t ntry = std::min<size_t>(viable.size(), 5);
-        a.s_begin = 0; a.s_end = std::min<int64_t>(e->S, tune_sites);
-        for (size_t i = 0; i < ntry; i++) {
-            const Cand &c = viable[i];
-            a.gstack = c.gstack ? 1 : 0; a.stack_depth = c.gstack ? 0 : e->stack_depth;
-            /* candidates may share a kernel function with different amounts of dynamic shared memory */
-            CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
-            float ms = 0.f;
-            for (int rep = 0; rep < 4; rep++) {      /* the first launch pays for loading the code; then the best of three */
-                float t = 0.f;
-                CK(e, cudaEventRecord(e->ev[3], e->stream));
-                c.k<<<grid_of(c), c.bd, c.smem, e->stream>>>(a, e->prog_h);
-                KCHECK(e);
-                CK(e, cudaEventRecord(e->ev[4], e->stream));
-                CK(e, cudaEventSynchronize(e->ev[4]));
-                CK(e, cudaEventElapsedTime(&t, e->ev[3], e->ev[4]));
-                if (rep == 1 || (rep > 1 && t < ms)) ms = t;
-            }
-            if (i == 0 || ms < best) { best = ms; pick = i; }
-        }
-        e->f4_tuned_version[tm] = e->program_version; e->f4_tuned_C[tm] = e->C; e->f4_tuned_K[tm] = e->K;
-        e->f4_tuned_pick[tm] = pick;
+        if (f4_tune(e, slot, a, longest, pick)) return -1;
         CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
         /* the marginal accumulators are added to by every launch: forget what the timing runs left there */
-        if (marg && a.block_marg)
+        if (kind == 2 && a.block_marg)
             CK(e, cudaMemsetAsync(e->d_block_marg.p, 0, sizeof(double) * (size_t)gmax * 16 * e->N * 4, e->stream));
-        if (gm) CK(e, cudaMemsetAsync(e->d_block_gmat.p, 0, sizeof(double) * (size_t)gmax * 16 * ngm, e->stream));
+        if (kind == 3) CK(e, cudaMemsetAsync(e->d_block_gmat.p, 0, sizeof(double) * (size_t)gmax * 16 * ngm, e->stream));
     }
     const Cand &use = viable[pick];
-    const int grid = grid_of(use);
+    const int grid = f4_grid(e, use, longest);
     {
         char nm[96];
         snprintf(nm, sizeof nm, "fused4_kernel<%d,%d,%d,%d,%d,%d>", e->C, kind, use.bd, use.staged, use.pack ? 1 : 0, use.cm ? 1 : 0);
@@ -1634,11 +1666,11 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     a.gstack = use.gstack ? 1 : 0; a.stack_depth = use.gstack ? 0 : e->stack_depth;
     CK(e, cudaFuncSetAttribute(use.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)use.smem));
     CK(e, cudaEventRecord(e->ev[3], e->stream));
-    for (size_t k = 0; k < nchunk; k++) {
+    for (size_t k = 0; k < L.nchunk; k++) {
         a.s_begin = bounds[k]; a.s_end = bounds[k + 1];
         a.block_ll = e->d_block_ll.as<double>() + k * (size_t)grid;
-        if (edge && !marg && !gm) a.block_edge = e->d_block_edge.as<double>() + k * (size_t)grid * e->E;
-        if (pipelined) {
+        if (kind == 1) a.block_edge = e->d_block_edge.as<double>() + k * (size_t)grid * e->E;
+        if (L.pipelined) {
             /* this chunk's codes and weights have arrived; bring them into the node-major layout */
             CK(e, cudaStreamWaitEvent(e->stream, e->chunk_ev[k], 0));
             if (launch_transpose(e, a.s_begin, a.s_end, e->pend_in_bytes)) return -1;
@@ -1653,8 +1685,22 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         cm_lock.unlock();
     }
     e->kernel_timed = true;
-    if (win) return 0;          /* run_fused_windows combines the windows, reduces and copies */
-    const bool shared_retry = pipelined && e->comm != nullptr;
+    L.use = &use;
+    L.grid = grid;
+    return 0;
+}
+
+/* n = 4, up to 4 rate categories: the fused launches, then their rows reduced (and all-reduced) into the sums */
+static int run_fused(plf_engine *e, Query &q)
+{
+    const int kind = f4_kind(q);
+    const size_t ngm = kind == 3 ? (size_t)e->C * e->E * 16 : 0;     /* mode 3: G[C][E][16] follows sum_ll */
+    if (prepare_sums(e, 2 + std::max((size_t)e->E + (size_t)e->N * e->n, ngm))) return -1;
+    F4Launch L;
+    if (f4_launch(e, q, kind, nullptr, L)) return -1;
+    const F4Args &a = L.a;
+    const int grid = L.grid;
+    const bool pipelined = L.pipelined, shared_retry = pipelined && e->comm != nullptr;
     if (shared_retry) {
         ENSURE(e, e->d_retry, sizeof(double));
         retry_word_kernel<<<1, 256, 0, e->stream>>>(e->d_err.as<int>() + 4, e->d_node_has_data.as<unsigned char>(), e->N,
@@ -1662,24 +1708,23 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         KCHECK(e);
     }
     if (pipelined && launch_flags_readback(e)) return -1;
-    if ((edge && !marg && q.site_edge) || (marg && q.site_marg)) {
+    if ((kind == 1 && q.site_edge) || (kind == 2 && q.site_marg)) {
         zero_lik_rows_kernel<<<(unsigned)((e->S + 255) / 256), 256, 0, e->stream>>>(
-            a.site_ll, a.site_w, 0, (int)e->S, a.error_flag, (edge && !marg) ? a.edge_site_out : nullptr, e->E,
-            marg ? a.marg_site_out : nullptr, e->N * 4);
+            a.site_ll, a.site_w, 0, (int)e->S, a.error_flag, kind == 1 ? a.edge_site_out : nullptr, e->E,
+            kind == 2 ? a.marg_site_out : nullptr, e->N * 4);
         KCHECK(e);
     }
-    const int rows = grid * (int)nchunk;
-    a.block_ll = e->d_block_ll.as<double>();
-    if (edge) a.block_edge = e->d_block_edge.as<double>();
+    const int rows = grid * (int)L.nchunk;
+    double *block_ll = e->d_block_ll.as<double>(), *block_edge = e->d_block_edge.as<double>();
     double *dsum = e->d_sum.as<double>();
     /* ll / ll + edge sums with a communicator: second-stage reduction and all-reduce are one kernel over peer memory */
-    const bool fuse_reduce = !marg && !gm && !q.site_edge && !pipelined && peer_path(e, 1 + (size_t)(edge ? e->E : 0));
+    const bool fuse_reduce = kind <= 1 && !q.site_edge && !pipelined && peer_path(e, 1 + (size_t)(kind ? e->E : 0));
     if (!fuse_reduce) {
-        sum_rows_kernel<<<1, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_ll, rows, 1, dsum);
+        sum_rows_kernel<<<1, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(block_ll, rows, 1, dsum);
         KCHECK(e);
     }
     size_t nsum = 1;
-    if (marg) {
+    if (kind == 2) {
         const int cols = e->N * 4;
         CK(e, cudaMemsetAsync(dsum + 1, 0, sizeof(double) * e->E, e->stream));
         if (q.site_marg) {
@@ -1689,24 +1734,24 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
                 KCHECK(e);
             }
         } else {
-            sum_rows_kernel<<<(cols + 31) / 32, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_marg, grid * (use.bd / 32), cols, dsum + 1 + e->E);
+            sum_rows_kernel<<<(cols + 31) / 32, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_marg, grid * (L.use->bd / 32), cols, dsum + 1 + e->E);
             KCHECK(e);
         }
         nsum = 1 + e->E + cols;
     }
-    if (gm) {
-        sum_rows_kernel<<<(unsigned)((ngm + 31) / 32), dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_gmat, grid * (use.bd / 32), (int)ngm, dsum + 1);
+    if (kind == 3) {
+        sum_rows_kernel<<<(unsigned)((ngm + 31) / 32), dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_gmat, grid * (L.use->bd / 32), (int)ngm, dsum + 1);
         KCHECK(e);
         nsum = 1 + ngm;
     }
-    if (edge && !marg && !gm && !q.site_edge) {
+    if (kind == 1 && !q.site_edge) {
         if (!fuse_reduce) {
-            sum_rows_kernel<<<(e->E + 31) / 32, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(a.block_edge, rows, e->E, dsum + 1);
+            sum_rows_kernel<<<(e->E + 31) / 32, dim3(32, PLF_ROW_GROUPS), 0, e->stream>>>(block_edge, rows, e->E, dsum + 1);
             KCHECK(e);
         }
         nsum = 1 + e->E;
     }
-    if (edge && !marg && q.site_edge && q.sum_edge) {
+    if (kind == 1 && q.site_edge && q.sum_edge) {
         /* per-site outputs requested together with sums: reduce the per-site rows with the weights */
         CK(e, cudaMemsetAsync(dsum + 1, 0, sizeof(double) * e->E, e->stream));
         wsum_rows_kernel<<<e->E, 256, 0, e->stream>>>(a.edge_site_out, a.site_w, 0, (int)e->S, dsum + 1, a.error_flag, 0);
@@ -1717,17 +1762,12 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
     if (fuse_reduce) {
         e->peer_seq++;
         peer_allreduce_kernel<<<1, 128 * PLF_ROW_GROUPS, 0, e->stream>>>(dsum, (int)nsum, e->peer_seq, e->rank, e->nranks, e->d_peer_ptrs.as<void *>(),
-                                                                         e->d_err.as<int>(), a.block_ll, edge ? a.block_edge : nullptr, rows, e->E);
+                                                                         e->d_err.as<int>(), block_ll, kind ? block_edge : nullptr, rows, e->E);
         KCHECK(e);
     } else if (finish_sums(e, dsum, nsum + (shared_retry ? 1 : 0))) return -1;
-    if (gm && (run_gmat_adjoint(e, dsum + 1) || copy_gmat_out(e, q))) return -1;
-    CK(e, cudaEventRecord(e->ev[2], e->stream));
-    std::vector<double> hs(nsum + 1, 0.0);
-    int herr = 0;
-    CK(e, cudaMemcpyAsync(hs.data(), dsum, sizeof(double) * (nsum + (shared_retry ? 1 : 0)), cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaMemcpyAsync(&herr, e->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-    if (q.site_ll) CK(e, cudaMemcpyAsync(q.site_ll, e->d_site_ll.p, sizeof(double) * e->S, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaStreamSynchronize(e->stream));
+    if (kind == 3 && (run_gmat_adjoint(e, dsum + 1) || copy_gmat_out(e, q))) return -1;
+    std::vector<double> hs; int herr = 0;
+    if (read_back(e, q, dsum, nsum + (shared_retry ? 1 : 0), hs, herr)) return -1;
     if (pipelined) {
         e->pend_active = false;
         if (data_has_bad_code(e)) { e->S = 0; FAIL(e, "plf_set_data_async: a character code is not a row of the definition table"); }
@@ -1738,12 +1778,8 @@ static int run_fused(plf_engine *e, Query &q, const F4Window *win = nullptr)
         if (changed || (shared_retry && hs[nsum] != 0.0)) return 1;
     }
     if (q.site_edge && copy_site_matrix(e, e->d_edge_site.as<double>(), e->E, e->S, q.site_edge)) return -1;
-    if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg || gm)) FAIL(e, "a site with non-zero weight has zero likelihood");
-    if (q.sum_ll) *q.sum_ll = hs[0];
-    if (q.sum_edge && !marg && nsum > 1) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * e->E);
-    if (marg && q.site_marg && copy_site_matrix(e, e->d_marg_site.as<double>(), e->N * 4, e->S, q.site_marg)) return -1;
-    if (marg && q.sum_marg) memcpy(q.sum_marg, hs.data() + 1 + e->E, sizeof(double) * e->N * 4);
+    if (unpack_sums(e, q, hs, herr)) return -1;
+    if (kind == 2 && q.site_marg && copy_site_matrix(e, e->d_marg_site.as<double>(), e->N * 4, e->S, q.site_marg)) return -1;
     return 0;
 }
 
@@ -1789,11 +1825,10 @@ static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
     const bool marg = q.want_marg, edge = q.want_edge && !marg;
     if (nwin > 16) FAIL(e, "more than 16 category windows");
     if (resolve_pending(e)) return -1;
+    if (prepare_sums(e, 2 + E + (size_t)N * 4)) return -1;
     ENSURE(e, e->f4w_ll, sizeof(double) * (size_t)nwin * S);
     if (edge) ENSURE(e, e->f4w_edge, sizeof(double) * (size_t)nwin * E * S);
     if (marg) ENSURE(e, e->f4w_marg, sizeof(double) * (size_t)nwin * N * 4 * S);
-    ENSURE(e, e->d_site_ll, sizeof(double) * S);
-    ENSURE(e, e->d_sum, sizeof(double) * (2 + E + (size_t)N * 4));
     float ms_total = 0.f;
     for (int w = 0; w < nwin; w++) {
         F4Window win;
@@ -1802,7 +1837,8 @@ static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
         win.site_edge = edge ? e->f4w_edge.as<double>() + (size_t)w * E * S : nullptr;
         win.site_marg = marg ? e->f4w_marg.as<double>() + (size_t)w * N * 4 * S : nullptr;
         e->C = std::min(wsize, Ctot - wsize * w);
-        const int rc = run_fused(e, q, &win);
+        F4Launch L;
+        const int rc = f4_launch(e, q, f4_kind(q), &win, L);
         e->C = Ctot;
         if (rc) return rc;
         float t = 0.f;
@@ -1829,21 +1865,109 @@ static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
     if (edge && q.sum_edge) { wsum_rows_kernel<<<E, 256, 0, e->stream>>>(e->f4w_edge.as<double>(), w, 0, (int)S, dsum + 1, e->d_err.as<int>(), 0); KCHECK(e); }
     if (marg && q.sum_marg) { wsum_rows_kernel<<<N * 4, 256, 0, e->stream>>>(e->f4w_marg.as<double>(), w, 0, (int)S, dsum + 1 + E, e->d_err.as<int>(), 0); KCHECK(e); }
     if (finish_sums(e, dsum, nsum)) return -1;
-    CK(e, cudaEventRecord(e->ev[2], e->stream));
-    std::vector<double> hs(nsum);
-    int herr = 0;
-    CK(e, cudaMemcpyAsync(hs.data(), dsum, sizeof(double) * nsum, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaMemcpyAsync(&herr, e->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-    if (q.site_ll) CK(e, cudaMemcpyAsync(q.site_ll, site_ll, sizeof(double) * S, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaStreamSynchronize(e->stream));
-    if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg)) FAIL(e, "a site with non-zero weight has zero likelihood");
-    if (q.sum_ll) *q.sum_ll = hs[0];
-    if (edge && q.sum_edge) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * E);
-    if (marg && q.sum_marg) memcpy(q.sum_marg, hs.data() + 1 + E, sizeof(double) * (size_t)N * 4);
+    std::vector<double> hs; int herr = 0;
+    if (read_back(e, q, dsum, nsum, hs, herr) || unpack_sums(e, q, hs, herr)) return -1;
     if (edge && q.site_edge && copy_site_matrix(e, e->f4w_edge.as<double>(), E, S, q.site_edge)) return -1;
     if (marg && q.site_marg && copy_site_matrix(e, e->f4w_marg.as<double>(), N * 4, S, q.site_marg)) return -1;
     e->ms_kernel_override = ms_total;
+    return 0;
+}
+
+/* 16 < n <= 64 on the generic path: tip tables (when they are small) and the GEMM edge order of the tile kernels */
+static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
+{
+    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    if (e->K <= 4096 && !getenv("PLF_NO_TIPTABLE")) {
+        /* tip tables (P_e def_k) so that tip children need no GEMM */
+        if (ensure_program(e)) return -1;
+        const int Et = (int)e->edge_of_tip.size();
+        std::vector<int> toe(E, -1);
+        for (int te = 0; te < Et; te++) toe[e->edge_of_tip[te]] = te;
+        ENSURE(e, e->d_tip_of_edge, sizeof(int) * E);
+        CK(e, cudaMemcpyAsync(e->d_tip_of_edge.p, toe.data(), sizeof(int) * E, cudaMemcpyHostToDevice, e->stream));
+        CK(e, cudaStreamSynchronize(e->stream));
+        const size_t cnt = (size_t)C * Et * e->K * n;
+        ENSURE(e, e->d_TPg, sizeof(double) * (cnt + 1));
+        if (cnt) {
+            tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
+                e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
+                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, 0, e->d_TPg.as<double>());
+            KCHECK(e);
+        }
+        a.TP = e->d_TPg.as<double>(); a.tip_of_edge = e->d_tip_of_edge.as<int>(); a.Et = Et;
+        if (q.want_edge && a.Fm && cnt) {
+            /* the same for the edge forms, so that tip edges need no GEMM in the outside pass either */
+            ENSURE(e, e->d_TFg, sizeof(double) * (cnt + 1));
+            tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
+                a.Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
+                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, a.f_zero_rowsum ? 1 : 2, e->d_TFg.as<double>());
+            KCHECK(e);
+            a.TF = e->d_TFg.as<double>();
+        }
+    }
+    /* GEMM edges in the order of the inside kernel's walk (reverse BFS, children in csr order) */
+    std::vector<int> toe(E, -1);
+    if (a.tip_of_edge) for (int te = 0; te < (int)e->edge_of_tip.size(); te++) toe[e->edge_of_tip[te]] = te;
+    std::vector<int> seq, pos(N, 0);
+    for (int u = 0; u < N; u++) pos[e->preorder[u]] = u;
+    for (int u = N - 1; u >= 0; u--) {
+        const int nd = e->preorder[u];
+        for (int idx = e->indptr[nd]; idx < e->indptr[nd + 1]; idx++) if (toe[idx] < 0) seq.push_back(idx);
+    }
+    const size_t nseq = seq.size();
+    for (size_t t = 0; t < nseq; t++) seq.push_back(pos[e->indices[seq[t]]]);    /* walk position of the child */
+    ENSURE(e, e->d_int_seq, sizeof(int) * (seq.size() + 1));
+    CK(e, cudaMemcpyAsync(e->d_int_seq.p, seq.data(), sizeof(int) * seq.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    a.int_seq = e->d_int_seq.as<int>(); a.n_int_seq = (int)nseq;
+    if (a.tip_of_edge && e->code_bytes == 1 && (size_t)a.Et * TL_TS <= 32 * 1024) {
+        a.tip_stage = 1;
+        a.tip_edge_csr = e->d_edge_of_tip.as<int>();
+    }
+    return 0;
+}
+
+/* tree navigation arrays of the Hessian kernel, on the device */
+static int upload_hess_tree(plf_engine *e, HessTree &ht)
+{
+    const int N = e->N, E = e->E;
+    std::vector<int> nav((size_t)3 * E + (size_t)4 * N, 0);
+    int *parent_node = nav.data(), *parent_edge = parent_node + E, *dfs_nodes = parent_edge + N, *dfs_pos = dfs_nodes + N,
+        *sub_end = dfs_pos + N, *sub_max = sub_end + N, *erank = sub_max + E;
+    for (int v = 0; v < N; v++) parent_edge[v] = -1;
+    for (int v = 0; v < N; v++)
+        for (int idx = e->indptr[v]; idx < e->indptr[v + 1]; idx++) { parent_node[idx] = v; parent_edge[e->indices[idx]] = idx; }
+    /* depth-first pre-order (children in csr order), subtree ends */
+    std::vector<int> st;
+    int pos = 0;
+    st.push_back(e->root);
+    while (!st.empty()) {
+        const int v = st.back(); st.pop_back();
+        dfs_pos[v] = pos; dfs_nodes[pos++] = v;
+        for (int idx = e->indptr[v + 1] - 1; idx >= e->indptr[v]; idx--) st.push_back(e->indices[idx]);
+    }
+    for (int p2 = N - 1; p2 >= 0; p2--) {
+        const int v = dfs_nodes[p2];
+        int end = p2 + 1;
+        for (int idx = e->indptr[v]; idx < e->indptr[v + 1]; idx++) end = std::max(end, sub_end[e->indices[idx]]);
+        sub_end[v] = end;
+    }
+    /* rank of an edge = BFS position of its child (csr indices follow the node labels, not the depth);
+     * largest rank below (and including) every edge, children before parents */
+    for (int u = 0; u < N; u++) { const int pe = parent_edge[e->preorder[u]]; if (pe >= 0) erank[pe] = u; }
+    for (int u = N - 1; u >= 0; u--) {
+        const int v = e->preorder[u], pe = parent_edge[v];
+        if (pe < 0) continue;
+        int mx = erank[pe];
+        for (int i2 = e->indptr[v]; i2 < e->indptr[v + 1]; i2++) mx = std::max(mx, sub_max[i2]);
+        sub_max[pe] = mx;
+    }
+    ENSURE(e, e->h_tree, sizeof(int) * nav.size());
+    CK(e, cudaMemcpyAsync(e->h_tree.p, nav.data(), sizeof(int) * nav.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    const int *d = e->h_tree.as<int>();
+    ht.parent_node = d; ht.parent_edge = d + E; ht.dfs_nodes = d + E + N; ht.dfs_pos = d + E + 2 * (size_t)N;
+    ht.sub_end = d + E + 3 * (size_t)N; ht.sub_max = d + E + 4 * (size_t)N; ht.erank = d + 2 * (size_t)E + 4 * (size_t)N;
     return 0;
 }
 
@@ -1852,8 +1976,9 @@ static int run_generic(plf_engine *e, Query &q)
     const int n = e->n, C = e->C, N = e->N, E = e->E;
     const bool gm = q.want_gmat;        /* plf_edge_expect_all: generic kernels only (generic_gmat_kernel) */
     const bool outside = q.want_edge || q.want_marg || gm;
-    e->last_kernel = (n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !gm) ? "tile_inside_kernel / tile_outside_kernel"
-                                                                               : "generic_inside_kernel / generic_outside_kernel";
+    /* 16 < n <= 64 (amino-acid, codon): inside pass on the FP64 tensor pipe (tile.cuh) */
+    const bool use_tile = n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess && !gm;
+    e->last_kernel = use_tile ? "tile_inside_kernel / tile_outside_kernel" : "generic_inside_kernel / generic_outside_kernel";
     const size_t ngm = gm ? (size_t)C * E * n * n : 0;     /* G[C][E][n][n] follows sum_ll */
     const size_t nsum_all = 1 + std::max((size_t)E + (size_t)N * n, ngm);
     /* chunk size from a memory budget */
@@ -1876,9 +2001,7 @@ static int run_generic(plf_engine *e, Query &q)
     ENSURE(e, e->g_cat_k, sizeof(int) * (size_t)C * Sc);
     ENSURE(e, e->g_site_m, sizeof(double) * Sc);
     ENSURE(e, e->g_site_k, sizeof(int) * Sc);
-    ENSURE(e, e->d_site_ll, sizeof(double) * e->S);
-    ENSURE(e, e->d_sum, sizeof(double) * nsum_all);
-    ENSURE(e, e->d_err, sizeof(int) * (N + 4));
+    if (prepare_sums(e, nsum_all)) return -1;
     if (gm) ENSURE(e, e->g_fe, sizeof(double) * (size_t)C * E * n * Sc);
     if (outside) {
         ENSURE(e, e->g_Fg, sizeof(double) * (size_t)C * N * n * Sc);
@@ -1886,13 +2009,8 @@ static int run_generic(plf_engine *e, Query &q)
     }
     if (q.want_edge) ENSURE(e, e->g_edge_out, sizeof(double) * (size_t)E * Sc);
     if (q.want_marg) ENSURE(e, e->g_marg_out, sizeof(double) * (size_t)N * n * Sc);
-    if (q.edge_mask_h) {
-        ENSURE(e, e->d_mask, E);
-        CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, E, cudaMemcpyHostToDevice, e->stream));
-    }
     double *dsum = e->d_sum.as<double>();
     CK(e, cudaMemsetAsync(dsum, 0, sizeof(double) * nsum_all, e->stream));
-    CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
 
     GenericArgs a;
     memset(&a, 0, sizeof(a));
@@ -1922,57 +2040,7 @@ static int run_generic(plf_engine *e, Query &q)
     if (smem_out > 48 * 1024) CK(e, cudaFuncSetAttribute(generic_outside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_out));
     if (smem_out > 227 * 1024) FAIL(e, "state count %d is too large for the generic kernels", n);
     const double *w = e->have_w ? e->d_site_w.as<double>() : nullptr;
-    /* 16 < n <= 64 (amino-acid, codon): inside pass on the FP64 tensor pipe (tile.cuh) */
-    const bool use_tile = n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess && !gm;
-    if (use_tile && e->K <= 4096 && !getenv("PLF_NO_TIPTABLE")) {
-        /* tip tables (P_e def_k) so that tip children need no GEMM */
-        if (ensure_program(e)) return -1;
-        const int Et = (int)e->edge_of_tip.size();
-        std::vector<int> toe(E, -1);
-        for (int te = 0; te < Et; te++) toe[e->edge_of_tip[te]] = te;
-        ENSURE(e, e->d_tip_of_edge, sizeof(int) * E);
-        CK(e, cudaMemcpyAsync(e->d_tip_of_edge.p, toe.data(), sizeof(int) * E, cudaMemcpyHostToDevice, e->stream));
-        CK(e, cudaStreamSynchronize(e->stream));
-        const size_t cnt = (size_t)C * Et * e->K * n;
-        ENSURE(e, e->d_TPg, sizeof(double) * (cnt + 1));
-        if (cnt) {
-            tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
-                e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, 0, e->d_TPg.as<double>());
-            KCHECK(e);
-        }
-        a.TP = e->d_TPg.as<double>(); a.tip_of_edge = e->d_tip_of_edge.as<int>(); a.Et = Et;
-        if (q.want_edge && a.Fm && cnt) {
-            /* the same for the edge forms, so that tip edges need no GEMM in the outside pass either */
-            ENSURE(e, e->d_TFg, sizeof(double) * (cnt + 1));
-            tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
-                a.Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, a.f_zero_rowsum ? 1 : 2, e->d_TFg.as<double>());
-            KCHECK(e);
-            a.TF = e->d_TFg.as<double>();
-        }
-    }
-    if (use_tile) {
-        /* GEMM edges in the order of the inside kernel's walk (reverse BFS, children in csr order) */
-        std::vector<int> toe(E, -1);
-        if (a.tip_of_edge) for (int te = 0; te < (int)e->edge_of_tip.size(); te++) toe[e->edge_of_tip[te]] = te;
-        std::vector<int> seq, pos(N, 0);
-        for (int u = 0; u < N; u++) pos[e->preorder[u]] = u;
-        for (int u = N - 1; u >= 0; u--) {
-            const int nd = e->preorder[u];
-            for (int idx = e->indptr[nd]; idx < e->indptr[nd + 1]; idx++) if (toe[idx] < 0) seq.push_back(idx);
-        }
-        const size_t nseq = seq.size();
-        for (size_t t = 0; t < nseq; t++) seq.push_back(pos[e->indices[seq[t]]]);    /* walk position of the child */
-        ENSURE(e, e->d_int_seq, sizeof(int) * (seq.size() + 1));
-        CK(e, cudaMemcpyAsync(e->d_int_seq.p, seq.data(), sizeof(int) * seq.size(), cudaMemcpyHostToDevice, e->stream));
-        CK(e, cudaStreamSynchronize(e->stream));
-        a.int_seq = e->d_int_seq.as<int>(); a.n_int_seq = (int)nseq;
-    }
-    if (use_tile && a.tip_of_edge && e->code_bytes == 1 && (size_t)a.Et * TL_TS <= 32 * 1024) {
-        a.tip_stage = 1;
-        a.tip_edge_csr = e->d_edge_of_tip.as<int>();
-    }
+    if (use_tile && prepare_tile(e, q, a)) return -1;
     /* padded state count of the tile kernels: 32 for amino-acid-sized models, 64 for codon-sized ones */
     const int tnp = (n <= 32 && !getenv("PLF_TILE_NP64")) ? 32 : 64, tnw = tnp / 8;
     const size_t smem_tile = sizeof(double) * (2 * tnp * TL_LS + tnw * TL_TS + TL_TS) + sizeof(int) * 2 * TL_TS +
@@ -1991,46 +2059,7 @@ static int run_generic(plf_engine *e, Query &q)
     int hgrid = 0;
     const size_t smem_hess = sizeof(double) * ((size_t)3 * n * PLF_TS + E);
     if (q.sum_hess) {
-        std::vector<int> nav((size_t)3 * E + (size_t)4 * N, 0);
-        int *parent_node = nav.data(), *parent_edge = parent_node + E, *dfs_nodes = parent_edge + N, *dfs_pos = dfs_nodes + N,
-            *sub_end = dfs_pos + N, *sub_max = sub_end + N, *erank = sub_max + E;
-        for (int v = 0; v < N; v++) parent_edge[v] = -1;
-        for (int v = 0; v < N; v++)
-            for (int idx = e->indptr[v]; idx < e->indptr[v + 1]; idx++) { parent_node[idx] = v; parent_edge[e->indices[idx]] = idx; }
-        {
-            /* depth-first pre-order (children in csr order), subtree ends */
-            std::vector<int> st;
-            int pos = 0;
-            st.push_back(e->root);
-            std::vector<int> order;
-            while (!st.empty()) {
-                const int v = st.back(); st.pop_back();
-                dfs_pos[v] = pos; dfs_nodes[pos++] = v;
-                for (int idx = e->indptr[v + 1] - 1; idx >= e->indptr[v]; idx--) st.push_back(e->indices[idx]);
-            }
-            for (int p2 = N - 1; p2 >= 0; p2--) {
-                const int v = dfs_nodes[p2];
-                int end = p2 + 1;
-                for (int idx = e->indptr[v]; idx < e->indptr[v + 1]; idx++) end = std::max(end, sub_end[e->indices[idx]]);
-                sub_end[v] = end;
-            }
-            /* rank of an edge = BFS position of its child (csr indices follow the node labels, not the depth);
-             * largest rank below (and including) every edge, children before parents */
-            for (int u = 0; u < N; u++) { const int pe = parent_edge[e->preorder[u]]; if (pe >= 0) erank[pe] = u; }
-            for (int u = N - 1; u >= 0; u--) {
-                const int v = e->preorder[u], pe = parent_edge[v];
-                if (pe < 0) continue;
-                int mx = erank[pe];
-                for (int i2 = e->indptr[v]; i2 < e->indptr[v + 1]; i2++) mx = std::max(mx, sub_max[i2]);
-                sub_max[pe] = mx;
-            }
-        }
-        ENSURE(e, e->h_tree, sizeof(int) * nav.size());
-        CK(e, cudaMemcpyAsync(e->h_tree.p, nav.data(), sizeof(int) * nav.size(), cudaMemcpyHostToDevice, e->stream));
-        CK(e, cudaStreamSynchronize(e->stream));
-        const int *d = e->h_tree.as<int>();
-        ht.parent_node = d; ht.parent_edge = d + E; ht.dfs_nodes = d + E + N; ht.dfs_pos = d + E + 2 * (size_t)N;
-        ht.sub_end = d + E + 3 * (size_t)N; ht.sub_max = d + E + 4 * (size_t)N; ht.erank = d + 2 * (size_t)E + 4 * (size_t)N;
+        if (upload_hess_tree(e, ht)) return -1;
         hgrid = (int)std::min<int64_t>((Sc + PLF_TS - 1) / PLF_TS, (int64_t)e->sm_count * 4);
         while (hgrid > 1 && (size_t)hgrid * E * E * sizeof(double) > ((size_t)2 << 30)) hgrid /= 2;
         ENSURE(e, e->h_part, sizeof(double) * (size_t)hgrid * E * E + 8);
@@ -2129,24 +2158,8 @@ static int run_generic(plf_engine *e, Query &q)
         KCHECK(e);
         if (finish_sums(e, e->h_out.as<double>(), (size_t)E * E)) return -1;
     }
-    CK(e, cudaEventRecord(e->ev[2], e->stream));
-    std::vector<double> hs(nsum);
-    int herr = 0;
-    CK(e, cudaMemcpyAsync(hs.data(), dsum, sizeof(double) * nsum, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaMemcpyAsync(&herr, e->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-    if (q.site_ll) CK(e, cudaMemcpyAsync(q.site_ll, e->d_site_ll.p, sizeof(double) * e->S, cudaMemcpyDeviceToHost, e->stream));
-    if (q.sum_hess) CK(e, cudaMemcpyAsync(q.sum_hess, e->h_out.p, sizeof(double) * (size_t)E * E, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaStreamSynchronize(e->stream));
-    if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
-    if ((herr & 2) && q.sum_hess) FAIL(e, "infeasible: a rate category with a non-zero rate has zero likelihood at a weighted site");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge || q.sum_marg || gm)) FAIL(e, "a site with non-zero weight has zero likelihood");
-    if (q.sum_hess) {
-        for (int i = 0; i < E; i++) for (int j = 0; j < i; j++) q.sum_hess[(size_t)j * E + i] = q.sum_hess[(size_t)i * E + j];
-    }
-    if (q.sum_ll) *q.sum_ll = hs[0];
-    if (q.sum_edge) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * E);
-    if (q.sum_marg) memcpy(q.sum_marg, hs.data() + 1 + E, sizeof(double) * (size_t)N * n);
-    return 0;
+    std::vector<double> hs; int herr = 0;
+    return (read_back(e, q, dsum, nsum, hs, herr) || unpack_sums(e, q, hs, herr)) ? -1 : 0;
 }
 
 /*
@@ -2235,7 +2248,7 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
 
 static int run_dmma(plf_engine *e, Query &q)
 {
-    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    const int n = e->n, C = e->C, E = e->E;
     const int NB = dm_blocks_for(n);
     if (ensure_dm_tables(e, NB, q.want_edge ? q.Fm : nullptr, q.f_zero_rowsum)) return -1;
     const int Ei = (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
@@ -2273,21 +2286,14 @@ static int run_dmma(plf_engine *e, Query &q)
     ENSURE(e, e->g_cat_k, sizeof(int) * (size_t)C * Sc);
     ENSURE(e, e->g_site_m, sizeof(double) * Sc);
     ENSURE(e, e->g_site_k, sizeof(int) * Sc);
-    ENSURE(e, e->d_site_ll, sizeof(double) * e->S);
-    ENSURE(e, e->d_sum, sizeof(double) * (1 + E));
-    ENSURE(e, e->d_err, sizeof(int) * (N + 4));
+    if (prepare_sums(e, 1 + E)) return -1;
     if (q.want_edge) {
         ENSURE(e, e->d_dm_slab, sizeof(double2) * (size_t)C * Ei * ngroups_max * NB * 32 + 16);
         ENSURE(e, e->d_dm_slabmeta, sizeof(int) * (size_t)C * Ei * ngroups_max * 32 + 16);
         ENSURE(e, e->g_edge_out, sizeof(double) * (size_t)E * Sc);
     }
-    if (q.edge_mask_h) {
-        ENSURE(e, e->d_mask, E);
-        CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, E, cudaMemcpyHostToDevice, e->stream));
-    }
     double *dsum = e->d_sum.as<double>();
     CK(e, cudaMemsetAsync(dsum, 0, sizeof(double) * (1 + E), e->stream));
-    CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
 
     DmArgs a;
     memset(&a, 0, sizeof(a));
@@ -2369,18 +2375,8 @@ static int run_dmma(plf_engine *e, Query &q)
     e->kernel_timed = true;
     const size_t nsum = 1 + E;
     if (finish_sums(e, dsum, nsum)) return -1;
-    CK(e, cudaEventRecord(e->ev[2], e->stream));
-    std::vector<double> hs(nsum);
-    int herr = 0;
-    CK(e, cudaMemcpyAsync(hs.data(), dsum, sizeof(double) * nsum, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaMemcpyAsync(&herr, e->d_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
-    if (q.site_ll) CK(e, cudaMemcpyAsync(q.site_ll, e->d_site_ll.p, sizeof(double) * e->S, cudaMemcpyDeviceToHost, e->stream));
-    CK(e, cudaStreamSynchronize(e->stream));
-    if (herr & 4) FAIL(e, "all-reduce over peer memory timed out (a rank is missing)");
-    if ((herr & 1) && (q.sum_ll || q.sum_edge)) FAIL(e, "a site with non-zero weight has zero likelihood");
-    if (q.sum_ll) *q.sum_ll = hs[0];
-    if (q.sum_edge) memcpy(q.sum_edge, hs.data() + 1, sizeof(double) * E);
-    return 0;
+    std::vector<double> hs; int herr = 0;
+    return (read_back(e, q, dsum, nsum, hs, herr) || unpack_sums(e, q, hs, herr)) ? -1 : 0;
 }
 
 /* common driver: matrices, path selection, timing.  Returns 1 when the query has to be repeated. */
@@ -2388,6 +2384,10 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
 {
     if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
     CK(e, cudaSetDevice(e->device));
+    if (q.edge_mask_h) {
+        ENSURE(e, e->d_mask, e->E);
+        CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, e->E, cudaMemcpyHostToDevice, e->stream));
+    }
     /* the edge matrices need the whole site likelihood: no category windows (n = 4 with C > 4 goes to the generic path) */
     bool use_fused = fused_applicable(e) && !q.sum_hess && !(q.want_gmat && e->C > 4);
     /* per-site marginals of a huge alignment: the generic path works in chunks of sites */
@@ -2408,10 +2408,6 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
     if (l_hi) {
         if (upload_L(e, l_hi, l_lo)) return -1;
         ENSURE(e, e->d_F, sizeof(double) * (size_t)e->C * e->E * e->n * e->n);
-        if (q.edge_mask_h) {
-            ENSURE(e, e->d_mask, e->E);
-            CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, e->E, cudaMemcpyHostToDevice, e->stream));
-        }
         if (run_expm(e, nullptr, nullptr, e->d_F.as<double>(), kind == PLF_KIND_TRANS ? 1 : 0,
                      q.edge_mask_h ? e->d_mask.as<unsigned char>() : nullptr, e->d_lhi.as<double>(), e->d_llo.as<double>())) return -1;
         q.Fm = e->d_F.as<double>(); q.f_zero_rowsum = 0; f_mode = 2;
@@ -2424,10 +2420,11 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
      * constant-memory kernels at the price of per-site outputs and a combination pass) */
     int wforce = 0;
     if (const char *wf = getenv("PLF_F4_WINDOW")) wforce = std::max(1, std::min(4, atoi(wf)));
-    int rc = use_fused ? ((!q.want_gmat && (e->C > 4 || (wforce && wforce < e->C))) ? run_fused_windows(e, q, wforce ? wforce : 4)
-                                                                                : run_fused(e, q))
-                       : (e->path != PLF_PATH_GENERIC && !q.sum_hess && !q.want_gmat && dmma_applicable(e, q)) ? run_dmma(e, q)
-                                                                                                              : run_generic(e, q);
+    int rc;
+    if (use_fused && !q.want_gmat && (e->C > 4 || (wforce && wforce < e->C))) rc = run_fused_windows(e, q, wforce ? wforce : 4);
+    else if (use_fused) rc = run_fused(e, q);
+    else if (e->path != PLF_PATH_GENERIC && !q.sum_hess && !q.want_gmat && dmma_applicable(e, q)) rc = run_dmma(e, q);
+    else rc = run_generic(e, q);
     if (rc) return rc;
     cudaEventElapsedTime(&e->ms_mat, e->ev[0], e->ev[1]);
     cudaEventElapsedTime(&e->ms_sites, e->ev[1], e->ev[2]);

@@ -383,10 +383,55 @@ def test_async_upload_matches_synchronous_upload():
     assert np.allclose(tot.sum(axis=1), w.sum(), rtol=1e-11)
 
 
+# What each forced index of PLF_F4_CONFIG_MARG / PLF_F4_CONFIG / PLF_F4_CONFIG_LL selects in
+# test_every_fused_configuration_agrees, per problem (taxa): the template arguments of fused4_kernel<...> for the
+# (marginal, edge forms, ll) query, None where no configuration fits.  The indices are positions in the candidate
+# tables of plf_engine.cu that tools/cfg_sweep.py and the recorded profiles refer to.  Recorded on an NVIDIA B200.
+FORCED_KERNELS = {
+    24: [
+        ("4,2,384,1,1,0", "4,1,512,2,1,1", "4,0,512,2,1,1"),
+        ("4,2,384,1,0,0", "4,1,512,2,0,1", "4,0,512,2,1,0"),
+        ("4,2,256,1,0,0", "4,1,384,2,0,1", "4,0,512,2,0,1"),
+        ("4,2,384,0,1,0", "4,1,384,2,1,0", "4,0,384,2,1,0"),
+        ("4,2,384,0,0,0", "4,1,384,1,0,0", "4,0,384,2,1,0"),
+        ("4,2,256,0,0,0", "4,1,512,1,0,0", "4,0,384,1,0,0"),
+        ("4,2,128,0,0,0", "4,1,256,2,0,0", "4,0,256,2,0,0"),
+        (None, "4,1,512,0,1,0", "4,0,256,2,0,0"),
+        (None, "4,1,384,0,1,0", "4,0,512,0,1,0"),
+        (None, "4,1,384,0,0,0", "4,0,384,0,1,0"),
+        (None, "4,1,256,0,0,0", "4,0,384,0,0,0"),
+        (None, "4,1,128,0,0,0", "4,0,256,0,0,0"),
+        (None, None, "4,0,128,0,0,0"),
+        (None, None, "4,0,128,0,0,0"),
+        (None, None, None),
+        (None, None, None),
+    ],
+    160: [
+        (None, None, None),
+        (None, None, None),
+        (None, None, None),
+        ("4,2,384,0,1,0", None, None),
+        ("4,2,384,0,0,0", None, None),
+        ("4,2,256,0,0,0", None, None),
+        ("4,2,128,0,0,0", None, None),
+        (None, "4,1,512,0,1,0", None),
+        (None, "4,1,384,0,1,0", "4,0,512,0,1,0"),
+        (None, "4,1,384,0,0,0", "4,0,384,0,1,0"),
+        (None, "4,1,256,0,0,0", "4,0,384,0,0,0"),
+        (None, "4,1,128,0,0,0", "4,0,256,0,0,0"),
+        (None, None, "4,0,128,0,0,0"),
+        (None, None, "4,0,128,0,0,0"),
+        (None, None, None),
+        (None, None, None),
+    ],
+}
+
+
 def test_every_fused_configuration_agrees(monkeypatch):
     """Each candidate configuration of the fused kernel (block size, staged / unstaged tables with prefetch,
     packed codes, constant-memory matrices, shared / global stack) is forced in turn on one problem and must
-    reproduce the sums of the default choice; the same for a tree too large for the constant-memory kernels."""
+    reproduce the sums of the default choice; the same for a tree too large for the constant-memory kernels.
+    Each index must also still select the kernel it selected when FORCED_KERNELS was recorded."""
     from phyly_b200.engine import EngineError
     for taxa, sites in ((24, 30000), (160, 6000)):
         b, pb = _problem(sites, taxa)
@@ -405,30 +450,34 @@ def test_every_fused_configuration_agrees(monkeypatch):
         scale = np.abs(want["sum_deriv"]).max()
         ran_edge = ran_ll = ran_mg = 0
         for i in range(16):
+            want_k = ["fused4_kernel<%s>" % k if k else None for k in FORCED_KERNELS[taxa][i]]
             monkeypatch.setenv("PLF_F4_CONFIG", str(i))
             monkeypatch.setenv("PLF_F4_CONFIG_LL", str(i))
             monkeypatch.setenv("PLF_F4_CONFIG_MARG", str(i))
             try:
                 got_mg = eng.marginal(per_site=False)[1]
             except EngineError as ex:
-                assert "no configuration fits" in str(ex), ex
+                assert "no configuration fits" in str(ex) and want_k[0] is None, (taxa, i, ex)
             else:
                 ran_mg += 1
+                assert eng.last_kernel_name() == want_k[0], (taxa, i)
                 assert np.allclose(got_mg, want_mg, rtol=1e-11, atol=1e-12 * np.abs(want_mg).max()), (taxa, i)
             try:
                 got = eng.deriv(per_site=False)
             except EngineError as ex:
-                assert "no configuration fits" in str(ex), ex
+                assert "no configuration fits" in str(ex) and want_k[1] is None, (taxa, i, ex)
             else:
                 ran_edge += 1
+                assert eng.last_kernel_name() == want_k[1], (taxa, i)
                 assert abs(got["sum_ll"] - want["sum_ll"]) <= 1e-12 * abs(want["sum_ll"]), (taxa, i)
                 assert np.all(np.abs(got["sum_deriv"] - want["sum_deriv"]) <= 1e-11 * np.abs(want["sum_deriv"]) + 1e-12 * scale), (taxa, i)
             try:
                 got_ll = eng.ll(per_site=False)[1]
             except EngineError as ex:
-                assert "no configuration fits" in str(ex), ex
+                assert "no configuration fits" in str(ex) and want_k[2] is None, (taxa, i, ex)
             else:
                 ran_ll += 1
+                assert eng.last_kernel_name() == want_k[2], (taxa, i)
                 assert abs(got_ll - want_ll) <= 1e-12 * abs(want_ll), (taxa, i)
         assert ran_edge >= 3 and ran_ll >= 3 and ran_mg >= 2, (taxa, ran_edge, ran_ll, ran_mg)
         eng.close()
