@@ -150,16 +150,14 @@ __global__ void dm_tip_table_kernel(const double *M, const double *defs, const u
     out[idx] = v;
 }
 
-/* four n-blocks (two packed pairs, chunk pc) of one contraction for the SG site groups of a warp:
- * em[r][i][h] = sum_k A[r][k] B[k][8 (4 pc + i) + ...]; every B fragment read from shared memory feeds 2 SG DMMAs */
-template <int NB, int SG>
-__device__ __forceinline__ void dm_gemm_chunk(const double (&A)[SG][2 * NB], const double2 *sl, int pc, double (&em)[SG][4][2])
+/* four n-blocks (two packed pairs, chunk pc) of one contraction for the 8 sites of a warp:
+ * em[i][h] = sum_k A[k] B[k][8 (4 pc + i) + ...]; every B fragment read from shared memory feeds 2 DMMAs */
+template <int NB>
+__device__ __forceinline__ void dm_gemm_chunk(const double (&A)[2 * NB], const double2 *sl, int pc, double (&em)[4][2])
 {
     constexpr int NBP = (NB + 1) / 2;
 #pragma unroll
-    for (int r = 0; r < SG; r++)
-#pragma unroll
-        for (int i = 0; i < 4; i++) { em[r][i][0] = 0.0; em[r][i][1] = 0.0; }
+    for (int i = 0; i < 4; i++) { em[i][0] = 0.0; em[i][1] = 0.0; }
 #pragma unroll
     for (int kk = 0; kk < 2 * NB; kk++) {
 #pragma unroll
@@ -167,11 +165,8 @@ __device__ __forceinline__ void dm_gemm_chunk(const double (&A)[SG][2 * NB], con
             const int nbp = 2 * pc + p;
             if (nbp < NBP) {
                 const double2 b = sl[(kk * NBP + nbp) * 32];
-#pragma unroll
-                for (int r = 0; r < SG; r++) {
-                    dm_dmma(em[r][2 * p][0], em[r][2 * p][1], A[r][kk], b.x);
-                    if (2 * nbp + 1 < NB) dm_dmma(em[r][2 * p + 1][0], em[r][2 * p + 1][1], A[r][kk], b.y);
-                }
+                dm_dmma(em[2 * p][0], em[2 * p][1], A[kk], b.x);
+                if (2 * nbp + 1 < NB) dm_dmma(em[2 * p + 1][0], em[2 * p + 1][1], A[kk], b.y);
             }
         }
     }
@@ -281,20 +276,18 @@ __device__ __forceinline__ void dm_prefetch(const void *p)
     asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
 }
 
-/* the warp's character codes of one tile: dst[row][8 SG sites] (site group r of the warp at bytes 8r..8r+7) */
-template <int SG>
+/* the warp's character codes of one tile: dst[row][8 sites] */
 __device__ __forceinline__ void dm_stage_codes(const DmArgs &a, unsigned char *my_codes, int sw, int lane)
 {
     __syncwarp();
     for (int r = lane; r < a.nrows; r += 32) {
         const unsigned char *src = a.codes + (size_t)a.code_row_node[r] * a.S + a.s0 + sw;
-        unsigned char *dst = my_codes + r * (8 * SG);
-        if (sw + 8 * SG <= a.Sc && ((reinterpret_cast<uintptr_t>(src) & 7) == 0)) {
-#pragma unroll
-            for (int i = 0; i < SG; i++) reinterpret_cast<uint2 *>(dst)[i] = reinterpret_cast<const uint2 *>(src)[i];
+        unsigned char *dst = my_codes + r * 8;
+        if (sw + 8 <= a.Sc && ((reinterpret_cast<uintptr_t>(src) & 7) == 0)) {
+            *reinterpret_cast<uint2 *>(dst) = *reinterpret_cast<const uint2 *>(src);
         } else {
             /* ragged end of the chunk: sites beyond it repeat the chunk's last site (their results are not written) */
-            for (int s = 0; s < 8 * SG; s++) dst[s] = src[(sw + s < a.Sc) ? s : (a.Sc - 1 - sw)];
+            for (int s = 0; s < 8; s++) dst[s] = src[(sw + s < a.Sc) ? s : (a.Sc - 1 - sw)];
         }
     }
     __syncwarp();
@@ -324,9 +317,9 @@ __device__ __forceinline__ int dm_site_max_hi(const double (&v)[2 * NB])
 
 /*
  * Inside pass.  grid = persistent CTAs (work item i = blockIdx.x + k gridDim.x -> tile i / C, category i % C),
- * NW warps of SG site groups (8 SG sites) each; NW SG = DM_GROUPS.
+ * NW = DM_GROUPS warps of one 8-site group each.
  */
-template <int NB, int NW, int SG>
+template <int NB, int NW>
 __global__ void __launch_bounds__(NW * 32, 1) dm_inside_kernel(const DmArgs a)
 {
     extern __shared__ __align__(128) unsigned char dm_smem[];
@@ -342,204 +335,162 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_inside_kernel(const DmArgs a)
     ring.total = my_items * a.Ei;
     ring.setup(dm_smem, tid);
     const DmProg prog = dm_stage_program(a, ring.after(), tid, NW * 32);
-    unsigned char *my_codes = prog.after + (size_t)warp * a.nrows * (8 * SG);
-    /* The warps of a scheduler run the same program and would stay in lock-step (all in a contraction, then all
-     * outside one, leaving the tensor pipe idle): start them a fraction of an op apart. */
-    if (a.stagger > 0) {
-        const long long t0 = clock64(), wait = (long long)(warp >> 2) * a.stagger;
-        while (clock64() - t0 < wait) { }
-    }
+    unsigned char *my_codes = prog.after + (size_t)warp * a.nrows * 8;
 
-    double2 *my_stack = a.stack + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (SG * NB * 32);
-    int *my_stack_meta = a.stack_meta + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (SG * 32);
+    double2 *my_stack = a.stack + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (NB * 32);
+    int *my_stack_meta = a.stack_meta + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * 32;
     long long G = 0;
 
     for (long long it = 0; it < my_items; it++) {
         const long long item = (long long)blockIdx.x + it * gridDim.x;
         const int tile = (int)(item / a.C), c = (int)(item % a.C);
-        int g0, cnt;
-        dm_tile(a, tile, g0, cnt);
-        const int nact = (cnt + SG - 1) / SG;
+        int g0, nact;                                       /* warps with sites: one per 8-site group of the tile */
+        dm_tile(a, tile, g0, nact);
         if (warp >= nact) {
             /* a short tile of the last wave: this warp has no sites; nothing after such a tile may overtake it */
             G += a.Ei;
             __syncthreads();
             continue;
         }
-        const int gw = g0 + warp * SG;                      /* first 8-site group of this warp (within the chunk) */
+        const int gw = g0 + warp;                           /* this warp's 8-site group (within the chunk) */
         const int sw = gw * 8;
-        dm_stage_codes<SG>(a, my_codes, sw, lane);
+        dm_stage_codes(a, my_codes, sw, lane);
 
         const double *TPc = a.TPf + (size_t)c * a.Et * a.K * W + q * 2 * NB;
-        double cur[SG][2 * NB];
-        int curk[SG], curc[SG], sp = 0;
+        double cur[2 * NB];
+        int curk = 0, curc = 1, sp = 0;
 #pragma unroll
-        for (int r = 0; r < SG; r++) {
-            curk[r] = 0; curc[r] = 1;
-#pragma unroll
-            for (int i = 0; i < 2 * NB; i++) cur[r][i] = 0.0;
-        }
+        for (int i = 0; i < 2 * NB; i++) cur[i] = 0.0;
 
 #pragma unroll 1
         for (int o = 0; o < a.nops; o++) {
             const DmOpV op = dm_op(prog, o);
             if (op.spill_before) {
-                double2 *st = my_stack + (size_t)sp * (SG * NB * 32) + lane;
+                double2 *st = my_stack + (size_t)sp * (NB * 32) + lane;
 #pragma unroll
-                for (int r = 0; r < SG; r++) {
-#pragma unroll
-                    for (int nb = 0; nb < NB; nb++) __stcg(st + (r * NB + nb) * 32, make_double2(cur[r][2 * nb], cur[r][2 * nb + 1]));
-                    my_stack_meta[(sp * SG + r) * 32 + lane] = curk[r] * 2 + curc[r];
-                }
+                for (int nb = 0; nb < NB; nb++) __stcg(st + nb * 32, make_double2(cur[2 * nb], cur[2 * nb + 1]));
+                my_stack_meta[sp * 32 + lane] = curk * 2 + curc;
                 sp++;
             }
-            double acc[SG][2 * NB];
-            int kacc[SG], cst[SG];
+            double acc[2 * NB];
+            int kacc = 0, cst = 1;
+            if (op.code_row >= 0) {
+                /* the node itself carries data (rare) */
+                const int code = my_codes[op.code_row * 8 + g];
+                const double2 *dp = reinterpret_cast<const double2 *>(a.defsf + (size_t)code * W + q * 2 * NB);
 #pragma unroll
-            for (int r = 0; r < SG; r++) {
-                kacc[r] = 0; cst[r] = 1;
-                if (op.code_row >= 0) {
-                    /* the node itself carries data (rare) */
-                    const int code = my_codes[op.code_row * (8 * SG) + 8 * r + g];
-                    const double2 *dp = reinterpret_cast<const double2 *>(a.defsf + (size_t)code * W + q * 2 * NB);
+                for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(dp + nb); acc[2 * nb] = v.x; acc[2 * nb + 1] = v.y; }
+                cst = prog.def_const[code];
+            } else {
 #pragma unroll
-                    for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(dp + nb); acc[r][2 * nb] = v.x; acc[r][2 * nb + 1] = v.y; }
-                    cst[r] = prog.def_const[code];
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 2 * NB; i++) acc[r][i] = 1.0;
-                }
+                for (int i = 0; i < 2 * NB; i++) acc[i] = 1.0;
             }
 #pragma unroll 1
             for (int j = 0; j < op.nchild; j++) {
                 const DmChV ch = dm_ch(prog, op.first_child + j);
-                int bc[SG];
+                int bc;
                 if (ch.kind == F4_KIND_TIP) {
+                    const int code = my_codes[ch.code_row * 8 + g];
+                    bc = prog.def_const[code];
+                    const double2 *tp = reinterpret_cast<const double2 *>(TPc + ((size_t)ch.mat * a.K + code) * W);
 #pragma unroll
-                    for (int r = 0; r < SG; r++) {
-                        const int code = my_codes[ch.code_row * (8 * SG) + 8 * r + g];
-                        bc[r] = prog.def_const[code];
-                        const double2 *tp = reinterpret_cast<const double2 *>(TPc + ((size_t)ch.mat * a.K + code) * W);
-#pragma unroll
-                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(tp + nb); acc[r][2 * nb] *= v.x; acc[r][2 * nb + 1] *= v.y; }
-                    }
+                    for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(tp + nb); acc[2 * nb] *= v.x; acc[2 * nb + 1] *= v.y; }
                 } else {
-                    int kb[SG];
+                    int kb;
                     if (ch.kind == F4_KIND_STACK) {
                         sp--;
-                        const double2 *st = my_stack + (size_t)sp * (SG * NB * 32) + lane;
+                        const double2 *st = my_stack + (size_t)sp * (NB * 32) + lane;
 #pragma unroll
-                        for (int r = 0; r < SG; r++) {
-#pragma unroll
-                            for (int nb = 0; nb < NB; nb++) { const double2 v = __ldcg(st + (r * NB + nb) * 32); cur[r][2 * nb] = v.x; cur[r][2 * nb + 1] = v.y; }
-                            const int meta = my_stack_meta[(sp * SG + r) * 32 + lane];
-                            kb[r] = meta >> 1; bc[r] = meta & 1;
-                        }
+                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldcg(st + nb * 32); cur[2 * nb] = v.x; cur[2 * nb + 1] = v.y; }
+                        const int meta = my_stack_meta[sp * 32 + lane];
+                        kb = meta >> 1; bc = meta & 1;
                     } else {
-#pragma unroll
-                        for (int r = 0; r < SG; r++) { kb[r] = curk[r]; bc[r] = curc[r]; }
+                        kb = curk; bc = curc;
                     }
                     /* a constant column maps to itself under a stochastic matrix (arb_mat_extras.c:84-91) */
-                    double v0[SG];
-#pragma unroll
-                    for (int r = 0; r < SG; r++) v0[r] = __shfl_sync(0xffffffffu, cur[r][0], lane & ~3);
+                    const double v0 = __shfl_sync(0xffffffffu, cur[0], lane & ~3);
                     const double2 *sl = ring.acquire(G, lane);
                     double2 *slab = nullptr;
                     if (a.slab) {
                         const size_t cell = ((size_t)c * a.Ei + ch.mat) * a.ngroups + (size_t)gw;
                         slab = a.slab + cell * (NB * 32) + lane;
-#pragma unroll
-                        for (int r = 0; r < SG; r++)
-                            if (gw + r < a.ngroups) a.slab_meta[(cell + r) * 32 + lane] = kb[r] * 2 + bc[r];
+                        if (gw < a.ngroups) a.slab_meta[cell * 32 + lane] = kb * 2 + bc;
                     }
 #pragma unroll
                     for (int pc = 0; pc < NCH; pc++) {
-                        double em[SG][4][2];
-                        dm_gemm_chunk<NB, SG>(cur, sl, pc, em);
+                        double em[4][2];
+                        dm_gemm_chunk<NB>(cur, sl, pc, em);
 #pragma unroll
-                        for (int r = 0; r < SG; r++) {
-#pragma unroll
-                            for (int i = 0; i < 4; i++) {
-                                const int nb = 4 * pc + i;
-                                if (nb < NB) {
-                                    if (bc[r]) {
-                                        em[r][i][0] = (8 * nb + 2 * q < a.n) ? v0[r] : 0.0;
-                                        em[r][i][1] = (8 * nb + 2 * q + 1 < a.n) ? v0[r] : 0.0;
-                                    }
-                                    if (slab && gw + r < a.ngroups) __stcs(slab + (r * NB + nb) * 32, make_double2(em[r][i][0], em[r][i][1]));
-                                    acc[r][2 * nb] *= em[r][i][0]; acc[r][2 * nb + 1] *= em[r][i][1];
+                        for (int i = 0; i < 4; i++) {
+                            const int nb = 4 * pc + i;
+                            if (nb < NB) {
+                                if (bc) {
+                                    em[i][0] = (8 * nb + 2 * q < a.n) ? v0 : 0.0;
+                                    em[i][1] = (8 * nb + 2 * q + 1 < a.n) ? v0 : 0.0;
                                 }
+                                if (slab && gw < a.ngroups) __stcs(slab + nb * 32, make_double2(em[i][0], em[i][1]));
+                                acc[2 * nb] *= em[i][0]; acc[2 * nb + 1] *= em[i][1];
                             }
                         }
                     }
                     ring.release(G, lane, nact);
                     G++;
-#pragma unroll
-                    for (int r = 0; r < SG; r++) kacc[r] += kb[r];
+                    kacc += kb;
                 }
                 /* per-site rescale after every second factor (non-negative doubles order like their high words) */
                 const bool resc = (j & 1) || j == op.nchild - 1;
+                cst &= bc;
+                if (resc) {
+                    const double sc = dm_scale_up(dm_site_max_hi<NB>(acc), kacc);
+                    if (sc != 1.0) {
 #pragma unroll
-                for (int r = 0; r < SG; r++) {
-                    cst[r] &= bc[r];
-                    if (resc) {
-                        const double sc = dm_scale_up(dm_site_max_hi<NB>(acc[r]), kacc[r]);
-                        if (sc != 1.0) {
-#pragma unroll
-                            for (int i = 0; i < 2 * NB; i++) acc[r][i] *= sc;
-                        }
+                        for (int i = 0; i < 2 * NB; i++) acc[i] *= sc;
                     }
                 }
             }
 #pragma unroll
-            for (int r = 0; r < SG; r++) {
-#pragma unroll
-                for (int i = 0; i < 2 * NB; i++) cur[r][i] = acc[r][i];
-                curk[r] = kacc[r]; curc[r] = cst[r];
-            }
+            for (int i = 0; i < 2 * NB; i++) cur[i] = acc[i];
+            curk = kacc; curc = cst;
         }
         /* root_prior_expectation (model.c:282-350) */
+        const double2 *rp = reinterpret_cast<const double2 *>(a.rootf + q * 2 * NB);
+        double lh = 0.0;
 #pragma unroll
-        for (int r = 0; r < SG; r++) {
-            const double2 *rp = reinterpret_cast<const double2 *>(a.rootf + q * 2 * NB);
-            double lh = 0.0;
-#pragma unroll
-            for (int nb = 0; nb < NB; nb++) { const double2 rv = __ldg(rp + nb); lh = fma(rv.x, cur[r][2 * nb], lh); lh = fma(rv.y, cur[r][2 * nb + 1], lh); }
-            lh += __shfl_xor_sync(0xffffffffu, lh, 1);
-            lh += __shfl_xor_sync(0xffffffffu, lh, 2);
-            const double v0 = __shfl_sync(0xffffffffu, cur[r][0], lane & ~3);
-            if (curc[r] && a.root_const_ok) lh = v0;
-            const int site = sw + 8 * r + g;
-            if (site < a.Sc && q == 0) {
-                a.cat_lh[(size_t)c * a.Sc + site] = lh;
-                a.cat_k[(size_t)c * a.Sc + site] = curk[r];
-            }
+        for (int nb = 0; nb < NB; nb++) { const double2 rv = __ldg(rp + nb); lh = fma(rv.x, cur[2 * nb], lh); lh = fma(rv.y, cur[2 * nb + 1], lh); }
+        lh += __shfl_xor_sync(0xffffffffu, lh, 1);
+        lh += __shfl_xor_sync(0xffffffffu, lh, 2);
+        const double v0 = __shfl_sync(0xffffffffu, cur[0], lane & ~3);
+        if (curc && a.root_const_ok) lh = v0;
+        const int site = sw + g;
+        if (site < a.Sc && q == 0) {
+            a.cat_lh[(size_t)c * a.Sc + site] = lh;
+            a.cat_k[(size_t)c * a.Sc + site] = curk;
         }
         if (nact < NW) __syncthreads();
     }
 }
 
-/* edge vector of a child at one site group of this warp: block nb of em (tip table or slab), its exponent and constant flag */
+/* edge vector of a child at the 8 sites of this warp: block nb of em (tip table or slab), its exponent and constant flag */
 struct DmChildRef {
     const double2 *p;       /* + nb * stride */
     int stride;
     int k, bc;
 };
 
-template <int NB, int SG>
-__device__ __forceinline__ DmChildRef dm_child_ref(const DmArgs &a, const DmProg &prog, const DmChV &ch, int c, int gw, int r, int lane, int g, int q,
+template <int NB>
+__device__ __forceinline__ DmChildRef dm_child_ref(const DmArgs &a, const DmProg &prog, const DmChV &ch, int c, int gw, int lane, int g, int q,
                                                    const unsigned char *my_codes)
 {
     DmChildRef ref;
     const int W = 8 * NB;
     if (ch.kind == F4_KIND_TIP) {
-        const int code = my_codes[ch.code_row * (8 * SG) + 8 * r + g];
+        const int code = my_codes[ch.code_row * 8 + g];
         ref.p = reinterpret_cast<const double2 *>(a.TPf + (((size_t)c * a.Et + ch.mat) * a.K + code) * W + q * 2 * NB);
         ref.stride = 1;
         ref.k = 0; ref.bc = prog.def_const[code];
     } else {
         /* groups beyond the chunk read the chunk's last group (their results are not written) */
-        const size_t cell = ((size_t)c * a.Ei + ch.mat) * a.ngroups + (size_t)min(gw + r, a.ngroups - 1);
+        const size_t cell = ((size_t)c * a.Ei + ch.mat) * a.ngroups + (size_t)min(gw, a.ngroups - 1);
         ref.p = a.slab + cell * (NB * 32) + lane;
         ref.stride = 32;
         const int meta = a.slab_meta[cell * 32 + lane];
@@ -574,9 +525,9 @@ __device__ __forceinline__ double dm_scale256(double x, int k)
  * that each (edge, site) output cell is accumulated by one thread.  Needs the slab of a keep-mode inside pass and
  * the combined site likelihoods (site_m, site_k).
  *
- * Per-warp stack entry: [SG][fn | z][NB][32] double2 and int4 meta [SG][32] {exponent, high word of max fn, csr edge, -}.
+ * Per-warp stack entry: [fn | z][NB][32] double2 and int4 meta [32] {exponent, high word of max fn, csr edge, -}.
  */
-template <int NB, int NW, int SG>
+template <int NB, int NW>
 __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
 {
     extern __shared__ __align__(128) unsigned char dm_smem[];
@@ -591,67 +542,48 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
     ring.total = my_items * a.C * 2 * a.Ei;
     ring.setup(dm_smem, tid);
     const DmProg prog = dm_stage_program(a, ring.after(), tid, NW * 32);
-    unsigned char *my_codes = prog.after + (size_t)warp * a.nrows * (8 * SG);
-    /* The warps of a scheduler run the same program and would stay in lock-step (all in a contraction, then all
-     * outside one, leaving the tensor pipe idle): start them a fraction of an op apart. */
-    if (a.stagger > 0) {
-        const long long t0 = clock64(), wait = (long long)(warp >> 2) * a.stagger;
-        while (clock64() - t0 < wait) { }
-    }
+    unsigned char *my_codes = prog.after + (size_t)warp * a.nrows * 8;
 
-    double2 *my_stack = a.stack + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (SG * 2 * NB * 32);
-    int4 *my_stack_meta = reinterpret_cast<int4 *>(a.stack_meta) + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (SG * 32);
+    double2 *my_stack = a.stack + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * (2 * NB * 32);
+    int4 *my_stack_meta = reinterpret_cast<int4 *>(a.stack_meta) + ((size_t)blockIdx.x * NW + warp) * a.stack_depth * 32;
     long long G = 0;
 
     for (long long it = 0; it < my_items; it++) {
         const int tile = (int)(blockIdx.x + it * gridDim.x);
-        int g0, cnt;
-        dm_tile(a, tile, g0, cnt);
-        const int nact = (cnt + SG - 1) / SG;
+        int g0, nact;
+        dm_tile(a, tile, g0, nact);
         if (warp >= nact) {
             G += (long long)a.C * 2 * a.Ei;
             __syncthreads();
             continue;
         }
-        const int gw = g0 + warp * SG;
+        const int gw = g0 + warp;
         const int sw = gw * 8;
-        dm_stage_codes<SG>(a, my_codes, sw, lane);
-        double sm[SG];
-        int sk[SG];
-        bool valid[SG];
-#pragma unroll
-        for (int r = 0; r < SG; r++) {
-            const int site = sw + 8 * r + g;
-            valid[r] = site < a.Sc;
-            sm[r] = valid[r] ? a.site_m[site] : 0.0;
-            sk[r] = valid[r] ? a.site_k[site] : 0;
-        }
+        dm_stage_codes(a, my_codes, sw, lane);
+        const int site = sw + g;
+        const bool valid = site < a.Sc;
+        const double sm = valid ? a.site_m[site] : 0.0;
+        const int sk = valid ? a.site_k[site] : 0;
 
 #pragma unroll 1
         for (int c = 0; c < a.C; c++) {
             const double *TFc = a.TFf + (size_t)c * a.Et * a.K * W + q * 2 * NB;
             int sp = 0;
-            double fn[SG][2 * NB];
-            int kf[SG];
-#pragma unroll
-            for (int r = 0; r < SG; r++) {
-                /* arbplfmarginal.c:184-191 / arbplfderiv.c:300-310: categories (and sites) of zero likelihood contribute nothing */
-                double coef = 0.0;
-                if (valid[r]) {
-                    const double prior = a.cat_prior[c];
-                    if (prior * a.cat_lh[(size_t)c * a.Sc + sw + 8 * r + g] > 0.0 && sm[r] > 0.0) coef = prior / sm[r];
-                }
-                kf[r] = -sk[r];
-                const double2 *rp = reinterpret_cast<const double2 *>(a.rootf + q * 2 * NB);
-#pragma unroll
-                for (int nb = 0; nb < NB; nb++) { const double2 rv = __ldg(rp + nb); fn[r][2 * nb] = rv.x * coef; fn[r][2 * nb + 1] = rv.y * coef; }
+            double fn[2 * NB];
+            /* arbplfmarginal.c:184-191 / arbplfderiv.c:300-310: categories (and sites) of zero likelihood contribute nothing */
+            double coef = 0.0;
+            if (valid) {
+                const double prior = a.cat_prior[c];
+                if (prior * a.cat_lh[(size_t)c * a.Sc + sw + g] > 0.0 && sm > 0.0) coef = prior / sm;
             }
+            int kf = -sk;
+            const double2 *rp = reinterpret_cast<const double2 *>(a.rootf + q * 2 * NB);
+#pragma unroll
+            for (int nb = 0; nb < NB; nb++) { const double2 rv = __ldg(rp + nb); fn[2 * nb] = rv.x * coef; fn[2 * nb + 1] = rv.y * coef; }
             bool fn_in_regs = true;               /* the root's fn was formed above */
 #pragma unroll 1
             for (int o = a.nops - 1; o >= 0; o--) {
                 const DmOpV op = dm_op(prog, o);
-                static_assert(SG == 1, "the outside pass is written for one site group per warp");
-                constexpr int r = 0;
                 const bool popped = (o != a.nops - 1);
                 const double2 *zp = nullptr;
                 int in_edge = -1, kz = 0;
@@ -662,21 +594,21 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                     const double2 *st = my_stack + (size_t)sp * (2 * NB * 32) + lane;
                     const int4 meta = my_stack_meta[sp * 32 + lane];
                     in_edge = meta.z; kz = meta.x;          /* z keeps the exponent it was computed with */
-                    kf[r] = meta.x;
+                    kf = meta.x;
                     int m = meta.y;
                     double sc = 1.0;
                     if (m > 0) {
-                        while (m < DM_HI_M256) { m += 0x10000000; sc *= DM_TWO_P256; kf[r] -= 1; }
-                        while (m >= DM_HI_P256) { m -= 0x10000000; sc *= DM_TWO_M256; kf[r] += 1; }
+                        while (m < DM_HI_M256) { m += 0x10000000; sc *= DM_TWO_P256; kf -= 1; }
+                        while (m >= DM_HI_P256) { m -= 0x10000000; sc *= DM_TWO_M256; kf += 1; }
                     }
                     if (fn_in_regs) {
                         if (sc != 1.0) {
 #pragma unroll
-                            for (int i = 0; i < 2 * NB; i++) fn[r][i] *= sc;
+                            for (int i = 0; i < 2 * NB; i++) fn[i] *= sc;
                         }
                     } else {
 #pragma unroll
-                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldcg(st + nb * 32); fn[r][2 * nb] = v.x * sc; fn[r][2 * nb + 1] = v.y * sc; }
+                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldcg(st + nb * 32); fn[2 * nb] = v.x * sc; fn[2 * nb + 1] = v.y * sc; }
                     }
                     zp = st + NB * 32;
                 }
@@ -684,7 +616,7 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
 
                 /* contraction of fe with (P_e, F_e) of an internal child: fn_b into `dst_fn` (registers, when the child is
                  * the next op's node) or into the stack entry, z_b always into the stack entry */
-                auto contract_and_push = [&](const double (&fe)[SG][2 * NB], int kfe, int edge, bool keep_fn) {
+                auto contract_and_push = [&](const double (&fe)[2 * NB], int kfe, int edge, bool keep_fn) {
                     double2 *st = my_stack + (size_t)sp * (2 * NB * 32) + lane;
                     int m = 0;
 #pragma unroll 1
@@ -692,18 +624,18 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                         const double2 *sl = ring.acquire(G, lane);
 #pragma unroll
                         for (int pc = 0; pc < NCH; pc++) {
-                            double em[SG][4][2];
-                            dm_gemm_chunk<NB, SG>(fe, sl, pc, em);
+                            double em[4][2];
+                            dm_gemm_chunk<NB>(fe, sl, pc, em);
 #pragma unroll
                             for (int i = 0; i < 4; i++) {
                                 const int nb = 4 * pc + i;
                                 if (nb < NB) {
                                     if (which == 0) {
-                                        m = max(m, max(__double2hiint(em[r][i][0]), __double2hiint(em[r][i][1])));
-                                        if (keep_fn) { fn[r][2 * nb] = em[r][i][0]; fn[r][2 * nb + 1] = em[r][i][1]; }
-                                        else __stcg(st + nb * 32, make_double2(em[r][i][0], em[r][i][1]));
+                                        m = max(m, max(__double2hiint(em[i][0]), __double2hiint(em[i][1])));
+                                        if (keep_fn) { fn[2 * nb] = em[i][0]; fn[2 * nb + 1] = em[i][1]; }
+                                        else __stcg(st + nb * 32, make_double2(em[i][0], em[i][1]));
                                     } else {
-                                        __stcg(st + (NB + nb) * 32, make_double2(em[r][i][0], em[r][i][1]));
+                                        __stcg(st + (NB + nb) * 32, make_double2(em[i][0], em[i][1]));
                                     }
                                 }
                             }
@@ -719,8 +651,8 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                 auto emit = [&](double x, int edge, int k) {
                     x += __shfl_xor_sync(0xffffffffu, x, 1);
                     x += __shfl_xor_sync(0xffffffffu, x, 2);
-                    if (valid[r] && q == 0 && (!a.edge_mask || a.edge_mask[edge])) {
-                        double *dst = a.edge_out + (size_t)edge * a.Sc + sw + 8 * r + g;
+                    if (valid && q == 0 && (!a.edge_mask || a.edge_mask[edge])) {
+                        double *dst = a.edge_out + (size_t)edge * a.Sc + sw + g;
                         /* the first category writes, the others add: no read-modify-write (a dependent global load) for C = 1 */
                         if (c == 0) *dst = dm_scale256(x, k);
                         else if (x != 0.0) *dst += dm_scale256(x, k);
@@ -742,13 +674,13 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                 if (op.nchild == 2 && op.code_row < 0) {
                     /* ---- two children, no data at the node: every vector is loaded once ---- */
                     const DmChV c0 = dm_ch(prog, op.first_child), c1 = dm_ch(prog, op.first_child + 1);
-                    const DmChildRef r0 = dm_child_ref<NB, SG>(a, prog, c0, c, gw, r, lane, g, q, my_codes);
-                    const DmChildRef r1 = dm_child_ref<NB, SG>(a, prog, c1, c, gw, r, lane, g, q, my_codes);
+                    const DmChildRef r0 = dm_child_ref<NB>(a, prog, c0, c, gw, lane, g, q, my_codes);
+                    const DmChildRef r1 = dm_child_ref<NB>(a, prog, c1, c, gw, lane, g, q, my_codes);
                     const bool int0 = c0.kind != F4_KIND_TIP, int1 = c1.kind != F4_KIND_TIP;
                     const double2 *tf0 = nullptr, *tf1 = nullptr;
-                    if (!int0) tf0 = reinterpret_cast<const double2 *>(TFc + ((size_t)c0.mat * a.K + my_codes[c0.code_row * (8 * SG) + 8 * r + g]) * W);
-                    if (!int1) tf1 = reinterpret_cast<const double2 *>(TFc + ((size_t)c1.mat * a.K + my_codes[c1.code_row * (8 * SG) + 8 * r + g]) * W);
-                    double fe[SG][2 * NB];
+                    if (!int0) tf0 = reinterpret_cast<const double2 *>(TFc + ((size_t)c0.mat * a.K + my_codes[c0.code_row * 8 + g]) * W);
+                    if (!int1) tf1 = reinterpret_cast<const double2 *>(TFc + ((size_t)c1.mat * a.K + my_codes[c1.code_row * 8 + g]) * W);
+                    double fe[2 * NB];
                     double xa = 0.0, x0 = 0.0, x1 = 0.0;
                     /* fe <- fn . em0 (the outside vector of child 1) when child 1 is internal, else fn . em1 (child 0's) */
 #pragma unroll
@@ -758,30 +690,30 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                             const double2 zz = __ldcg(zp + nb * 32);
                             xa = fma(zz.x, v0.x * v1.x, xa); xa = fma(zz.y, v0.y * v1.y, xa);
                         }
-                        const double f0x = fn[r][2 * nb] * v1.x, f0y = fn[r][2 * nb + 1] * v1.y;     /* child 0: fn . em1 */
-                        const double f1x = fn[r][2 * nb] * v0.x, f1y = fn[r][2 * nb + 1] * v0.y;     /* child 1: fn . em0 */
+                        const double f0x = fn[2 * nb] * v1.x, f0y = fn[2 * nb + 1] * v1.y;     /* child 0: fn . em1 */
+                        const double f1x = fn[2 * nb] * v0.x, f1y = fn[2 * nb + 1] * v0.y;     /* child 1: fn . em0 */
                         if (!int0) { const double2 t = __ldg(tf0 + nb); x0 = fma(t.x, f0x, x0); x0 = fma(t.y, f0y, x0); }
                         if (!int1) { const double2 t = __ldg(tf1 + nb); x1 = fma(t.x, f1x, x1); x1 = fma(t.y, f1y, x1); }
-                        if (int1) { fe[r][2 * nb] = f1x; fe[r][2 * nb + 1] = f1y; }
-                        else { fe[r][2 * nb] = f0x; fe[r][2 * nb + 1] = f0y; }
+                        if (int1) { fe[2 * nb] = f1x; fe[2 * nb + 1] = f1y; }
+                        else { fe[2 * nb] = f0x; fe[2 * nb + 1] = f0y; }
                     }
                     if (popped) {
                         if (a.f_zero_rowsum && (r0.bc & r1.bc)) xa = 0.0;
                         emit(xa, in_edge, kz + r0.k + r1.k);
                     }
-                    if (!int0) emit(x0, c0.edge, kf[r] + r1.k);
-                    if (!int1) emit(x1, c1.edge, kf[r] + r0.k);
+                    if (!int0) emit(x0, c0.edge, kf + r1.k);
+                    if (!int1) emit(x1, c1.edge, kf + r0.k);
                     if (int1) {
                         /* both internal: child 1 first (it goes to the stack), then child 0 with em1 loaded again */
-                        int kfe = kf[r] + r0.k;
-                        dm_rescale_both<NB>(fe[r], kfe);
+                        int kfe = kf + r0.k;
+                        dm_rescale_both<NB>(fe, kfe);
                         contract_and_push(fe, kfe, c1.edge, false);
 #pragma unroll
-                        for (int nb = 0; nb < NB; nb++) { const double2 v1 = r1.p[nb * r1.stride]; fe[r][2 * nb] = fn[r][2 * nb] * v1.x; fe[r][2 * nb + 1] = fn[r][2 * nb + 1] * v1.y; }
+                        for (int nb = 0; nb < NB; nb++) { const double2 v1 = r1.p[nb * r1.stride]; fe[2 * nb] = fn[2 * nb] * v1.x; fe[2 * nb + 1] = fn[2 * nb + 1] * v1.y; }
                     }
                     if (int0) {
-                        int kfe = kf[r] + r1.k;
-                        dm_rescale_both<NB>(fe[r], kfe);
+                        int kfe = kf + r1.k;
+                        dm_rescale_both<NB>(fe, kfe);
                         contract_and_push(fe, kfe, c0.edge, true);
                         fn_in_regs = true;
                     }
@@ -794,7 +726,7 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                     double La[2 * NB];
                     int kL = 0, cstL = 1;
                     if (op.code_row >= 0) {
-                        const int code = my_codes[op.code_row * (8 * SG) + 8 * r + g];
+                        const int code = my_codes[op.code_row * 8 + g];
                         const double2 *dp = reinterpret_cast<const double2 *>(a.defsf + (size_t)code * W + q * 2 * NB);
 #pragma unroll
                         for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(dp + nb); La[2 * nb] = v.x; La[2 * nb + 1] = v.y; }
@@ -805,7 +737,7 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                     }
 #pragma unroll 1
                     for (int j = 0; j < op.nchild; j++) {
-                        const DmChildRef ref = dm_child_ref<NB, SG>(a, prog, dm_ch(prog, op.first_child + j), c, gw, r, lane, g, q, my_codes);
+                        const DmChildRef ref = dm_child_ref<NB>(a, prog, dm_ch(prog, op.first_child + j), c, gw, lane, g, q, my_codes);
 #pragma unroll
                         for (int nb = 0; nb < NB; nb++) { const double2 v = ref.p[nb * ref.stride]; La[2 * nb] *= v.x; La[2 * nb + 1] *= v.y; }
                         kL += ref.k; cstL &= ref.bc;
@@ -825,37 +757,37 @@ __global__ void __launch_bounds__(NW * 32, 1) dm_outside_kernel(const DmArgs a)
                 }
                 /* fn_a . data_a */
                 if (op.code_row >= 0) {
-                    const int code = my_codes[op.code_row * (8 * SG) + 8 * r + g];
+                    const int code = my_codes[op.code_row * 8 + g];
                     const double2 *dp = reinterpret_cast<const double2 *>(a.defsf + (size_t)code * W + q * 2 * NB);
 #pragma unroll
-                    for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(dp + nb); fn[r][2 * nb] *= v.x; fn[r][2 * nb + 1] *= v.y; }
+                    for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(dp + nb); fn[2 * nb] *= v.x; fn[2 * nb + 1] *= v.y; }
                 }
                 /* children: tips in any order, internal ones from the last to the first so that the stack unwinds in
                  * the reverse of the inside pass */
 #pragma unroll 1
                 for (int j = op.nchild - 1; j >= 0; j--) {
                     const DmChV ch = dm_ch(prog, op.first_child + j);
-                    double fe[SG][2 * NB];
-                    int kfe = kf[r];
+                    double fe[2 * NB];
+                    int kfe = kf;
 #pragma unroll
-                    for (int i = 0; i < 2 * NB; i++) fe[r][i] = fn[r][i];
+                    for (int i = 0; i < 2 * NB; i++) fe[i] = fn[i];
                     int nmul = 0;
 #pragma unroll 1
                     for (int j2 = 0; j2 < op.nchild; j2++) {
                         if (j2 == j) continue;
-                        const DmChildRef ref = dm_child_ref<NB, SG>(a, prog, dm_ch(prog, op.first_child + j2), c, gw, r, lane, g, q, my_codes);
+                        const DmChildRef ref = dm_child_ref<NB>(a, prog, dm_ch(prog, op.first_child + j2), c, gw, lane, g, q, my_codes);
 #pragma unroll
-                        for (int nb = 0; nb < NB; nb++) { const double2 v = ref.p[nb * ref.stride]; fe[r][2 * nb] *= v.x; fe[r][2 * nb + 1] *= v.y; }
+                        for (int nb = 0; nb < NB; nb++) { const double2 v = ref.p[nb * ref.stride]; fe[2 * nb] *= v.x; fe[2 * nb + 1] *= v.y; }
                         kfe += ref.k;
-                        if ((++nmul & 1) == 0) dm_rescale_both<NB>(fe[r], kfe);
+                        if ((++nmul & 1) == 0) dm_rescale_both<NB>(fe, kfe);
                     }
-                    dm_rescale_both<NB>(fe[r], kfe);
+                    dm_rescale_both<NB>(fe, kfe);
                     if (ch.kind == F4_KIND_TIP) {
-                        const int code = my_codes[ch.code_row * (8 * SG) + 8 * r + g];
+                        const int code = my_codes[ch.code_row * 8 + g];
                         const double2 *tf = reinterpret_cast<const double2 *>(TFc + ((size_t)ch.mat * a.K + code) * W);
                         double x = 0.0;
 #pragma unroll
-                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(tf + nb); x = fma(v.x, fe[r][2 * nb], x); x = fma(v.y, fe[r][2 * nb + 1], x); }
+                        for (int nb = 0; nb < NB; nb++) { const double2 v = __ldg(tf + nb); x = fma(v.x, fe[2 * nb], x); x = fma(v.y, fe[2 * nb + 1], x); }
                         emit(x, ch.edge, kfe);
                     } else {
                         contract_and_push(fe, kfe, ch.edge, false);
@@ -922,32 +854,30 @@ cudaError_t dm_tip_table(const double *M, const double *defs, const unsigned cha
     return cudaGetLastError();
 }
 
-template <int NB, int SG>
+template <int NB>
 static cudaError_t dm_launch_t(const DmArgs &a, int grid, bool outside, cudaStream_t st)
 {
-    constexpr int NW = DM_GROUPS / SG;
+    constexpr int NW = DM_GROUPS;
     const size_t smem = dm_smem_bytes(NB, a.R, a.nrows, a.nops, a.nchildren);
     cudaError_t r;
     if (outside) {
-        r = cudaFuncSetAttribute(dm_outside_kernel<NB, NW, SG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        r = cudaFuncSetAttribute(dm_outside_kernel<NB, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (r != cudaSuccess) return r;
-        dm_outside_kernel<NB, NW, SG><<<grid, NW * 32, smem, st>>>(a);
+        dm_outside_kernel<NB, NW><<<grid, NW * 32, smem, st>>>(a);
     } else {
-        r = cudaFuncSetAttribute(dm_inside_kernel<NB, NW, SG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        r = cudaFuncSetAttribute(dm_inside_kernel<NB, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (r != cudaSuccess) return r;
-        dm_inside_kernel<NB, NW, SG><<<grid, NW * 32, smem, st>>>(a);
+        dm_inside_kernel<NB, NW><<<grid, NW * 32, smem, st>>>(a);
     }
     return cudaGetLastError();
 }
 
 static cudaError_t dm_launch(const DmArgs &a, int NB, int grid, bool outside, cudaStream_t st)
 {
-    /* a.sg: site groups per warp.  Only 1 (16 warps of 8 sites) is instantiated: with 2 (8 warps of 16 sites, every B
-     * fragment feeding two site groups) the shared-memory traffic halves but the kernel is no faster (measured). */
-    switch (NB * 10 + a.sg) {
-    case 31: return dm_launch_t<3, 1>(a, grid, outside, st);
-    case 41: return dm_launch_t<4, 1>(a, grid, outside, st);
-    case 81: return dm_launch_t<8, 1>(a, grid, outside, st);
+    switch (NB) {
+    case 3: return dm_launch_t<3>(a, grid, outside, st);
+    case 4: return dm_launch_t<4>(a, grid, outside, st);
+    case 8: return dm_launch_t<8>(a, grid, outside, st);
     default: return cudaErrorInvalidValue;
     }
 }

@@ -13,7 +13,7 @@
 #include "f4prog.h"
 
 #define DM_MAX_R 8        /* slots of the matrix ring */
-#define DM_GROUPS 16      /* 8-site groups per full tile (16 warps of one group or 8 warps of two) */
+#define DM_GROUPS 16      /* 8-site groups per full tile, one warp each */
 #define DM_TILE (8 * DM_GROUPS)
 
 struct DmArgs {
@@ -38,8 +38,6 @@ struct DmArgs {
     int ntiles;                      /* tiles of the chunk: tiles_full of DM_GROUPS 8-site groups, the rest of tail_gs groups */
     int tiles_full, tail_gs;
     int R;                           /* ring slots in use (2..DM_MAX_R) */
-    int sg;                          /* site groups per warp (1) */
-    int stagger;                     /* clocks between the start of successive warps of a scheduler */
     int stack_depth;                 /* entries of the per-warp stacks */
     double2 *stack;                  /* inside: [ctas][groups][depth][NB][32]; outside: [ctas][groups][depth][2][NB][32] */
     int *stack_meta;                 /* inside: [ctas][groups][depth][32];     outside: [ctas][groups][depth][32][4] */

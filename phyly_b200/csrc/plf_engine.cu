@@ -200,13 +200,8 @@ struct plf_engine {
 
 /* input of PLF_CODES_PACKED4: two codes per byte, node 2j in the low nibble of byte j, rows of (N + 1) / 2 bytes */
 struct Packed4 { unsigned char b; };
-template <typename TIn> __device__ __forceinline__ int load_code(const TIn *in, int64_t s, int nd, int N) { return (int)in[(size_t)s * N + nd]; }
-template <> __device__ __forceinline__ int load_code<Packed4>(const Packed4 *in, int64_t s, int nd, int N)
-{
-    return (in[(size_t)s * ((N + 1) >> 1) + (nd >> 1)].b >> ((nd & 1) * 4)) & 15;
-}
 
-/* codes_in[S][N] (1 or 4 bytes, or packed nibbles) -> codes[N][S] (1 or 4 bytes); also flags nodes that carry data */
+/* codes_in[S][N] (4 bytes) -> codes[N][S] (1 or 4 bytes); also flags nodes that carry data */
 template <typename TIn, typename TOut>
 __global__ void transpose_codes_kernel(const TIn *in, TOut *out, int64_t s_begin, int64_t s_end, int64_t S, int N,
                                        const unsigned char *def_ones, int *node_flags, int K, int *bad_code)
@@ -217,7 +212,7 @@ __global__ void transpose_codes_kernel(const TIn *in, TOut *out, int64_t s_begin
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {
         int64_t s = s0 + r;
         int nd = n0 + threadIdx.x;
-        tile[r][threadIdx.x] = (s < s_end && nd < N) ? load_code<TIn>(in, s, nd, N) : -1;
+        tile[r][threadIdx.x] = (s < s_end && nd < N) ? (int)in[(size_t)s * N + nd] : -1;
     }
     __syncthreads();
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {
@@ -934,7 +929,7 @@ static int launch_transpose(plf_engine *e, int64_t s0, int64_t s1, int in_bytes)
     int *flags = e->d_err.as<int>() + 4;
     int *bad = e->d_err.as<int>() + 1;          /* set when a code is not a row of the definition table */
     dim3 blk(32, 8), grid((unsigned)((s1 - s0 + 31) / 32), (unsigned)((N + 31) / 32));
-    if ((in_bytes == PLF_CODES_PACKED4 || in_bytes == 1) && !getenv("PLF_OLD_TRANSPOSE")) {
+    if (in_bytes == PLF_CODES_PACKED4 || in_bytes == 1) {
         /* rows of 128 sites through shared memory; the row pitch is an odd number of words (conflict-free columns) */
         const int nt = std::min(N, TR_NODES);
         const int pad_words = ((nt + 3) / 4) | 1;
@@ -946,13 +941,7 @@ static int launch_transpose(plf_engine *e, int64_t s0, int64_t s1, int in_bytes)
         else
             transpose_codes_rows_kernel<Packed4><<<g, 256, smem, e->stream>>>(
                 e->d_codes_in.as<Packed4>(), e->d_codes.as<unsigned char>(), s0, s1, S, N, e->d_def_ones.as<unsigned char>(), flags, e->K, bad, pad_words);
-    } else if (in_bytes == PLF_CODES_PACKED4)
-        transpose_codes_kernel<Packed4, unsigned char><<<grid, blk, 0, e->stream>>>(
-            e->d_codes_in.as<Packed4>(), e->d_codes.as<unsigned char>(), s0, s1, S, N, e->d_def_ones.as<unsigned char>(), flags, e->K, bad);
-    else if (in_bytes == 1)
-        transpose_codes_kernel<unsigned char, unsigned char><<<grid, blk, 0, e->stream>>>(
-            e->d_codes_in.as<unsigned char>(), e->d_codes.as<unsigned char>(), s0, s1, S, N, e->d_def_ones.as<unsigned char>(), flags, e->K, bad);
-    else if (e->code_bytes == 1)
+    } else if (e->code_bytes == 1)
         transpose_codes_kernel<int, unsigned char><<<grid, blk, 0, e->stream>>>(
             e->d_codes_in.as<int>(), e->d_codes.as<unsigned char>(), s0, s1, S, N, e->d_def_ones.as<unsigned char>(), flags, e->K, bad);
     else
@@ -1147,12 +1136,6 @@ struct Query {
     bool want_gmat = false;
     double *dwell_out = nullptr, *trans_out = nullptr;  /* [E][n][n] */
 };
-
-static bool fused_applicable(const plf_engine *e)
-{
-    /* more than 4 rate categories (Gamma4+I, Gamma8 ...) run as windows of <= 4 (run_fused_windows) */
-    return e->n == 4 && e->C <= 16 && e->code_bytes == 1 && e->K <= 256 && e->max_degree <= F4_MAXD;
-}
 
 static int ensure_program(plf_engine *e)
 {
@@ -1468,7 +1451,7 @@ static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool 
         slot->cands = std::move(viable);
     }
     const std::vector<Cand> &viable = slot->cands;
-    const bool can_tune = viable.size() > 1 && e->S >= f4_tune_sites(e) / 2 && !getenv("PLF_F4_NOTUNE");
+    const bool can_tune = viable.size() > 1 && e->S >= f4_tune_sites(e) / 2;
     pick = 0; tune = false;
     if (can_tune && slot->tuned_version == e->program_version && slot->tuned_C == e->C && slot->tuned_K == e->K &&
         slot->tuned_pick < viable.size())
@@ -1818,13 +1801,13 @@ __global__ void f4_combine_windows_kernel(int nwin, int64_t S, double *w_ll /*[n
  * per-site outputs -- and combined per site.  The site likelihood is a sum over categories, L = sum_w L_w, and every
  * per-site output a likelihood-weighted mean, x = sum_w x_w L_w / L, so the combination is exact up to rounding.
  */
-static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
+static int run_fused_windows(plf_engine *e, Query &q)
 {
+    const int wsize = 4;
     const int Ctot = e->C, nwin = (Ctot + wsize - 1) / wsize, E = e->E, N = e->N;
     const int64_t S = e->S;
     const bool marg = q.want_marg, edge = q.want_edge && !marg;
     if (nwin > 16) FAIL(e, "more than 16 category windows");
-    if (resolve_pending(e)) return -1;
     if (prepare_sums(e, 2 + E + (size_t)N * 4)) return -1;
     ENSURE(e, e->f4w_ll, sizeof(double) * (size_t)nwin * S);
     if (edge) ENSURE(e, e->f4w_edge, sizeof(double) * (size_t)nwin * E * S);
@@ -1877,7 +1860,7 @@ static int run_fused_windows(plf_engine *e, Query &q, int wsize = 4)
 static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
 {
     const int n = e->n, C = e->C, N = e->N, E = e->E;
-    if (e->K <= 4096 && !getenv("PLF_NO_TIPTABLE")) {
+    if (e->K <= 4096) {
         /* tip tables (P_e def_k) so that tip children need no GEMM */
         if (ensure_program(e)) return -1;
         const int Et = (int)e->edge_of_tip.size();
@@ -1971,13 +1954,12 @@ static int upload_hess_tree(plf_engine *e, HessTree &ht)
     return 0;
 }
 
-static int run_generic(plf_engine *e, Query &q)
+/* use_tile: 16 < n <= 64 (amino-acid, codon), inside pass on the FP64 tensor pipe (tile.cuh) */
+static int run_generic(plf_engine *e, Query &q, bool use_tile)
 {
     const int n = e->n, C = e->C, N = e->N, E = e->E;
     const bool gm = q.want_gmat;        /* plf_edge_expect_all: generic kernels only (generic_gmat_kernel) */
     const bool outside = q.want_edge || q.want_marg || gm;
-    /* 16 < n <= 64 (amino-acid, codon): inside pass on the FP64 tensor pipe (tile.cuh) */
-    const bool use_tile = n > 16 && n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess && !gm;
     e->last_kernel = use_tile ? "tile_inside_kernel / tile_outside_kernel" : "generic_inside_kernel / generic_outside_kernel";
     const size_t ngm = gm ? (size_t)C * E * n * n : 0;     /* G[C][E][n][n] follows sum_ll */
     const size_t nsum_all = 1 + std::max((size_t)E + (size_t)N * n, ngm);
@@ -2042,7 +2024,7 @@ static int run_generic(plf_engine *e, Query &q)
     const double *w = e->have_w ? e->d_site_w.as<double>() : nullptr;
     if (use_tile && prepare_tile(e, q, a)) return -1;
     /* padded state count of the tile kernels: 32 for amino-acid-sized models, 64 for codon-sized ones */
-    const int tnp = (n <= 32 && !getenv("PLF_TILE_NP64")) ? 32 : 64, tnw = tnp / 8;
+    const int tnp = n <= 32 ? 32 : 64, tnw = tnp / 8;
     const size_t smem_tile = sizeof(double) * (2 * tnp * TL_LS + tnw * TL_TS + TL_TS) + sizeof(int) * 2 * TL_TS +
                              (a.tip_stage ? (size_t)a.Et * TL_TS : 0) + 16;
     const size_t smem_tile_out = sizeof(double) * (tnp * TL_LS + tnw * TL_TS + 3 * TL_TS) + sizeof(int) * 6 * TL_TS;
@@ -2162,15 +2144,6 @@ static int run_generic(plf_engine *e, Query &q)
     return (read_back(e, q, dsum, nsum, hs, herr) || unpack_sums(e, q, hs, herr)) ? -1 : 0;
 }
 
-/*
- * 16 < n <= 64 (amino-acid, codon models), ll and edge-form queries: the FP64 tensor-pipe kernels of dmma.cu.
- * Marginals of such models stay on the tile / generic kernels.
- */
-static bool dmma_applicable(const plf_engine *e, const Query &q)
-{
-    return dm_blocks_for(e->n) != 0 && !q.want_marg && e->code_bytes == 1 && e->K <= 256 && !getenv("PLF_NO_DMMA");
-}
-
 static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_rowsum)
 {
     if (ensure_program(e)) return -1;
@@ -2246,6 +2219,7 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
     return 0;
 }
 
+/* 16 < n <= 64 (amino-acid, codon models), ll and edge-form queries: the FP64 tensor-pipe kernels of dmma.cu */
 static int run_dmma(plf_engine *e, Query &q)
 {
     const int n = e->n, C = e->C, E = e->E;
@@ -2257,7 +2231,6 @@ static int run_dmma(plf_engine *e, Query &q)
     /* ring slots that fit beside the warps' code tiles */
     const int nops = (int)e->ops.size(), nch = (int)e->children.size();
     int R = 3;      /* measured (2..6): 3 is best by 1-3 %; shared memory not used by the ring is L1 for the tip tables and the slab */
-    if (const char *s = getenv("PLF_DM_R")) R = std::max(2, std::min(DM_MAX_R, atoi(s)));
     while (R > 2 && dm_smem_bytes(NB, R, nrows, nops, nch) > 227 * 1024) R--;
     if (dm_smem_bytes(NB, R, nrows, nops, nch) > 227 * 1024) FAIL(e, "tree too large for the tensor-pipe kernels (%d code rows)", nrows);
 
@@ -2276,7 +2249,6 @@ static int run_dmma(plf_engine *e, Query &q)
         Sc = std::min<int64_t>(e->S, groups * 8 / DM_TILE * DM_TILE);
     }
     Sc = std::min<int64_t>(Sc, (int64_t)1 << 24);
-    if (const char *s = getenv("PLF_DM_CHUNK")) Sc = std::min<int64_t>(Sc, std::max<int64_t>(DM_TILE, atoll(s) / DM_TILE * DM_TILE));
     const int64_t ngroups_max = (Sc + 7) / 8;
 
     const int grid_max = e->sm_count;
@@ -2306,9 +2278,6 @@ static int run_dmma(plf_engine *e, Query &q)
     a.root_const_ok = (e->root_mode == PLF_ROOT_UNIFORM || e->root_mode == PLF_ROOT_EQUILIBRIUM) ? 1 : 0;
     a.cat_lh = e->g_cat_lh.as<double>(); a.cat_k = e->g_cat_k.as<int>();
     a.R = R;
-    a.sg = 1;
-    a.stagger = 0;          /* measured 0..8000 clocks: no effect on either kernel */
-    if (const char *sg = getenv("PLF_DM_STAGGER")) a.stagger = atoi(sg);
     a.stack = e->d_dm_stack.as<double2>(); a.stack_meta = e->d_dm_stackmeta.as<int>();
     a.Of = e->d_dm_Of.as<double>(); a.TFf = e->d_dmTFf.as<double>();
     a.cat_prior = e->d_cat_prior.as<double>();
@@ -2379,6 +2348,37 @@ static int run_dmma(plf_engine *e, Query &q)
     return (read_back(e, q, dsum, nsum, hs, herr) || unpack_sums(e, q, hs, herr)) ? -1 : 0;
 }
 
+enum class QueryPath { fused, fused_windows, dmma, tile, generic };
+
+/* The kernels a query runs.  An upload in flight is resolved here, before the tree program is built, unless the query
+ * takes the single-window fused path: only run_fused overlaps an upload, and it repeats the query when the upload
+ * changes which nodes carry data. */
+static int choose_path(plf_engine *e, const Query &q, QueryPath &path)
+{
+    const bool generic_only = e->path == PLF_PATH_GENERIC;
+    /* the edge matrices need the whole site likelihood: no category windows (n = 4 with C > 4 goes to the generic
+     * path); per-site marginals of a huge alignment: the generic path works in chunks of sites */
+    bool fused = e->n == 4 && e->C <= 16 && e->code_bytes == 1 && e->K <= 256 && e->max_degree <= F4_MAXD && !generic_only &&
+                 !q.sum_hess && !(q.want_gmat && e->C > 4) &&
+                 !(q.want_marg && q.site_marg && (size_t)e->N * 4 * e->S * sizeof(double) > ((size_t)32 << 30));
+    const bool windows = e->C > 4 && !q.want_gmat;
+    const bool overlap = fused && !windows && e->node_has_data_h.size() == (size_t)e->N;
+    if (!overlap && resolve_pending(e)) return -1;
+    if (fused) {
+        if (ensure_program(e)) return -1;
+        fused = fused_fits(e, q.want_edge || q.want_marg || q.want_gmat);
+    }
+    if (!fused && resolve_pending(e)) return -1;
+    if (e->path == PLF_PATH_FUSED4 && !fused) FAIL(e, "the fused 4-state path does not apply to this query");
+    if (fused) path = windows ? QueryPath::fused_windows : QueryPath::fused;
+    else if (!generic_only && !q.sum_hess && !q.want_gmat && !q.want_marg && dm_blocks_for(e->n) != 0 && e->code_bytes == 1 &&
+             e->K <= 256)
+        path = QueryPath::dmma;
+    else if (e->n > 16 && e->n <= TL_NP && !getenv("PLF_NO_TILE") && !q.sum_hess && !q.want_gmat) path = QueryPath::tile;
+    else path = QueryPath::generic;
+    return 0;
+}
+
 /* common driver: matrices, path selection, timing.  Returns 1 when the query has to be repeated. */
 static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_hi, const double *l_lo, int kind)
 {
@@ -2388,19 +2388,9 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
         ENSURE(e, e->d_mask, e->E);
         CK(e, cudaMemcpyAsync(e->d_mask.p, q.edge_mask_h, e->E, cudaMemcpyHostToDevice, e->stream));
     }
-    /* the edge matrices need the whole site likelihood: no category windows (n = 4 with C > 4 goes to the generic path) */
-    bool use_fused = fused_applicable(e) && !q.sum_hess && !(q.want_gmat && e->C > 4);
-    /* per-site marginals of a huge alignment: the generic path works in chunks of sites */
-    if (q.want_marg && q.site_marg && (size_t)e->N * 4 * e->S * sizeof(double) > ((size_t)32 << 30)) use_fused = false;
-    if (e->path == PLF_PATH_GENERIC) use_fused = false;
-    /* an upload in flight is overlapped with the fused kernel only; it needs a program built for earlier data */
-    if (e->pend_active && !(use_fused && e->node_has_data_h.size() == (size_t)e->N) && resolve_pending(e)) return -1;
-    if (use_fused) {
-        if (ensure_program(e)) return -1;
-        if (!fused_fits(e, q.want_edge || q.want_marg || q.want_gmat)) use_fused = false;
-    }
-    if (!use_fused && resolve_pending(e)) return -1;
-    if (e->path == PLF_PATH_FUSED4 && !use_fused) FAIL(e, "the fused 4-state path does not apply to this query");
+    QueryPath path;
+    if (choose_path(e, q, path)) return -1;
+    const bool fused = path == QueryPath::fused || path == QueryPath::fused_windows;
     CK(e, cudaEventRecord(e->ev[0], e->stream));
     if (ensure_matrices(e, need_D)) return -1;
     int f_mode = 2;
@@ -2412,19 +2402,17 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
                      q.edge_mask_h ? e->d_mask.as<unsigned char>() : nullptr, e->d_lhi.as<double>(), e->d_llo.as<double>())) return -1;
         q.Fm = e->d_F.as<double>(); q.f_zero_rowsum = 0; f_mode = 2;
     }
-    if (use_fused && ensure_tip_tables(e, q.want_edge ? q.Fm : nullptr, f_mode, q.want_marg)) return -1;
+    if (fused && ensure_tip_tables(e, q.want_edge ? q.Fm : nullptr, f_mode, q.want_marg)) return -1;
     CK(e, cudaEventRecord(e->ev[1], e->stream));
     e->kernel_timed = false;
     e->ms_kernel_override = -1.f;
-    /* PLF_F4_WINDOW=<w> forces windows of w categories (experiments: smaller windows let larger trees use the
-     * constant-memory kernels at the price of per-site outputs and a combination pass) */
-    int wforce = 0;
-    if (const char *wf = getenv("PLF_F4_WINDOW")) wforce = std::max(1, std::min(4, atoi(wf)));
     int rc;
-    if (use_fused && !q.want_gmat && (e->C > 4 || (wforce && wforce < e->C))) rc = run_fused_windows(e, q, wforce ? wforce : 4);
-    else if (use_fused) rc = run_fused(e, q);
-    else if (e->path != PLF_PATH_GENERIC && !q.sum_hess && !q.want_gmat && dmma_applicable(e, q)) rc = run_dmma(e, q);
-    else rc = run_generic(e, q);
+    switch (path) {
+    case QueryPath::fused: rc = run_fused(e, q); break;
+    case QueryPath::fused_windows: rc = run_fused_windows(e, q); break;
+    case QueryPath::dmma: rc = run_dmma(e, q); break;
+    default: rc = run_generic(e, q, path == QueryPath::tile); break;
+    }
     if (rc) return rc;
     cudaEventElapsedTime(&e->ms_mat, e->ev[0], e->ev[1]);
     cudaEventElapsedTime(&e->ms_sites, e->ev[1], e->ev[2]);

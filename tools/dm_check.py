@@ -59,8 +59,7 @@ def compare(name, eng):
 if __name__ == "__main__":
     Q, pi = _codon_model()
     worst = 0.0
-    for sgv in (("1",) if len(sys.argv) <= 3 else ()):
-        os.environ["PLF_DM_SG"] = sgv
+    if len(sys.argv) <= 3:
         eng, s, N = make(61, Q, 16, 300, 21)
         worst = max(worst, compare("codon 16x300", eng)); eng.close()
         eng, s, N = make(61, Q, 70, 1037, 31)
@@ -83,7 +82,6 @@ if __name__ == "__main__":
         eng, s, N = make(30, Qb, 33, 555, 6, mixture={"rates": [0.2, 1.0, 2.5], "prior": [0.3, 0.4, 0.3]})
         worst = max(worst, compare("n=30 33x555 C=3", eng)); eng.close()
         print(json.dumps({"worst": worst}), flush=True)
-    os.environ.pop("PLF_DM_SG", None)
     taxa = int(sys.argv[1]) if len(sys.argv) > 1 else 256
     S = int(sys.argv[2]) if len(sys.argv) > 2 else 100000
     eng, s, N = make(61, Q, taxa, S, 21, missing=0.0, rate=0.05)
@@ -107,21 +105,6 @@ if __name__ == "__main__":
     print(json.dumps({"what": "cfg4 ll+deriv", "ms_matrices": ms_mat, "ms_sites": ms_sites, "ms_kernels": ms_k,
                       "updates_per_s": S * Eg / (ms_sites * 1e-3), "tflops_gemm_edges": 3 * flops / (ms_k * 1e-3) / 1e12,
                       "sum_ll": r["sum_ll"], "d0": float(r["sum_deriv"][0])}), flush=True)
-    for R, SGv in ((2, 3000), (3, 3000), (4, 3000), (2, 0), (6, 3000)):
-        os.environ["PLF_DM_R"] = str(R)
-        os.environ["PLF_DM_STAGGER"] = str(SGv)
-        t = []
-        for kind in ("ll", "deriv"):
-            for it in range(3):
-                if kind == "ll":
-                    eng.ll(per_site=False)
-                else:
-                    eng.deriv(per_site=False)
-                ms_k = eng.last_kernel_ms()
-            t.append(ms_k)
-        print(json.dumps({"ring_slots": R, "stagger": SGv, "ms_ll": t[0], "ms_ll_deriv": t[1]}), flush=True)
-    del os.environ["PLF_DM_R"]
-    del os.environ["PLF_DM_STAGGER"]
     eng.set_path(E.PATH_GENERIC)
     if S <= 20000:
         g = eng.deriv(per_site=False)
