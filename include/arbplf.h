@@ -41,6 +41,8 @@ char *arbplf_em_update(const char *json_in, int *retcode);
 
 /* arbplf-ll answered with an enclosure {"lower": table, "upper": table} (certified mode, directed rounding) */
 char *arbplf_ll_certified(const char *json_in, int *retcode);
+/* arbplf-deriv answered the same way (both tables in the format of arbplf-deriv) */
+char *arbplf_deriv_certified(const char *json_in, int *retcode);
 
 char *arbplf_hess(const char *json_in, int *retcode);
 char *arbplf_inv_hess(const char *json_in, int *retcode);

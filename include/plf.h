@@ -150,6 +150,22 @@ int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q, double *s
                      double *sum_lo, double *sum_hi);
 
 /*
+ * Certified mode for plf_deriv: site_lo[s][e] <= d log L_s / d edge_rate_e <= site_hi[s][e] (csr edge order) for the
+ * edges with edge_mask[idx] != 0 (NULL = all); unrequested edges are 0 in both bounds.  sum_lo / sum_hi [E] enclose
+ * sum_s w_s d[s][e]; they are summed on the device in a fixed order (the same bits on every call), a negative weight
+ * swapping the bounds it multiplies.  Any output may be NULL.  The input uncertainties are those of plf_ll_certified.
+ * Rate matrix derivatives r_c Q P_e come from R = P - 1 P_0 (R 1 = 0, so Q P = Q R and R(y)^2 = R(2y)): R is enclosed
+ * where the scaled Taylor series is, then squared, so a long branch keeps its relative width (csrc/certified.cuh).
+ * Certified: the bounds contain the exact derivative of the model given to the engine within those uncertainties.
+ * Not certified: the host's inputs beyond them; and after plf_comm_init the sums cover this engine's sites only (no
+ * directed-rounding all-reduce).  A site of non-zero weight whose likelihood enclosure reaches 0 makes the sums an
+ * error ("a site with non-zero weight has zero likelihood"); its per-site bounds are -inf / +inf.  At most 75 states
+ * ("state count ... is too large for the certified kernels" otherwise).
+ */
+int plf_deriv_certified(plf_engine *e, double delta_rate, double delta_q, const unsigned char *edge_mask /*[E] or NULL*/,
+                        double *site_lo /*[S][E]*/, double *site_hi /*[S][E]*/, double *sum_lo /*[E]*/, double *sum_hi /*[E]*/);
+
+/*
  * Second order (arbplfhess.c:502-829): sum_ll = sum_s w_s log L_s, sum_deriv[E] its gradient and sum_hess[E][E] its
  * Hessian with respect to the edge rate coefficients (csr edge order, full symmetric matrix).  sum_ll and sum_deriv
  * may be NULL.  A rate category with a non-zero rate and zero likelihood at a weighted site is an error

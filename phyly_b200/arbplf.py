@@ -51,10 +51,12 @@ for _n in _NAMES:
 arbplf_model_summary = _bind("model_summary")
 # certified mode (not in the reference module, whose every output is certified): arbplf-ll answered with an enclosure
 arbplf_ll_certified = _bind("ll_certified")
+# and arbplf-deriv, whose derivative bounds certify their sign
+arbplf_deriv_certified = _bind("deriv_certified")
 
 
 def set_device(device):
     _lib.load().arbplf_set_device(int(device))
 
 
-__all__ = ["arbplf_" + n for n in _NAMES] + ["arbplf_model_summary", "arbplf_ll_certified", "set_device"]
+__all__ = ["arbplf_" + n for n in _NAMES] + ["arbplf_model_summary", "arbplf_ll_certified", "arbplf_deriv_certified", "set_device"]

@@ -15,13 +15,22 @@
  * exp(x Q) = (e^{-beta} exp(B))^(2^s), beta = mu / 2^s <= 1.  The Taylor polynomial of degree K of exp(B) with all
  * operations rounded down is a lower bound; rounded up and increased by the bound beta^(K+1)/(K+1)!/(1 - beta/(K+2)) of
  * the remainder (B has row sums beta) it is an upper bound; squaring keeps both (non-negative matrices).
+ *
+ * Derivatives (plf_deriv_certified) are signed: d L_c / d t_e = r_c fe^T Q P_e L_b.  Q P is not formed from [Plo, Phi],
+ * whose width on a long branch is as large as Q P itself.  With R(y) = P(y) - 1 P_0(y) (row 0 subtracted from every
+ * row; R 1 = 0), R(y)^2 = R(2y) and Q P = Q R, so R is enclosed at the scaled level y = x / 2^s, where its entries are
+ * O(beta) and not O(e^{-lambda x}), squared s times in signed interval arithmetic (cert_imul), and D = r_c Q R(x).
+ * cert_outside_kernel restates generic_outside_kernel on non-negative intervals (one exponent for both bounds, as in
+ * cert_inside_kernel); only the edge form fe^T D L_b is signed.  cert_deriv_site_kernel sums the categories and
+ * divides by the site likelihood enclosure of cert_site_kernel.
  */
 #pragma once
 #include <stdint.h>
 #include "plf_consts.h"
 
-#define CERT_TS 64          /* sites per CTA in cert_inside_kernel */
+#define CERT_TS 64          /* sites per CTA in cert_inside_kernel and cert_outside_kernel */
 #define CERT_TAYLOR 26
+#define CERT_GROUP 1024     /* sites per partial sum of plf_deriv_certified: chunks are multiples of it */
 
 __device__ __forceinline__ double cert_down(double x, int ulps)
 {
@@ -34,10 +43,88 @@ __device__ __forceinline__ double cert_up(double x, int ulps)
     return x;
 }
 
-/* one CTA per (edge, category); ws: 8 n^2 doubles per CTA */
+/* [lo, hi] = [alo, ahi] * [blo, bhi], signs arbitrary */
+__device__ __forceinline__ void cert_imul(double alo, double ahi, double blo, double bhi, double &lo, double &hi)
+{
+    lo = fmin(fmin(__dmul_rd(alo, blo), __dmul_rd(alo, bhi)), fmin(__dmul_rd(ahi, blo), __dmul_rd(ahi, bhi)));
+    hi = fmax(fmax(__dmul_ru(alo, blo), __dmul_ru(alo, bhi)), fmax(__dmul_ru(ahi, blo), __dmul_ru(ahi, bhi)));
+}
+
+/* [lo, hi] = [alo, ahi] * [blo, bhi] with blo >= 0 */
+__device__ __forceinline__ void cert_mul_pos(double alo, double ahi, double blo, double bhi, double &lo, double &hi)
+{
+    lo = __dmul_rd(alo, alo >= 0.0 ? blo : bhi);
+    hi = __dmul_ru(ahi, ahi >= 0.0 ? bhi : blo);
+}
+
+/*
+ * D = r Q R(x) from R at the scaled level (in Rlo / Rhi, s squarings to go); W: 2 n^2 doubles of workspace.  Q is the
+ * interval matrix of cert_expm_kernel without the factor x: off the diagonal the enclosure of q_ij, on it minus the sum
+ * of that row's enclosures.  r = 0 gives D = 0 exactly.
+ */
+__device__ void cert_deriv_matrix(int n, int s, double r, double delta_rate, double delta_q, const double *q_hi, const double *q_lo,
+                                  double *Rlo, double *Rhi, double *Wlo, double *Whi, double *Dlo, double *Dhi)
+{
+    const int nn = n * n;
+    if (r == 0.0) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { Dlo[idx] = 0.0; Dhi[idx] = 0.0; }
+        return;
+    }
+    for (int q = 0; q < s; q++) {
+        __syncthreads();
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const int i = idx / n, j = idx - i * n;
+            double lo = 0.0, hi = 0.0;
+            for (int m = 0; m < n; m++) {
+                double pl, ph;
+                cert_imul(Rlo[i * n + m], Rhi[i * n + m], Rlo[m * n + j], Rhi[m * n + j], pl, ph);
+                lo = __dadd_rd(lo, pl); hi = __dadd_ru(hi, ph);
+            }
+            Wlo[idx] = lo; Whi[idx] = hi;
+        }
+        __syncthreads();
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { Rlo[idx] = Wlo[idx]; Rhi[idx] = Whi[idx]; }
+    }
+    __syncthreads();
+    /* the enclosure of Q into W */
+    for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+        const int i = idx / n, j = idx - i * n;
+        if (i != j) {
+            const double qd = __dadd_rd(q_hi[idx], q_lo ? q_lo[idx] : 0.0), qu = __dadd_ru(q_hi[idx], q_lo ? q_lo[idx] : 0.0);
+            Wlo[idx] = fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q)));
+            Whi[idx] = __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q));
+        } else {
+            double rlo = 0.0, rhi = 0.0;
+            for (int k = 0; k < n; k++) {
+                if (k == i) continue;
+                const double qd = __dadd_rd(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0), qu = __dadd_ru(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0);
+                rlo = __dadd_rd(rlo, fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q))));
+                rhi = __dadd_ru(rhi, __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q)));
+            }
+            Wlo[idx] = -rhi; Whi[idx] = -rlo;
+        }
+    }
+    __syncthreads();
+    const double rl = __dmul_rd(r, __dsub_rd(1.0, delta_rate)), rh = __dmul_ru(r, __dadd_ru(1.0, delta_rate));
+    for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+        const int i = idx / n, j = idx - i * n;
+        double lo = 0.0, hi = 0.0;
+        for (int m = 0; m < n; m++) {
+            double pl, ph;
+            cert_imul(Wlo[i * n + m], Whi[i * n + m], Rlo[m * n + j], Rhi[m * n + j], pl, ph);
+            lo = __dadd_rd(lo, pl); hi = __dadd_ru(hi, ph);
+        }
+        double dl, dh;
+        cert_mul_pos(lo, hi, rl, rh, dl, dh);
+        Dlo[idx] = dl; Dhi[idx] = dh;
+    }
+}
+
+/* one CTA per (edge, category); ws: 8 n^2 doubles per CTA.  Dlo / Dhi (or NULL): enclosure of r_c Q P_e as well. */
 __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, const double *q_hi, const double *q_lo,
                                                         const double *edge_rate, const double *cat_rate, double delta_rate,
-                                                        double delta_q, double *ws, double *Plo, double *Phi)
+                                                        double delta_q, double *ws, double *Plo, double *Phi,
+                                                        double *Dlo, double *Dhi)
 {
     const int e = blockIdx.x, c = blockIdx.y, nn = n * n;
     double *base = ws + ((size_t)c * E + e) * 8 * nn;
@@ -69,6 +156,15 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
     const int s = sh_s;
     if (!(mu > 0.0)) {          /* zero rate or zero length: the identity, exactly */
         for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { const double v = (idx / n == idx % n) ? 1.0 : 0.0; outlo[idx] = v; outhi[idx] = v; }
+        if (!Dlo) return;
+        /* R = I - 1 e_0^T, exactly */
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const int i = idx / n, j = idx - i * n;
+            const double v = (i == j ? 1.0 : 0.0) - (j == 0 ? 1.0 : 0.0);
+            Blo[idx] = v; Bhi[idx] = v;
+        }
+        cert_deriv_matrix(n, 0, r, delta_rate, delta_q, q_hi, q_lo, Blo, Bhi, Tlo, Thi,
+                          Dlo + ((size_t)c * E + e) * nn, Dhi + ((size_t)c * E + e) * nn);
         return;
     }
     const double sc = scalbn(1.0, -s);
@@ -125,6 +221,14 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
         Shi[idx] = __dmul_ru(__dadd_ru(Shi[idx], rem), ehi);
     }
     __syncthreads();
+    if (Dlo) {
+        /* R(y) = P(y) - 1 P_0(y) at the scaled level into B (free after the Taylor stage); row 0 is exactly 0 */
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const int i = idx / n, j = idx - i * n;
+            Blo[idx] = i == 0 ? 0.0 : __dsub_rd(Slo[idx], Shi[j]);
+            Bhi[idx] = i == 0 ? 0.0 : __dsub_ru(Shi[idx], Slo[j]);
+        }
+    }
     for (int q = 0; q < s; q++) {
         for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
             const int i = idx / n, j = idx - i * n;
@@ -140,6 +244,8 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
         __syncthreads();
     }
     for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { outlo[idx] = fmax(0.0, Slo[idx]); outhi[idx] = fmin(1.0, Shi[idx]); }
+    if (Dlo) cert_deriv_matrix(n, s, r, delta_rate, delta_q, q_hi, q_lo, Blo, Bhi, Tlo, Thi,
+                               Dlo + ((size_t)c * E + e) * nn, Dhi + ((size_t)c * E + e) * nn);
 }
 
 struct CertArgs {
@@ -157,6 +263,16 @@ struct CertArgs {
     int *Kg; unsigned char *Cg;        /* [C][N][Sc] */
     double *cat_lo, *cat_hi; int *cat_k;   /* [C][Sc] */
     double *site_lo, *site_hi;         /* [S] enclosures of the site log-likelihoods */
+    /* plf_deriv_certified only (NULL otherwise) */
+    double *site_mlo, *site_mhi; int *site_k;   /* [Sc] the site likelihood enclosure [mlo, mhi] 2^(256 k) */
+    const double *Dlo, *Dhi;           /* [C][E][n][n] enclosures of r_c Q P_e */
+    const double *cat_rate;            /* [C] */
+    const unsigned char *edge_mask;    /* [E] or NULL */
+    double *Flo, *Fhi; int *FK;        /* [C][N][n][Sc] outside vectors (mantissas), [C][N][Sc] their exponents */
+    double *xlo, *xhi; int *xk;        /* [C][E][Sc] edge forms fe^T D L_b (mantissas), [C][E][Sc] exponents */
+    const double *site_w;              /* [S] or NULL */
+    double *out_lo, *out_hi;           /* [E][Sc] enclosures of d log L_s / d t_e */
+    int *err;                          /* bit 0: a site of non-zero weight whose likelihood enclosure reaches 0 */
 };
 
 /* interval restatement of generic_inside_kernel: thread = (site, category), blockIdx.y = category */
@@ -276,4 +392,227 @@ __global__ void cert_site_kernel(CertArgs a)
     lhi = __dadd_ru(lhi, __dmul_ru(kd, k0 <= 0 ? c_lo : c_hi));
     a.site_lo[a.s0 + s] = llo;
     a.site_hi[a.s0 + s] = lhi;
+    if (a.site_mlo) { a.site_mlo[s] = lo; a.site_mhi[s] = hi; a.site_k[s] = k0; }
+}
+
+/* x 2^(256 k), any sign and any k, rounded down (down = 1) or up; exact whenever the result is representable */
+__device__ __forceinline__ double cert_scale_signed(double x, int k, int down)
+{
+    if (x == 0.0 || k == 0) return x;
+    const int kk = max(-16, min(16, k));
+    const double y = scalbn(x, PLF_SCALE_BITS * kk);
+    if (kk == k && isfinite(y) && scalbn(y, -PLF_SCALE_BITS * kk) == x) return y;
+    if (y == 0.0) return (down == (x < 0.0)) ? (down ? -__longlong_as_double(1LL) : __longlong_as_double(1LL)) : 0.0;
+    return down ? cert_down(y, 1) : cert_up(y, 1);
+}
+
+/* rescale a non-negative interval vector (stride CERT_TS) by powers of 2^256 until max(hi) lies in [2^-256, 2^256] */
+__device__ __forceinline__ void cert_rescale(double *lo, double *hi, int n, double mx, int &k)
+{
+    while (mx > 0.0 && mx < PLF_TWO_M256) {            /* exact */
+        for (int i = 0; i < n; i++) { lo[i * CERT_TS] *= PLF_TWO_P256; hi[i * CERT_TS] *= PLF_TWO_P256; }
+        mx *= PLF_TWO_P256; k -= 1;
+    }
+    while (mx > PLF_TWO_P256 && mx < INFINITY) {        /* the low bounds may lose bits: round them down */
+        for (int i = 0; i < n; i++) { lo[i * CERT_TS] = __dmul_rd(lo[i * CERT_TS], PLF_TWO_M256); hi[i * CERT_TS] = __dmul_ru(hi[i * CERT_TS], PLF_TWO_M256); }
+        mx *= PLF_TWO_M256; k += 1;
+    }
+}
+
+/*
+ * Interval restatement of generic_outside_kernel: thread = (site, category), blockIdx.y = category.  Writes the edge
+ * form fe^T D L_b of every requested edge to xlo / xhi / xk.  A category with zero likelihood at the site writes
+ * nothing (cert_deriv_site_kernel skips it); a category of rate 0 and a child whose vector is an exact constant column
+ * (D 1 = 0) give 0 exactly.  The sibling edge vectors P L are recomputed from the inside vectors.
+ */
+__global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
+{
+    extern __shared__ double csm[];
+    const int tid = threadIdx.x;
+    const int s = blockIdx.x * CERT_TS + tid;
+    const int c = blockIdx.y;
+    if (s >= a.Sc) return;
+    const int n = a.n, Sc = a.Sc;
+    const int64_t gs = a.s0 + s;
+    if (!(a.prior_hi[c] * a.cat_hi[(size_t)c * Sc + s] > 0.0)) return;
+    double *tlo = csm + tid, *thi = csm + (size_t)n * CERT_TS + tid;
+    double *flo = csm + (size_t)2 * n * CERT_TS + tid, *fhi = csm + (size_t)3 * n * CERT_TS + tid;
+    double *ylo = csm + (size_t)4 * n * CERT_TS + tid, *yhi = csm + (size_t)5 * n * CERT_TS + tid;
+    const size_t cN = (size_t)c * a.t.N, cE = (size_t)c * a.t.E, nn = (size_t)n * n;
+    const bool zero_rate = a.cat_rate[c] == 0.0;
+    {
+        double *Fl = a.Flo + ((cN + a.t.root) * n) * Sc + s, *Fh = a.Fhi + ((cN + a.t.root) * n) * Sc + s;
+        for (int i = 0; i < n; i++) { Fl[(size_t)i * Sc] = a.root_lo[i]; Fh[(size_t)i * Sc] = a.root_hi[i]; }
+        a.FK[(cN + a.t.root) * Sc + s] = 0;
+    }
+    for (int u = 0; u < a.t.N; u++) {
+        const int nd = a.t.preorder[u];
+        const int start = a.t.indptr[nd], stop = a.t.indptr[nd + 1];
+        if (start == stop) continue;
+        const double *Fl = a.Flo + ((cN + nd) * n) * Sc + s, *Fh = a.Fhi + ((cN + nd) * n) * Sc + s;
+        const int ka = a.FK[(cN + nd) * Sc + s];
+        if (a.t.node_has_data[nd]) {
+            const int code = plf_code_at(a.codes, a.code_bytes, a.S, nd, gs);
+            for (int i = 0; i < n; i++) {
+                const double d = a.defs[(size_t)code * n + i];
+                tlo[i * CERT_TS] = __dmul_rd(Fl[(size_t)i * Sc], d); thi[i * CERT_TS] = __dmul_ru(Fh[(size_t)i * Sc], d);
+            }
+        } else {
+            for (int i = 0; i < n; i++) { tlo[i * CERT_TS] = Fl[(size_t)i * Sc]; thi[i * CERT_TS] = Fh[(size_t)i * Sc]; }
+        }
+        for (int idx = start; idx < stop; idx++) {
+            const int b = a.t.indices[idx];
+            int kfe = ka;
+            for (int i = 0; i < n; i++) { flo[i * CERT_TS] = tlo[i * CERT_TS]; fhi[i * CERT_TS] = thi[i * CERT_TS]; }
+            for (int idx2 = start; idx2 < stop; idx2++) {
+                if (idx2 == idx) continue;
+                const int b2 = a.t.indices[idx2];
+                const double *Lbl = a.Llo + ((cN + b2) * n) * Sc + s, *Lbh = a.Lhi + ((cN + b2) * n) * Sc + s;
+                for (int k = 0; k < n; k++) { ylo[k * CERT_TS] = Lbl[(size_t)k * Sc]; yhi[k * CERT_TS] = Lbh[(size_t)k * Sc]; }
+                const int bc = a.Cg[(cN + b2) * Sc + s];
+                const double *Pl = a.Plo + (cE + idx2) * nn, *Ph = a.Phi + (cE + idx2) * nn;
+                double mx = 0.0;
+                for (int i = 0; i < n; i++) {
+                    double elo, ehi;
+                    if (bc) {
+                        elo = ylo[0]; ehi = yhi[0];
+                    } else {
+                        elo = 0.0; ehi = 0.0;
+                        for (int k = 0; k < n; k++) {
+                            elo = __fma_rd(Pl[i * n + k], ylo[k * CERT_TS], elo);
+                            ehi = __fma_ru(Ph[i * n + k], yhi[k * CERT_TS], ehi);
+                        }
+                    }
+                    const double xl = __dmul_rd(flo[i * CERT_TS], elo), xh = __dmul_ru(fhi[i * CERT_TS], ehi);
+                    flo[i * CERT_TS] = xl; fhi[i * CERT_TS] = xh;
+                    mx = fmax(mx, xh);
+                }
+                kfe += a.Kg[(cN + b2) * Sc + s];
+                cert_rescale(flo, fhi, n, mx, kfe);
+            }
+            const int kb = a.Kg[(cN + b) * Sc + s];
+            if (!a.edge_mask || a.edge_mask[idx]) {
+                /* fe^T (D L_b): first the signed interval vector D L_b, then its product with the non-negative fe */
+                double xl = 0.0, xh = 0.0;
+                if (!zero_rate && !a.Cg[(cN + b) * Sc + s]) {
+                    const double *Lbl = a.Llo + ((cN + b) * n) * Sc + s, *Lbh = a.Lhi + ((cN + b) * n) * Sc + s;
+                    for (int k = 0; k < n; k++) { ylo[k * CERT_TS] = Lbl[(size_t)k * Sc]; yhi[k * CERT_TS] = Lbh[(size_t)k * Sc]; }
+                    const double *Dl = a.Dlo + (cE + idx) * nn, *Dh = a.Dhi + (cE + idx) * nn;
+                    for (int i = 0; i < n; i++) {
+                        double vl = 0.0, vh = 0.0;
+                        for (int k = 0; k < n; k++) {
+                            double pl, ph;
+                            cert_mul_pos(Dl[i * n + k], Dh[i * n + k], ylo[k * CERT_TS], yhi[k * CERT_TS], pl, ph);
+                            vl = __dadd_rd(vl, pl); vh = __dadd_ru(vh, ph);
+                        }
+                        double pl, ph;
+                        cert_mul_pos(vl, vh, flo[i * CERT_TS], fhi[i * CERT_TS], pl, ph);
+                        xl = __dadd_rd(xl, pl); xh = __dadd_ru(xh, ph);
+                    }
+                }
+                a.xlo[(cE + idx) * Sc + s] = xl;
+                a.xhi[(cE + idx) * Sc + s] = xh;
+                a.xk[(cE + idx) * Sc + s] = kfe + kb;
+            }
+            /* outside vector of b: P^T fe (internal children only) */
+            if (a.t.indptr[b] != a.t.indptr[b + 1]) {
+                const double *Pl = a.Plo + (cE + idx) * nn, *Ph = a.Phi + (cE + idx) * nn;
+                double mx = 0.0;
+                for (int j = 0; j < n; j++) {
+                    double lo = 0.0, hi = 0.0;
+                    for (int i = 0; i < n; i++) {
+                        lo = __fma_rd(Pl[i * n + j], flo[i * CERT_TS], lo);
+                        hi = __fma_ru(Ph[i * n + j], fhi[i * CERT_TS], hi);
+                    }
+                    ylo[j * CERT_TS] = lo; yhi[j * CERT_TS] = hi;
+                    mx = fmax(mx, hi);
+                }
+                int kfb = kfe;
+                cert_rescale(ylo, yhi, n, mx, kfb);
+                double *Fbl = a.Flo + ((cN + b) * n) * Sc + s, *Fbh = a.Fhi + ((cN + b) * n) * Sc + s;
+                for (int j = 0; j < n; j++) { Fbl[(size_t)j * Sc] = ylo[j * CERT_TS]; Fbh[(size_t)j * Sc] = yhi[j * CERT_TS]; }
+                a.FK[(cN + b) * Sc + s] = kfb;
+            }
+        }
+    }
+}
+
+/*
+ * Per (site, edge): sum_c prior_c x_c 2^(256 (xk_c - k0)) over the categories of non-zero likelihood, divided by the
+ * site likelihood enclosure [mlo, mhi] 2^(256 k0).  grid (sites / 128, E).  Unrequested edges are 0 exactly; a site
+ * whose likelihood enclosure reaches 0 gets [-inf, +inf] (and bit 0 of err if its weight is not 0).
+ */
+__global__ void cert_deriv_site_kernel(CertArgs a)
+{
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    const int e = blockIdx.y, E = a.t.E;
+    if (s >= a.Sc) return;
+    const int Sc = a.Sc;
+    const double mlo = a.site_mlo[s], mhi = a.site_mhi[s];
+    const int k0 = a.site_k[s];
+    if (e == 0 && !(mlo > 0.0) && (a.site_w ? a.site_w[a.s0 + s] : 1.0) != 0.0) atomicOr(a.err, 1);
+    double lo = 0.0, hi = 0.0;
+    if (!a.edge_mask || a.edge_mask[e]) {
+        if (!(mlo > 0.0)) {
+            lo = -INFINITY; hi = INFINITY;
+        } else {
+            double nlo = 0.0, nhi = 0.0;
+            for (int c = 0; c < a.C; c++) {
+                if (!(a.prior_hi[c] * a.cat_hi[(size_t)c * Sc + s] > 0.0)) continue;
+                const size_t at = ((size_t)c * E + e) * Sc + s;
+                double tl, th;
+                cert_mul_pos(a.xlo[at], a.xhi[at], a.prior_lo[c], a.prior_hi[c], tl, th);
+                const int dk = a.xk[at] - k0;
+                nlo = __dadd_rd(nlo, cert_scale_signed(tl, dk, 1));
+                nhi = __dadd_ru(nhi, cert_scale_signed(th, dk, 0));
+            }
+            lo = __ddiv_rd(nlo, nlo >= 0.0 ? mhi : mlo);
+            hi = __ddiv_ru(nhi, nhi >= 0.0 ? mlo : mhi);
+            if (lo == 0.0) lo = 0.0;            /* no -0.0 */
+            if (hi == 0.0) hi = 0.0;
+        }
+    }
+    a.out_lo[(size_t)e * Sc + s] = lo;
+    a.out_hi[(size_t)e * Sc + s] = hi;
+}
+
+/*
+ * Weighted sums of the enclosures, per group of CERT_GROUP sites and edge, in a fixed order (the same bits on every
+ * call, whatever the chunking): grid (groups of the chunk, E), one warp.  A negative weight swaps the bounds.
+ */
+__global__ void __launch_bounds__(32) cert_deriv_group_sum_kernel(CertArgs a, double *part_lo, double *part_hi)
+{
+    const int g = blockIdx.x, e = blockIdx.y, lane = threadIdx.x, E = a.t.E, Sc = a.Sc;
+    const int s1 = min(Sc, (g + 1) * CERT_GROUP);
+    double lo = 0.0, hi = 0.0;
+    for (int s = g * CERT_GROUP + lane; s < s1; s += 32) {
+        const double w = a.site_w ? a.site_w[a.s0 + s] : 1.0;
+        if (w == 0.0) continue;
+        const double l = a.out_lo[(size_t)e * Sc + s], h = a.out_hi[(size_t)e * Sc + s];
+        lo = __dadd_rd(lo, __dmul_rd(w, w > 0.0 ? l : h));
+        hi = __dadd_ru(hi, __dmul_ru(w, w > 0.0 ? h : l));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lo = __dadd_rd(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = __dadd_ru(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if (lane == 0) {
+        const size_t at = (size_t)(a.s0 / CERT_GROUP + g) * E + e;
+        part_lo[at] = lo; part_hi[at] = hi;
+    }
+}
+
+/* sum_lo[e] / sum_hi[e]: the groups' partial sums in order */
+__global__ void cert_deriv_total_kernel(const double *part_lo, const double *part_hi, int groups, int E, double *sum_lo, double *sum_hi)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= E) return;
+    double lo = 0.0, hi = 0.0;
+    for (int g = 0; g < groups; g++) {
+        lo = __dadd_rd(lo, part_lo[(size_t)g * E + e]);
+        hi = __dadd_ru(hi, part_hi[(size_t)g * E + e]);
+    }
+    sum_lo[e] = lo == 0.0 ? 0.0 : lo;           /* no -0.0 (a rounded-down sum of zeros) */
+    sum_hi[e] = hi == 0.0 ? 0.0 : hi;
 }

@@ -9,6 +9,7 @@
  * reference's outer, precision-agnostic layer: schema validation, selection /
  * aggregation weights and the output table.
  */
+#include <fenv.h>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -720,6 +721,97 @@ char *arbplf_ll_certified(const char *json_in, int *retcode)
 done:
     free(lo); free(hi); free(slo); free(shi); free(t_lo); free(t_hi);
     axis_clear(&ax[0]); reduction_clear(&r_site);
+    return finish(&c, out, rc, retcode);
+}
+
+/* ------------------------------------------------------------------ */
+/* arbplf-deriv, certified mode                                        */
+/* ------------------------------------------------------------------ */
+
+/* [*lo, *hi] += w [xlo, xhi], rounded outwards on the host (a negative weight swaps the bounds it multiplies) */
+static void acc_bounds(double *lo, double *hi, double w, double xlo, double xhi)
+{
+    const int old = fegetround();
+    volatile double t;
+    fesetround(FE_DOWNWARD);
+    t = w * (w >= 0.0 ? xlo : xhi);
+    t = *lo + t;
+    *lo = t;
+    fesetround(FE_UPWARD);
+    t = w * (w >= 0.0 ? xhi : xlo);
+    t = *hi + t;
+    *hi = t;
+    fesetround(old);
+}
+
+/*
+ * The same request as arbplf-deriv, answered with an enclosure: {"lower": <table>, "upper": <table>}, both tables in
+ * the format of arbplf-deriv (plf_deriv_certified).  Site aggregation is the engine's weighted sum; edge aggregation
+ * combines the per-edge bounds here with directed rounding.  As in arbplf-ll-certified the weights are the doubles of
+ * the reduction step (an "avg" weight 1 / count included).
+ */
+char *arbplf_deriv_certified(const char *json_in, int *retcode)
+{
+    static const char *const keys[] = {"model_and_data", "?site_reduction", "?edge_reduction", NULL};
+    const jv *v[3];
+    ctx c;
+    reduction r_site, r_edge; reduction_init(&r_site); reduction_init(&r_edge);
+    axis ax[2]; memset(ax, 0, sizeof ax);
+    double *lo = NULL, *hi = NULL, *blo = NULL, *bhi = NULL;
+    unsigned char *mask = NULL;
+    char *out = NULL, *t_lo = NULL, *t_hi = NULL;
+    int rc = -1;
+    if (ctx_parse(&c, json_in, keys, v)) goto done;
+    const int E = c.m.E;
+    const int64_t S = c.m.S;
+    if (reduction_parse(&r_site, (int)S, "site", v[1])) goto done;
+    if (reduction_parse(&r_edge, E, "edge", v[2])) goto done;
+    if (axis_init(&ax[0], "site", (int)S, &r_site) || axis_init(&ax[1], "edge", E, &r_edge)) goto done;
+    const size_t edge_ext = ax[1].aggregated ? 1 : (size_t)E;
+    {
+        size_t cells = (ax[0].aggregated ? 1 : (size_t)S) * edge_ext;
+        lo = calloc(cells ? cells : 1, sizeof(double));
+        hi = calloc(cells ? cells : 1, sizeof(double));
+    }
+    if (S > 0 && E > 0) {
+        if (ctx_load(&c)) goto done;
+        mask = edge_mask_csr(&c.m, &ax[1]);
+        const double d_rate = 4e-15, d_q = 8.673617379884035e-19;       /* 2^-60 */
+        const int64_t rows = ax[0].aggregated ? 1 : S;
+        blo = malloc(sizeof(double) * (size_t)rows * E);
+        bhi = malloc(sizeof(double) * (size_t)rows * E);
+        int r;
+        if (ax[0].aggregated) r = plf_set_site_weights(c.e, ax[0].w) || plf_deriv_certified(c.e, d_rate, d_q, mask, NULL, NULL, blo, bhi);
+        else r = plf_set_site_weights(c.e, NULL) || plf_deriv_certified(c.e, d_rate, d_q, mask, blo, bhi, NULL, NULL);
+        if (r) { fprintf(stderr, "error: %s\n", plf_last_error(c.e)); goto done; }
+        for (int64_t s = 0; s < rows; s++) {
+            if (!ax[0].aggregated && !ax[0].requested[s]) continue;
+            for (int e = 0; e < E; e++) {
+                if (!ax[1].requested[e]) continue;
+                const double xl = blo[(size_t)s * E + c.m.order[e]], xh = bhi[(size_t)s * E + c.m.order[e]];
+                if (!isfinite(xl) || !isfinite(xh)) {
+                    if (ax[0].aggregated) fprintf(stderr, "error: a requested site has zero likelihood\n");
+                    else fprintf(stderr, "error: site %lld has zero likelihood\n", (long long)s);
+                    goto done;
+                }
+                if (ax[1].aggregated) acc_bounds(&lo[s], &hi[s], ax[1].w[e], xl, xh);
+                else { lo[(size_t)s * edge_ext + e] = xl; hi[(size_t)s * edge_ext + e] = xh; }
+            }
+        }
+    }
+    phase_compute_done(&c);
+    t_lo = table_to_json(ax, 2, lo);
+    t_hi = table_to_json(ax, 2, hi);
+    {
+        jbuf b; jbuf_init(&b);
+        jbuf_puts(&b, "{\"lower\": "); jbuf_puts(&b, t_lo); jbuf_puts(&b, ", \"upper\": "); jbuf_puts(&b, t_hi); jbuf_puts(&b, "}");
+        out = jbuf_take(&b);
+    }
+    rc = 0;
+done:
+    free(lo); free(hi); free(blo); free(bhi); free(mask); free(t_lo); free(t_hi);
+    axis_clear(&ax[0]); axis_clear(&ax[1]);
+    reduction_clear(&r_site); reduction_clear(&r_edge);
     return finish(&c, out, rc, retcode);
 }
 

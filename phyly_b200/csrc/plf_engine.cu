@@ -167,6 +167,7 @@ struct plf_engine {
     DevBuf g_Lg, g_Kg, g_Cg, g_Eg, g_Fg, g_FK, g_cat_lh, g_cat_k, g_site_m, g_site_k, g_edge_out, g_marg_out, g_tr;
     DevBuf h_Yg, h_dFg, h_dFk, h_part, h_gram, h_tree, h_out;
     DevBuf c_Plo, c_Phi, c_ws, c_cat_hi, c_site_lo, c_site_hi, c_small;
+    DevBuf c_Dlo, c_Dhi, c_Flo, c_Fhi, c_FK, c_xlo, c_xhi, c_xk, c_mlo, c_mhi, c_mk, c_olo, c_ohi, c_part, c_sums, c_err;
 
     /* timing / accounting */
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -2529,26 +2530,26 @@ extern "C" int plf_get_frechet_matrices(plf_engine *e, const double *l_hi, const
 static double cert_lo_h(double v, double d) { return v <= 0.0 ? 0.0 : std::nextafter(v * (1.0 - d), -INFINITY); }
 static double cert_hi_h(double v, double d) { return v <= 0.0 ? 0.0 : std::nextafter(v * (1.0 + d), INFINITY); }
 
-extern "C" int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q, double *site_lo, double *site_hi,
-                                double *sum_lo, double *sum_hi)
+/* Enclosures of the transition matrices (and, with D, of r_c Q P_e) on the device, and those of the root weights and
+ * the category priors in c_small = [root_lo | root_hi | prior_lo | prior_hi] (exact when they are the user's own numbers) */
+static int cert_prepare(plf_engine *e, double delta_rate, double delta_q, bool with_D)
 {
-    if (!e) return -1;
-    if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
-    if (!(delta_rate >= 0.0) || !(delta_q >= 0.0) || delta_rate > 1e-3 || delta_q > 1e-3) FAIL(e, "plf_ll_certified: bad input uncertainties");
-    CK(e, cudaSetDevice(e->device));
-    if (resolve_pending(e)) return -1;
-    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    const int n = e->n, C = e->C, E = e->E;
     const size_t nn = (size_t)n * n;
     ENSURE(e, e->c_Plo, sizeof(double) * C * E * nn + 8);
     ENSURE(e, e->c_Phi, sizeof(double) * C * E * nn + 8);
     ENSURE(e, e->c_ws, sizeof(double) * C * E * 8 * nn + 8);
+    if (with_D) {
+        ENSURE(e, e->c_Dlo, sizeof(double) * C * E * nn + 8);
+        ENSURE(e, e->c_Dhi, sizeof(double) * C * E * nn + 8);
+    }
     if (E > 0) {
         cert_expm_kernel<<<dim3(E, C), 128, 0, e->stream>>>(n, E, C, e->d_qhi.as<double>(), e->d_qlo.as<double>(), e->d_edge_rates.as<double>(),
                                                             e->d_cat_rates.as<double>(), delta_rate, delta_q, e->c_ws.as<double>(),
-                                                            e->c_Plo.as<double>(), e->c_Phi.as<double>());
+                                                            e->c_Plo.as<double>(), e->c_Phi.as<double>(),
+                                                            with_D ? e->c_Dlo.as<double>() : nullptr, with_D ? e->c_Dhi.as<double>() : nullptr);
         KCHECK(e);
     }
-    /* enclosures of the root weights and of the category priors (exact when they are the user's own numbers) */
     std::vector<double> small(2 * (size_t)n + 2 * (size_t)C);
     double *rlo = small.data(), *rhi = rlo + n, *plo = rhi + n, *phi = plo + C;
     for (int i = 0; i < n; i++) {
@@ -2561,6 +2562,19 @@ extern "C" int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q
     ENSURE(e, e->c_small, sizeof(double) * small.size());
     CK(e, cudaMemcpyAsync(e->c_small.p, small.data(), sizeof(double) * small.size(), cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+extern "C" int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q, double *site_lo, double *site_hi,
+                                double *sum_lo, double *sum_hi)
+{
+    if (!e) return -1;
+    if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
+    if (!(delta_rate >= 0.0) || !(delta_q >= 0.0) || delta_rate > 1e-3 || delta_q > 1e-3) FAIL(e, "plf_ll_certified: bad input uncertainties");
+    CK(e, cudaSetDevice(e->device));
+    if (resolve_pending(e)) return -1;
+    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    if (cert_prepare(e, delta_rate, delta_q, false)) return -1;
 
     const size_t per_site = (size_t)C * ((size_t)2 * N * n * 8 + (size_t)N * 5 + 24) + 16;
     size_t free_b = 0, total_b = 0;
@@ -2641,6 +2655,123 @@ extern "C" int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q
         if (bad) FAIL(e, "a site with non-zero weight has zero likelihood");
         if (sum_lo) *sum_lo = acc_lo;
         if (sum_hi) *sum_hi = acc_hi;
+    }
+    return 0;
+}
+
+extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delta_q, const unsigned char *edge_mask,
+                                   double *site_lo, double *site_hi, double *sum_lo, double *sum_hi)
+{
+    if (!e) return -1;
+    if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
+    if (!(delta_rate >= 0.0) || !(delta_q >= 0.0) || delta_rate > 1e-3 || delta_q > 1e-3) FAIL(e, "plf_deriv_certified: bad input uncertainties");
+    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    const size_t smem_in = sizeof(double) * 4 * n * CERT_TS, smem_out = sizeof(double) * 6 * n * CERT_TS;
+    if (smem_out > 227 * 1024) FAIL(e, "state count %d is too large for the certified kernels", n);
+    CK(e, cudaSetDevice(e->device));
+    if (resolve_pending(e)) return -1;
+    if (E == 0) return 0;
+    if (cert_prepare(e, delta_rate, delta_q, true)) return -1;
+    ENSURE(e, e->d_mask, (size_t)E);
+    if (edge_mask) CK(e, cudaMemcpyAsync(e->d_mask.p, edge_mask, (size_t)E, cudaMemcpyHostToDevice, e->stream));
+
+    /* inside and outside vectors, edge forms, the site likelihood enclosure and the per-site output of a chunk */
+    const size_t per_site = (size_t)C * ((size_t)4 * N * n * 8 + (size_t)N * 9 + (size_t)E * 20 + 24) + (size_t)E * 16 + 24;
+    size_t free_b = 0, total_b = 0;
+    CK(e, cudaMemGetInfo(&free_b, &total_b));
+    const size_t held = e->g_Lg.cap + e->g_Fg.cap + e->c_Flo.cap + e->c_Fhi.cap + e->c_xlo.cap + e->c_xhi.cap + e->c_olo.cap + e->c_ohi.cap;
+    const size_t budget = std::min<size_t>((size_t)24 << 30, free_b / 2 + held);
+    int64_t Sc = std::max<int64_t>(CERT_GROUP, std::min<int64_t>(e->S, (int64_t)(budget / per_site)));
+    Sc = std::min<int64_t>(Sc, 1 << 20);
+    if (Sc < e->S) Sc = (Sc / CERT_GROUP) * CERT_GROUP;
+    Sc = std::min<int64_t>(Sc, e->S);
+    ENSURE(e, e->g_Lg, sizeof(double) * (size_t)C * N * n * Sc);
+    ENSURE(e, e->g_Fg, sizeof(double) * (size_t)C * N * n * Sc);
+    ENSURE(e, e->g_Kg, sizeof(int) * (size_t)C * N * Sc);
+    ENSURE(e, e->g_Cg, (size_t)C * N * Sc);
+    ENSURE(e, e->g_cat_lh, sizeof(double) * (size_t)C * Sc);
+    ENSURE(e, e->c_cat_hi, sizeof(double) * (size_t)C * Sc);
+    ENSURE(e, e->g_cat_k, sizeof(int) * (size_t)C * Sc);
+    ENSURE(e, e->c_site_lo, sizeof(double) * e->S);
+    ENSURE(e, e->c_site_hi, sizeof(double) * e->S);
+    ENSURE(e, e->c_Flo, sizeof(double) * (size_t)C * N * n * Sc);
+    ENSURE(e, e->c_Fhi, sizeof(double) * (size_t)C * N * n * Sc);
+    ENSURE(e, e->c_FK, sizeof(int) * (size_t)C * N * Sc);
+    ENSURE(e, e->c_xlo, sizeof(double) * (size_t)C * E * Sc);
+    ENSURE(e, e->c_xhi, sizeof(double) * (size_t)C * E * Sc);
+    ENSURE(e, e->c_xk, sizeof(int) * (size_t)C * E * Sc);
+    ENSURE(e, e->c_mlo, sizeof(double) * Sc);
+    ENSURE(e, e->c_mhi, sizeof(double) * Sc);
+    ENSURE(e, e->c_mk, sizeof(int) * Sc);
+    ENSURE(e, e->c_olo, sizeof(double) * (size_t)E * Sc);
+    ENSURE(e, e->c_ohi, sizeof(double) * (size_t)E * Sc);
+    const int64_t groups = (e->S + CERT_GROUP - 1) / CERT_GROUP;
+    ENSURE(e, e->c_part, sizeof(double) * 2 * (size_t)groups * E);
+    ENSURE(e, e->c_sums, sizeof(double) * 2 * (size_t)E);
+    ENSURE(e, e->c_err, sizeof(int));
+    CK(e, cudaMemsetAsync(e->c_err.p, 0, sizeof(int), e->stream));
+
+    CertArgs a;
+    memset(&a, 0, sizeof(a));
+    a.t.N = N; a.t.E = E; a.t.root = e->root;
+    a.t.indptr = e->d_indptr.as<int>(); a.t.indices = e->d_indices.as<int>(); a.t.preorder = e->d_preorder.as<int>();
+    a.t.node_has_data = e->d_node_has_data.as<unsigned char>();
+    a.n = n; a.C = C; a.K = e->K; a.S = e->S;
+    a.codes = e->d_codes.p; a.code_bytes = e->code_bytes;
+    a.defs = e->d_defs.as<double>(); a.def_const = e->d_def_const.as<unsigned char>();
+    a.Plo = e->c_Plo.as<double>(); a.Phi = e->c_Phi.as<double>();
+    a.root_mode = e->root_mode;
+    a.root_lo = e->c_small.as<double>(); a.root_hi = a.root_lo + n; a.prior_lo = a.root_hi + n; a.prior_hi = a.prior_lo + C;
+    a.Llo = e->g_Lg.as<double>(); a.Lhi = e->g_Fg.as<double>(); a.Kg = e->g_Kg.as<int>(); a.Cg = e->g_Cg.as<unsigned char>();
+    a.cat_lo = e->g_cat_lh.as<double>(); a.cat_hi = e->c_cat_hi.as<double>(); a.cat_k = e->g_cat_k.as<int>();
+    a.site_lo = e->c_site_lo.as<double>(); a.site_hi = e->c_site_hi.as<double>();
+    a.site_mlo = e->c_mlo.as<double>(); a.site_mhi = e->c_mhi.as<double>(); a.site_k = e->c_mk.as<int>();
+    a.Dlo = e->c_Dlo.as<double>(); a.Dhi = e->c_Dhi.as<double>();
+    a.cat_rate = e->d_cat_rates.as<double>();
+    a.edge_mask = edge_mask ? e->d_mask.as<unsigned char>() : nullptr;
+    a.Flo = e->c_Flo.as<double>(); a.Fhi = e->c_Fhi.as<double>(); a.FK = e->c_FK.as<int>();
+    a.xlo = e->c_xlo.as<double>(); a.xhi = e->c_xhi.as<double>(); a.xk = e->c_xk.as<int>();
+    a.site_w = e->have_w ? e->d_site_w.as<double>() : nullptr;
+    a.out_lo = e->c_olo.as<double>(); a.out_hi = e->c_ohi.as<double>();
+    a.err = e->c_err.as<int>();
+    if (smem_in > 48 * 1024) CK(e, cudaFuncSetAttribute(cert_inside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_in));
+    if (smem_out > 48 * 1024) CK(e, cudaFuncSetAttribute(cert_outside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_out));
+    e->last_kernel = "cert_expm_kernel + cert_inside_kernel + cert_outside_kernel";
+    const bool sums = sum_lo || sum_hi;
+    double *part_lo = e->c_part.as<double>(), *part_hi = part_lo + (size_t)groups * E;
+    for (int64_t s0 = 0; s0 < e->S; s0 += Sc) {
+        a.s0 = s0; a.Sc = (int)std::min<int64_t>(Sc, e->S - s0);
+        const unsigned tiles = (unsigned)((a.Sc + CERT_TS - 1) / CERT_TS);
+        cert_inside_kernel<<<dim3(tiles, C), CERT_TS, smem_in, e->stream>>>(a);
+        KCHECK(e);
+        cert_site_kernel<<<(a.Sc + 255) / 256, 256, 0, e->stream>>>(a);
+        KCHECK(e);
+        cert_outside_kernel<<<dim3(tiles, C), CERT_TS, smem_out, e->stream>>>(a);
+        KCHECK(e);
+        cert_deriv_site_kernel<<<dim3((a.Sc + 127) / 128, E), 128, 0, e->stream>>>(a);
+        KCHECK(e);
+        if (sums) {
+            cert_deriv_group_sum_kernel<<<dim3((a.Sc + CERT_GROUP - 1) / CERT_GROUP, E), 32, 0, e->stream>>>(a, part_lo, part_hi);
+            KCHECK(e);
+        }
+        /* per-site outputs of the chunk, [E][Sc] on the device -> rows s0.. of [S][E] on the host */
+        if (site_lo && copy_site_matrix(e, a.out_lo, E, a.Sc, site_lo + (size_t)s0 * E)) return -1;
+        if (site_hi && copy_site_matrix(e, a.out_hi, E, a.Sc, site_hi + (size_t)s0 * E)) return -1;
+    }
+    double *d_sums = e->c_sums.as<double>();
+    if (sums) {
+        cert_deriv_total_kernel<<<(E + 127) / 128, 128, 0, e->stream>>>(part_lo, part_hi, (int)groups, E, d_sums, d_sums + E);
+        KCHECK(e);
+    }
+    std::vector<double> sums_h(sums ? 2 * (size_t)E : 0);
+    int err = 0;
+    if (sums) CK(e, cudaMemcpyAsync(sums_h.data(), d_sums, sizeof(double) * 2 * E, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaMemcpyAsync(&err, e->c_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    if (sums) {
+        if (err & 1) FAIL(e, "a site with non-zero weight has zero likelihood");
+        if (sum_lo) memcpy(sum_lo, sums_h.data(), sizeof(double) * E);
+        if (sum_hi) memcpy(sum_hi, sums_h.data() + E, sizeof(double) * E);
     }
     return 0;
 }
