@@ -43,6 +43,12 @@ char *arbplf_em_update(const char *json_in, int *retcode);
 char *arbplf_ll_certified(const char *json_in, int *retcode);
 /* arbplf-deriv answered the same way (both tables in the format of arbplf-deriv) */
 char *arbplf_deriv_certified(const char *json_in, int *retcode);
+/* arbplf-marginal, arbplf-dwell and arbplf-trans answered the same way (each in its program's table format); site
+ * aggregation is the engine's weighted sum, node, state, edge and transition aggregation are done with directed rounding
+ * on the host or folded into the Frechet direction as the uncertified programs fold them (signed weights allowed) */
+char *arbplf_marginal_certified(const char *json_in, int *retcode);
+char *arbplf_dwell_certified(const char *json_in, int *retcode);
+char *arbplf_trans_certified(const char *json_in, int *retcode);
 
 char *arbplf_hess(const char *json_in, int *retcode);
 char *arbplf_inv_hess(const char *json_in, int *retcode);

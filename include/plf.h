@@ -166,6 +166,27 @@ int plf_deriv_certified(plf_engine *e, double delta_rate, double delta_q, const 
                         double *site_lo /*[S][E]*/, double *site_hi /*[S][E]*/, double *sum_lo /*[E]*/, double *sum_hi /*[E]*/);
 
 /*
+ * Certified mode for plf_marginal and plf_edge_expect: enclosures of exactly what those return, with the input
+ * uncertainties, the errors, the 75-state limit, the fixed-order device sums and the sums after plf_comm_init (this
+ * engine's sites only) of plf_deriv_certified.  Any output may be NULL.
+ *   plf_marginal_certified: site_lo[s][v][i] <= marg <= site_hi[s][v][i] for every node v (root and leaves included)
+ *     and state i; sum_lo / sum_hi [N][n] enclose sum_s w_s marg.  A state that a node's data excludes is 0.0 in both
+ *     bounds.
+ *   plf_edge_expect_certified: the same for the edge expectations of direction L = l_hi + l_lo (l_lo may be NULL) and
+ *     kind PLF_KIND_DWELL or PLF_KIND_TRANS (any other kind is an error); unrequested edges (edge_mask) are 0.0 in
+ *     both bounds.  L may have entries of both signs (F is linear in L: F(L+) - F(L-), the second only when L has a
+ *     negative entry); each entry is taken within the relative delta_q, as a TRANS direction holds entries of Q.
+ * The Frechet matrices F = the top-right block of exp([[A, L], [0, A]]), A = r_c t_e Q, are enclosed by the Taylor
+ * series of the shifted block matrix, whose terms are non-negative for L >= 0 (csrc/certified.cuh).
+ */
+int plf_marginal_certified(plf_engine *e, double delta_rate, double delta_q, double *site_lo /*[S][N][n]*/,
+                           double *site_hi /*[S][N][n]*/, double *sum_lo /*[N][n]*/, double *sum_hi /*[N][n]*/);
+int plf_edge_expect_certified(plf_engine *e, double delta_rate, double delta_q, int kind,
+                              const double *l_hi /*[n*n]*/, const double *l_lo /*[n*n] or NULL*/,
+                              const unsigned char *edge_mask /*[E] or NULL*/,
+                              double *site_lo /*[S][E]*/, double *site_hi /*[S][E]*/, double *sum_lo /*[E]*/, double *sum_hi /*[E]*/);
+
+/*
  * Second order (arbplfhess.c:502-829): sum_ll = sum_s w_s log L_s, sum_deriv[E] its gradient and sum_hess[E][E] its
  * Hessian with respect to the edge rate coefficients (csr edge order, full symmetric matrix).  sum_ll and sum_deriv
  * may be NULL.  A rate category with a non-zero rate and zero likelihood at a weighted site is an error

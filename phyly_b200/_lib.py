@@ -63,6 +63,10 @@ def load():
     lib.plf_ll_certified.restype = c.c_int
     lib.plf_deriv_certified.argtypes = [P, c.c_double, c.c_double, P, P, P, P, P]
     lib.plf_deriv_certified.restype = c.c_int
+    lib.plf_marginal_certified.argtypes = [P, c.c_double, c.c_double, P, P, P, P]
+    lib.plf_marginal_certified.restype = c.c_int
+    lib.plf_edge_expect_certified.argtypes = [P, c.c_double, c.c_double, c.c_int, P, P, P, P, P, P, P]
+    lib.plf_edge_expect_certified.restype = c.c_int
     lib.plf_hess.argtypes = [P, P, P, P]
     lib.plf_hess.restype = c.c_int
     lib.plf_comm_unique_id.argtypes = [c.c_char_p]

@@ -53,10 +53,16 @@ arbplf_model_summary = _bind("model_summary")
 arbplf_ll_certified = _bind("ll_certified")
 # and arbplf-deriv, whose derivative bounds certify their sign
 arbplf_deriv_certified = _bind("deriv_certified")
+# and arbplf-marginal, arbplf-dwell, arbplf-trans
+arbplf_marginal_certified = _bind("marginal_certified")
+arbplf_dwell_certified = _bind("dwell_certified")
+arbplf_trans_certified = _bind("trans_certified")
 
 
 def set_device(device):
     _lib.load().arbplf_set_device(int(device))
 
 
-__all__ = ["arbplf_" + n for n in _NAMES] + ["arbplf_model_summary", "arbplf_ll_certified", "arbplf_deriv_certified", "set_device"]
+__all__ = ["arbplf_" + n for n in _NAMES] + ["arbplf_model_summary", "arbplf_ll_certified", "arbplf_deriv_certified",
+                                            "arbplf_marginal_certified", "arbplf_dwell_certified", "arbplf_trans_certified",
+                                            "set_device"]

@@ -23,6 +23,10 @@
  * cert_outside_kernel restates generic_outside_kernel on non-negative intervals (one exponent for both bounds, as in
  * cert_inside_kernel); only the edge form fe^T D L_b is signed.  cert_deriv_site_kernel sums the categories and
  * divides by the site likelihood enclosure of cert_site_kernel.
+ *
+ * Edge expectations (plf_edge_expect_certified) take the Frechet matrices of cert_frechet_kernel in place of D, without
+ * D's literal-zero shortcuts; marginals (plf_marginal_certified) replace every node's outside vector by fa_v .* L_v in
+ * the outside pass.  Both are non-negative apart from a signed direction L = L+ - L-.
  */
 #pragma once
 #include <stdint.h>
@@ -30,7 +34,7 @@
 
 #define CERT_TS 64          /* sites per CTA in cert_inside_kernel and cert_outside_kernel */
 #define CERT_TAYLOR 26
-#define CERT_GROUP 1024     /* sites per partial sum of plf_deriv_certified: chunks are multiples of it */
+#define CERT_GROUP 1024     /* sites per partial sum of the certified outside queries: chunks are multiples of it */
 
 __device__ __forceinline__ double cert_down(double x, int ulps)
 {
@@ -120,6 +124,58 @@ __device__ void cert_deriv_matrix(int n, int s, double r, double delta_rate, dou
     }
 }
 
+/* thread 0 of the CTA: x = r t in [xlo, xhi] and mu >= max_i x sum_{j != i} q_ij, both rounded up */
+__device__ __forceinline__ void cert_shift(int n, const double *q_hi, const double *q_lo, double r, double t, double delta_rate,
+                                           double delta_q, double &xlo, double &xhi, double &mu)
+{
+    xlo = __dmul_rd(__dmul_rd(r, __dsub_rd(1.0, delta_rate)), t);
+    xhi = __dmul_ru(__dmul_ru(r, __dadd_ru(1.0, delta_rate)), t);
+    mu = 0.0;
+    for (int i = 0; i < n; i++) {
+        double rs = 0.0;
+        for (int j = 0; j < n; j++) {
+            if (j == i) continue;
+            const double q = __dmul_ru(__dadd_ru(q_hi[i * n + j], q_lo ? q_lo[i * n + j] : 0.0), __dadd_ru(1.0, delta_q));
+            rs = __dadd_ru(rs, q);
+        }
+        mu = fmax(mu, __dmul_ru(xhi, rs));
+    }
+}
+
+/* [Blo, Bhi] = (x Q + mu I) sc, sc a power of two */
+__device__ __forceinline__ void cert_shifted_matrix(int n, const double *q_hi, const double *q_lo, double delta_q, double xlo,
+                                                    double xhi, double mu, double sc, double *Blo, double *Bhi)
+{
+    for (int idx = threadIdx.x; idx < n * n; idx += blockDim.x) {
+        const int i = idx / n, j = idx - i * n;
+        double lo, hi;
+        if (i != j) {
+            const double qd = __dadd_rd(q_hi[idx], q_lo ? q_lo[idx] : 0.0), qu = __dadd_ru(q_hi[idx], q_lo ? q_lo[idx] : 0.0);
+            lo = __dmul_rd(xlo, fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q))));
+            hi = __dmul_ru(xhi, __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q)));
+        } else {
+            double rlo = 0.0, rhi = 0.0;
+            for (int k = 0; k < n; k++) {
+                if (k == i) continue;
+                const double qd = __dadd_rd(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0), qu = __dadd_ru(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0);
+                rlo = __dadd_rd(rlo, fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q))));
+                rhi = __dadd_ru(rhi, __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q)));
+            }
+            lo = fmax(0.0, __dsub_rd(mu, __dmul_ru(xhi, rhi)));
+            hi = __dsub_ru(mu, __dmul_rd(xlo, rlo));
+        }
+        Blo[idx] = lo * sc; Bhi[idx] = hi * sc;               /* exact: a power of two */
+    }
+}
+
+/* b^(K+1) / (K+1)! / (1 - b / (K+2)), rounded up: the remainder of the Taylor series of exp(M), M >= 0 of row sums <= b <= 1 */
+__device__ __forceinline__ double cert_taylor_rem(double b)
+{
+    double rem = 1.0;
+    for (int k = 1; k <= CERT_TAYLOR + 1; k++) rem = __ddiv_ru(__dmul_ru(rem, b), (double)k);
+    return __ddiv_ru(rem, __dsub_rd(1.0, __ddiv_ru(b, (double)(CERT_TAYLOR + 2))));
+}
+
 /* one CTA per (edge, category); ws: 8 n^2 doubles per CTA.  Dlo / Dhi (or NULL): enclosure of r_c Q P_e as well. */
 __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, const double *q_hi, const double *q_lo,
                                                         const double *edge_rate, const double *cat_rate, double delta_rate,
@@ -135,18 +191,8 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
     __shared__ int sh_s;
     const double r = cat_rate[c], t = edge_rate[e];
     if (threadIdx.x == 0) {
-        const double xlo = __dmul_rd(__dmul_rd(r, __dsub_rd(1.0, delta_rate)), t);
-        const double xhi = __dmul_ru(__dmul_ru(r, __dadd_ru(1.0, delta_rate)), t);
-        double mu = 0.0;
-        for (int i = 0; i < n; i++) {
-            double rs = 0.0;
-            for (int j = 0; j < n; j++) {
-                if (j == i) continue;
-                const double q = __dmul_ru(__dadd_ru(q_hi[i * n + j], q_lo ? q_lo[i * n + j] : 0.0), __dadd_ru(1.0, delta_q));
-                rs = __dadd_ru(rs, q);
-            }
-            mu = fmax(mu, __dmul_ru(xhi, rs));
-        }
+        double xlo, xhi, mu;
+        cert_shift(n, q_hi, q_lo, r, t, delta_rate, delta_q, xlo, xhi, mu);
         int s = 0;
         if (mu > 1.0) { int ex; frexp(mu, &ex); s = ex; }
         sh_mu = mu; sh_s = s; sh_xlo = xlo; sh_xhi = xhi;
@@ -169,26 +215,9 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
     }
     const double sc = scalbn(1.0, -s);
     /* B, term_0 = sum_0 = I */
+    cert_shifted_matrix(n, q_hi, q_lo, delta_q, xlo, xhi, mu, sc, Blo, Bhi);
     for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
-        const int i = idx / n, j = idx - i * n;
-        double lo, hi;
-        if (i != j) {
-            const double qd = __dadd_rd(q_hi[idx], q_lo ? q_lo[idx] : 0.0), qu = __dadd_ru(q_hi[idx], q_lo ? q_lo[idx] : 0.0);
-            lo = __dmul_rd(xlo, fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q))));
-            hi = __dmul_ru(xhi, __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q)));
-        } else {
-            double rlo = 0.0, rhi = 0.0;
-            for (int k = 0; k < n; k++) {
-                if (k == i) continue;
-                const double qd = __dadd_rd(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0), qu = __dadd_ru(q_hi[i * n + k], q_lo ? q_lo[i * n + k] : 0.0);
-                rlo = __dadd_rd(rlo, fmax(0.0, __dmul_rd(qd, __dsub_rd(1.0, delta_q))));
-                rhi = __dadd_ru(rhi, __dmul_ru(fmax(0.0, qu), __dadd_ru(1.0, delta_q)));
-            }
-            lo = fmax(0.0, __dsub_rd(mu, __dmul_ru(xhi, rhi)));
-            hi = __dsub_ru(mu, __dmul_rd(xlo, rlo));
-        }
-        Blo[idx] = lo * sc; Bhi[idx] = hi * sc;               /* exact: a power of two */
-        const double id = (i == j) ? 1.0 : 0.0;
+        const double id = (idx / n == idx % n) ? 1.0 : 0.0;
         Tlo[idx] = id; Thi[idx] = id; Slo[idx] = id; Shi[idx] = id;
     }
     __syncthreads();
@@ -211,9 +240,7 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
     }
     /* remainder of the series and the scalar e^{-beta} */
     const double beta = mu * sc;                               /* exact, <= 1 */
-    double rem = 1.0;
-    for (int k = 1; k <= CERT_TAYLOR + 1; k++) rem = __ddiv_ru(__dmul_ru(rem, beta), (double)k);
-    rem = __ddiv_ru(rem, __dsub_rd(1.0, __ddiv_ru(beta, (double)(CERT_TAYLOR + 2))));
+    const double rem = cert_taylor_rem(beta);
     const double ev = exp(-beta);
     const double elo = cert_down(ev, 3), ehi = cert_up(ev, 3);
     for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
@@ -248,6 +275,156 @@ __global__ void __launch_bounds__(128) cert_expm_kernel(int n, int E, int C, con
                                Dlo + ((size_t)c * E + e) * nn, Dhi + ((size_t)c * E + e) * nn);
 }
 
+/*
+ * [Ylo, Yhi] encloses the Frechet block F(L) = the top-right block of exp([[A, L], [0, A]]), A = x Q, for a direction
+ * [Llo, Lhi] >= 0 of row sums <= lnorm.  With B = (A + mu I) / 2^s >= 0 and L_s = L / 2^s, the shifted block matrix
+ * [[B, L_s], [0, B]] is non-negative with row sums <= b = (mu + lnorm) / 2^s <= 1; its Taylor terms are X_k = B X_{k-1} / k
+ * and Y_k = (B Y_{k-1} + L_s X_{k-1}) / k, the remainder of every entry is cert_taylor_rem(b), and e^{-beta} (X, Y) is
+ * squared s times as (X, Y) <- (X X, X Y + Y X).  Everything is non-negative: round down for Ylo, up for Yhi.
+ * W: 14 n^2 doubles of workspace.  mu = 0 (x = 0, or Q = 0) gives F = L exactly.
+ */
+__device__ void cert_frechet_pos(int n, const double *q_hi, const double *q_lo, double delta_q, double xlo, double xhi,
+                                 double mu, double lnorm, const double *Llo, const double *Lhi, double *W, double *Ylo, double *Yhi)
+{
+    const int nn = n * n;
+    if (!(mu > 0.0)) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { Ylo[idx] = Llo[idx]; Yhi[idx] = Lhi[idx]; }
+        __syncthreads();
+        return;
+    }
+    double *Blo = W, *Bhi = W + nn, *Xlo = W + 2 * nn, *Xhi = W + 3 * nn, *Tlo = W + 4 * nn, *Thi = W + 5 * nn;
+    double *SXlo = W + 6 * nn, *SXhi = W + 7 * nn, *Ulo = W + 8 * nn, *Uhi = W + 9 * nn, *Vlo = W + 10 * nn, *Vhi = W + 11 * nn;
+    double *Lslo = W + 12 * nn, *Lshi = W + 13 * nn;
+    const double bsum = __dadd_ru(mu, lnorm);
+    int s = 0;
+    if (bsum > 1.0) { int ex; frexp(bsum, &ex); s = ex; }
+    const double sc = scalbn(1.0, -s);
+    cert_shifted_matrix(n, q_hi, q_lo, delta_q, xlo, xhi, mu, sc, Blo, Bhi);
+    for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+        const double id = (idx / n == idx % n) ? 1.0 : 0.0;
+        Xlo[idx] = id; Xhi[idx] = id; SXlo[idx] = id; SXhi[idx] = id;
+        Tlo[idx] = 0.0; Thi[idx] = 0.0; Ylo[idx] = 0.0; Yhi[idx] = 0.0;
+        Lslo[idx] = __dmul_rd(Llo[idx], sc); Lshi[idx] = __dmul_ru(Lhi[idx], sc);
+    }
+    __syncthreads();
+    /* Taylor terms: X in (X, SX), Y_k in T, their sum in Y */
+    for (int k = 1; k <= CERT_TAYLOR; k++) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const int i = idx / n, j = idx - i * n;
+            double xl = 0.0, xh = 0.0, yl = 0.0, yh = 0.0;
+            for (int m = 0; m < n; m++) {
+                xl = __fma_rd(Blo[i * n + m], Xlo[m * n + j], xl);
+                xh = __fma_ru(Bhi[i * n + m], Xhi[m * n + j], xh);
+                yl = __fma_rd(Blo[i * n + m], Tlo[m * n + j], yl);
+                yh = __fma_ru(Bhi[i * n + m], Thi[m * n + j], yh);
+                yl = __fma_rd(Lslo[i * n + m], Xlo[m * n + j], yl);
+                yh = __fma_ru(Lshi[i * n + m], Xhi[m * n + j], yh);
+            }
+            Ulo[idx] = __ddiv_rd(xl, (double)k); Uhi[idx] = __ddiv_ru(xh, (double)k);
+            Vlo[idx] = __ddiv_rd(yl, (double)k); Vhi[idx] = __ddiv_ru(yh, (double)k);
+        }
+        __syncthreads();
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            Xlo[idx] = Ulo[idx]; Xhi[idx] = Uhi[idx]; Tlo[idx] = Vlo[idx]; Thi[idx] = Vhi[idx];
+            SXlo[idx] = __dadd_rd(SXlo[idx], Ulo[idx]); SXhi[idx] = __dadd_ru(SXhi[idx], Uhi[idx]);
+            Ylo[idx] = __dadd_rd(Ylo[idx], Vlo[idx]); Yhi[idx] = __dadd_ru(Yhi[idx], Vhi[idx]);
+        }
+        __syncthreads();
+    }
+    /* remainder of both blocks and the scalar e^{-beta} */
+    const double rem = cert_taylor_rem(bsum * sc);             /* bsum * sc: exact, <= 1 */
+    const double ev = exp(-(mu * sc));
+    const double elo = cert_down(ev, 3), ehi = cert_up(ev, 3);
+    for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+        SXlo[idx] = __dmul_rd(SXlo[idx], elo); SXhi[idx] = __dmul_ru(__dadd_ru(SXhi[idx], rem), ehi);
+        Ylo[idx] = __dmul_rd(Ylo[idx], elo); Yhi[idx] = __dmul_ru(__dadd_ru(Yhi[idx], rem), ehi);
+    }
+    __syncthreads();
+    for (int q = 0; q < s; q++) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const int i = idx / n, j = idx - i * n;
+            double xl = 0.0, xh = 0.0, yl = 0.0, yh = 0.0;
+            for (int m = 0; m < n; m++) {
+                xl = __fma_rd(SXlo[i * n + m], SXlo[m * n + j], xl);
+                xh = __fma_ru(SXhi[i * n + m], SXhi[m * n + j], xh);
+                yl = __fma_rd(SXlo[i * n + m], Ylo[m * n + j], yl);
+                yh = __fma_ru(SXhi[i * n + m], Yhi[m * n + j], yh);
+                yl = __fma_rd(Ylo[i * n + m], SXlo[m * n + j], yl);
+                yh = __fma_ru(Yhi[i * n + m], SXhi[m * n + j], yh);
+            }
+            Ulo[idx] = xl; Uhi[idx] = fmin(1.0, xh); Vlo[idx] = yl; Vhi[idx] = yh;
+        }
+        __syncthreads();
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            SXlo[idx] = Ulo[idx]; SXhi[idx] = Uhi[idx]; Ylo[idx] = Vlo[idx]; Yhi[idx] = Vhi[idx];
+        }
+        __syncthreads();
+    }
+}
+
+/*
+ * Enclosures of the Frechet matrices of plf_edge_expect: one CTA per (edge, category), ws: 18 n^2 doubles per CTA.
+ * F is linear in L = L+ - L-; each entry l_hi + l_lo is widened by the relative delta_q (a TRANS direction holds entries
+ * of the scaled Q), and F(L-) is formed only when L has a negative entry.  trans: F x, x in [xlo, xhi] (f_scale_mode 1
+ * of expm_dd_kernel); x = 0 gives F = L (DWELL) or F = 0 (TRANS) exactly.  Unrequested edges are 0.
+ */
+__global__ void __launch_bounds__(128) cert_frechet_kernel(int n, int E, int C, const double *q_hi, const double *q_lo,
+                                                           const double *edge_rate, const double *cat_rate, double delta_rate,
+                                                           double delta_q, const double *l_hi, const double *l_lo, int trans,
+                                                           const unsigned char *edge_mask, double *ws, double *Flo, double *Fhi)
+{
+    const int e = blockIdx.x, c = blockIdx.y, nn = n * n;
+    double *outlo = Flo + ((size_t)c * E + e) * nn, *outhi = Fhi + ((size_t)c * E + e) * nn;
+    if (edge_mask && !edge_mask[e]) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { outlo[idx] = 0.0; outhi[idx] = 0.0; }
+        return;
+    }
+    double *base = ws + ((size_t)c * E + e) * 18 * nn;
+    double *Ylo = base + 14 * nn, *Yhi = base + 15 * nn, *Llo = base + 16 * nn, *Lhi = base + 17 * nn;
+    __shared__ double sh_mu, sh_xlo, sh_xhi, sh_lnorm;
+    if (threadIdx.x == 0) {
+        double xlo, xhi, mu;
+        cert_shift(n, q_hi, q_lo, cat_rate[c], edge_rate[e], delta_rate, delta_q, xlo, xhi, mu);
+        sh_mu = mu; sh_xlo = xlo; sh_xhi = xhi;
+    }
+    __syncthreads();
+    const double mu = sh_mu, xlo = sh_xlo, xhi = sh_xhi;
+    if (trans && !(xhi > 0.0)) {
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) { outlo[idx] = 0.0; outhi[idx] = 0.0; }
+        return;
+    }
+    for (int neg = 0; neg < 2; neg++) {
+        /* [Llo, Lhi]: the enclosure of L+ (neg = 0) or of L- (neg = 1) */
+        int any = 0;
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            const double vd = __dadd_rd(l_hi[idx], l_lo ? l_lo[idx] : 0.0), vu = __dadd_ru(l_hi[idx], l_lo ? l_lo[idx] : 0.0);
+            const double pd = neg ? -vu : vd, pu = neg ? -vd : vu;
+            Llo[idx] = fmax(0.0, __dmul_rd(pd, __dsub_rd(1.0, delta_q)));
+            Lhi[idx] = __dmul_ru(fmax(0.0, pu), __dadd_ru(1.0, delta_q));
+            any |= Lhi[idx] > 0.0;
+        }
+        if (!__syncthreads_or(any) && neg) break;
+        if (threadIdx.x == 0) {
+            double ln = 0.0;
+            for (int i = 0; i < n; i++) {
+                double rs = 0.0;
+                for (int j = 0; j < n; j++) rs = __dadd_ru(rs, Lhi[i * n + j]);
+                ln = fmax(ln, rs);
+            }
+            sh_lnorm = ln;
+        }
+        __syncthreads();
+        cert_frechet_pos(n, q_hi, q_lo, delta_q, xlo, xhi, mu, sh_lnorm, Llo, Lhi, base, Ylo, Yhi);
+        for (int idx = threadIdx.x; idx < nn; idx += blockDim.x) {
+            double lo = Ylo[idx], hi = Yhi[idx];
+            if (trans) cert_mul_pos(lo, hi, xlo, xhi, lo, hi);
+            if (!neg) { outlo[idx] = lo; outhi[idx] = hi; }
+            else { outlo[idx] = __dsub_rd(outlo[idx], hi); outhi[idx] = __dsub_ru(outhi[idx], lo); }
+        }
+        __syncthreads();
+    }
+}
+
 struct CertArgs {
     TreeDev t;
     int n, C, K;
@@ -263,15 +440,17 @@ struct CertArgs {
     int *Kg; unsigned char *Cg;        /* [C][N][Sc] */
     double *cat_lo, *cat_hi; int *cat_k;   /* [C][Sc] */
     double *site_lo, *site_hi;         /* [S] enclosures of the site log-likelihoods */
-    /* plf_deriv_certified only (NULL otherwise) */
+    /* the outside queries only: plf_deriv_certified, plf_edge_expect_certified, plf_marginal_certified (NULL otherwise) */
     double *site_mlo, *site_mhi; int *site_k;   /* [Sc] the site likelihood enclosure [mlo, mhi] 2^(256 k) */
-    const double *Dlo, *Dhi;           /* [C][E][n][n] enclosures of r_c Q P_e */
+    const double *Dlo, *Dhi;           /* [C][E][n][n] enclosures of the edge matrices: r_c Q P_e, or Frechet matrices */
+    int deriv;                         /* the edge matrices are r_c Q P_e: D 1 = 0 and D = 0 at rate 0 (literal zeros) */
+    int marg;                          /* replace every node's outside vector (leaves included) by fa_v .* L_v */
     const double *cat_rate;            /* [C] */
     const unsigned char *edge_mask;    /* [E] or NULL */
     double *Flo, *Fhi; int *FK;        /* [C][N][n][Sc] outside vectors (mantissas), [C][N][Sc] their exponents */
-    double *xlo, *xhi; int *xk;        /* [C][E][Sc] edge forms fe^T D L_b (mantissas), [C][E][Sc] exponents */
+    double *xlo, *xhi; int *xk;        /* [C][E][Sc] edge forms fe^T D L_b (mantissas), [C][E][Sc] exponents; NULL: none */
     const double *site_w;              /* [S] or NULL */
-    double *out_lo, *out_hi;           /* [E][Sc] enclosures of d log L_s / d t_e */
+    double *out_lo, *out_hi;           /* [cols][Sc] per-site enclosures (columns: edges, or node x state) */
     int *err;                          /* bit 0: a site of non-zero weight whose likelihood enclosure reaches 0 */
 };
 
@@ -421,9 +600,12 @@ __device__ __forceinline__ void cert_rescale(double *lo, double *hi, int n, doub
 
 /*
  * Interval restatement of generic_outside_kernel: thread = (site, category), blockIdx.y = category.  Writes the edge
- * form fe^T D L_b of every requested edge to xlo / xhi / xk.  A category with zero likelihood at the site writes
- * nothing (cert_deriv_site_kernel skips it); a category of rate 0 and a child whose vector is an exact constant column
- * (D 1 = 0) give 0 exactly.  The sibling edge vectors P L are recomputed from the inside vectors.
+ * form fe^T D L_b of every requested edge to xlo / xhi / xk (unless xlo is NULL).  A category with zero likelihood at
+ * the site writes nothing (cert_deriv_site_kernel skips it); for the derivative (deriv) a category of rate 0 and a child
+ * whose vector is an exact constant column (D 1 = 0) give 0 exactly -- properties of D that a Frechet matrix does not
+ * have.  With marg, every node's outside vector fa_v is replaced by the marginal product fa_v .* L_v (exponent
+ * k_a + k_v) once its children have used it; the leaves get outside vectors too.  The sibling edge vectors P L are
+ * recomputed from the inside vectors.
  */
 __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
 {
@@ -439,7 +621,7 @@ __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
     double *flo = csm + (size_t)2 * n * CERT_TS + tid, *fhi = csm + (size_t)3 * n * CERT_TS + tid;
     double *ylo = csm + (size_t)4 * n * CERT_TS + tid, *yhi = csm + (size_t)5 * n * CERT_TS + tid;
     const size_t cN = (size_t)c * a.t.N, cE = (size_t)c * a.t.E, nn = (size_t)n * n;
-    const bool zero_rate = a.cat_rate[c] == 0.0;
+    const bool zero_rate = a.deriv && a.cat_rate[c] == 0.0;
     {
         double *Fl = a.Flo + ((cN + a.t.root) * n) * Sc + s, *Fh = a.Fhi + ((cN + a.t.root) * n) * Sc + s;
         for (int i = 0; i < n; i++) { Fl[(size_t)i * Sc] = a.root_lo[i]; Fh[(size_t)i * Sc] = a.root_hi[i]; }
@@ -448,17 +630,29 @@ __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
     for (int u = 0; u < a.t.N; u++) {
         const int nd = a.t.preorder[u];
         const int start = a.t.indptr[nd], stop = a.t.indptr[nd + 1];
-        if (start == stop) continue;
-        const double *Fl = a.Flo + ((cN + nd) * n) * Sc + s, *Fh = a.Fhi + ((cN + nd) * n) * Sc + s;
+        if (start == stop && !a.marg) continue;
+        double *Fl = a.Flo + ((cN + nd) * n) * Sc + s, *Fh = a.Fhi + ((cN + nd) * n) * Sc + s;
         const int ka = a.FK[(cN + nd) * Sc + s];
-        if (a.t.node_has_data[nd]) {
-            const int code = plf_code_at(a.codes, a.code_bytes, a.S, nd, gs);
-            for (int i = 0; i < n; i++) {
-                const double d = a.defs[(size_t)code * n + i];
-                tlo[i * CERT_TS] = __dmul_rd(Fl[(size_t)i * Sc], d); thi[i * CERT_TS] = __dmul_ru(Fh[(size_t)i * Sc], d);
+        if (start != stop) {
+            if (a.t.node_has_data[nd]) {
+                const int code = plf_code_at(a.codes, a.code_bytes, a.S, nd, gs);
+                for (int i = 0; i < n; i++) {
+                    const double d = a.defs[(size_t)code * n + i];
+                    tlo[i * CERT_TS] = __dmul_rd(Fl[(size_t)i * Sc], d); thi[i * CERT_TS] = __dmul_ru(Fh[(size_t)i * Sc], d);
+                }
+            } else {
+                for (int i = 0; i < n; i++) { tlo[i * CERT_TS] = Fl[(size_t)i * Sc]; thi[i * CERT_TS] = Fh[(size_t)i * Sc]; }
             }
-        } else {
-            for (int i = 0; i < n; i++) { tlo[i * CERT_TS] = Fl[(size_t)i * Sc]; thi[i * CERT_TS] = Fh[(size_t)i * Sc]; }
+        }
+        if (a.marg) {
+            /* fa_v .* L_v in place of fa_v, which the children below take from t */
+            const double *Ll = a.Llo + ((cN + nd) * n) * Sc + s, *Lh = a.Lhi + ((cN + nd) * n) * Sc + s;
+            for (int i = 0; i < n; i++) {
+                Fl[(size_t)i * Sc] = __dmul_rd(Fl[(size_t)i * Sc], Ll[(size_t)i * Sc]);
+                Fh[(size_t)i * Sc] = __dmul_ru(Fh[(size_t)i * Sc], Lh[(size_t)i * Sc]);
+            }
+            a.FK[(cN + nd) * Sc + s] = ka + a.Kg[(cN + nd) * Sc + s];
+            if (start == stop) continue;
         }
         for (int idx = start; idx < stop; idx++) {
             const int b = a.t.indices[idx];
@@ -491,10 +685,10 @@ __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
                 cert_rescale(flo, fhi, n, mx, kfe);
             }
             const int kb = a.Kg[(cN + b) * Sc + s];
-            if (!a.edge_mask || a.edge_mask[idx]) {
+            if (a.xlo && (!a.edge_mask || a.edge_mask[idx])) {
                 /* fe^T (D L_b): first the signed interval vector D L_b, then its product with the non-negative fe */
                 double xl = 0.0, xh = 0.0;
-                if (!zero_rate && !a.Cg[(cN + b) * Sc + s]) {
+                if (!zero_rate && !(a.deriv && a.Cg[(cN + b) * Sc + s])) {
                     const double *Lbl = a.Llo + ((cN + b) * n) * Sc + s, *Lbh = a.Lhi + ((cN + b) * n) * Sc + s;
                     for (int k = 0; k < n; k++) { ylo[k * CERT_TS] = Lbl[(size_t)k * Sc]; yhi[k * CERT_TS] = Lbh[(size_t)k * Sc]; }
                     const double *Dl = a.Dlo + (cE + idx) * nn, *Dh = a.Dhi + (cE + idx) * nn;
@@ -514,8 +708,8 @@ __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
                 a.xhi[(cE + idx) * Sc + s] = xh;
                 a.xk[(cE + idx) * Sc + s] = kfe + kb;
             }
-            /* outside vector of b: P^T fe (internal children only) */
-            if (a.t.indptr[b] != a.t.indptr[b + 1]) {
+            /* outside vector of b: P^T fe (internal children only, unless marg) */
+            if (a.marg || a.t.indptr[b] != a.t.indptr[b + 1]) {
                 const double *Pl = a.Plo + (cE + idx) * nn, *Ph = a.Phi + (cE + idx) * nn;
                 double mx = 0.0;
                 for (int j = 0; j < n; j++) {
@@ -538,14 +732,16 @@ __global__ void __launch_bounds__(CERT_TS) cert_outside_kernel(CertArgs a)
 }
 
 /*
- * Per (site, edge): sum_c prior_c x_c 2^(256 (xk_c - k0)) over the categories of non-zero likelihood, divided by the
- * site likelihood enclosure [mlo, mhi] 2^(256 k0).  grid (sites / 128, E).  Unrequested edges are 0 exactly; a site
- * whose likelihood enclosure reaches 0 gets [-inf, +inf] (and bit 0 of err if its weight is not 0).
+ * Per (site, column): sum_c prior_c x_c 2^(256 (xk_c - k0)) over the categories of non-zero likelihood, divided by the
+ * site likelihood enclosure [mlo, mhi] 2^(256 k0).  Column e of category c has its mantissas at x[(c cols + e) Sc + s]
+ * and its exponent at xk[(c cols / cpk + e / cpk) Sc + s]: the edge forms (cols = E, cpk = 1) or the marginal products
+ * (cols = N n, cpk = n).  grid (sites / 128, columns e0..).  Unrequested edges are 0 exactly; a site whose likelihood
+ * enclosure reaches 0 gets [-inf, +inf] (and bit 0 of err if its weight is not 0).
  */
-__global__ void cert_deriv_site_kernel(CertArgs a)
+__global__ void cert_deriv_site_kernel(CertArgs a, const double *x_lo, const double *x_hi, const int *x_k, int cols, int cpk, int e0)
 {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
-    const int e = blockIdx.y, E = a.t.E;
+    const int e = e0 + blockIdx.y;
     if (s >= a.Sc) return;
     const int Sc = a.Sc;
     const double mlo = a.site_mlo[s], mhi = a.site_mhi[s];
@@ -559,10 +755,10 @@ __global__ void cert_deriv_site_kernel(CertArgs a)
             double nlo = 0.0, nhi = 0.0;
             for (int c = 0; c < a.C; c++) {
                 if (!(a.prior_hi[c] * a.cat_hi[(size_t)c * Sc + s] > 0.0)) continue;
-                const size_t at = ((size_t)c * E + e) * Sc + s;
+                const size_t at = ((size_t)c * cols + e) * Sc + s;
                 double tl, th;
-                cert_mul_pos(a.xlo[at], a.xhi[at], a.prior_lo[c], a.prior_hi[c], tl, th);
-                const int dk = a.xk[at] - k0;
+                cert_mul_pos(x_lo[at], x_hi[at], a.prior_lo[c], a.prior_hi[c], tl, th);
+                const int dk = x_k[((size_t)c * (cols / cpk) + e / cpk) * Sc + s] - k0;
                 nlo = __dadd_rd(nlo, cert_scale_signed(tl, dk, 1));
                 nhi = __dadd_ru(nhi, cert_scale_signed(th, dk, 0));
             }
@@ -577,12 +773,12 @@ __global__ void cert_deriv_site_kernel(CertArgs a)
 }
 
 /*
- * Weighted sums of the enclosures, per group of CERT_GROUP sites and edge, in a fixed order (the same bits on every
- * call, whatever the chunking): grid (groups of the chunk, E), one warp.  A negative weight swaps the bounds.
+ * Weighted sums of the enclosures, per group of CERT_GROUP sites and column, in a fixed order (the same bits on every
+ * call, whatever the chunking): grid (groups of the chunk, columns e0..), one warp.  A negative weight swaps the bounds.
  */
-__global__ void __launch_bounds__(32) cert_deriv_group_sum_kernel(CertArgs a, double *part_lo, double *part_hi)
+__global__ void __launch_bounds__(32) cert_deriv_group_sum_kernel(CertArgs a, int cols, int e0, double *part_lo, double *part_hi)
 {
-    const int g = blockIdx.x, e = blockIdx.y, lane = threadIdx.x, E = a.t.E, Sc = a.Sc;
+    const int g = blockIdx.x, e = e0 + blockIdx.y, lane = threadIdx.x, Sc = a.Sc;
     const int s1 = min(Sc, (g + 1) * CERT_GROUP);
     double lo = 0.0, hi = 0.0;
     for (int s = g * CERT_GROUP + lane; s < s1; s += 32) {
@@ -598,7 +794,7 @@ __global__ void __launch_bounds__(32) cert_deriv_group_sum_kernel(CertArgs a, do
         hi = __dadd_ru(hi, __shfl_xor_sync(0xffffffffu, hi, o));
     }
     if (lane == 0) {
-        const size_t at = (size_t)(a.s0 / CERT_GROUP + g) * E + e;
+        const size_t at = (size_t)(a.s0 / CERT_GROUP + g) * cols + e;
         part_lo[at] = lo; part_hi[at] = hi;
     }
 }

@@ -744,6 +744,60 @@ static void acc_bounds(double *lo, double *hi, double w, double xlo, double xhi)
     fesetround(old);
 }
 
+/* {"lower": <table>, "upper": <table>} */
+static char *bounds_to_json(const axis *ax, int ndim, const double *lo, const double *hi)
+{
+    char *t_lo = table_to_json(ax, ndim, lo), *t_hi = table_to_json(ax, ndim, hi);
+    jbuf b; jbuf_init(&b);
+    jbuf_puts(&b, "{\"lower\": "); jbuf_puts(&b, t_lo); jbuf_puts(&b, ", \"upper\": "); jbuf_puts(&b, t_hi); jbuf_puts(&b, "}");
+    free(t_lo); free(t_hi);
+    return jbuf_take(&b);
+}
+
+/* the relative input uncertainties of every certified program (plf.h): rate_c t_e, and Q and the priors (2^-60) */
+#define CERT_D_RATE 4e-15
+#define CERT_D_Q 8.673617379884035e-19
+
+/*
+ * The certified counterpart of edge_pass: one engine call (kind < 0: plf_deriv_certified, else plf_edge_expect_certified
+ * with direction L) fills [lo, hi] over (site, user edge) at third-axis coordinate `third` (extent third_n); site
+ * aggregation is the engine's weighted sum, edge aggregation acc_bounds.
+ */
+static int edge_pass_certified(ctx *c, int kind, const double *l_hi, const double *l_lo, const axis *ax_site,
+                               const axis *ax_edge, const unsigned char *mask, double *lo, double *hi, int third, int third_n)
+{
+    const plf_model *m = &c->m;
+    const int E = m->E;
+    const int64_t rows = ax_site->aggregated ? 1 : m->S;
+    const size_t edge_ext = ax_edge->aggregated ? 1 : (size_t)E;
+    double *blo = malloc(sizeof(double) * (size_t)rows * (E > 0 ? E : 1)), *bhi = malloc(sizeof(double) * (size_t)rows * (E > 0 ? E : 1));
+    int rc = -1, r;
+    double *slo = ax_site->aggregated ? NULL : blo, *shi = ax_site->aggregated ? NULL : bhi;
+    double *tlo = ax_site->aggregated ? blo : NULL, *thi = ax_site->aggregated ? bhi : NULL;
+    if (plf_set_site_weights(c->e, ax_site->aggregated ? ax_site->w : NULL)) r = -1;
+    else if (kind < 0) r = plf_deriv_certified(c->e, CERT_D_RATE, CERT_D_Q, mask, slo, shi, tlo, thi);
+    else r = plf_edge_expect_certified(c->e, CERT_D_RATE, CERT_D_Q, kind, l_hi, l_lo, mask, slo, shi, tlo, thi);
+    if (r) { fprintf(stderr, "error: %s\n", plf_last_error(c->e)); goto done; }
+    for (int64_t s = 0; s < rows; s++) {
+        if (!ax_site->aggregated && !ax_site->requested[s]) continue;
+        for (int e = 0; e < E; e++) {
+            if (!ax_edge->requested[e]) continue;
+            const double xl = blo[(size_t)s * E + m->order[e]], xh = bhi[(size_t)s * E + m->order[e]];
+            if (!isfinite(xl) || !isfinite(xh)) {
+                if (ax_site->aggregated) fprintf(stderr, "error: a requested site has zero likelihood\n");
+                else fprintf(stderr, "error: site %lld has zero likelihood\n", (long long)s);
+                goto done;
+            }
+            if (ax_edge->aggregated) acc_bounds(&lo[(size_t)s * third_n + third], &hi[(size_t)s * third_n + third], ax_edge->w[e], xl, xh);
+            else { lo[((size_t)s * edge_ext + e) * third_n + third] = xl; hi[((size_t)s * edge_ext + e) * third_n + third] = xh; }
+        }
+    }
+    rc = 0;
+done:
+    free(blo); free(bhi);
+    return rc;
+}
+
 /*
  * The same request as arbplf-deriv, answered with an enclosure: {"lower": <table>, "upper": <table>}, both tables in
  * the format of arbplf-deriv (plf_deriv_certified).  Site aggregation is the engine's weighted sum; edge aggregation
@@ -757,9 +811,9 @@ char *arbplf_deriv_certified(const char *json_in, int *retcode)
     ctx c;
     reduction r_site, r_edge; reduction_init(&r_site); reduction_init(&r_edge);
     axis ax[2]; memset(ax, 0, sizeof ax);
-    double *lo = NULL, *hi = NULL, *blo = NULL, *bhi = NULL;
+    double *lo = NULL, *hi = NULL;
     unsigned char *mask = NULL;
-    char *out = NULL, *t_lo = NULL, *t_hi = NULL;
+    char *out = NULL;
     int rc = -1;
     if (ctx_parse(&c, json_in, keys, v)) goto done;
     const int E = c.m.E;
@@ -767,51 +821,216 @@ char *arbplf_deriv_certified(const char *json_in, int *retcode)
     if (reduction_parse(&r_site, (int)S, "site", v[1])) goto done;
     if (reduction_parse(&r_edge, E, "edge", v[2])) goto done;
     if (axis_init(&ax[0], "site", (int)S, &r_site) || axis_init(&ax[1], "edge", E, &r_edge)) goto done;
-    const size_t edge_ext = ax[1].aggregated ? 1 : (size_t)E;
     {
-        size_t cells = (ax[0].aggregated ? 1 : (size_t)S) * edge_ext;
+        size_t cells = (ax[0].aggregated ? 1 : (size_t)S) * (ax[1].aggregated ? 1 : (size_t)E);
         lo = calloc(cells ? cells : 1, sizeof(double));
         hi = calloc(cells ? cells : 1, sizeof(double));
     }
     if (S > 0 && E > 0) {
         if (ctx_load(&c)) goto done;
         mask = edge_mask_csr(&c.m, &ax[1]);
-        const double d_rate = 4e-15, d_q = 8.673617379884035e-19;       /* 2^-60 */
+        if (edge_pass_certified(&c, -1, NULL, NULL, &ax[0], &ax[1], mask, lo, hi, 0, 1)) goto done;
+    }
+    phase_compute_done(&c);
+    out = bounds_to_json(ax, 2, lo, hi);
+    rc = 0;
+done:
+    free(lo); free(hi); free(mask);
+    axis_clear(&ax[0]); axis_clear(&ax[1]);
+    reduction_clear(&r_site); reduction_clear(&r_edge);
+    return finish(&c, out, rc, retcode);
+}
+
+/* ------------------------------------------------------------------ */
+/* arbplf-marginal / arbplf-dwell / arbplf-trans, certified mode       */
+/* ------------------------------------------------------------------ */
+
+/*
+ * The same request as arbplf-marginal, answered with {"lower", "upper"} tables in its format (plf_marginal_certified).
+ * Site aggregation is the engine's weighted sum; node and state aggregation multiply the bounds by each weight in turn
+ * and add them up with directed rounding.
+ */
+char *arbplf_marginal_certified(const char *json_in, int *retcode)
+{
+    static const char *const keys[] = {"model_and_data", "?site_reduction", "?node_reduction", "?state_reduction", NULL};
+    const jv *v[4];
+    ctx c;
+    reduction r_site, r_node, r_state;
+    reduction_init(&r_site); reduction_init(&r_node); reduction_init(&r_state);
+    axis ax[3]; memset(ax, 0, sizeof ax);
+    double *lo = NULL, *hi = NULL, *blo = NULL, *bhi = NULL;
+    char *out = NULL;
+    int rc = -1;
+    if (ctx_parse(&c, json_in, keys, v)) goto done;
+    const int N = c.m.N, n = c.m.n;
+    const int64_t S = c.m.S;
+    if (reduction_parse(&r_site, (int)S, "site", v[1])) goto done;
+    if (reduction_parse(&r_node, N, "node", v[2])) goto done;
+    if (reduction_parse(&r_state, n, "state", v[3])) goto done;
+    if (axis_init(&ax[0], "site", (int)S, &r_site) || axis_init(&ax[1], "node", N, &r_node) ||
+        axis_init(&ax[2], "state", n, &r_state)) goto done;
+    const size_t e1 = ax[1].aggregated ? 1 : (size_t)N, e2 = ax[2].aggregated ? 1 : (size_t)n;
+    lo = calloc((ax[0].aggregated ? 1 : (size_t)(S > 0 ? S : 1)) * e1 * e2, sizeof(double));
+    hi = calloc((ax[0].aggregated ? 1 : (size_t)(S > 0 ? S : 1)) * e1 * e2, sizeof(double));
+    if (S > 0) {
+        if (ctx_load(&c)) goto done;
         const int64_t rows = ax[0].aggregated ? 1 : S;
-        blo = malloc(sizeof(double) * (size_t)rows * E);
-        bhi = malloc(sizeof(double) * (size_t)rows * E);
+        blo = malloc(sizeof(double) * (size_t)rows * N * n);
+        bhi = malloc(sizeof(double) * (size_t)rows * N * n);
         int r;
-        if (ax[0].aggregated) r = plf_set_site_weights(c.e, ax[0].w) || plf_deriv_certified(c.e, d_rate, d_q, mask, NULL, NULL, blo, bhi);
-        else r = plf_set_site_weights(c.e, NULL) || plf_deriv_certified(c.e, d_rate, d_q, mask, blo, bhi, NULL, NULL);
+        if (ax[0].aggregated) r = plf_set_site_weights(c.e, ax[0].w) || plf_marginal_certified(c.e, CERT_D_RATE, CERT_D_Q, NULL, NULL, blo, bhi);
+        else r = plf_set_site_weights(c.e, NULL) || plf_marginal_certified(c.e, CERT_D_RATE, CERT_D_Q, blo, bhi, NULL, NULL);
         if (r) { fprintf(stderr, "error: %s\n", plf_last_error(c.e)); goto done; }
         for (int64_t s = 0; s < rows; s++) {
             if (!ax[0].aggregated && !ax[0].requested[s]) continue;
-            for (int e = 0; e < E; e++) {
-                if (!ax[1].requested[e]) continue;
-                const double xl = blo[(size_t)s * E + c.m.order[e]], xh = bhi[(size_t)s * E + c.m.order[e]];
-                if (!isfinite(xl) || !isfinite(xh)) {
-                    if (ax[0].aggregated) fprintf(stderr, "error: a requested site has zero likelihood\n");
-                    else fprintf(stderr, "error: site %lld has zero likelihood\n", (long long)s);
-                    goto done;
+            for (int a = 0; a < N; a++) {
+                if (!ax[1].requested[a]) continue;
+                for (int j = 0; j < n; j++) {
+                    if (!ax[2].requested[j]) continue;
+                    double xl = blo[((size_t)s * N + a) * n + j], xh = bhi[((size_t)s * N + a) * n + j];
+                    if (!isfinite(xl) || !isfinite(xh)) { fprintf(stderr, "error: a requested site has zero likelihood\n"); goto done; }
+                    if (ax[1].aggregated) { double tl = 0.0, th = 0.0; acc_bounds(&tl, &th, ax[1].w[a], xl, xh); xl = tl; xh = th; }
+                    const size_t off = ((size_t)s * e1 + (ax[1].aggregated ? 0 : a)) * e2 + (ax[2].aggregated ? 0 : j);
+                    acc_bounds(&lo[off], &hi[off], ax[2].aggregated ? ax[2].w[j] : 1.0, xl, xh);
                 }
-                if (ax[1].aggregated) acc_bounds(&lo[s], &hi[s], ax[1].w[e], xl, xh);
-                else { lo[(size_t)s * edge_ext + e] = xl; hi[(size_t)s * edge_ext + e] = xh; }
             }
         }
     }
     phase_compute_done(&c);
-    t_lo = table_to_json(ax, 2, lo);
-    t_hi = table_to_json(ax, 2, hi);
-    {
-        jbuf b; jbuf_init(&b);
-        jbuf_puts(&b, "{\"lower\": "); jbuf_puts(&b, t_lo); jbuf_puts(&b, ", \"upper\": "); jbuf_puts(&b, t_hi); jbuf_puts(&b, "}");
-        out = jbuf_take(&b);
-    }
+    out = bounds_to_json(ax, 3, lo, hi);
     rc = 0;
 done:
-    free(lo); free(hi); free(blo); free(bhi); free(mask); free(t_lo); free(t_hi);
-    axis_clear(&ax[0]); axis_clear(&ax[1]);
-    reduction_clear(&r_site); reduction_clear(&r_edge);
+    free(lo); free(hi); free(blo); free(bhi);
+    for (int i = 0; i < 3; i++) axis_clear(&ax[i]);
+    reduction_clear(&r_site); reduction_clear(&r_node); reduction_clear(&r_state);
+    return finish(&c, out, rc, retcode);
+}
+
+/* The same request as arbplf-dwell, answered with {"lower", "upper"} tables in its format (plf_edge_expect_certified);
+ * state aggregation is folded into the direction as arbplf-dwell folds it, signed weights included. */
+char *arbplf_dwell_certified(const char *json_in, int *retcode)
+{
+    static const char *const keys[] = {"model_and_data", "?site_reduction", "?edge_reduction", "?state_reduction", NULL};
+    const jv *v[4];
+    ctx c;
+    reduction r_site, r_edge, r_state;
+    reduction_init(&r_site); reduction_init(&r_edge); reduction_init(&r_state);
+    axis ax[3]; memset(ax, 0, sizeof ax);
+    double *lo = NULL, *hi = NULL, *L = NULL;
+    unsigned char *mask = NULL;
+    char *out = NULL;
+    int rc = -1;
+    if (ctx_parse(&c, json_in, keys, v)) goto done;
+    const int n = c.m.n, E = c.m.E;
+    const int64_t S = c.m.S;
+    if (reduction_parse(&r_site, (int)S, "site", v[1])) goto done;
+    if (reduction_parse(&r_edge, E, "edge", v[2])) goto done;
+    if (reduction_parse(&r_state, n, "state", v[3])) goto done;
+    if (axis_init(&ax[0], "site", (int)S, &r_site) || axis_init(&ax[1], "edge", E, &r_edge) ||
+        axis_init(&ax[2], "state", n, &r_state)) goto done;
+    const int state_agg = ax[2].aggregated;
+    const int third_n = state_agg ? 1 : n;
+    {
+        size_t cells = (ax[0].aggregated ? 1 : (size_t)(S > 0 ? S : 1)) * (ax[1].aggregated ? 1 : (size_t)E) * third_n;
+        lo = calloc(cells ? cells : 1, sizeof(double));
+        hi = calloc(cells ? cells : 1, sizeof(double));
+    }
+    if (S > 0) {
+        if (ctx_load(&c)) goto done;
+        mask = edge_mask_csr(&c.m, &ax[1]);
+        L = calloc((size_t)n * n, sizeof(double));
+        if (state_agg) {
+            for (int s = 0; s < n; s++) L[s * n + s] = ax[2].w[s];     /* arbplfdwell.c:173-178 */
+            if (edge_pass_certified(&c, PLF_KIND_DWELL, L, NULL, &ax[0], &ax[1], mask, lo, hi, 0, 1)) goto done;
+        } else {
+            for (int s = 0; s < n; s++) {
+                if (!ax[2].requested[s]) continue;
+                memset(L, 0, sizeof(double) * n * n);
+                L[s * n + s] = 1.0;                                     /* arbplfdwell.c:133 */
+                if (edge_pass_certified(&c, PLF_KIND_DWELL, L, NULL, &ax[0], &ax[1], mask, lo, hi, s, n)) goto done;
+            }
+        }
+    }
+    phase_compute_done(&c);
+    out = bounds_to_json(ax, state_agg ? 2 : 3, lo, hi);
+    rc = 0;
+done:
+    free(lo); free(hi); free(L); free(mask);
+    for (int i = 0; i < 3; i++) axis_clear(&ax[i]);
+    reduction_clear(&r_site); reduction_clear(&r_edge); reduction_clear(&r_state);
+    return finish(&c, out, rc, retcode);
+}
+
+/* The same request as arbplf-trans, answered with {"lower", "upper"} tables in its format (plf_edge_expect_certified);
+ * transition aggregation is folded into the direction (sum_k w_k E_{a_k b_k}) .* Q as arbplf-trans folds it, signed
+ * weights included.  The weights of a repeated pair are added in double-double, so that the direction stays within the
+ * engine's relative delta_q of the exact one. */
+char *arbplf_trans_certified(const char *json_in, int *retcode)
+{
+    static const char *const keys[] = {"model_and_data", "?site_reduction", "?edge_reduction", "?trans_reduction", NULL};
+    const jv *v[4];
+    ctx c;
+    reduction r_site, r_edge, r_trans;
+    reduction_init(&r_site); reduction_init(&r_edge); reduction_init(&r_trans);
+    axis ax[3]; memset(ax, 0, sizeof ax);
+    double *lo = NULL, *hi = NULL, *Lh = NULL, *Ll = NULL;
+    dd_t *W = NULL;
+    unsigned char *mask = NULL;
+    char *out = NULL;
+    int rc = -1;
+    if (ctx_parse(&c, json_in, keys, v)) goto done;
+    const int n = c.m.n, E = c.m.E;
+    const int64_t S = c.m.S;
+    if (reduction_parse(&r_site, (int)S, "site", v[1])) goto done;
+    if (reduction_parse(&r_edge, E, "edge", v[2])) goto done;
+    if (reduction_parse_pairs(&r_trans, n, "trans", v[3])) goto done;
+    const int T = r_trans.selection_len;
+    if (axis_init(&ax[0], "site", (int)S, &r_site) || axis_init(&ax[1], "edge", E, &r_edge) ||
+        axis_init(&ax[2], "trans", T, &r_trans)) goto done;
+    ax[2].ncomp = 2;
+    ax[2].comp_name[0] = "first_state"; ax[2].comp_name[1] = "second_state";
+    ax[2].comp_idx[0] = r_trans.first_idx; ax[2].comp_idx[1] = r_trans.second_idx;
+    const int trans_agg = ax[2].aggregated;
+    const int third_n = trans_agg ? 1 : (T > 0 ? T : 1);
+    {
+        size_t cells = (ax[0].aggregated ? 1 : (size_t)(S > 0 ? S : 1)) * (ax[1].aggregated ? 1 : (size_t)E) * third_n;
+        lo = calloc(cells ? cells : 1, sizeof(double));
+        hi = calloc(cells ? cells : 1, sizeof(double));
+    }
+    if (S > 0) {
+        if (ctx_load(&c)) goto done;
+        mask = edge_mask_csr(&c.m, &ax[1]);
+        Lh = calloc((size_t)n * n, sizeof(double));
+        Ll = calloc((size_t)n * n, sizeof(double));
+        if (trans_agg) {
+            /* L = (sum_k w_k E_{a_k b_k}) .* Q / divisor  (arbplftrans.c:179-193) */
+            W = calloc((size_t)n * n, sizeof(dd_t));
+            for (int k = 0; k < T; k++) {
+                dd_t *x = &W[r_trans.first_idx[k] * n + r_trans.second_idx[k]];
+                *x = dd_add(*x, dd_make(ax[2].w[k], 0.0));
+            }
+            for (int i = 0; i < n * n; i++) {
+                dd_t q = dd_mul(dd_make(c.d.q_hi[i], c.d.q_lo[i]), W[i]);
+                Lh[i] = q.hi; Ll[i] = q.lo;
+            }
+            if (edge_pass_certified(&c, PLF_KIND_TRANS, Lh, Ll, &ax[0], &ax[1], mask, lo, hi, 0, 1)) goto done;
+        } else {
+            for (int k = 0; k < T; k++) {
+                if (!ax[2].requested[k]) continue;
+                memset(Lh, 0, sizeof(double) * n * n); memset(Ll, 0, sizeof(double) * n * n);
+                int idx = r_trans.first_idx[k] * n + r_trans.second_idx[k];
+                Lh[idx] = c.d.q_hi[idx]; Ll[idx] = c.d.q_lo[idx];      /* arbplftrans.c:133-134 */
+                if (edge_pass_certified(&c, PLF_KIND_TRANS, Lh, Ll, &ax[0], &ax[1], mask, lo, hi, k, third_n)) goto done;
+            }
+        }
+    }
+    phase_compute_done(&c);
+    out = bounds_to_json(ax, trans_agg ? 2 : 3, lo, hi);
+    rc = 0;
+done:
+    free(lo); free(hi); free(Lh); free(Ll); free(W); free(mask);
+    for (int i = 0; i < 3; i++) axis_clear(&ax[i]);
+    reduction_clear(&r_site); reduction_clear(&r_edge); reduction_clear(&r_trans);
     return finish(&c, out, rc, retcode);
 }
 

@@ -2659,24 +2659,32 @@ extern "C" int plf_ll_certified(plf_engine *e, double delta_rate, double delta_q
     return 0;
 }
 
-extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delta_q, const unsigned char *edge_mask,
-                                   double *site_lo, double *site_hi, double *sum_lo, double *sum_hi)
+/* the checks every certified outside query makes before it launches anything */
+static int cert_check(plf_engine *e, const char *what, double delta_rate, double delta_q)
 {
-    if (!e) return -1;
     if (e->S == 0 || e->n == 0 || e->N == 0) FAIL(e, "engine is not fully configured (tree, model and data are required)");
-    if (!(delta_rate >= 0.0) || !(delta_q >= 0.0) || delta_rate > 1e-3 || delta_q > 1e-3) FAIL(e, "plf_deriv_certified: bad input uncertainties");
-    const int n = e->n, C = e->C, N = e->N, E = e->E;
-    const size_t smem_in = sizeof(double) * 4 * n * CERT_TS, smem_out = sizeof(double) * 6 * n * CERT_TS;
-    if (smem_out > 227 * 1024) FAIL(e, "state count %d is too large for the certified kernels", n);
-    CK(e, cudaSetDevice(e->device));
-    if (resolve_pending(e)) return -1;
-    if (E == 0) return 0;
-    if (cert_prepare(e, delta_rate, delta_q, true)) return -1;
-    ENSURE(e, e->d_mask, (size_t)E);
-    if (edge_mask) CK(e, cudaMemcpyAsync(e->d_mask.p, edge_mask, (size_t)E, cudaMemcpyHostToDevice, e->stream));
+    if (!(delta_rate >= 0.0) || !(delta_q >= 0.0) || delta_rate > 1e-3 || delta_q > 1e-3) FAIL(e, "%s: bad input uncertainties", what);
+    if (sizeof(double) * 6 * e->n * CERT_TS > 227 * 1024) FAIL(e, "state count %d is too large for the certified kernels", e->n);
+    return 0;
+}
 
+enum CertOutside { CERT_DERIV, CERT_EXPECT, CERT_MARGINAL };
+
+/*
+ * The site passes of the certified outside queries, after cert_prepare (and, for the edge forms, the edge matrices in
+ * c_Dlo / c_Dhi and the mask in d_mask): per chunk the inside pass, the site likelihood enclosure, the outside pass,
+ * the per-site columns (edges, or node x state for CERT_MARGINAL) and their group sums; then the totals and the
+ * read-back.  Per-site output [S][cols], sums [cols].
+ */
+static int cert_outside_query(plf_engine *e, CertOutside what, const unsigned char *edge_mask, double *site_lo, double *site_hi,
+                              double *sum_lo, double *sum_hi)
+{
+    const int n = e->n, C = e->C, N = e->N, E = e->E;
+    const bool edges = what != CERT_MARGINAL;
+    const int cols = edges ? E : N * n;
+    const size_t smem_in = sizeof(double) * 4 * n * CERT_TS, smem_out = sizeof(double) * 6 * n * CERT_TS;
     /* inside and outside vectors, edge forms, the site likelihood enclosure and the per-site output of a chunk */
-    const size_t per_site = (size_t)C * ((size_t)4 * N * n * 8 + (size_t)N * 9 + (size_t)E * 20 + 24) + (size_t)E * 16 + 24;
+    const size_t per_site = (size_t)C * ((size_t)4 * N * n * 8 + (size_t)N * 9 + (edges ? (size_t)E * 20 : 0) + 24) + (size_t)cols * 16 + 24;
     size_t free_b = 0, total_b = 0;
     CK(e, cudaMemGetInfo(&free_b, &total_b));
     const size_t held = e->g_Lg.cap + e->g_Fg.cap + e->c_Flo.cap + e->c_Fhi.cap + e->c_xlo.cap + e->c_xhi.cap + e->c_olo.cap + e->c_ohi.cap;
@@ -2697,17 +2705,19 @@ extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delt
     ENSURE(e, e->c_Flo, sizeof(double) * (size_t)C * N * n * Sc);
     ENSURE(e, e->c_Fhi, sizeof(double) * (size_t)C * N * n * Sc);
     ENSURE(e, e->c_FK, sizeof(int) * (size_t)C * N * Sc);
-    ENSURE(e, e->c_xlo, sizeof(double) * (size_t)C * E * Sc);
-    ENSURE(e, e->c_xhi, sizeof(double) * (size_t)C * E * Sc);
-    ENSURE(e, e->c_xk, sizeof(int) * (size_t)C * E * Sc);
+    if (edges) {
+        ENSURE(e, e->c_xlo, sizeof(double) * (size_t)C * E * Sc);
+        ENSURE(e, e->c_xhi, sizeof(double) * (size_t)C * E * Sc);
+        ENSURE(e, e->c_xk, sizeof(int) * (size_t)C * E * Sc);
+    }
     ENSURE(e, e->c_mlo, sizeof(double) * Sc);
     ENSURE(e, e->c_mhi, sizeof(double) * Sc);
     ENSURE(e, e->c_mk, sizeof(int) * Sc);
-    ENSURE(e, e->c_olo, sizeof(double) * (size_t)E * Sc);
-    ENSURE(e, e->c_ohi, sizeof(double) * (size_t)E * Sc);
+    ENSURE(e, e->c_olo, sizeof(double) * (size_t)cols * Sc);
+    ENSURE(e, e->c_ohi, sizeof(double) * (size_t)cols * Sc);
     const int64_t groups = (e->S + CERT_GROUP - 1) / CERT_GROUP;
-    ENSURE(e, e->c_part, sizeof(double) * 2 * (size_t)groups * E);
-    ENSURE(e, e->c_sums, sizeof(double) * 2 * (size_t)E);
+    ENSURE(e, e->c_part, sizeof(double) * 2 * (size_t)groups * cols);
+    ENSURE(e, e->c_sums, sizeof(double) * 2 * (size_t)cols);
     ENSURE(e, e->c_err, sizeof(int));
     CK(e, cudaMemsetAsync(e->c_err.p, 0, sizeof(int), e->stream));
 
@@ -2726,19 +2736,22 @@ extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delt
     a.cat_lo = e->g_cat_lh.as<double>(); a.cat_hi = e->c_cat_hi.as<double>(); a.cat_k = e->g_cat_k.as<int>();
     a.site_lo = e->c_site_lo.as<double>(); a.site_hi = e->c_site_hi.as<double>();
     a.site_mlo = e->c_mlo.as<double>(); a.site_mhi = e->c_mhi.as<double>(); a.site_k = e->c_mk.as<int>();
-    a.Dlo = e->c_Dlo.as<double>(); a.Dhi = e->c_Dhi.as<double>();
+    if (edges) {
+        a.Dlo = e->c_Dlo.as<double>(); a.Dhi = e->c_Dhi.as<double>();
+        a.xlo = e->c_xlo.as<double>(); a.xhi = e->c_xhi.as<double>(); a.xk = e->c_xk.as<int>();
+        a.edge_mask = edge_mask ? e->d_mask.as<unsigned char>() : nullptr;
+    }
+    a.deriv = what == CERT_DERIV;
+    a.marg = what == CERT_MARGINAL;
     a.cat_rate = e->d_cat_rates.as<double>();
-    a.edge_mask = edge_mask ? e->d_mask.as<unsigned char>() : nullptr;
     a.Flo = e->c_Flo.as<double>(); a.Fhi = e->c_Fhi.as<double>(); a.FK = e->c_FK.as<int>();
-    a.xlo = e->c_xlo.as<double>(); a.xhi = e->c_xhi.as<double>(); a.xk = e->c_xk.as<int>();
     a.site_w = e->have_w ? e->d_site_w.as<double>() : nullptr;
     a.out_lo = e->c_olo.as<double>(); a.out_hi = e->c_ohi.as<double>();
     a.err = e->c_err.as<int>();
     if (smem_in > 48 * 1024) CK(e, cudaFuncSetAttribute(cert_inside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_in));
     if (smem_out > 48 * 1024) CK(e, cudaFuncSetAttribute(cert_outside_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_out));
-    e->last_kernel = "cert_expm_kernel + cert_inside_kernel + cert_outside_kernel";
     const bool sums = sum_lo || sum_hi;
-    double *part_lo = e->c_part.as<double>(), *part_hi = part_lo + (size_t)groups * E;
+    double *part_lo = e->c_part.as<double>(), *part_hi = part_lo + (size_t)groups * cols;
     for (int64_t s0 = 0; s0 < e->S; s0 += Sc) {
         a.s0 = s0; a.Sc = (int)std::min<int64_t>(Sc, e->S - s0);
         const unsigned tiles = (unsigned)((a.Sc + CERT_TS - 1) / CERT_TS);
@@ -2748,32 +2761,93 @@ extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delt
         KCHECK(e);
         cert_outside_kernel<<<dim3(tiles, C), CERT_TS, smem_out, e->stream>>>(a);
         KCHECK(e);
-        cert_deriv_site_kernel<<<dim3((a.Sc + 127) / 128, E), 128, 0, e->stream>>>(a);
-        KCHECK(e);
-        if (sums) {
-            cert_deriv_group_sum_kernel<<<dim3((a.Sc + CERT_GROUP - 1) / CERT_GROUP, E), 32, 0, e->stream>>>(a, part_lo, part_hi);
+        for (int e0 = 0; e0 < cols; e0 += 65535) {          /* the grid's y extent */
+            const dim3 site_grid((a.Sc + 127) / 128, std::min(cols - e0, 65535)), group_grid((a.Sc + CERT_GROUP - 1) / CERT_GROUP, site_grid.y);
+            if (edges) cert_deriv_site_kernel<<<site_grid, 128, 0, e->stream>>>(a, a.xlo, a.xhi, a.xk, E, 1, e0);
+            else cert_deriv_site_kernel<<<site_grid, 128, 0, e->stream>>>(a, a.Flo, a.Fhi, a.FK, cols, n, e0);
             KCHECK(e);
+            if (sums) {
+                cert_deriv_group_sum_kernel<<<group_grid, 32, 0, e->stream>>>(a, cols, e0, part_lo, part_hi);
+                KCHECK(e);
+            }
         }
-        /* per-site outputs of the chunk, [E][Sc] on the device -> rows s0.. of [S][E] on the host */
-        if (site_lo && copy_site_matrix(e, a.out_lo, E, a.Sc, site_lo + (size_t)s0 * E)) return -1;
-        if (site_hi && copy_site_matrix(e, a.out_hi, E, a.Sc, site_hi + (size_t)s0 * E)) return -1;
+        /* per-site outputs of the chunk, [cols][Sc] on the device -> rows s0.. of [S][cols] on the host */
+        if (site_lo && copy_site_matrix(e, a.out_lo, cols, a.Sc, site_lo + (size_t)s0 * cols)) return -1;
+        if (site_hi && copy_site_matrix(e, a.out_hi, cols, a.Sc, site_hi + (size_t)s0 * cols)) return -1;
     }
     double *d_sums = e->c_sums.as<double>();
     if (sums) {
-        cert_deriv_total_kernel<<<(E + 127) / 128, 128, 0, e->stream>>>(part_lo, part_hi, (int)groups, E, d_sums, d_sums + E);
+        cert_deriv_total_kernel<<<(cols + 127) / 128, 128, 0, e->stream>>>(part_lo, part_hi, (int)groups, cols, d_sums, d_sums + cols);
         KCHECK(e);
     }
-    std::vector<double> sums_h(sums ? 2 * (size_t)E : 0);
+    std::vector<double> sums_h(sums ? 2 * (size_t)cols : 0);
     int err = 0;
-    if (sums) CK(e, cudaMemcpyAsync(sums_h.data(), d_sums, sizeof(double) * 2 * E, cudaMemcpyDeviceToHost, e->stream));
+    if (sums) CK(e, cudaMemcpyAsync(sums_h.data(), d_sums, sizeof(double) * 2 * cols, cudaMemcpyDeviceToHost, e->stream));
     CK(e, cudaMemcpyAsync(&err, e->c_err.p, sizeof(int), cudaMemcpyDeviceToHost, e->stream));
     CK(e, cudaStreamSynchronize(e->stream));
     if (sums) {
         if (err & 1) FAIL(e, "a site with non-zero weight has zero likelihood");
-        if (sum_lo) memcpy(sum_lo, sums_h.data(), sizeof(double) * E);
-        if (sum_hi) memcpy(sum_hi, sums_h.data() + E, sizeof(double) * E);
+        if (sum_lo) memcpy(sum_lo, sums_h.data(), sizeof(double) * cols);
+        if (sum_hi) memcpy(sum_hi, sums_h.data() + cols, sizeof(double) * cols);
     }
     return 0;
+}
+
+extern "C" int plf_deriv_certified(plf_engine *e, double delta_rate, double delta_q, const unsigned char *edge_mask,
+                                   double *site_lo, double *site_hi, double *sum_lo, double *sum_hi)
+{
+    if (!e) return -1;
+    if (cert_check(e, "plf_deriv_certified", delta_rate, delta_q)) return -1;
+    CK(e, cudaSetDevice(e->device));
+    if (resolve_pending(e)) return -1;
+    if (e->E == 0) return 0;
+    if (cert_prepare(e, delta_rate, delta_q, true)) return -1;
+    ENSURE(e, e->d_mask, (size_t)e->E);
+    if (edge_mask) CK(e, cudaMemcpyAsync(e->d_mask.p, edge_mask, (size_t)e->E, cudaMemcpyHostToDevice, e->stream));
+    e->last_kernel = "cert_expm_kernel + cert_inside_kernel + cert_outside_kernel";
+    return cert_outside_query(e, CERT_DERIV, edge_mask, site_lo, site_hi, sum_lo, sum_hi);
+}
+
+extern "C" int plf_edge_expect_certified(plf_engine *e, double delta_rate, double delta_q, int kind, const double *l_hi,
+                                         const double *l_lo, const unsigned char *edge_mask, double *site_lo, double *site_hi,
+                                         double *sum_lo, double *sum_hi)
+{
+    if (!e) return -1;
+    if (cert_check(e, "plf_edge_expect_certified", delta_rate, delta_q)) return -1;
+    if (kind != PLF_KIND_DWELL && kind != PLF_KIND_TRANS) FAIL(e, "plf_edge_expect_certified: invalid kind %d", kind);
+    if (!l_hi) FAIL(e, "plf_edge_expect_certified: l_hi is required");
+    CK(e, cudaSetDevice(e->device));
+    if (resolve_pending(e)) return -1;
+    const int n = e->n, C = e->C, E = e->E;
+    if (E == 0) return 0;
+    const size_t nn = (size_t)n * n;
+    ENSURE(e, e->c_ws, sizeof(double) * C * E * 18 * nn + 8);
+    ENSURE(e, e->c_Dlo, sizeof(double) * C * E * nn + 8);
+    ENSURE(e, e->c_Dhi, sizeof(double) * C * E * nn + 8);
+    if (cert_prepare(e, delta_rate, delta_q, false)) return -1;
+    ENSURE(e, e->d_mask, (size_t)E);
+    if (edge_mask) CK(e, cudaMemcpyAsync(e->d_mask.p, edge_mask, (size_t)E, cudaMemcpyHostToDevice, e->stream));
+    if (upload_L(e, l_hi, l_lo)) return -1;
+    cert_frechet_kernel<<<dim3(E, C), 128, 0, e->stream>>>(n, E, C, e->d_qhi.as<double>(), e->d_qlo.as<double>(), e->d_edge_rates.as<double>(),
+                                                           e->d_cat_rates.as<double>(), delta_rate, delta_q, e->d_lhi.as<double>(),
+                                                           l_lo ? e->d_llo.as<double>() : nullptr, kind == PLF_KIND_TRANS,
+                                                           edge_mask ? e->d_mask.as<unsigned char>() : nullptr, e->c_ws.as<double>(),
+                                                           e->c_Dlo.as<double>(), e->c_Dhi.as<double>());
+    KCHECK(e);
+    e->last_kernel = "cert_expm_kernel + cert_frechet_kernel + cert_inside_kernel + cert_outside_kernel";
+    return cert_outside_query(e, CERT_EXPECT, edge_mask, site_lo, site_hi, sum_lo, sum_hi);
+}
+
+extern "C" int plf_marginal_certified(plf_engine *e, double delta_rate, double delta_q, double *site_lo, double *site_hi,
+                                      double *sum_lo, double *sum_hi)
+{
+    if (!e) return -1;
+    if (cert_check(e, "plf_marginal_certified", delta_rate, delta_q)) return -1;
+    CK(e, cudaSetDevice(e->device));
+    if (resolve_pending(e)) return -1;
+    if (cert_prepare(e, delta_rate, delta_q, false)) return -1;
+    e->last_kernel = "cert_expm_kernel + cert_inside_kernel + cert_outside_kernel";
+    return cert_outside_query(e, CERT_MARGINAL, nullptr, site_lo, site_hi, sum_lo, sum_hi);
 }
 
 /* ------------------------------------------------------------------ */

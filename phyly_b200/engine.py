@@ -221,6 +221,28 @@ class Engine:
         self._ck(self._lib.plf_deriv_certified(self._h, delta_rate, delta_q, _ptr(m), _ptr(lo), _ptr(hi), _ptr(slo), _ptr(shi)))
         return dict(site_lo=lo, site_hi=hi, sum_lo=slo, sum_hi=shi)
 
+    def marginal_certified(self, per_site=True, delta_rate=4e-15, delta_q=2.0 ** -60):
+        """Enclosures of the posterior marginals [S, N, n] (None unless per_site) and of their weighted sums [N, n]:
+        dict(site_lo, site_hi, sum_lo, sum_hi)."""
+        lo = np.zeros((self.S, self.N, self.n)) if per_site else None
+        hi = np.zeros((self.S, self.N, self.n)) if per_site else None
+        slo = np.zeros((self.N, self.n))
+        shi = np.zeros((self.N, self.n))
+        self._ck(self._lib.plf_marginal_certified(self._h, delta_rate, delta_q, _ptr(lo), _ptr(hi), _ptr(slo), _ptr(shi)))
+        return dict(site_lo=lo, site_hi=hi, sum_lo=slo, sum_hi=shi)
+
+    def edge_expect_certified(self, kind, L, edge_mask=None, per_site=True, L_lo=None, delta_rate=4e-15, delta_q=2.0 ** -60):
+        """Enclosures of edge_expect(kind, L): per site [S, E] (csr order; None unless per_site) and the weighted sums [E],
+        dict(site_lo, site_hi, sum_lo, sum_hi).  L may have entries of both signs; unrequested edges are 0 in both bounds."""
+        m = None if edge_mask is None else np.ascontiguousarray(edge_mask, dtype=np.uint8)
+        lo = np.zeros((self.S, self.E)) if per_site else None
+        hi = np.zeros((self.S, self.E)) if per_site else None
+        slo = np.zeros(self.E)
+        shi = np.zeros(self.E)
+        self._ck(self._lib.plf_edge_expect_certified(self._h, delta_rate, delta_q, kind, _ptr(_f64(L)), _ptr(_f64(L_lo)), _ptr(m),
+                                                     _ptr(lo), _ptr(hi), _ptr(slo), _ptr(shi)))
+        return dict(site_lo=lo, site_hi=hi, sum_lo=slo, sum_hi=shi)
+
     def hess(self):
         """sum_ll, gradient [E] and Hessian [E, E] of the weighted log likelihood w.r.t. the edge rates (csr order)."""
         ll = np.zeros(1)
