@@ -9,6 +9,7 @@
 #define F4_KIND_TIP 0
 #define F4_KIND_CUR 1
 #define F4_KIND_STACK 2
+#define F4_KIND_CHERRY 3     /* a node whose two children are tips, folded into per-code-pair tables (ll / edge forms) */
 
 struct F4Op {
     int node;
@@ -23,10 +24,11 @@ struct F4Child {
     int kind;
     int slot;            /* scratch slot if internal, else -1 */
     int mat;             /* internal child: index into the compact internal-edge matrices;
-                            tip child: index into the compact tip tables */
-    int code_row;        /* tip child: row of the codes tile */
+                            tip child: index into the compact tip tables; cherry: index of its tables */
+    int code_row;        /* tip child: row of the codes tile; cherry: row of its first tip */
     int edge;            /* csr idx (output position) */
     int node;            /* the child node (output position of its marginal) */
-    int pad[2];
+    int code_row_b;      /* cherry: row of its second tip */
+    int tip_edge;        /* cherry: csr idx of the edge to its first tip (the second's is tip_edge + 1) */
 };
 

@@ -123,24 +123,6 @@ __device__ __forceinline__ void f4_ld4(const double *__restrict__ p, double out[
     out[0] = a.x; out[1] = a.y; out[2] = b.x; out[3] = b.y;
 }
 
-/* number of 2^256 up-scalings applied so that max(v) >= 2^-256 (v >= 0) */
-__device__ __forceinline__ int f4_rescale_up(double v[4])
-{
-    /* non-negative doubles order like their high words */
-    int h = max(max(__double2hiint(v[0]), __double2hiint(v[1])), max(__double2hiint(v[2]), __double2hiint(v[3])));
-    int s = 0;
-    if (h < 0x2FF00000) {          /* high word of 2^-256 */
-        double m = fmax(fmax(v[0], v[1]), fmax(v[2], v[3]));
-        while (m > 0.0 && m < PLF_TWO_M256 && s < 3) {
-#pragma unroll
-            for (int i = 0; i < 4; i++) v[i] *= PLF_TWO_P256;
-            m *= PLF_TWO_P256;
-            s++;
-        }
-    }
-    return s;
-}
-
 __device__ __forceinline__ double f4_warp_sum(double x)
 {
 #pragma unroll
@@ -182,7 +164,7 @@ __device__ __forceinline__ void f4_prefetch_tables(const F4Args &a, const F4Chil
 #pragma unroll
             for (int c = 0; c < C; c++) f4_prefetch(tf + c * tpstride);
         }
-    } else if (lane < C) {
+    } else if (nc.kind != F4_KIND_CHERRY && lane < C) {
         f4_prefetch(Pint + lane * pstride + nc.mat * 16);
         if (WITH_F) f4_prefetch(Fint + lane * pstride + nc.mat * 16);
     }
@@ -212,6 +194,26 @@ __device__ __forceinline__ double f4_warp_sum2(double a, double b, int lane)
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) keep += __shfl_xor_sync(0xffffffffu, keep, o);
     return keep;
+}
+
+/* sums of N values (N = 2, 4, 8) over the warp in one reduce-scatter butterfly: the sum of v[k] lands in lane k * 32 / N.
+ * Every sum is added in the order of f4_warp_sum (offsets 16, 8, ..., 1), so it has the same bits. */
+template <int N>
+__device__ __forceinline__ double f4_warp_sum_n(double v[N], int lane)
+{
+#pragma unroll
+    for (int h = N / 2, o = 16; h >= 1; h >>= 1, o >>= 1) {
+        const bool hi = lane & o;
+#pragma unroll
+        for (int k = 0; k < h; k++) {
+            const double keep = hi ? v[k + h] : v[k], send = hi ? v[k] : v[k + h];
+            v[k] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        }
+    }
+    double r = v[0];
+#pragma unroll
+    for (int o = 16 / N; o > 0; o >>= 1) r += __shfl_xor_sync(0xffffffffu, r, o);
+    return r;
 }
 
 /*
@@ -249,25 +251,51 @@ __device__ __forceinline__ void f4_gm_add(double *row, const double fe[4], const
     if (!(lane & 1)) row[lane >> 1] += sum;
 }
 
+/* x[0] += sc fe.z_a, x[1] += sc fe.z_b with sc = 2^(256 s), s the cherry's rescale count */
+__device__ __forceinline__ void f4_cherry_tips(const double fe[4], const double z[8], int s, double *x)
+{
+    double f[4] = {fe[0], fe[1], fe[2], fe[3]};
+    if (s) {
+        const double sc = __hiloint2double((1023 + PLF_SCALE_BITS * s) << 20, 0);
+#pragma unroll
+        for (int i = 0; i < 4; i++) f[i] *= sc;
+    }
+    double xa = f[0] * z[0], xb = f[0] * z[4];
+#pragma unroll
+    for (int i = 1; i < 4; i++) { xa = fma(f[i], z[i], xa); xb = fma(f[i], z[4 + i], xb); }
+    x[0] += xa; x[1] += xb;
+}
+
 /*
  * Outside step specialised for a node with exactly two children of kinds (K0, K1) in
- * {(CUR, TIP), (CUR, STACK), (TIP, TIP)}: straight-line code, no filler factors.
+ * {(CUR, TIP), (CUR, STACK), (TIP, TIP)} and, with folded cherries (mode 1), {(CUR, CHERRY), (CHERRY, CHERRY),
+ * (CHERRY, TIP)}: straight-line code, no filler factors.  x[0], x[1] take the values of the children's edges,
+ * x[2], x[3] those of the tip edges of a cherry c0 and x[4], x[5] of a cherry c1.
  */
 template <int C, int BD, int K0, int K1, bool PACK, bool CM, bool MARG, bool GM>
 __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, const F4Child &c0, const F4Child &c1,
                                             bool from_slot, double *cur, const unsigned char *tile, const double *defs_s,
                                             const double *Pint, const double *Fint, const double *TP, const double *TF,
+                                            const double *chEm, const unsigned int *chW,
                                             int pstride, int tpstride, size_t T, size_t gtid, int tid,
-                                            double &x0, double &x1, double *mgo, double *accG)
+                                            double *x, double *mgo, double *accG)
 {
+    constexpr bool CH0 = K0 == F4_KIND_CHERRY, CH1 = K1 == F4_KIND_CHERRY;
+    const int K2 = a.K * a.K;
     double basev[4] = {1.0, 1.0, 1.0, 1.0};
     const bool has_base = op.code_row >= 0;
     if (has_base) f4_ld4(defs_s + f4_code<BD, PACK>(tile, op.code_row, tid) * 4, basev);
     const unsigned int sword_a = a.scratchS[(size_t)op.slot * T + gtid];
     int code0 = 0, code1 = 0, bc0 = 0, bc1 = 0;
-    if (K0 == F4_KIND_TIP) code0 = f4_code<BD, PACK>(tile, c0.code_row, tid); else bc0 = (a.scratchS[(size_t)c0.slot * T + gtid] >> 6) & 1;
-    if (K1 == F4_KIND_TIP) code1 = f4_code<BD, PACK>(tile, c1.code_row, tid); else bc1 = (a.scratchS[(size_t)c1.slot * T + gtid] >> 6) & 1;
-    x0 = 0.0; x1 = 0.0;
+    unsigned int w0 = 0, w1 = 0;     /* a cherry: its scale word; code0 / code1 its code pair */
+    if (K0 == F4_KIND_TIP) code0 = f4_code<BD, PACK>(tile, c0.code_row, tid);
+    else if (CH0) { code0 = f4_code<BD, PACK>(tile, c0.code_row, tid) * a.K + f4_code<BD, PACK>(tile, c0.code_row_b, tid); w0 = chW[c0.mat * K2 + code0]; }
+    else bc0 = (a.scratchS[(size_t)c0.slot * T + gtid] >> 6) & 1;
+    if (K1 == F4_KIND_TIP) code1 = f4_code<BD, PACK>(tile, c1.code_row, tid);
+    else if (CH1) { code1 = f4_code<BD, PACK>(tile, c1.code_row, tid) * a.K + f4_code<BD, PACK>(tile, c1.code_row_b, tid); w1 = chW[c1.mat * K2 + code1]; }
+    else bc1 = (a.scratchS[(size_t)c1.slot * T + gtid] >> 6) & 1;
+#pragma unroll
+    for (int i = 0; i < 6; i++) x[i] = 0.0;
     /* marginal mode: posterior state distribution of this node and of its tip children, summed over categories */
     double mg[4] = {0.0, 0.0, 0.0, 0.0}, mt0[4] = {0.0, 0.0, 0.0, 0.0}, mt1[4] = {0.0, 0.0, 0.0, 0.0};
     const int ptstride = a.Et * 16;
@@ -276,11 +304,11 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
     for (int c = 0; c < C; c++) {
         /* loads of this category first */
         double l0[4], l1[4], fa[4];
-        if (K0 != F4_KIND_TIP) {
+        if (K0 != F4_KIND_TIP && !CH0) {
             double4 v = f4_slab_ld(&a.scratch[((size_t)c0.slot * C + c) * T + gtid]);
             l0[0] = v.x; l0[1] = v.y; l0[2] = v.z; l0[3] = v.w;
         }
-        if (K1 != F4_KIND_TIP) {
+        if (K1 != F4_KIND_TIP && !CH1) {
             double4 v = f4_slab_ld(&a.scratch[((size_t)c1.slot * C + c) * T + gtid]);
             l1[0] = v.x; l1[1] = v.y; l1[2] = v.z; l1[3] = v.w;
         }
@@ -301,10 +329,14 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
 #pragma unroll
             for (int i = 0; i < 4; i++) fa[i] *= sc;
         }
-        double em0[4], y0[4], em1[4], y1[4];
+        double em0[4], y0[4], em1[4], y1[4], z0[8], z1[8];
         if (K0 == F4_KIND_TIP) {
             f4_ld4(TP + c * tpstride + (c0.mat * a.K + code0) * 4, em0);
             if (!MARG && !GM) f4_ld4(TF + c * tpstride + (c0.mat * a.K + code0) * 4, y0);
+        } else if (CH0) {
+            const size_t ent = ((size_t)c * a.nch + c0.mat) * K2 + code0;
+            f4_ld4(chEm + ent * 4, em0);
+            f4_ld4(a.chOut + ent * 16 + 4, y0); f4_ld4(a.chOut + ent * 16 + 8, z0); f4_ld4(a.chOut + ent * 16 + 12, z0 + 4);
         } else {
             f4_mv<CM, 0>(Pint, c * pstride + c0.mat * 16, l0, em0);
             if (!MARG && !GM) f4_mv<CM, 1>(Fint, c * pstride + c0.mat * 16, l0, y0);
@@ -316,6 +348,10 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
         if (K1 == F4_KIND_TIP) {
             f4_ld4(TP + c * tpstride + (c1.mat * a.K + code1) * 4, em1);
             if (!MARG && !GM) f4_ld4(TF + c * tpstride + (c1.mat * a.K + code1) * 4, y1);
+        } else if (CH1) {
+            const size_t ent = ((size_t)c * a.nch + c1.mat) * K2 + code1;
+            f4_ld4(chEm + ent * 4, em1);
+            f4_ld4(a.chOut + ent * 16 + 4, y1); f4_ld4(a.chOut + ent * 16 + 8, z1); f4_ld4(a.chOut + ent * 16 + 12, z1 + 4);
         } else {
             f4_mv<CM, 0>(Pint, c * pstride + c1.mat * 16, l1, em1);
             if (!MARG && !GM) f4_mv<CM, 1>(Fint, c * pstride + c1.mat * 16, l1, y1);
@@ -336,10 +372,13 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
         } else if (!MARG) {
             double xv = fe0[0] * y0[0];
             xv = fma(fe0[1], y0[1], xv); xv = fma(fe0[2], y0[2], xv); xv = fma(fe0[3], y0[3], xv);
-            x0 += xv;
+            x[0] += xv;
             xv = fe1[0] * y1[0];
             xv = fma(fe1[1], y1[1], xv); xv = fma(fe1[2], y1[2], xv); xv = fma(fe1[3], y1[3], xv);
-            x1 += xv;
+            x[1] += xv;
+            /* a cherry's tip edges: fe scaled like the cherry's own outside vector, times z_a and z_b */
+            if (CH0) f4_cherry_tips(fe0, z0, (w0 >> (8 * c)) & 63, x + 2);
+            if (CH1) f4_cherry_tips(fe1, z1, (w1 >> (8 * c)) & 63, x + 4);
         } else {
 #pragma unroll
             for (int i = 0; i < 4; i++) mg[i] = fma(fe0[i], em0[i], mg[i]);
@@ -357,7 +396,7 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
                 for (int i = 0; i < 4; i++) mt1[i] += fb[i];
             }
         }
-        if (K0 != F4_KIND_TIP) {
+        if (K0 != F4_KIND_TIP && !CH0) {
             double fb[4];
             f4_mvt<CM>(Pint, c * pstride + c0.mat * 16, fe0, fb);
             if (K0 == F4_KIND_CUR) {
@@ -367,7 +406,7 @@ __device__ __forceinline__ void f4_outside2(const F4Args &a, const F4Op &op, con
                 f4_slab_st(&a.scratch[((size_t)c0.slot * C + c) * T + gtid], fb[0], fb[1], fb[2], fb[3]);
             }
         }
-        if (K1 != F4_KIND_TIP) {
+        if (K1 != F4_KIND_TIP && !CH1) {
             double fb[4];
             f4_mvt<CM>(Pint, c * pstride + c1.mat * 16, fe1, fb);
             /* the child's inside vector is dead after this op: its slot carries fn down */
@@ -637,6 +676,7 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
     constexpr bool EDGE = MODE != 0;     /* an outside pass runs */
     constexpr bool MARG = MODE == 2;     /* ... and produces node marginals instead of per-edge forms */
     constexpr bool GM = MODE == 3;       /* ... or the per-edge outer-product matrices (no edge-form tables) */
+    constexpr bool FOLD = MODE <= 1;     /* the program may carry folded cherries (F4_KIND_CHERRY) */
     extern __shared__ __align__(16) unsigned char f4_smem[];
     const int tid = threadIdx.x;
     constexpr int bd = BD;
@@ -665,6 +705,9 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
     unsigned char *tile = f4_smem + off; off = f4_align16(off + (size_t)(PACK ? (a.ncode_rows + 1) / 2 : a.ncode_rows) * bd);
     unsigned char *dconst = f4_smem + off; off = f4_align16(off + a.K);
     double *defs_s = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + sizeof(double) * 4 * a.K);
+    const int K2 = a.K * a.K, nchE = FOLD ? 4 * C * a.nch * K2 : 0, nchW = FOLD ? a.nch * K2 : 0;
+    double *chEm = reinterpret_cast<double *>(f4_smem + off); off = f4_align16(off + sizeof(double) * nchE);
+    unsigned int *chW = reinterpret_cast<unsigned int *>(f4_smem + off); off = f4_align16(off + sizeof(unsigned int) * nchW);
     const double *Pint = a.Pint, *TP = a.TP, *Fint = a.Fint, *TF = a.TF;
     if (STAGED) {
         const size_t nP = CM ? 0 : (size_t)C * a.Ei * 16, nT = (size_t)C * a.Et * a.K * 4;
@@ -686,6 +729,8 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
     }
     for (int i = tid; i < a.K; i += bd) dconst[i] = a.def_const[i];
     for (int i = tid; i < 4 * a.K; i += bd) defs_s[i] = a.defs[i];
+    for (int i = tid; i < nchE; i += bd) chEm[i] = a.chEm[i];
+    for (int i = tid; i < nchW; i += bd) chW[i] = a.chW[i];
     if (EDGE && !MARG && !GM) for (int i = tid; i < nwarp * a.E; i += bd) accE[i] = 0.0;
     double *accM = MARG ? a.block_marg + ((size_t)blockIdx.x * nwarp + warp) * ((size_t)a.N * 4) : nullptr;
     double *accG = GM ? a.block_gmat + ((size_t)blockIdx.x * nwarp + warp) * ((size_t)C * a.E * 16) : nullptr;
@@ -781,6 +826,16 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
                     const double *tp = TP + (ch.mat * a.K + code) * 4;
 #pragma unroll
                     for (int c = 0; c < C; c++) f4_ld4(tp + c * tpstride, em[c]);
+                } else if (FOLD && ch.kind == F4_KIND_CHERRY) {
+                    /* the cherry's P_e L_b and scale word by its code pair: its rescale counts go to the node's */
+                    const int pr = f4_code<BD, PACK>(tile, ch.code_row, tid) * a.K + f4_code<BD, PACK>(tile, ch.code_row_b, tid);
+                    const unsigned int wd = chW[ch.mat * K2 + pr];
+                    bc = (wd >> 6) & 1;
+#pragma unroll
+                    for (int c = 0; c < C; c++) {
+                        f4_ld4(chEm + ((c * a.nch + ch.mat) * K2 + pr) * 4, em[c]);
+                        ktot[c] -= (wd >> (8 * c)) & 63;
+                    }
                 } else {
                     double v[C][4];
                     if (ch.kind == F4_KIND_CUR) {
@@ -909,10 +964,15 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
                 }
                 for (int j = 0; j < nx.nchild; j++) {
                     const F4Child nc = F4_CH(nx.first_child + j);
-                    if (nc.kind != F4_KIND_TIP) {
+                    if (nc.kind == F4_KIND_CUR || nc.kind == F4_KIND_STACK) {
                         f4_prefetch(&a.scratchS[(size_t)nc.slot * T + gtid]);
 #pragma unroll
                         for (int c = 0; c < C; c++) f4_prefetch(&a.scratch[((size_t)nc.slot * C + c) * T + gtid]);
+                    } else if (FOLD && nc.kind == F4_KIND_CHERRY) {
+                        /* the cherry's line of the outside table (128 bytes per category) */
+                        const int pr = f4_code<BD, PACK>(tile, nc.code_row, tid) * a.K + f4_code<BD, PACK>(tile, nc.code_row_b, tid);
+#pragma unroll
+                        for (int c = 0; c < C; c++) f4_prefetch(a.chOut + (((size_t)c * a.nch + nc.mat) * K2 + pr) * 16);
                     }
                     if (STAGED == 0 && !CM)
                         f4_prefetch_tables<C, BD, PACK, !MARG && !GM>(a, nc, tile, Pint, Fint, TP, TF, pstride, tpstride, tid, lane);
@@ -920,16 +980,46 @@ __global__ void __launch_bounds__(BD) fused4_kernel(const F4Args a, const __grid
             }
             if (op.nchild == 2) {
                 const F4Child c0 = F4_CH(op.first_child), c1 = F4_CH(op.first_child + 1);
-                double x0, x1, mgo[12];
-                if (c0.kind == F4_KIND_CUR && c1.kind == F4_KIND_TIP)
-                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_TIP, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
-                else if (c0.kind == F4_KIND_CUR)
-                    f4_outside2<C, BD, F4_KIND_CUR, F4_KIND_STACK, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                   pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
-                else
-                    f4_outside2<C, BD, F4_KIND_TIP, F4_KIND_TIP, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF,
-                                                                 pstride, tpstride, (size_t)T, (size_t)gtid, tid, x0, x1, mgo, accG);
+                double x[6], mgo[12];
+#define F4_OUT2(K0, K1) f4_outside2<C, BD, K0, K1, PACK, CM, MARG, GM>(a, op, c0, c1, from_slot, cur, tile, defs_s, Pint, Fint, TP, TF, \
+                                                                   chEm, chW, pstride, tpstride, (size_t)T, (size_t)gtid, tid, x, mgo, accG)
+                if (MODE == 1 && (c0.kind == F4_KIND_CHERRY || c1.kind == F4_KIND_CHERRY)) {
+                    /* a folded cherry adds its two tip edges: four or six edge values, summed in one butterfly */
+                    double xs[8];
+                    int ed[8];
+                    const bool two = c0.kind == F4_KIND_CHERRY && c1.kind == F4_KIND_CHERRY;
+                    if (two) F4_OUT2(F4_KIND_CHERRY, F4_KIND_CHERRY);
+                    else if (c0.kind == F4_KIND_CUR) F4_OUT2(F4_KIND_CUR, F4_KIND_CHERRY);
+                    else F4_OUT2(F4_KIND_CHERRY, F4_KIND_TIP);
+                    const F4Child &ch = c0.kind == F4_KIND_CHERRY ? c0 : c1;
+                    const int ne = two ? 6 : 4;
+                    ed[0] = c0.edge; ed[1] = c1.edge; ed[2] = ch.tip_edge; ed[3] = ch.tip_edge + 1;
+                    ed[4] = c1.tip_edge; ed[5] = c1.tip_edge + 1; ed[6] = ed[7] = 0;
+                    xs[0] = x[0]; xs[1] = x[1];
+                    xs[2] = (c0.kind == F4_KIND_CHERRY) ? x[2] : x[4]; xs[3] = (c0.kind == F4_KIND_CHERRY) ? x[3] : x[5];
+                    xs[4] = x[4]; xs[5] = x[5]; xs[6] = xs[7] = 0.0;
+                    bool me[8];
+#pragma unroll
+                    for (int k = 0; k < 8; k++) {
+                        me[k] = k < ne && (!a.edge_mask || a.edge_mask[ed[k]]);
+                        if (!me[k]) xs[k] = 0.0;
+                    }
+                    if (a.edge_site_out) {
+#pragma unroll
+                        for (int k = 0; k < 8; k++) if (valid && me[k]) a.edge_site_out[(size_t)ed[k] * a.S + site] = xs[k];
+                    } else {
+                        /* (the butterfly runs whatever the mask says, as in the two-edge case below) */
+                        const double r = f4_warp_sum_n<8>(xs, lane);
+#pragma unroll
+                        for (int k = 0; k < 8; k++) if (lane == 4 * k && me[k]) accE[warp * a.E + ed[k]] += r;
+                    }
+                    continue;
+                }
+                if (c0.kind == F4_KIND_CUR && c1.kind == F4_KIND_TIP) F4_OUT2(F4_KIND_CUR, F4_KIND_TIP);
+                else if (c0.kind == F4_KIND_CUR) F4_OUT2(F4_KIND_CUR, F4_KIND_STACK);
+                else F4_OUT2(F4_KIND_TIP, F4_KIND_TIP);
+#undef F4_OUT2
+                const double x0 = x[0], x1 = x[1];
                 if (MARG) {
                     f4_marg_out(a, accM, op.node, mgo, valid, site, lane);
                     if (c0.kind == F4_KIND_TIP) f4_marg_out(a, accM, c0.node, mgo + 4, valid, site, lane);

@@ -43,6 +43,10 @@ struct F4Args {
     double *block_edge;              /* [grid][E] */
     int *error_flag;
     double *block_gmat;              /* mode 3: [grid * warps][C][E][16], zeroed by the host, accumulated here */
+    int nch;                         /* folded cherries (F4_KIND_CHERRY children; modes 0 and 1), tables by code pair p: */
+    const double *chEm;              /* [C][nch][K*K][4]: the vector the parent multiplies in (staged in shared memory) */
+    const unsigned int *chW;         /* [nch][K*K]: scale word, the layout of scratchS (staged in shared memory) */
+    const double *chOut;             /* mode 1: [C][nch][K*K][16]: chEm, y, z_a, z_b (f4_tables_kernel), read through L1 */
 };
 
 /*

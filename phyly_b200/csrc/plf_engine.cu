@@ -108,6 +108,22 @@ struct F4Slot {
     int tuned_C = 0, tuned_K = 0;
 };
 
+/*
+ * A post-order program of the fused kernels (build_program) with its device copy and its tables: the compact matrices
+ * of the internal-child edges (Pint, Fint), the tip tables (TP, TF) and, for folded cherries, per (category, cherry,
+ * code pair) the inside vector the parent sees (chEm), the scale word (chW) and the line of the outside pass (chOut).
+ */
+struct F4Program {
+    std::vector<F4Op> ops;
+    std::vector<F4Child> children;
+    std::vector<int> edge_of_int, edge_of_tip;
+    std::vector<int> cherry;          /* folded cherries: csr idx of the cherry's edge and of its first tip edge */
+    int stack_depth = 0, nslots = 0;
+    DevBuf d_ops, d_children, d_edge_of_int, d_edge_of_tip, d_cherry, d_TP, d_TF, d_Pint, d_Fint, d_chEm, d_chW, d_chOut;
+    bool TP_valid = false;            /* TP, Pint (and chEm, chW) hold the current matrices */
+    int ncherry() const { return (int)cherry.size() / 2; }
+};
+
 struct plf_engine {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -144,14 +160,14 @@ struct plf_engine {
     int pend_in_bytes = 1;
     unsigned char *flags_pinned = nullptr;
 
-    /* fused program */
-    std::vector<F4Op> ops;
-    std::vector<F4Child> children;
-    DevBuf d_ops, d_children, d_TP, d_TF, d_Pint, d_Fint, d_Ptip, d_block_marg, d_marg_site, d_edge_of_int, d_edge_of_tip, d_code_row_node, d_tip_of_edge, d_TPg, d_TFg, d_int_seq;
-    std::vector<int> edge_of_int, edge_of_tip, code_row_node;
+    /* fused programs: prog for every query (and the DMMA kernels), fold with the cherries folded into tables for the
+     * ll and edge-form queries when they are worth it (f4_use_fold); both read the tile rows of code_row_node */
+    F4Program prog, fold;
+    DevBuf d_Ptip, d_block_marg, d_marg_site, d_code_row_node, d_tip_of_edge, d_TPg, d_TFg, d_int_seq;
+    std::vector<int> code_row_node;
     std::vector<unsigned char> node_has_data_h;
-    int stack_depth = 0, nslots = 0, max_degree = 0;
-    bool TP_valid = false, program_dirty = true;
+    int max_degree = 0;
+    bool program_dirty = true;
     bool dm_valid = false;       /* packed matrices / tip tables of the DMMA kernels (dmma.cuh) */
     DevBuf d_dmPf, d_dmTPf, d_dmTFf, d_dm_defsf, d_dm_rootf, d_dm_stack, d_dm_stackmeta, d_dm_slab, d_dm_slabmeta, d_dm_Of, d_dm_oidx, d_dm_otr, d_dm_ops, d_dm_ch;
     int dm_out_depth = 0;
@@ -507,16 +523,91 @@ __global__ void compact_matrices_kernel(const double *M, const int *edge_of, int
     out[idx] = M[((size_t)c * E + edge_of[ie]) * 16 + k];
 }
 
-/* the tables of the fused 4-state kernel in one launch: tip tables and compact internal-edge matrices of P and,
- * when Fm is given, of the edge-form matrices (four launches of the two kernels above otherwise) */
+/* entry i of the tip table of 4-state matrix M (mode 0: P, 1: derivative, 2: other edge forms) for character k */
+__device__ __forceinline__ double f4_tip_entry(const double *M, const double *defs, const unsigned char *def_const, int c, int E,
+                                               int edge, int i, int k, int mode)
+{
+    const double *row = M + (((size_t)c * E + edge) * 4 + i) * 4;
+    const double *d = defs + (size_t)k * 4;
+    if (def_const[k] && mode == 0) return d[0];
+    if (def_const[k] && mode == 1) return 0.0;
+    double v = 0.0;
+    for (int j = 0; j < 4; j++) v = fma(row[j], d[j], v);
+    return v;
+}
+
+/* out = M v in the order of the fused kernel's f4_mv */
+__device__ __forceinline__ void f4_table_mv(const double *M, const double v[4], double out[4])
+{
+    for (int i = 0; i < 4; i++) {
+        double r = M[4 * i] * v[0];
+        r = fma(M[4 * i + 1], v[1], r);
+        r = fma(M[4 * i + 2], v[2], r);
+        r = fma(M[4 * i + 3], v[3], r);
+        out[i] = r;
+    }
+}
+
+/*
+ * The tables of the fused 4-state kernel in one launch: tip tables and compact internal-edge matrices of P and, when Fm
+ * is given, of the edge-form matrices (four launches of the two kernels above otherwise), then the tables of the nch
+ * folded cherries (build_program), one thread per (category c, cherry j, code pair p = k_a K + k_b):
+ *   chEm[c][j][p]  = the vector the parent multiplies in: P_e L_b with L_b = TP_a[k_a] .* TP_b[k_b] rescaled (f4_rescale_up),
+ *                    or L_b itself when both characters are constant -- computed as the kernel computes it for an internal
+ *                    child, so the same bits;
+ *   chW[j][p]      = the cherry's scale word: byte c = rescale count | constant flag << 6 (the layout of scratchS; each
+ *                    thread writes its byte, the last category's also the unused ones);
+ *   chOut[c][j][p] = 16 doubles: chEm, y = F_e L_b (0 for a constant cherry when F has zero row sums) and
+ *                    z_a = P_e (TP_b[k_b] .* TF_a[k_a]), z_b = P_e (TP_a[k_a] .* TF_b[k_b]): with the outside vector fe of
+ *                    the cherry's edge the three edge values are fe.y and 2^(256 s) fe.z_a, 2^(256 s) fe.z_b.
+ * cherry[2 j], cherry[2 j + 1]: csr idx of the cherry's edge and of its first tip edge (the second's is one more).
+ */
 __global__ void f4_tables_kernel(const double *P, const double *Fm, const double *defs, const unsigned char *def_const,
                                  const int *edge_of_tip, const int *edge_of_int, int C, int E, int Et, int Ei, int K, int f_mode,
-                                 double *TP, double *Pint, double *TF, double *Fint)
+                                 double *TP, double *Pint, double *TF, double *Fint,
+                                 const int *cherry, int nch, double *chEm, unsigned int *chW, double *chOut)
 {
     const size_t cntT = (size_t)C * Et * K * 4, cntP = (size_t)C * Ei * 16;
     size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const size_t per = cntT + cntP;
-    if (idx >= per * (Fm ? 2 : 1)) return;
+    if (idx >= per * (Fm ? 2 : 1)) {
+        idx -= per * (Fm ? 2 : 1);
+        const int K2 = K * K;
+        if (idx >= (size_t)C * nch * K2) return;
+        const size_t jp = idx % ((size_t)nch * K2);
+        const int c = (int)(idx / ((size_t)nch * K2)), j = (int)(jp / K2), p = (int)(jp % K2), ka = p / K, kb = p % K;
+        const int ce = cherry[2 * j], ta = cherry[2 * j + 1];
+        const bool cst = def_const[ka] && def_const[kb];
+        double pa[4], pb[4], L[4], em[4];
+        for (int i = 0; i < 4; i++) {
+            pa[i] = f4_tip_entry(P, defs, def_const, c, E, ta, i, ka, 0);
+            pb[i] = f4_tip_entry(P, defs, def_const, c, E, ta + 1, i, kb, 0);
+            L[i] = pa[i];
+            L[i] *= pb[i];
+        }
+        const int sc = f4_rescale_up(L);
+        unsigned char *wbyte = reinterpret_cast<unsigned char *>(chW + jp);
+        wbyte[c] = (unsigned char)(sc | (cst ? 64 : 0));
+        if (c == C - 1) for (int u = C; u < 4; u++) wbyte[u] = 0;
+        const double *Pe = P + ((size_t)c * E + ce) * 16;
+        if (cst) for (int i = 0; i < 4; i++) em[i] = L[i];
+        else f4_table_mv(Pe, L, em);
+        const size_t ent = ((size_t)c * nch + j) * K2 + p;
+        for (int i = 0; i < 4; i++) chEm[ent * 4 + i] = em[i];
+        if (Fm) {
+            double y[4], wa[4], wb[4], *o = chOut + ent * 16;
+            f4_table_mv(Fm + ((size_t)c * E + ce) * 16, L, y);
+            if (cst && f_mode == 1) for (int i = 0; i < 4; i++) y[i] = 0.0;
+            for (int i = 0; i < 4; i++) {
+                wa[i] = pb[i] * f4_tip_entry(Fm, defs, def_const, c, E, ta, i, ka, f_mode);
+                wb[i] = pa[i] * f4_tip_entry(Fm, defs, def_const, c, E, ta + 1, i, kb, f_mode);
+            }
+            f4_table_mv(Pe, wa, o + 8);
+            f4_table_mv(Pe, wb, o + 12);
+            for (int i = 0; i < 4; i++) { o[i] = em[i]; o[4 + i] = y[i]; }
+        }
+        return;
+    }
     const bool second = idx >= per;
     if (second) idx -= per;
     const double *M = second ? Fm : P;
@@ -525,13 +616,7 @@ __global__ void f4_tables_kernel(const double *P, const double *Fm, const double
         const int i = (int)(idx % 4); size_t r = idx / 4;
         const int k = (int)(r % K); r /= K;
         const int te = (int)(r % Et), c = (int)(r / Et);
-        const double *row = M + (((size_t)c * E + edge_of_tip[te]) * 4 + i) * 4;
-        const double *d = defs + (size_t)k * 4;
-        double v;
-        if (def_const[k] && mode == 0) v = d[0];
-        else if (def_const[k] && mode == 1) v = 0.0;
-        else { v = 0.0; for (int j = 0; j < 4; j++) v = fma(row[j], d[j], v); }
-        (second ? TF : TP)[idx] = v;
+        (second ? TF : TP)[idx] = f4_tip_entry(M, defs, def_const, c, E, edge_of_tip[te], i, k, mode);
     } else {
         idx -= cntT;
         const int k = (int)(idx & 15); const size_t r = idx >> 4;
@@ -594,7 +679,9 @@ extern "C" void plf_destroy(plf_engine *e)
     DevBuf *bufs[] = {&e->d_indptr, &e->d_indices, &e->d_preorder, &e->d_node_has_data, &e->d_qhi, &e->d_qlo,
                       &e->d_edge_rates, &e->d_cat_rates, &e->d_cat_prior, &e->d_root_vec, &e->d_P, &e->d_D, &e->d_F,
                       &e->d_lhi, &e->d_llo, &e->d_expm_ws, &e->d_codes_in, &e->d_codes, &e->d_defs, &e->d_def_const,
-                      &e->d_def_ones, &e->d_site_w, &e->d_ops, &e->d_children, &e->d_TP, &e->d_TF, &e->d_Ptip, &e->d_block_marg, &e->d_marg_site, &e->d_scratch,
+                      &e->d_def_ones, &e->d_site_w, &e->prog.d_ops, &e->prog.d_children, &e->prog.d_TP, &e->prog.d_TF, &e->fold.d_ops,
+                      &e->fold.d_children, &e->fold.d_edge_of_int, &e->fold.d_edge_of_tip, &e->fold.d_cherry, &e->fold.d_TP,
+                      &e->fold.d_TF, &e->fold.d_Pint, &e->fold.d_Fint, &e->fold.d_chEm, &e->fold.d_chW, &e->fold.d_chOut, &e->d_Ptip, &e->d_block_marg, &e->d_marg_site, &e->d_scratch,
                       &e->d_scratchS, &e->d_block_ll, &e->d_block_edge, &e->d_edge_site, &e->d_sum, &e->d_site_ll,
                       &e->d_err, &e->d_mask, &e->g_Lg, &e->g_Kg, &e->g_Cg, &e->g_Eg, &e->g_Fg, &e->g_FK, &e->g_cat_lh,
                       &e->g_cat_k, &e->g_site_m, &e->g_site_k, &e->g_edge_out, &e->g_marg_out, &e->g_tr};
@@ -657,20 +744,35 @@ extern "C" int64_t plf_launch_count(plf_engine *e, int reset)
 /* tree                                                                */
 /* ------------------------------------------------------------------ */
 
-static int build_program(plf_engine *e)
+/*
+ * The post-order program of the fused kernels into p.  With fold, a cherry -- an internal node other than the root whose
+ * two children are tips, under a parent with two children, neither node carrying data of its own -- is no op of the
+ * program: its parent carries it as an F4_KIND_CHERRY child that reads per-code-pair tables (f4_tables_kernel).  The
+ * parent multiplies two factors and no data row, so the order of its children does not change the bits: the
+ * log-likelihood keeps those of the unfolded program.  Tile rows are shared: the rows of e->code_row_node are kept
+ * and extended.
+ */
+static int build_program(plf_engine *e, F4Program &p, bool fold)
 {
     const int N = e->N;
     std::vector<int> need(N, 0), slot(N, -1);
     std::vector<std::vector<int>> ichild(N);   /* internal children (csr edge idx) sorted for visiting */
     e->max_degree = 0;
     auto is_leaf = [&](int v) { return e->indptr[v] == e->indptr[v + 1]; };
+    auto has_data = [&](int v) { return !e->node_has_data_h.empty() && e->node_has_data_h[v]; };
+    std::vector<int> parent(N, -1);
+    for (int a = 0; a < N; a++) for (int idx = e->indptr[a]; idx < e->indptr[a + 1]; idx++) parent[e->indices[idx]] = a;
+    auto deg = [&](int v) { return e->indptr[v + 1] - e->indptr[v]; };
+    auto is_cherry = [&](int v) {
+        return fold && v != e->root && deg(v) == 2 && is_leaf(e->indices[e->indptr[v]]) && is_leaf(e->indices[e->indptr[v] + 1]) &&
+               !has_data(v) && deg(parent[v]) == 2 && !has_data(parent[v]);
+    };
     for (int u = N - 1; u >= 0; u--) {
         int a = e->preorder[u];
-        int deg = e->indptr[a + 1] - e->indptr[a];
-        e->max_degree = std::max(e->max_degree, deg);
+        e->max_degree = std::max(e->max_degree, deg(a));
         std::vector<int> &ic = ichild[a];
         for (int idx = e->indptr[a]; idx < e->indptr[a + 1]; idx++)
-            if (!is_leaf(e->indices[idx])) ic.push_back(idx);
+            if (!is_leaf(e->indices[idx]) && !is_cherry(e->indices[idx])) ic.push_back(idx);
         std::stable_sort(ic.begin(), ic.end(), [&](int x, int y) { return need[e->indices[x]] > need[e->indices[y]]; });
         int nd = 0;
         for (size_t j = 0; j < ic.size(); j++) nd = std::max(nd, (int)j + need[e->indices[ic[j]]]);
@@ -694,10 +796,11 @@ static int build_program(plf_engine *e)
             }
         }
     }
-    e->ops.clear(); e->children.clear();
-    e->edge_of_int.clear(); e->edge_of_tip.clear(); e->code_row_node.clear();
+    p.ops.clear(); p.children.clear();
+    p.edge_of_int.clear(); p.edge_of_tip.clear(); p.cherry.clear();
     for (size_t o = 0; o < order.size(); o++) slot[order[o]] = (int)o;
     std::vector<int> code_row(N, -1);
+    for (size_t r = 0; r < e->code_row_node.size(); r++) code_row[e->code_row_node[r]] = (int)r;
     auto row_of = [&](int node) {
         if (code_row[node] < 0) { code_row[node] = (int)e->code_row_node.size(); e->code_row_node.push_back(node); }
         return code_row[node];
@@ -707,8 +810,8 @@ static int build_program(plf_engine *e)
     for (size_t o = 0; o < order.size(); o++) {
         int a = order[o];
         F4Op op;
-        op.node = a; op.first_child = (int)e->children.size(); op.nchild = 0; op.slot = (int)o;
-        op.code_row = (!e->node_has_data_h.empty() && e->node_has_data_h[a]) ? row_of(a) : -1;
+        op.node = a; op.first_child = (int)p.children.size(); op.nchild = 0; op.slot = (int)o;
+        op.code_row = has_data(a) ? row_of(a) : -1;
         op.spill_before = 0;
         const std::vector<int> &ic = ichild[a];
         int cur_edge = -1;
@@ -721,9 +824,9 @@ static int build_program(plf_engine *e)
         auto add_internal = [&](int idx, int b, int kind) {
             F4Child ch;
             memset(&ch, 0, sizeof(ch));
-            ch.kind = kind; ch.slot = slot[b]; ch.mat = (int)e->edge_of_int.size(); ch.code_row = -1; ch.edge = idx; ch.node = b;
-            e->edge_of_int.push_back(idx);
-            e->children.push_back(ch); op.nchild++;
+            ch.kind = kind; ch.slot = slot[b]; ch.mat = (int)p.edge_of_int.size(); ch.code_row = -1; ch.edge = idx; ch.node = b;
+            p.edge_of_int.push_back(idx);
+            p.children.push_back(ch); op.nchild++;
         };
         if (cur_edge != -1) add_internal(cur_edge, cur, F4_KIND_CUR);
         size_t nstack = ic.size() - (cur_edge != -1 ? 1 : 0);
@@ -737,20 +840,32 @@ static int build_program(plf_engine *e)
         }
         for (int idx = e->indptr[a]; idx < e->indptr[a + 1]; idx++) {
             int b = e->indices[idx];
+            if (is_cherry(b)) {
+                F4Child ch;
+                memset(&ch, 0, sizeof(ch));
+                const int ta = e->indptr[b];
+                ch.kind = F4_KIND_CHERRY; ch.slot = -1; ch.mat = p.ncherry(); ch.edge = idx; ch.node = b;
+                ch.code_row = row_of(e->indices[ta]); ch.code_row_b = row_of(e->indices[ta + 1]); ch.tip_edge = ta;
+                p.cherry.push_back(idx); p.cherry.push_back(ta);
+                p.children.push_back(ch); op.nchild++;
+            }
+        }
+        for (int idx = e->indptr[a]; idx < e->indptr[a + 1]; idx++) {
+            int b = e->indices[idx];
             if (is_leaf(b)) {
                 F4Child ch;
                 memset(&ch, 0, sizeof(ch));
-                ch.kind = F4_KIND_TIP; ch.slot = -1; ch.mat = (int)e->edge_of_tip.size(); ch.code_row = row_of(b); ch.edge = idx; ch.node = b;
-                e->edge_of_tip.push_back(idx);
-                e->children.push_back(ch); op.nchild++;
+                ch.kind = F4_KIND_TIP; ch.slot = -1; ch.mat = (int)p.edge_of_tip.size(); ch.code_row = row_of(b); ch.edge = idx; ch.node = b;
+                p.edge_of_tip.push_back(idx);
+                p.children.push_back(ch); op.nchild++;
             }
         }
-        e->ops.push_back(op);
+        p.ops.push_back(op);
         cur = a;
     }
     if (!stk.empty()) { e->err = "internal error: fused program leaves a non-empty stack"; return -1; }
-    e->stack_depth = maxdepth;
-    e->nslots = (int)order.size();
+    p.stack_depth = maxdepth;
+    p.nslots = (int)order.size();
     return 0;
 }
 
@@ -793,7 +908,7 @@ extern "C" int plf_set_tree(plf_engine *e, int node_count, const int *indptr, co
     CK(e, cudaMemcpyAsync(e->d_indices.p, indices, sizeof(int) * E, cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaMemcpyAsync(e->d_preorder.p, preorder, sizeof(int) * N, cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaStreamSynchronize(e->stream));
-    e->P_valid = e->D_valid = e->TP_valid = e->dm_valid = false;
+    e->P_valid = e->D_valid = e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     e->S = 0;   /* data must be (re)set after the tree */
     return 0;
 }
@@ -840,7 +955,7 @@ extern "C" int plf_set_model(plf_engine *e, int n, int C, const double *q_hi, co
     CK(e, cudaMemcpyAsync(e->d_cat_prior.p, e->cat_prior.data(), sizeof(double) * C, cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaMemcpyAsync(e->d_root_vec.p, e->root_vec.data(), sizeof(double) * n, cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaStreamSynchronize(e->stream));
-    e->P_valid = e->D_valid = e->TP_valid = e->dm_valid = false;
+    e->P_valid = e->D_valid = e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     return 0;
 }
 
@@ -855,7 +970,7 @@ extern "C" int plf_set_edge_rates(plf_engine *e, const double *edge_rates)
     /* no wait here: a copy from pageable memory has left the host buffer (for the driver's staging area) when the call
      * returns, and everything that reads d_edge_rates is launched on the same stream */
     CK(e, cudaMemcpyAsync(e->d_edge_rates.p, e->edge_rates.data(), sizeof(double) * e->E, cudaMemcpyHostToDevice, e->stream));
-    e->P_valid = e->D_valid = e->TP_valid = e->dm_valid = false;
+    e->P_valid = e->D_valid = e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     return 0;
 }
 
@@ -901,7 +1016,7 @@ static int ensure_matrices(plf_engine *e, bool need_D)
     if (run_expm(e, e->d_P.as<double>(), need_D ? e->d_D.as<double>() : nullptr, nullptr, 0, nullptr, nullptr, nullptr)) return -1;
     e->P_valid = true;
     if (need_D) e->D_valid = true;
-    e->TP_valid = e->dm_valid = false;
+    e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     return 0;
 }
 
@@ -1034,7 +1149,7 @@ static int set_data_common(plf_engine *e, int64_t S, int K, const double *defs, 
     if (!e->flags_pinned) CK(e, cudaMallocHost((void **)&e->flags_pinned, 1 << 16));
     if (N > (1 << 16) - 8) FAIL(e, "plf_set_data: more than 65528 nodes");
     e->S = S; e->K = K; e->code_bytes = dev_bytes;
-    e->TP_valid = e->dm_valid = false;
+    e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     e->have_w = false;
     CK(e, cudaMemcpyAsync(e->d_defs.p, defs, sizeof(double) * K * n, cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaMemcpyAsync(e->d_def_const.p, dconst.data(), K, cudaMemcpyHostToDevice, e->stream));
@@ -1138,32 +1253,88 @@ struct Query {
     double *dwell_out = nullptr, *trans_out = nullptr;  /* [E][n][n] */
 };
 
+static int upload_program(plf_engine *e, F4Program &p)
+{
+    ENSURE(e, p.d_ops, sizeof(F4Op) * p.ops.size());
+    ENSURE(e, p.d_children, sizeof(F4Child) * p.children.size());
+    ENSURE(e, p.d_edge_of_int, sizeof(int) * (p.edge_of_int.size() + 1));
+    ENSURE(e, p.d_edge_of_tip, sizeof(int) * (p.edge_of_tip.size() + 1));
+    ENSURE(e, p.d_cherry, sizeof(int) * (p.cherry.size() + 1));
+    CK(e, cudaMemcpyAsync(p.d_ops.p, p.ops.data(), sizeof(F4Op) * p.ops.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaMemcpyAsync(p.d_children.p, p.children.data(), sizeof(F4Child) * p.children.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaMemcpyAsync(p.d_edge_of_int.p, p.edge_of_int.data(), sizeof(int) * p.edge_of_int.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaMemcpyAsync(p.d_edge_of_tip.p, p.edge_of_tip.data(), sizeof(int) * p.edge_of_tip.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaMemcpyAsync(p.d_cherry.p, p.cherry.data(), sizeof(int) * p.cherry.size(), cudaMemcpyHostToDevice, e->stream));
+    return 0;
+}
+
 static int ensure_program(plf_engine *e)
 {
     if (!e->program_dirty) return 0;
-    if (build_program(e)) return -1;
-    ENSURE(e, e->d_ops, sizeof(F4Op) * e->ops.size());
-    ENSURE(e, e->d_children, sizeof(F4Child) * e->children.size());
-    ENSURE(e, e->d_edge_of_int, sizeof(int) * (e->edge_of_int.size() + 1));
-    ENSURE(e, e->d_edge_of_tip, sizeof(int) * (e->edge_of_tip.size() + 1));
+    e->code_row_node.clear();
+    if (build_program(e, e->prog, false) || build_program(e, e->fold, true)) return -1;
+    if (upload_program(e, e->prog) || upload_program(e, e->fold)) return -1;
     ENSURE(e, e->d_code_row_node, sizeof(int) * (e->code_row_node.size() + 1));
-    CK(e, cudaMemcpyAsync(e->d_ops.p, e->ops.data(), sizeof(F4Op) * e->ops.size(), cudaMemcpyHostToDevice, e->stream));
-    CK(e, cudaMemcpyAsync(e->d_children.p, e->children.data(), sizeof(F4Child) * e->children.size(), cudaMemcpyHostToDevice, e->stream));
-    CK(e, cudaMemcpyAsync(e->d_edge_of_int.p, e->edge_of_int.data(), sizeof(int) * e->edge_of_int.size(), cudaMemcpyHostToDevice, e->stream));
-    CK(e, cudaMemcpyAsync(e->d_edge_of_tip.p, e->edge_of_tip.data(), sizeof(int) * e->edge_of_tip.size(), cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaMemcpyAsync(e->d_code_row_node.p, e->code_row_node.data(), sizeof(int) * e->code_row_node.size(), cudaMemcpyHostToDevice, e->stream));
     CK(e, cudaStreamSynchronize(e->stream));
     e->program_dirty = false;
     e->program_version++;
-    e->TP_valid = e->dm_valid = false;
+    e->prog.TP_valid = e->fold.TP_valid = e->dm_valid = false;
     return 0;
 }
 
-/* compact matrices of the internal-child edges and tip tables for the fused kernel */
-static int ensure_tip_tables(plf_engine *e, const double *Fm, int f_mode, bool want_ptip = false)
+/*
+ * Whether an ll (kind 0) or edge-form (kind 1) query runs the folded program: it has cherries, the model at most four
+ * categories (one launch; the scale word has a byte per category), and the tables the kernel stages in shared memory
+ * -- C nch K^2 inside vectors and nch K^2 scale words -- stay within F4_FOLD_SMEM and leave the smallest configuration
+ * room.  Beyond that (many characters: probability-array data with many distinct rows, a large tree) today's program
+ * runs.
+ */
+#define F4_FOLD_SMEM (80 * 1024)
+static size_t f4_smem_bytes(const plf_engine *e, const F4Program &p, int kind, int bd, int staged, bool pack = false, bool cm = false,
+                            bool gstack = false);
+static size_t f4_fold_bytes(const plf_engine *e, const F4Program &p)
+{
+    const size_t K2 = (size_t)e->K * e->K;
+    return f4_align16(sizeof(double) * 4 * std::min(e->C, 4) * p.ncherry() * K2) + f4_align16(sizeof(unsigned int) * p.ncherry() * K2);
+}
+static bool f4_use_fold(const plf_engine *e, int kind)
+{
+    return kind <= 1 && e->C <= 4 && e->fold.ncherry() > 0 && f4_fold_bytes(e, e->fold) <= F4_FOLD_SMEM &&
+           f4_smem_bytes(e, e->fold, 1, 128, 0) <= 227 * 1024;
+}
+
+/* compact matrices of the internal-child edges and tip tables for the fused kernel: of the folded program (with its
+ * cherry tables, one launch) when the query runs it, else of the engine's program */
+static int ensure_tip_tables(plf_engine *e, const double *Fm, int f_mode, bool want_ptip, bool fold)
 {
     if (ensure_program(e)) return -1;
-    const int Ei = (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
+    if (fold) {
+        F4Program &p = e->fold;
+        if (p.TP_valid && !Fm) return 0;
+        const int Ei = (int)p.edge_of_int.size(), Et = (int)p.edge_of_tip.size(), nch = p.ncherry();
+        const size_t cntT = (size_t)e->C * Et * e->K * 4, cntP = (size_t)e->C * Ei * 16, nent = (size_t)e->C * nch * e->K * e->K;
+        ENSURE(e, p.d_TP, sizeof(double) * (cntT + 1));
+        ENSURE(e, p.d_Pint, sizeof(double) * (cntP + 1));
+        ENSURE(e, p.d_chEm, sizeof(double) * 4 * nent);
+        ENSURE(e, p.d_chW, sizeof(unsigned int) * (size_t)nch * e->K * e->K);
+        if (Fm) {
+            ENSURE(e, p.d_TF, sizeof(double) * (cntT + 1));
+            ENSURE(e, p.d_Fint, sizeof(double) * (cntP + 1));
+            ENSURE(e, p.d_chOut, sizeof(double) * 16 * nent);
+        }
+        const size_t total = (Fm ? 2 : 1) * (cntT + cntP) + nent;
+        const int threads = 256;
+        f4_tables_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, e->stream>>>(
+            e->d_P.as<double>(), Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), p.d_edge_of_tip.as<int>(),
+            p.d_edge_of_int.as<int>(), e->C, e->E, Et, Ei, e->K, f_mode, p.d_TP.as<double>(), p.d_Pint.as<double>(),
+            p.d_TF.as<double>(), p.d_Fint.as<double>(), p.d_cherry.as<int>(), nch, p.d_chEm.as<double>(),
+            p.d_chW.as<unsigned int>(), p.d_chOut.as<double>());
+        KCHECK(e);
+        p.TP_valid = true;
+        return 0;
+    }
+    const int Ei = (int)e->prog.edge_of_int.size(), Et = (int)e->prog.edge_of_tip.size();
     const size_t cntT = (size_t)e->C * Et * e->K * e->n, cntP = (size_t)e->C * Ei * 16;
     const int threads = 256;
     if (want_ptip) {
@@ -1172,53 +1343,53 @@ static int ensure_tip_tables(plf_engine *e, const double *Fm, int f_mode, bool w
         ENSURE(e, e->d_Ptip, sizeof(double) * (cntPt + 1));
         if (cntPt) {
             compact_matrices_kernel<<<(unsigned)((cntPt + threads - 1) / threads), threads, 0, e->stream>>>(
-                e->d_P.as<double>(), e->d_edge_of_tip.as<int>(), e->C, e->E, Et, e->d_Ptip.as<double>());
+                e->d_P.as<double>(), e->prog.d_edge_of_tip.as<int>(), e->C, e->E, Et, e->d_Ptip.as<double>());
             KCHECK(e);
         }
     }
-    if (!e->TP_valid && Fm && cntT && cntP && e->n == 4) {
+    if (!e->prog.TP_valid && Fm && cntT && cntP && e->n == 4) {
         /* the usual case of an optimisation step (matrices changed, edge forms wanted): one launch for all four tables */
-        ENSURE(e, e->d_TP, sizeof(double) * (cntT + 1));
-        ENSURE(e, e->d_Pint, sizeof(double) * (cntP + 1));
-        ENSURE(e, e->d_TF, sizeof(double) * (cntT + 1));
-        ENSURE(e, e->d_Fint, sizeof(double) * (cntP + 1));
+        ENSURE(e, e->prog.d_TP, sizeof(double) * (cntT + 1));
+        ENSURE(e, e->prog.d_Pint, sizeof(double) * (cntP + 1));
+        ENSURE(e, e->prog.d_TF, sizeof(double) * (cntT + 1));
+        ENSURE(e, e->prog.d_Fint, sizeof(double) * (cntP + 1));
         const size_t total = 2 * (cntT + cntP);
         f4_tables_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, e->stream>>>(
-            e->d_P.as<double>(), Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->d_edge_of_tip.as<int>(),
-            e->d_edge_of_int.as<int>(), e->C, e->E, Et, Ei, e->K, f_mode, e->d_TP.as<double>(), e->d_Pint.as<double>(),
-            e->d_TF.as<double>(), e->d_Fint.as<double>());
+            e->d_P.as<double>(), Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->prog.d_edge_of_tip.as<int>(),
+            e->prog.d_edge_of_int.as<int>(), e->C, e->E, Et, Ei, e->K, f_mode, e->prog.d_TP.as<double>(), e->prog.d_Pint.as<double>(),
+            e->prog.d_TF.as<double>(), e->prog.d_Fint.as<double>(), nullptr, 0, nullptr, nullptr, nullptr);
         KCHECK(e);
-        e->TP_valid = true;
+        e->prog.TP_valid = true;
         return 0;
     }
-    if (!e->TP_valid) {
-        ENSURE(e, e->d_TP, sizeof(double) * (cntT + 1));
-        ENSURE(e, e->d_Pint, sizeof(double) * (cntP + 1));
+    if (!e->prog.TP_valid) {
+        ENSURE(e, e->prog.d_TP, sizeof(double) * (cntT + 1));
+        ENSURE(e, e->prog.d_Pint, sizeof(double) * (cntP + 1));
         if (cntT) {
             tip_table_kernel<<<(unsigned)((cntT + threads - 1) / threads), threads, 0, e->stream>>>(
                 e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), e->C, e->E, Et, e->K, e->n, 0, e->d_TP.as<double>());
+                e->prog.d_edge_of_tip.as<int>(), e->C, e->E, Et, e->K, e->n, 0, e->prog.d_TP.as<double>());
             KCHECK(e);
         }
         if (cntP) {
             compact_matrices_kernel<<<(unsigned)((cntP + threads - 1) / threads), threads, 0, e->stream>>>(
-                e->d_P.as<double>(), e->d_edge_of_int.as<int>(), e->C, e->E, Ei, e->d_Pint.as<double>());
+                e->d_P.as<double>(), e->prog.d_edge_of_int.as<int>(), e->C, e->E, Ei, e->prog.d_Pint.as<double>());
             KCHECK(e);
         }
-        e->TP_valid = true;
+        e->prog.TP_valid = true;
     }
     if (Fm) {
-        ENSURE(e, e->d_TF, sizeof(double) * (cntT + 1));
-        ENSURE(e, e->d_Fint, sizeof(double) * (cntP + 1));
+        ENSURE(e, e->prog.d_TF, sizeof(double) * (cntT + 1));
+        ENSURE(e, e->prog.d_Fint, sizeof(double) * (cntP + 1));
         if (cntT) {
             tip_table_kernel<<<(unsigned)((cntT + threads - 1) / threads), threads, 0, e->stream>>>(
                 Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), e->C, e->E, Et, e->K, e->n, f_mode, e->d_TF.as<double>());
+                e->prog.d_edge_of_tip.as<int>(), e->C, e->E, Et, e->K, e->n, f_mode, e->prog.d_TF.as<double>());
             KCHECK(e);
         }
         if (cntP) {
             compact_matrices_kernel<<<(unsigned)((cntP + threads - 1) / threads), threads, 0, e->stream>>>(
-                Fm, e->d_edge_of_int.as<int>(), e->C, e->E, Ei, e->d_Fint.as<double>());
+                Fm, e->prog.d_edge_of_int.as<int>(), e->C, e->E, Ei, e->prog.d_Fint.as<double>());
             KCHECK(e);
         }
     }
@@ -1318,14 +1489,14 @@ static cudaEvent_t g_cm_done[64];
 static int f4_kind(const Query &q) { return q.want_gmat ? 3 : (q.want_marg ? 2 : (q.want_edge ? 1 : 0)); }
 
 /* mirrors the shared-memory carve-up at the top of fused4_kernel */
-static size_t f4_smem_bytes(const plf_engine *e, int kind, int bd, int staged, bool pack = false, bool cm = false,
-                            bool gstack = false)
+static size_t f4_smem_bytes(const plf_engine *e, const F4Program &p, int kind, int bd, int staged, bool pack, bool cm,
+                            bool gstack)
 {
-    const int sdepth = gstack ? 0 : e->stack_depth;
-    const int C = std::min(e->C, 4), Ei = cm ? 0 : (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
+    const int sdepth = gstack ? 0 : p.stack_depth;
+    const int C = std::min(e->C, 4), Ei = cm ? 0 : (int)p.edge_of_int.size(), Et = (int)p.edge_of_tip.size();
     size_t off = 0;
-    off = f4_align16(off + (cm ? 0 : sizeof(F4Op) * e->ops.size()));
-    off = f4_align16(off + (cm ? 0 : sizeof(F4Child) * e->children.size()));
+    off = f4_align16(off + (cm ? 0 : sizeof(F4Op) * p.ops.size()));
+    off = f4_align16(off + (cm ? 0 : sizeof(F4Child) * p.children.size()));
     off = f4_align16(off + sizeof(double) * 4 * C * bd);
     off = f4_align16(off + (kind == 1 ? sizeof(double) * (bd / 32) * e->E : 0));
     off = f4_align16(off + (kind ? 0 : sizeof(double) * 4 * C * bd * sdepth));
@@ -1333,6 +1504,7 @@ static size_t f4_smem_bytes(const plf_engine *e, int kind, int bd, int staged, b
     off = f4_align16(off + (pack ? (e->code_row_node.size() + 1) / 2 : e->code_row_node.size()) * bd);
     off = f4_align16(off + e->K);
     off = f4_align16(off + sizeof(double) * 4 * e->K);
+    if (kind <= 1) off += f4_fold_bytes(e, p);
     const size_t nP = (size_t)C * Ei * 16 * sizeof(double), nT = (size_t)C * Et * e->K * 4 * sizeof(double);
     const size_t nF = kind == 2 ? (size_t)C * Et * 16 * sizeof(double) : nP;
     if (staged) off += nP + nT + ((kind == 1 || kind == 2) ? nF : 0) + ((kind == 1 && staged == 2) ? nT : 0);
@@ -1342,7 +1514,7 @@ static size_t f4_smem_bytes(const plf_engine *e, int kind, int bd, int staged, b
 /* an outside pass is checked with the layout of the edge forms, the largest unstaged one */
 static bool fused_fits(const plf_engine *e, bool outside)
 {
-    return f4_smem_bytes(e, outside ? 1 : 0, 128, 0) <= 227 * 1024;
+    return f4_smem_bytes(e, e->prog, outside ? 1 : 0, 128, 0) <= 227 * 1024;
 }
 
 /* dwell[e] = sum_c W[c][e], trans[e] = sum_c rate_c t_e W[c][e] (categories in order) */
@@ -1422,17 +1594,17 @@ static int64_t f4_tune_sites(const plf_engine *e) { return (int64_t)e->sm_count 
  * made of each instantiation (tools/check_cm_uniform.sh), so the first large query times the leading candidates on a
  * sample of the sites and keeps the fastest.
  */
-static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool &tune)
+static int f4_choose(plf_engine *e, const F4Program &p, int kind, F4Slot *&slot, size_t &pick, bool &tune)
 {
     slot = &e->f4_slot[5 * kind + e->C];
     const char *force = getenv(kind >= 2 ? "PLF_F4_CONFIG_MARG" : (kind ? "PLF_F4_CONFIG" : "PLF_F4_CONFIG_LL"));
     const std::string cand_key = std::to_string(e->program_version) + "/" + std::to_string(e->C) + "/" + std::to_string(e->K) + "/" +
-                                 std::to_string(e->E) + "/" + (force ? force : "");
+                                 std::to_string(e->E) + "/" + (force ? force : "") + (&p == &e->fold ? "/fold" : "");
     if (slot->cand_key != cand_key) {
         const bool can_pack = e->K <= 16;
-        bool can_cm = (size_t)e->C * e->edge_of_int.size() * 16 <= F4_CM_MAXD && e->ops.size() <= F4_CM_MAXOPS &&
-                      e->children.size() <= F4_CM_MAXCH && e->device < 64;
-        for (const F4Op &op : e->ops) if (op.nchild != 2) can_cm = false;     /* CM kernels carry the two-children step only */
+        bool can_cm = (size_t)e->C * p.edge_of_int.size() * 16 <= F4_CM_MAXD && p.ops.size() <= F4_CM_MAXOPS &&
+                      p.children.size() <= F4_CM_MAXCH && e->device < 64;
+        for (const F4Op &op : p.ops) if (op.nchild != 2) can_cm = false;     /* CM kernels carry the two-children step only */
         const std::vector<F4Config> &cfgs = f4_configs[std::min(kind, 2)];
         std::vector<Cand> viable;
         size_t smem = 0;
@@ -1441,7 +1613,7 @@ static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool 
             if ((force && atoi(force) != i) || (f.pack && !can_pack) || (f.cm && !can_cm)) continue;
             Cand c{f, f4_get_kernel(f.bd, f.staged, f.pack, f.cm, e->C, kind), 0, 0};
             if (!c.k) continue;
-            c.smem = smem = f4_smem_bytes(e, kind, c.bd, c.staged, c.pack, c.cm, c.gstack);
+            c.smem = smem = f4_smem_bytes(e, p, kind, c.bd, c.staged, c.pack, c.cm, c.gstack);
             if (c.smem > 227 * 1024) continue;
             CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
             CK(e, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.per_sm, c.k, c.bd, c.smem));
@@ -1450,6 +1622,7 @@ static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool 
         if (viable.empty()) FAIL(e, "fused kernel: no configuration fits (C = %d, %zu bytes of shared memory)", e->C, smem);
         slot->cand_key = cand_key;
         slot->cands = std::move(viable);
+        slot->tuned_version = ~(uint64_t)0;      /* a pick among other candidates */
     }
     const std::vector<Cand> &viable = slot->cands;
     const bool can_tune = viable.size() > 1 && e->S >= f4_tune_sites(e) / 2;
@@ -1468,30 +1641,38 @@ static int f4_choose(plf_engine *e, int kind, F4Slot *&slot, size_t &pick, bool 
  * outputs go to these device buffers. */
 struct F4Window { int c0; double *site_ll, *site_edge, *site_marg; };
 
+/* the program a fused query of this kind runs (category windows: the engine's) */
+static const F4Program &f4_program(const plf_engine *e, int kind, const F4Window *win)
+{
+    return (!win && f4_use_fold(e, kind)) ? e->fold : e->prog;
+}
+
 /* what the reduction of a fused query needs from its launches */
 struct F4Launch { F4Args a; const Cand *use; int grid; size_t nchunk; bool pipelined; };
 
 /* the arguments of a fused launch that do not depend on its configuration */
-static void f4_fill_args(const plf_engine *e, const Query &q, int kind, const F4Window *win, F4Args &a)
+static void f4_fill_args(const plf_engine *e, const F4Program &p, const Query &q, int kind, const F4Window *win, F4Args &a)
 {
     memset(&a, 0, sizeof(a));
-    a.nops = (int)e->ops.size(); a.nchildren = (int)e->children.size();
-    a.ops = e->d_ops.as<F4Op>(); a.children = e->d_children.as<F4Child>();
+    a.nops = (int)p.ops.size(); a.nchildren = (int)p.children.size();
+    a.ops = p.d_ops.as<F4Op>(); a.children = p.d_children.as<F4Child>();
     a.E = e->E; a.K = e->K; a.S = e->S; a.N = e->N;
-    a.Ei = (int)e->edge_of_int.size(); a.Et = (int)e->edge_of_tip.size();
+    a.Ei = (int)p.edge_of_int.size(); a.Et = (int)p.edge_of_tip.size();
     a.ncode_rows = (int)e->code_row_node.size();
     a.code_row_node = e->d_code_row_node.as<int>();
     a.codes = e->d_codes.as<unsigned char>();
     a.defs = e->d_defs.as<double>(); a.def_const = e->d_def_const.as<unsigned char>();
-    a.Pint = e->d_Pint.as<double>(); a.TP = e->d_TP.as<double>();
-    a.Fint = kind == 2 ? e->d_Ptip.as<double>() : (kind == 1 ? e->d_Fint.as<double>() : nullptr);
-    a.TF = kind == 1 ? e->d_TF.as<double>() : nullptr;
+    a.Pint = p.d_Pint.as<double>(); a.TP = p.d_TP.as<double>();
+    a.Fint = kind == 2 ? e->d_Ptip.as<double>() : (kind == 1 ? p.d_Fint.as<double>() : nullptr);
+    a.TF = kind == 1 ? p.d_TF.as<double>() : nullptr;
     a.f_zero_rowsum = q.f_zero_rowsum;
     a.cat_prior = e->d_cat_prior.as<double>();
     a.root_mode = e->root_mode;
     for (int i = 0; i < 4; i++) a.root_vec[i] = e->root_vec[i];
     a.site_w = e->have_w ? e->d_site_w.as<double>() : nullptr;
-    a.stack_depth = e->stack_depth; a.nslots = e->nslots;
+    a.stack_depth = p.stack_depth; a.nslots = p.nslots;
+    a.nch = p.ncherry();
+    a.chEm = p.d_chEm.as<double>(); a.chW = p.d_chW.as<unsigned int>(); a.chOut = kind == 1 ? p.d_chOut.as<double>() : nullptr;
     if (win) {
         /* the tables are laid out [category][...]: a window is a pointer offset */
         const size_t c0 = (size_t)win->c0;
@@ -1509,7 +1690,7 @@ static int f4_grid(const plf_engine *e, const Cand &c, int64_t longest)
 }
 
 /* times each leading candidate on the first sites (results are overwritten by the real run) and keeps the fastest */
-static int f4_tune(plf_engine *e, F4Slot *slot, F4Args &a, int64_t longest, size_t &pick)
+static int f4_tune(plf_engine *e, const F4Program &p, F4Slot *slot, F4Args &a, int64_t longest, size_t &pick)
 {
     const std::vector<Cand> &viable = slot->cands;
     float best = 0.f;
@@ -1517,7 +1698,7 @@ static int f4_tune(plf_engine *e, F4Slot *slot, F4Args &a, int64_t longest, size
     a.s_begin = 0; a.s_end = std::min<int64_t>(e->S, f4_tune_sites(e));
     for (size_t i = 0; i < ntry; i++) {
         const Cand &c = viable[i];
-        a.gstack = c.gstack ? 1 : 0; a.stack_depth = c.gstack ? 0 : e->stack_depth;
+        a.gstack = c.gstack ? 1 : 0; a.stack_depth = c.gstack ? 0 : p.stack_depth;
         /* candidates may share a kernel function with different amounts of dynamic shared memory */
         CK(e, cudaFuncSetAttribute(c.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
         float ms = 0.f;
@@ -1545,11 +1726,12 @@ static int f4_tune(plf_engine *e, F4Slot *slot, F4Args &a, int64_t longest, size
  */
 static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *win, F4Launch &L)
 {
+    const F4Program &p = f4_program(e, kind, win);
     F4Slot *slot = nullptr; size_t pick = 0; bool tune = false;
-    if (f4_choose(e, kind, slot, pick, tune)) return -1;
+    if (f4_choose(e, p, kind, slot, pick, tune)) return -1;
     const std::vector<Cand> &viable = slot->cands;
     F4Args &a = L.a;
-    f4_fill_args(e, q, kind, win, a);
+    f4_fill_args(e, p, q, kind, win, a);
     L.pipelined = e->pend_active;
     std::vector<int64_t> bounds;
     if (L.pipelined) bounds = e->pend_bounds; else { bounds.push_back(0); bounds.push_back(e->S); }
@@ -1574,8 +1756,8 @@ static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *wi
     /* the site log-likelihoods are always kept: the zero-likelihood check of every query kind reads them */
     a.site_ll = win ? win->site_ll : e->d_site_ll.as<double>();
     if (kind) {
-        ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * e->nslots * Tmax);
-        ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)e->nslots * Tmax);
+        ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * p.nslots * Tmax);
+        ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)p.nslots * Tmax);
         if (kind == 1) ENSURE(e, e->d_block_edge, sizeof(double) * (size_t)gmax * e->E * L.nchunk);
         a.scratch = e->d_scratch.as<double4>(); a.scratchS = e->d_scratchS.as<unsigned int>();
         a.block_edge = e->d_block_edge.as<double>();
@@ -1608,9 +1790,9 @@ static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *wi
             a.edge_site_out = e->d_edge_site.as<double>();
         }
     }
-    if (!kind && any_gstack && e->stack_depth > 0) {
-        ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * e->stack_depth * Tmax);
-        ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)e->stack_depth * Tmax);
+    if (!kind && any_gstack && p.stack_depth > 0) {
+        ENSURE(e, e->d_scratch, sizeof(double4) * (size_t)e->C * p.stack_depth * Tmax);
+        ENSURE(e, e->d_scratchS, sizeof(unsigned int) * (size_t)p.stack_depth * Tmax);
         a.scratch = e->d_scratch.as<double4>(); a.scratchS = e->d_scratchS.as<unsigned int>();
     }
     std::unique_lock<std::mutex> cm_lock(g_cm_mutex, std::defer_lock);
@@ -1623,17 +1805,17 @@ static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *wi
     if (any_cm) {
         /* program as a kernel parameter, matrices into the constant bank (ordered against other engines) */
         memset(&e->prog_h, 0, sizeof(F4Prog));
-        memcpy(e->prog_h.ops, e->ops.data(), sizeof(F4Op) * e->ops.size());
-        memcpy(e->prog_h.ch, e->children.data(), sizeof(F4Child) * e->children.size());
+        memcpy(e->prog_h.ops, p.ops.data(), sizeof(F4Op) * p.ops.size());
+        memcpy(e->prog_h.ch, p.children.data(), sizeof(F4Child) * p.children.size());
         cm_lock.lock();
         if (!g_cm_done[e->device]) CK(e, cudaEventCreateWithFlags(&g_cm_done[e->device], cudaEventDisableTiming));
         CK(e, cudaStreamWaitEvent(e->stream, g_cm_done[e->device], 0));
         cm_guard.ev = &g_cm_done[e->device]; cm_guard.st = e->stream;
-        const size_t nP = sizeof(double) * (size_t)e->C * e->edge_of_int.size() * 16;
+        const size_t nP = sizeof(double) * (size_t)e->C * p.edge_of_int.size() * 16;
         CK(e, f4_upload_const(a.Pint, kind ? a.Fint : nullptr, nP, e->stream));
     }
     if (tune) {
-        if (f4_tune(e, slot, a, longest, pick)) return -1;
+        if (f4_tune(e, p, slot, a, longest, pick)) return -1;
         CK(e, cudaMemsetAsync(e->d_err.p, 0, sizeof(int), e->stream));
         /* the marginal accumulators are added to by every launch: forget what the timing runs left there */
         if (kind == 2 && a.block_marg)
@@ -1647,7 +1829,7 @@ static int f4_launch(plf_engine *e, const Query &q, int kind, const F4Window *wi
         snprintf(nm, sizeof nm, "fused4_kernel<%d,%d,%d,%d,%d,%d>", e->C, kind, use.bd, use.staged, use.pack ? 1 : 0, use.cm ? 1 : 0);
         e->last_kernel = nm;
     }
-    a.gstack = use.gstack ? 1 : 0; a.stack_depth = use.gstack ? 0 : e->stack_depth;
+    a.gstack = use.gstack ? 1 : 0; a.stack_depth = use.gstack ? 0 : p.stack_depth;
     CK(e, cudaFuncSetAttribute(use.k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)use.smem));
     CK(e, cudaEventRecord(e->ev[3], e->stream));
     for (size_t k = 0; k < L.nchunk; k++) {
@@ -1864,9 +2046,9 @@ static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
     if (e->K <= 4096) {
         /* tip tables (P_e def_k) so that tip children need no GEMM */
         if (ensure_program(e)) return -1;
-        const int Et = (int)e->edge_of_tip.size();
+        const int Et = (int)e->prog.edge_of_tip.size();
         std::vector<int> toe(E, -1);
-        for (int te = 0; te < Et; te++) toe[e->edge_of_tip[te]] = te;
+        for (int te = 0; te < Et; te++) toe[e->prog.edge_of_tip[te]] = te;
         ENSURE(e, e->d_tip_of_edge, sizeof(int) * E);
         CK(e, cudaMemcpyAsync(e->d_tip_of_edge.p, toe.data(), sizeof(int) * E, cudaMemcpyHostToDevice, e->stream));
         CK(e, cudaStreamSynchronize(e->stream));
@@ -1875,7 +2057,7 @@ static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
         if (cnt) {
             tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
                 e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, 0, e->d_TPg.as<double>());
+                e->prog.d_edge_of_tip.as<int>(), C, E, Et, e->K, n, 0, e->d_TPg.as<double>());
             KCHECK(e);
         }
         a.TP = e->d_TPg.as<double>(); a.tip_of_edge = e->d_tip_of_edge.as<int>(); a.Et = Et;
@@ -1884,14 +2066,14 @@ static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
             ENSURE(e, e->d_TFg, sizeof(double) * (cnt + 1));
             tip_table_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->stream>>>(
                 a.Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(),
-                e->d_edge_of_tip.as<int>(), C, E, Et, e->K, n, a.f_zero_rowsum ? 1 : 2, e->d_TFg.as<double>());
+                e->prog.d_edge_of_tip.as<int>(), C, E, Et, e->K, n, a.f_zero_rowsum ? 1 : 2, e->d_TFg.as<double>());
             KCHECK(e);
             a.TF = e->d_TFg.as<double>();
         }
     }
     /* GEMM edges in the order of the inside kernel's walk (reverse BFS, children in csr order) */
     std::vector<int> toe(E, -1);
-    if (a.tip_of_edge) for (int te = 0; te < (int)e->edge_of_tip.size(); te++) toe[e->edge_of_tip[te]] = te;
+    if (a.tip_of_edge) for (int te = 0; te < (int)e->prog.edge_of_tip.size(); te++) toe[e->prog.edge_of_tip[te]] = te;
     std::vector<int> seq, pos(N, 0);
     for (int u = 0; u < N; u++) pos[e->preorder[u]] = u;
     for (int u = N - 1; u >= 0; u--) {
@@ -1906,7 +2088,7 @@ static int prepare_tile(plf_engine *e, const Query &q, GenericArgs &a)
     a.int_seq = e->d_int_seq.as<int>(); a.n_int_seq = (int)nseq;
     if (a.tip_of_edge && e->code_bytes == 1 && (size_t)a.Et * TL_TS <= 32 * 1024) {
         a.tip_stage = 1;
-        a.tip_edge_csr = e->d_edge_of_tip.as<int>();
+        a.tip_edge_csr = e->prog.d_edge_of_tip.as<int>();
     }
     return 0;
 }
@@ -2149,7 +2331,7 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
 {
     if (ensure_program(e)) return -1;
     const int n = e->n, C = e->C, E = e->E, K = e->K;
-    const int Ei = (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
+    const int Ei = (int)e->prog.edge_of_int.size(), Et = (int)e->prog.edge_of_tip.size();
     const size_t slot = dm_slot_doubles_host(NB), W = 8 * (size_t)NB;
     if (!e->dm_valid) {
         ENSURE(e, e->d_dmPf, sizeof(double) * ((size_t)C * Ei * slot + 1));
@@ -2160,11 +2342,11 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
          * P_e then F_e (negative index = second source), all transposed */
         std::vector<int> oidx, otr;
         int depth = 0, sp = 0;
-        for (int o = (int)e->ops.size() - 1; o >= 0; o--) {
-            const F4Op &op = e->ops[o];
-            if (o != (int)e->ops.size() - 1) sp--;
+        for (int o = (int)e->prog.ops.size() - 1; o >= 0; o--) {
+            const F4Op &op = e->prog.ops[o];
+            if (o != (int)e->prog.ops.size() - 1) sp--;
             for (int j = op.nchild - 1; j >= 0; j--) {
-                const F4Child &ch = e->children[op.first_child + j];
+                const F4Child &ch = e->prog.children[op.first_child + j];
                 if (ch.kind == F4_KIND_TIP) continue;
                 oidx.push_back(ch.edge); oidx.push_back(-(ch.edge + 1));
                 otr.push_back(1); otr.push_back(1);
@@ -2174,11 +2356,11 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
         }
         e->dm_out_depth = std::max(depth, 1);
         /* the program in the compact form the kernels stage in shared memory */
-        std::vector<int4> ops4(e->ops.size()), ch4(e->children.size());
-        for (size_t o = 0; o < e->ops.size(); o++)
-            ops4[o] = make_int4(e->ops[o].first_child, e->ops[o].nchild, e->ops[o].code_row, e->ops[o].spill_before);
-        for (size_t j = 0; j < e->children.size(); j++)
-            ch4[j] = make_int4(e->children[j].kind, e->children[j].mat, e->children[j].code_row, e->children[j].edge);
+        std::vector<int4> ops4(e->prog.ops.size()), ch4(e->prog.children.size());
+        for (size_t o = 0; o < e->prog.ops.size(); o++)
+            ops4[o] = make_int4(e->prog.ops[o].first_child, e->prog.ops[o].nchild, e->prog.ops[o].code_row, e->prog.ops[o].spill_before);
+        for (size_t j = 0; j < e->prog.children.size(); j++)
+            ch4[j] = make_int4(e->prog.children[j].kind, e->prog.children[j].mat, e->prog.children[j].code_row, e->prog.children[j].edge);
         ENSURE(e, e->d_dm_ops, sizeof(int4) * (ops4.size() + 1));
         ENSURE(e, e->d_dm_ch, sizeof(int4) * (ch4.size() + 1));
         CK(e, cudaMemcpyAsync(e->d_dm_ops.p, ops4.data(), sizeof(int4) * ops4.size(), cudaMemcpyHostToDevice, e->stream));
@@ -2198,9 +2380,9 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
         CK(e, cudaMemcpyAsync(e->d_dm_otr.p, otr.data(), sizeof(int) * otr.size(), cudaMemcpyHostToDevice, e->stream));
         CK(e, cudaMemcpyAsync(e->d_dm_rootf.p, rootf.data(), sizeof(double) * W, cudaMemcpyHostToDevice, e->stream));
         CK(e, cudaStreamSynchronize(e->stream));
-        CK(e, dm_pack(e->d_P.as<double>(), nullptr, e->d_edge_of_int.as<int>(), nullptr, Ei, C, E, n, NB, e->d_dmPf.as<double>(), e->stream));
+        CK(e, dm_pack(e->d_P.as<double>(), nullptr, e->prog.d_edge_of_int.as<int>(), nullptr, Ei, C, E, n, NB, e->d_dmPf.as<double>(), e->stream));
         e->launches++;
-        CK(e, dm_tip_table(e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->d_edge_of_tip.as<int>(),
+        CK(e, dm_tip_table(e->d_P.as<double>(), e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->prog.d_edge_of_tip.as<int>(),
                            C, E, Et, K, n, NB, 0, e->d_dmTPf.as<double>(), e->stream));
         e->launches++;
         CK(e, dm_tip_table(nullptr, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), nullptr,
@@ -2213,7 +2395,7 @@ static int ensure_dm_tables(plf_engine *e, int NB, const double *Fm, int f_zero_
         ENSURE(e, e->d_dmTFf, sizeof(double) * ((size_t)C * Et * K * W + 1));
         CK(e, dm_pack(e->d_P.as<double>(), Fm, e->d_dm_oidx.as<int>(), e->d_dm_otr.as<int>(), 2 * Ei, C, E, n, NB, e->d_dm_Of.as<double>(), e->stream));
         e->launches++;
-        CK(e, dm_tip_table(Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->d_edge_of_tip.as<int>(),
+        CK(e, dm_tip_table(Fm, e->d_defs.as<double>(), e->d_def_const.as<unsigned char>(), e->prog.d_edge_of_tip.as<int>(),
                            C, E, Et, K, n, NB, f_zero_rowsum ? 1 : 2, e->d_dmTFf.as<double>(), e->stream));
         e->launches++;
     }
@@ -2226,11 +2408,11 @@ static int run_dmma(plf_engine *e, Query &q)
     const int n = e->n, C = e->C, E = e->E;
     const int NB = dm_blocks_for(n);
     if (ensure_dm_tables(e, NB, q.want_edge ? q.Fm : nullptr, q.f_zero_rowsum)) return -1;
-    const int Ei = (int)e->edge_of_int.size(), Et = (int)e->edge_of_tip.size();
+    const int Ei = (int)e->prog.edge_of_int.size(), Et = (int)e->prog.edge_of_tip.size();
     const int nrows = (int)e->code_row_node.size();
 
     /* ring slots that fit beside the warps' code tiles */
-    const int nops = (int)e->ops.size(), nch = (int)e->children.size();
+    const int nops = (int)e->prog.ops.size(), nch = (int)e->prog.children.size();
     int R = 3;      /* measured (2..6): 3 is best by 1-3 %; shared memory not used by the ring is L1 for the tip tables and the slab */
     while (R > 2 && dm_smem_bytes(NB, R, nrows, nops, nch) > 227 * 1024) R--;
     if (dm_smem_bytes(NB, R, nrows, nops, nch) > 227 * 1024) FAIL(e, "tree too large for the tensor-pipe kernels (%d code rows)", nrows);
@@ -2253,8 +2435,8 @@ static int run_dmma(plf_engine *e, Query &q)
     const int64_t ngroups_max = (Sc + 7) / 8;
 
     const int grid_max = e->sm_count;
-    ENSURE(e, e->d_dm_stack, sizeof(double2) * (size_t)grid_max * DM_GROUPS * std::max(1, std::max(e->stack_depth, q.want_edge ? 2 * e->dm_out_depth : 0)) * NB * 32);
-    ENSURE(e, e->d_dm_stackmeta, sizeof(int) * (size_t)grid_max * DM_GROUPS * std::max(1, std::max(e->stack_depth, q.want_edge ? 4 * e->dm_out_depth : 0)) * 32);
+    ENSURE(e, e->d_dm_stack, sizeof(double2) * (size_t)grid_max * DM_GROUPS * std::max(1, std::max(e->prog.stack_depth, q.want_edge ? 2 * e->dm_out_depth : 0)) * NB * 32);
+    ENSURE(e, e->d_dm_stackmeta, sizeof(int) * (size_t)grid_max * DM_GROUPS * std::max(1, std::max(e->prog.stack_depth, q.want_edge ? 4 * e->dm_out_depth : 0)) * 32);
     ENSURE(e, e->g_cat_lh, sizeof(double) * (size_t)C * Sc);
     ENSURE(e, e->g_cat_k, sizeof(int) * (size_t)C * Sc);
     ENSURE(e, e->g_site_m, sizeof(double) * Sc);
@@ -2306,7 +2488,7 @@ static int run_dmma(plf_engine *e, Query &q)
         dm_tiling(a.ngroups, C, grid_max, &a.tiles_full, &a.tail_gs, &a.ntiles);
         a.slab = q.want_edge ? e->d_dm_slab.as<double2>() : nullptr;
         a.slab_meta = q.want_edge ? e->d_dm_slabmeta.as<int>() : nullptr;
-        a.stack_depth = std::max(1, e->stack_depth);
+        a.stack_depth = std::max(1, e->prog.stack_depth);
         const long long items = (long long)a.ntiles * C;
         CK(e, dm_launch_inside(a, NB, (int)std::min<long long>(grid_max, items), e->stream));
         e->launches++;
@@ -2403,7 +2585,7 @@ static int run_query_once(plf_engine *e, Query &q, bool need_D, const double *l_
                      q.edge_mask_h ? e->d_mask.as<unsigned char>() : nullptr, e->d_lhi.as<double>(), e->d_llo.as<double>())) return -1;
         q.Fm = e->d_F.as<double>(); q.f_zero_rowsum = 0; f_mode = 2;
     }
-    if (fused && ensure_tip_tables(e, q.want_edge ? q.Fm : nullptr, f_mode, q.want_marg)) return -1;
+    if (fused && ensure_tip_tables(e, q.want_edge ? q.Fm : nullptr, f_mode, q.want_marg, f4_use_fold(e, f4_kind(q)))) return -1;
     CK(e, cudaEventRecord(e->ev[1], e->stream));
     e->kernel_timed = false;
     e->ms_kernel_override = -1.f;
